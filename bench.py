@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py - throughput of the UML training step on B200 (contract in the task statement).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--workload cfg3]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--workload cfg3] [--dump-outputs DIR]
 
 Metric (BASELINE.json): UML train samples/sec (image + text rows consumed per second).
 Workload at N=1 (``config.workload``): cfg3 = ImageNet full-data shapes, "ViT-L/14" 768-d features,
@@ -334,6 +334,25 @@ def make_model(wl, dev, txt_bank):
     return model, opt, sch
 
 
+DUMP_MAX_ELEMS = 1 << 22  # 16 MB of float32 per array; with at most two such arrays (img_proj, head) a dump stays < 64 MB
+
+
+def dump_outputs(out_dir, model, stats):
+    """--dump-outputs: what the timed steps hand to their caller after the last one - the model's parameters (float32)
+    and that step's loss / accuracy record (float64 scalars) - as out_dir/<name>.npy.  An array of more than
+    DUMP_MAX_ELEMS elements is stored as the same seeded sample of its flattened elements in every run."""
+    import numpy as np
+
+    os.makedirs(out_dir, exist_ok=True)
+    arrays = {name: p.detach().float().cpu().numpy() for name, p in model.named_parameters()}
+    arrays.update({k: np.float64(v) for k, v in stats.items()})
+    for name, a in arrays.items():
+        if a.size > DUMP_MAX_ELEMS:
+            keep = np.sort(np.random.default_rng(0).choice(a.size, DUMP_MAX_ELEMS, replace=False))
+            a = a.reshape(-1)[keep]
+        np.save(os.path.join(out_dir, name + ".npy"), a)
+
+
 def _stage(msg):
     if os.environ.get("UML_BENCH_VERBOSE"):
         print(f"[bench] {msg}", file=sys.stderr, flush=True)
@@ -475,6 +494,8 @@ def run_ours(args, wl, rank, world, dev):
         sampler.close()
     ktimes = engine.kernel_times_ms()
     loss_tail = engine.read_log([W + K - 1])[0]
+    if args.dump_outputs and rank == 0:  # before the breakdown steps below train the model further
+        dump_outputs(args.dump_outputs, model, loss_tail)
     # per-kernel breakdown of the step from a few extra (untimed) steps with every kernel bracketed
     engine.prepare_profile(16)
     step(W + K, 16)
@@ -950,7 +971,15 @@ def main():
                          "H2D, fp32 torch ops on the device) - the like-for-like GPU baseline of SURVEY 8d")
     ap.add_argument("--precision", type=str, default="auto", choices=["auto", "fp32", "bf16"])
     ap.add_argument("--cpu-seconds", type=float, default=20.0, help="budget of the cpu_baseline leg")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write the trained parameters and the last timed step's losses and "
+                         "accuracies as DIR/<name>.npy (the inputs are seeded: two builds can be compared file by file)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and (args.impl == "reference" or args.workload in ("cfg1", "cfg2_sweep", "cfg5", "eval")):
+        ap.error("--dump-outputs covers the training step of our implementation: --impl ours with workload "
+                 + ", ".join(sorted(WORKLOADS)))
     args.warmup = max(args.warmup, 3)
     if args.workload == "eval":
         if args.impl == "reference":

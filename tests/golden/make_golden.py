@@ -9,6 +9,7 @@ the files are reproducible.
 """
 from __future__ import annotations
 
+import json
 import os
 import sys
 
@@ -274,6 +275,13 @@ def text_and_init():
     return fx
 
 
+def reference_defaults():
+    """The reference's hyper-parameter presets and the defaults of its command-line parser."""
+    ns = rh.load_vision_language()
+    from engine.config import parser  # the reference's, via the harness' sys.path
+    return {"HYPER_DICT": ns.default.HYPER_DICT, "parser_defaults": vars(parser.parse_args([]))}
+
+
 def gaussian():
     gm = rh.load_gaussian()
     cfg = dict(seed=42, num_samples=64, dim_c=10, dim_x=5, dim_y=5, dim_obs=12, noise_std=0.09,
@@ -349,6 +357,8 @@ def main():
     misc.update(gaussian())
     np.savez_compressed(os.path.join(OUT, "misc.npz"), **misc)
     print("misc keys", len(misc))
+    with open(os.path.join(OUT, "reference_defaults.json"), "w") as f:
+        json.dump(reference_defaults(), f, indent=1, sort_keys=True)
 
 
 if __name__ == "__main__":

@@ -1,6 +1,7 @@
 """Host-side logic of the product against the golden vectors recorded from the reference - runs
 without a GPU: sampler RNG protocol, text-bank selection, LR schedule, presets, path layout."""
 import ast
+import json
 import os
 
 import numpy as np
@@ -17,6 +18,9 @@ from uml_b200 import features as F
 
 GOLDEN = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden")
 M = np.load(os.path.join(GOLDEN, "misc.npz"), allow_pickle=False)
+# the reference's HYPER_DICT and parser.parse_args([]) (make_golden.py)
+with open(os.path.join(GOLDEN, "reference_defaults.json")) as _f:
+    REF_DEFAULTS = json.load(_f)
 
 
 def _bank(n):
@@ -124,12 +128,9 @@ def test_paths_and_names_match_reference():
 
 
 def test_presets_equal_reference_when_available():
-    from oracle import ref_harness as rh
     assert set(HYPER_DICT) == {"full_ds_full_model_finetune", "clip_linear", "linear", "audio"}
     assert HYPER_DICT["clip_linear"]["batch_size"] == [32] and HYPER_DICT["linear"]["learnable_temp"] == [True]
-    if not rh.reference_available():
-        pytest.skip("reference tree not present")
-    assert rh.load_vision_language().default.HYPER_DICT == HYPER_DICT
+    assert REF_DEFAULTS["HYPER_DICT"] == HYPER_DICT
 
 
 def test_bank_files_round_trip(tmp_path):
@@ -155,13 +156,7 @@ def test_config_parser_defaults_match_reference_when_available():
     from uml_b200.engine.config import parser
     ours = vars(parser.parse_args([]))
     assert ours["logit"] == 4.60517 and ours["num_workers"] == 4 and ours["modality"] == "image"
-    from oracle import ref_harness as rh
-    if not rh.reference_available():
-        pytest.skip("reference tree not present")
-    rh.load_vision_language()
-    from engine.config import parser as ref_parser  # the reference's, via the harness' sys.path
-    ref = vars(ref_parser.parse_args([]))
-    for k, v in ref.items():
+    for k, v in REF_DEFAULTS["parser_defaults"].items():
         assert ours[k] == v, k
 
 
