@@ -400,9 +400,39 @@ typedef struct {
  * the last batch of an epoch is short) with learning rates lr[i*n_heads + k] (host array).                      */
 int uml_sweep_run(const uml_sweep_args* args /*host*/, int32_t n_steps, const int64_t* rows /*host*/,
                   const float* lr /*host*/, void* stream);
-/* kernels launched by uml_sweep_run in this process so far (modulo 2^31): three per step when the tensor-core dW launch
- * carries the statistics warp, four otherwise */
+/* kernels launched by uml_sweep_run and uml_sweep_adapter_run in this process so far (modulo 2^31): three per step when
+ * the tensor-core dW launch carries the statistics warp, four otherwise; see uml_sweep_adapter_run for its count */
 int uml_sweep_launch_count(void);
+
+/* The same lock-step sweep for UML heads with an image adapter and / or learnable temperatures (head.py:39-98: the
+ * reference's `linear` preset over unimodal encoders, engine/optimizer/default.py:17-31).  Per head k and step:
+ *   Z_k = X_img Wp_k^T,  logits = [Z_k ; X_txt] W_k^T * scale_k,  dZ_k = G_k[image rows] W_k (W_k before its update),
+ *   W_k, scale_k and Wp_k updated with the head's rule (the four parameters share one parameter group).
+ * `args` describes the head exactly as for uml_sweep_run; args->dim is the head's input width D (= the adapter's output),
+ * bank[0] holds image rows of img_dim floats when there is an adapter, bank[1] text rows of D floats.
+ * One step of all heads is five launches: Z, logits + softmax / CE over [Z; X_txt] (+ per-row d loss / d scale), dZ,
+ * head dW + update + statistics (+ temperature update), adapter dWp + update; without an adapter, or in a step without
+ * image rows, Z, dZ and dWp are skipped (two launches).
+ * Contract, checked before anything touches the device: tensor-core forms only - dim % 4 == 0, img_dim % 4 == 0, 16-byte
+ * aligned slabs, banks, G, Z and dZ with strides that are multiples of 4; max_rows <= 64; n_classes <= 1024.           */
+typedef struct {
+  int32_t  img_dim;         /* Dv, width of the image rows; 0 = no adapter (image rows go straight to the head)          */
+  float*   W;               /* [n_heads][adapter_stride] adapter weights, each a [dim][img_dim] matrix (img_proj.weight) */
+  float*   m;               /* exp_avg | momentum buffers, same layout                                                 */
+  float*   v;               /* exp_avg_sq (unused for SGD)                                                             */
+  int64_t  adapter_stride;
+  float*   Z;               /* scratch [n_heads][max_img_rows][ldz]: adapter output                                    */
+  float*   dZ;              /* scratch [n_heads][max_img_rows][ldz]: its gradient                                      */
+  int64_t  ldz, max_img_rows;
+  float*   scale_param;     /* [n_heads][2] learnable temperatures (image, text); NULL: the fixed args->scale           */
+  float*   scale_m;         /* [n_heads][2] optimizer state of the temperatures                                        */
+  float*   scale_v;
+  float*   row_dscale;      /* scratch [n_heads][max_rows] (with scale_param)                                          */
+  void*    ev[10];          /* optional cudaEvent_t pairs around the five launch sites of the LAST step: Z, logits +
+                               softmax / CE, dZ, head dW + update + statistics, adapter dWp + update                   */
+} uml_sweep_adapter_args;
+int uml_sweep_adapter_run(const uml_sweep_args* args /*host*/, const uml_sweep_adapter_args* adapter /*host*/,
+                          int32_t n_steps, const int64_t* rows /*host*/, const float* lr /*host*/, void* stream);
 
 /* ---- sampler: the epoch permutation on the host, bit-exact with torch.randperm(n, generator=
  * torch.Generator().manual_seed(seed)) on the CPU - what RandomSampler draws once per epoch for the

@@ -69,6 +69,13 @@ class SweepArgs(C.Structure):
                 ("active", C.c_uint8 * SWEEP_MAX_HEADS), ("ev", c_vp * 8)]
 
 
+class SweepAdapterArgs(C.Structure):
+    """uml_sweep_adapter_args"""
+    _fields_ = [("img_dim", c_i32), ("W", c_vp), ("m", c_vp), ("v", c_vp), ("adapter_stride", c_i64), ("Z", c_vp),
+                ("dZ", c_vp), ("ldz", c_i64), ("max_img_rows", c_i64), ("scale_param", c_vp), ("scale_m", c_vp),
+                ("scale_v", c_vp), ("row_dscale", c_vp), ("ev", c_vp * 10)]
+
+
 # name -> argtypes; every function returns int except uml_last_error
 PROTOTYPES = {
     "uml_abi_version": [],
@@ -139,6 +146,7 @@ PROTOTYPES = {
                       c_f64, c_f64, c_f64, c_f64, c_i64, c_vp, c_vp, c_vp],
     "uml_gauss_eval": [c_vp, c_i32, c_i32, c_i32, c_vp, c_vp, c_i64, c_vp, c_vp, c_vp],
     "uml_sweep_run": [C.POINTER(SweepArgs), c_i32, c_vp, c_vp, c_vp],
+    "uml_sweep_adapter_run": [C.POINTER(SweepArgs), C.POINTER(SweepAdapterArgs), c_i32, c_vp, c_vp, c_vp],
     "uml_randperm_i64": [C.c_uint64, c_i64, c_vp],
     "uml_randperm_begin": [c_vp, C.c_uint64, c_i64, c_vp],
     "uml_randperm_advance": [c_vp, c_i64],

@@ -59,9 +59,21 @@ struct SweepDev {
   int kind, first_step;
   float beta1, beta2, eps, momentum, bc2_sqrt_inv;
   float lr[kMaxHeads], step_size[kMaxHeads], decay[kMaxHeads], wd[kMaxHeads];
+  // adapter heads (uml_sweep_adapter_run): image row r of head k is zrows[k * z_stride + r * z_ld] (the adapter output Z)
+  // instead of a bank row; labels still come through the permutation.  NULL: bank rows.
+  const float* zrows;
+  int64_t z_ld, z_stride;
+  // learnable temperatures: [K][2] (image, text) parameters and optimizer state; NULL: the fixed scale[]
+  float* scale_dev;
+  float* scale_m;
+  float* scale_v;
+  float* row_dscale;  // [K][row_stride] per-row d loss / d scale, written by the fused softmax epilogue
 };
 
 __device__ __forceinline__ bool head_active(const SweepDev& p, int head) { return (p.active_mask >> head) & 1u; }
+__device__ __forceinline__ float seg_scale(const SweepDev& p, int head, bool is_txt) {
+  return p.scale_dev ? p.scale_dev[2 * head + (is_txt ? 1 : 0)] : p.scale[is_txt ? 1 : 0];
+}
 
 // bank row and bank label of logical row r (image run first, then the text run) of head `head`
 __device__ __forceinline__ int64_t bank_row(const SweepDev& p, int head, int64_t r, bool& is_txt) {
@@ -71,6 +83,7 @@ __device__ __forceinline__ int64_t bank_row(const SweepDev& p, int head, int64_t
   return pm[(is_txt ? p.pos[1] : p.pos[0]) + l];
 }
 __device__ __forceinline__ const float* row_ptr(const SweepDev& p, int head, int64_t r) {
+  if (p.zrows != nullptr && r < p.n0) return p.zrows + head * p.z_stride + r * p.z_ld;
   bool s;
   const int64_t src = bank_row(p, head, r, s);
   return (s ? p.bank[1] : p.bank[0]) + src * (s ? p.ld[1] : p.ld[0]);
@@ -756,7 +769,10 @@ __global__ void __launch_bounds__(256, 2) sweep_logits_tc_kernel(const __grid_co
     __shared__ int pub_arg[BN];                 //                            first maximal class of the tile
     __shared__ float row_scale[BN], row_gcoef[BN], row_lab[BN];
     __shared__ int row_label[BN], row_arg[BN];
+    __shared__ float row_weight[BN], row_n[BN], pub_ds[BN];  // learnable temperatures: d loss / d scale of the row
     float* tile = reinterpret_cast<float*>(smem);  // [BN][BM]
+    float* raw_tile = tile + BN * BM;               // [BN][BM] unscaled logits (learnable temperatures only)
+    const bool want_ds = p.scale_dev != nullptr;
     if (t < BN) {
       const int64_t r = m0 + t;
       row_label[t] = -1;
@@ -766,9 +782,12 @@ __global__ void __launch_bounds__(256, 2) sweep_logits_tc_kernel(const __grid_co
         bool is_txt;
         const int64_t src = bank_row(p, head, r, is_txt);
         row_label[t] = static_cast<int>((is_txt ? p.labels[1] : p.labels[0])[src]);
-        const float sc = is_txt ? p.scale[1] : p.scale[0];
+        const float sc = seg_scale(p, head, is_txt);
+        const float w = is_txt ? p.alpha[head] : 1.f;
         row_scale[t] = sc;
-        row_gcoef[t] = (is_txt ? p.alpha[head] : 1.f) * sc / static_cast<float>(is_txt ? p.n1 : p.n0);
+        row_gcoef[t] = w * sc / static_cast<float>(is_txt ? p.n1 : p.n0);
+        row_weight[t] = w;
+        row_n[t] = static_cast<float>(is_txt ? p.n1 : p.n0);
       }
     }
     __syncthreads();
@@ -778,6 +797,7 @@ __global__ void __launch_bounds__(256, 2) sweep_logits_tc_kernel(const __grid_co
       for (int i = 0; i < 32; ++i) {
         const int rl = h * 32 + i;
         tile[rl * BM + cl] = (c0 + cl < C) ? __uint_as_float(v[i]) * row_scale[rl] : -INFINITY;
+        if (want_ds) raw_tile[rl * BM + cl] = (c0 + cl < C) ? __uint_as_float(v[i]) : 0.f;
       }
     }
     __syncthreads();
@@ -872,6 +892,15 @@ __global__ void __launch_bounds__(256, 2) sweep_logits_tc_kernel(const __grid_co
       const float4 e4 = *reinterpret_cast<const float4*>(tile + rl * BM + 4 * lane);
       float pr[4] = {e4.x * inv, e4.y * inv, e4.z * inv, e4.w * inv};
       const int cb = c0 + 4 * lane;
+      float ds = 0.f;
+      if (want_ds) {  // softmax_ce_grad_row's  sum_c (p_c - y_c) raw_c  (simt.cu), tile part: lanes in a shuffle tree
+        const float4 r4 = *reinterpret_cast<const float4*>(raw_tile + rl * BM + 4 * lane);
+        const float raw[4] = {r4.x, r4.y, r4.z, r4.w};
+#pragma unroll
+        for (int k = 0; k < 4; ++k) ds = fmaf(pr[k] - (cb + k == label ? 1.f : 0.f), raw[k], ds);
+        ds = warp_sum(ds);
+        if (lane == 0) pub_ds[rl] = ds;
+      }
 #pragma unroll
       for (int k = 0; k < 4; ++k) {
         if (cb + k == label) pr[k] -= 1.f;
@@ -889,6 +918,15 @@ __global__ void __launch_bounds__(256, 2) sweep_logits_tc_kernel(const __grid_co
       if (label >= cb && label < cb + 4) {
         p.row_loss[head * p.row_stride + r] = logf(sum) - row_lab[rl];
         p.row_correct[head * p.row_stride + r] = (row_arg[rl] == label) ? 1 : 0;
+      }
+    }
+    if (want_ds) {  // the row's tiles in class order, by the first tile of the cluster
+      cluster_sync_all();
+      const int rl = warp * 8 + (lane & 7);
+      if (blockIdx.x == 0 && lane < 8 && m0 + rl < R) {
+        float s = 0.f;
+        for (uint32_t k = 0; k < n_tiles; ++k) s += ld_cluster_f32(mapa_cta(smem_u32(&pub_ds[rl]), k));
+        p.row_dscale[head * p.row_stride + m0 + rl] = s * row_weight[rl] / row_n[rl];
       }
     }
     cluster_sync_all();  // nobody leaves while a neighbour may still read its published values
@@ -1029,28 +1067,42 @@ __global__ void __launch_bounds__(kNT + 64, 1)
 
   if (warp == kWarps + 1) {
     // ------------------------------------------------ statistics warp: what sweep_stats_kernel computes, in a warp that
-    // would otherwise not exist (running head a belongs to CTA a mod gridDim.x; lanes stride over the rows, shuffle tree)
-    const int n_act = __popc(p.active_mask);
+    // would otherwise not exist (running head a belongs to CTA a mod gridDim.x; lanes stride over the rows, shuffle tree).
+    // With learnable temperatures it also sums the rows' d loss / d scale and steps the head's two scales with the
+    // head's optimizer rule (the scales share the weights' parameter group: same lr, decay, betas and step count); the
+    // next read of a scale is the next step's logits launch.  stats == NULL (adapter update launch): nothing to do.
+    const int n_act = p.stats ? __popc(p.active_mask) : 0;
     for (int a = blockIdx.x; a < n_act; a += gridDim.x) {
       const int hd = __fns(p.active_mask, 0, a + 1);
       for (int sg = 0; sg < 2; ++sg) {
         const int64_t beg = sg ? p.n0 : 0, n = sg ? p.n1 : p.n0;
         const float* rl = p.row_loss + hd * p.row_stride + beg;
         const int32_t* rc = p.row_correct + hd * p.row_stride + beg;
-        float ls = 0.f;
+        const float* rd = p.scale_dev ? p.row_dscale + hd * p.row_stride + beg : nullptr;
+        float ls = 0.f, ds = 0.f;
         int hits = 0;
         for (int64_t i = lane; i < n; i += 32) {
           ls += rl[i];
           hits += rc[i];
+          if (rd) ds += rd[i];
         }
         ls = warp_sum(ls);
+        ds = warp_sum(ds);
         hits = warp_sum_i(hits);
         if (lane == 0) {
           uml_seg_stats& o = p.stats[hd * 2 + sg];
           o.loss_mean = n > 0 ? ls / static_cast<float>(n) : 0.f;
-          o.dscale = 0.f;
+          o.dscale = ds;
           o.correct = hits;
           o.n = static_cast<int32_t>(n);
+          if (rd && n > 0) {  // (a modality without rows leaves its scale without a gradient: torch skips it)
+            float w = p.scale_dev[2 * hd + sg], m = p.scale_m[2 * hd + sg];
+            float v = p.kind == 3 ? 0.f : p.scale_v[2 * hd + sg];
+            update_one(p, p.lr[hd], p.step_size[hd], p.decay[hd], p.wd[hd], w, m, v, ds);
+            p.scale_dev[2 * hd + sg] = w;
+            p.scale_m[2 * hd + sg] = m;
+            if (p.kind != 3) p.scale_v[2 * hd + sg] = v;
+          }
         }
       }
     }
@@ -1226,6 +1278,149 @@ __global__ void __launch_bounds__(kNT + 64, 1)
   tc_fence_before();
   __syncthreads();
   if (warp == 1) tmem_dealloc(tmem_base, 128);
+}
+
+// 5t. adapter back-propagation dZ_k = G_k[image rows] . W_k, with W_k before the step's update (the head launch updates
+//     it after this one), transposed tile: D[dim, row] = W_k^T[128 dims, classes] . G_k^T[classes, 64 rows]
+//     grid (ceil(D/128), K).  A = weight rows read along the dims: MN-major, SWIZZLE_128B_BASE32B like the dW kernel's
+//     feature tile (k-blocks of 32 classes: four 4 KB boxes of 32 classes x 32 dims); B = G rows, K-major SWIZZLE_128B
+//     like the logits kernel's row tile.  Two stages, the next block's loads in registers while this one is split and
+//     multiplied, as in the logits kernel; the accumulation order is fixed by the instruction stream (no atomics), so a
+//     head's dZ does not depend on its slot.
+constexpr int kTcDzStage = 48 * 1024;  // W hi 16 KB | W lo 16 KB | G hi 8 KB | G lo 8 KB
+constexpr int kTcDzSmemBytes = 2 * kTcDzStage + 1024 + 64;
+
+__global__ void __launch_bounds__(256, 2)
+    sweep_dz_tc_kernel(const __grid_constant__ SweepDev p, float* __restrict__ dZ, int64_t ldz, int64_t dz_stride) {
+  constexpr int BM = 128, BN = 64, BK = 32, S = 2;
+  const int head = blockIdx.y;
+  if (!head_active(p, head)) return;
+  extern __shared__ unsigned char tc_smem_raw[];
+  unsigned char* smem = reinterpret_cast<unsigned char*>((reinterpret_cast<uintptr_t>(tc_smem_raw) + 1023) & ~uintptr_t(1023));
+  uint64_t* empty_bar = reinterpret_cast<uint64_t*>(smem + S * kTcDzStage);
+  uint64_t* tfull_bar = empty_bar + S;
+  uint32_t* tmem_slot = reinterpret_cast<uint32_t*>(tfull_bar + 1);
+  const int t = threadIdx.x, warp = t >> 5, lane = t & 31;
+  const int64_t R = p.n0;  // image rows only (<= 64, launcher)
+  const int d0 = blockIdx.x * BM;
+  const int D = p.dim, C = p.n_classes;
+  const float* __restrict__ W = p.W + head * p.head_stride;
+  const float* __restrict__ G = p.G + head * p.g_stride;
+  if (t == 0) {
+    for (int s = 0; s < S; ++s) mbar_init(&empty_bar[s], 1);
+    mbar_init(tfull_bar, 1);
+    fence_barrier_init();
+  }
+  if (warp == 1) tmem_alloc(tmem_slot, 64);
+  tc_fence_before();
+  __syncthreads();
+  tc_fence_after();
+  const uint32_t tmem_base = *tmem_slot;
+
+  // this thread's 16-byte chunks of a k-block: four of the weight tile (32 classes x 128 dims, a warp per class row),
+  // two of the G tile (64 rows x 32 classes, eight threads per row)
+  int wrow[4], wcol[4], grow[2], gch[2];
+  uint32_t woff[4], goff[2];
+#pragma unroll
+  for (int i = 0; i < 4; ++i) {
+    const int f = t + 256 * i, j = f & 31;
+    wrow[i] = f >> 5;
+    wcol[i] = d0 + 4 * j;
+    woff[i] = static_cast<uint32_t>((j >> 3) * 4096) + sw128_b32(wrow[i], j & 7);
+  }
+#pragma unroll
+  for (int i = 0; i < 2; ++i) {
+    const int f = t + 256 * i;
+    grow[i] = f >> 3;
+    gch[i] = f & 7;
+    goff[i] = sw128(grow[i], gch[i]);
+  }
+  auto load = [&](int kb, float4 (&r)[6]) {
+#pragma unroll
+    for (int i = 0; i < 4; ++i) {
+      const int c = kb * BK + wrow[i];
+      r[i] = (c < C && wcol[i] < D) ? __ldg(reinterpret_cast<const float4*>(W + static_cast<int64_t>(c) * D + wcol[i]))
+                                    : make_float4(0.f, 0.f, 0.f, 0.f);
+    }
+#pragma unroll
+    for (int i = 0; i < 2; ++i) {
+      const int c = kb * BK + 4 * gch[i];
+      float4 x = make_float4(0.f, 0.f, 0.f, 0.f);
+      if (grow[i] < R && c < C) {  // (ldg % 4 == 0: the chunk stays inside the row; columns >= C are not written by the
+        x = *reinterpret_cast<const float4*>(G + grow[i] * p.ldg + c);  //  logits launch and must not enter the sum)
+        if (c + 1 >= C) x.y = 0.f;
+        if (c + 2 >= C) x.z = 0.f;
+        if (c + 3 >= C) x.w = 0.f;
+      }
+      r[4 + i] = x;
+    }
+  };
+
+  const int nk = (C + BK - 1) / BK;
+  constexpr uint32_t idesc = make_idesc_tf32(BM, BN, 1, 0);
+  float4 cur[6], nxt[6];
+  load(0, cur);
+#pragma unroll 1
+  for (int kb = 0; kb < nk; ++kb) {
+    if (kb + 1 < nk) load(kb + 1, nxt);
+    const int s = kb & (S - 1);
+    if (kb >= S) mbar_wait_or_trap(&empty_bar[s], static_cast<uint32_t>((kb / S) - 1) & 1u);
+    unsigned char* st = smem + s * kTcDzStage;
+#pragma unroll
+    for (int i = 0; i < 4; ++i) {
+      float4 hi, lo;
+      split_tf32(cur[i], hi, lo);
+      *reinterpret_cast<float4*>(st + woff[i]) = hi;
+      *reinterpret_cast<float4*>(st + 16384 + woff[i]) = lo;
+    }
+#pragma unroll
+    for (int i = 0; i < 2; ++i) {
+      float4 hi, lo;
+      split_tf32(cur[4 + i], hi, lo);
+      *reinterpret_cast<float4*>(st + 32768 + goff[i]) = hi;
+      *reinterpret_cast<float4*>(st + 40960 + goff[i]) = lo;
+    }
+    fence_proxy_async();
+    __syncthreads();
+    if (t == 0) {
+      tc_fence_after();
+      const uint32_t a_hi = smem_u32(st), a_lo = a_hi + 16384, b_hi = a_hi + 32768, b_lo = a_hi + 40960;
+#pragma unroll
+      for (int k = 0; k < BK / 8; ++k) {  // A: 8 classes = two 4-row atoms (SBO 512 B), next 32 dims one 4 KB box further
+        const uint64_t dah = make_smem_desc(a_hi + k * 1024, 4096, 512, kLayoutSw128Base32);
+        const uint64_t dal = make_smem_desc(a_lo + k * 1024, 4096, 512, kLayoutSw128Base32);
+        const uint64_t dbh = make_smem_desc(b_hi + k * 32, 16, 1024, kLayoutSw128);
+        const uint64_t dbl = make_smem_desc(b_lo + k * 32, 16, 1024, kLayoutSw128);
+        umma_tf32(tmem_base, dal, dbh, idesc, (kb | k) != 0);
+        umma_tf32(tmem_base, dah, dbl, idesc, 1);
+        umma_tf32(tmem_base, dah, dbh, idesc, 1);
+      }
+      umma_commit(&empty_bar[s]);
+      if (kb == nk - 1) umma_commit(tfull_bar);
+    }
+#pragma unroll
+    for (int i = 0; i < 6; ++i) cur[i] = nxt[i];
+  }
+
+  // epilogue: TMEM lane = dim, column = row; warp w reads lane quadrant w % 4, rows 32 (w / 4) ..
+  mbar_wait_or_trap(tfull_bar, 0);
+  tc_fence_after();
+  const int q = warp & 3, h = warp >> 2;
+  uint32_t v[32];
+  tmem_ld32(tmem_base + (static_cast<uint32_t>(q * 32) << 16) + h * 32, v);
+  tmem_ld_wait();
+  const int d = d0 + q * 32 + lane;
+  if (d < D) {
+    float* __restrict__ out = dZ + head * dz_stride + d;
+#pragma unroll
+    for (int i = 0; i < 32; ++i) {
+      const int64_t r = h * 32 + i;
+      if (r < R) out[r * ldz] = __uint_as_float(v[i]);  // a warp stores 32 consecutive dims of one row
+    }
+  }
+  tc_fence_before();
+  __syncthreads();
+  if (warp == 1) tmem_dealloc(tmem_base, 64);
 }
 
 // ---------------------------------------------------------------------------------------------------------------
@@ -1455,6 +1650,219 @@ int uml_sweep_run(const uml_sweep_args* a, int32_t n_steps, const int64_t* rows,
       ++g_sweep_launches;
     }
     if (mark(7)) return 1;
+    pos[0] += n0;
+    pos[1] += n1;
+  }
+  return 0;
+}
+
+static bool aligned16(const void* ptr) { return (reinterpret_cast<uintptr_t>(ptr) & 15) == 0; }
+
+int uml_sweep_adapter_run(const uml_sweep_args* a, const uml_sweep_adapter_args* ad, int32_t n_steps, const int64_t* rows,
+                          const float* lr, void* stream) {
+  using namespace uml;
+  using namespace uml::sweep;
+  UML_REQUIRE(a && ad && rows && lr && n_steps >= 0, "sweep_adapter_run: null argument");
+  const int K = a->n_heads;
+  UML_REQUIRE(K >= 1 && K <= kMaxHeads, "sweep_adapter_run: 1..%d heads", kMaxHeads);
+  UML_REQUIRE(a->dim > 0 && a->n_classes > 0 && a->ldg >= a->n_classes, "sweep_adapter_run: bad shape");
+  UML_REQUIRE(a->kind >= 1 && a->kind <= 3, "sweep_adapter_run: optimizer kind must be 1 (AdamW), 2 (Adam) or 3 (SGD)");
+  UML_REQUIRE(a->W && a->m && (a->kind == 3 || a->v) && a->G && a->row_loss && a->row_correct && a->stats,
+              "sweep_adapter_run: null buffer");
+  UML_REQUIRE(a->head_stride >= static_cast<int64_t>(a->n_classes) * a->dim, "sweep_adapter_run: head_stride too small");
+  const bool adapter = ad->img_dim > 0, temps = ad->scale_param != nullptr;
+  // tensor-core forms only: 16-byte rows and operands, one 64-row feature tile, softmax / CE in the logits epilogue
+  UML_REQUIRE(a->dim % 4 == 0 && ad->img_dim % 4 == 0 && ad->img_dim >= 0, "sweep_adapter_run: dims must be multiples of 4");
+  UML_REQUIRE(a->n_classes <= 1024, "sweep_adapter_run: at most 1024 classes (softmax / CE in the logits epilogue)");
+  UML_REQUIRE(a->max_rows >= 1 && a->max_rows <= 64, "sweep_adapter_run: at most 64 rows per step (max_rows %lld)",
+              static_cast<long long>(a->max_rows));
+  UML_REQUIRE(a->head_stride % 4 == 0 && aligned16(a->W) && aligned16(a->m) && aligned16(a->v) && aligned16(a->G) &&
+                  a->ldg % 4 == 0,
+              "sweep_adapter_run: W, m, v, G must be 16-byte aligned with strides that are multiples of 4");
+  for (int s = 0; s < 2; ++s)
+    UML_REQUIRE(!a->bank[s] || (aligned16(a->bank[s]) && a->bank_ld[s] % 4 == 0),
+                "sweep_adapter_run: bank %d rows must be 16-byte aligned", s);
+  if (adapter) {
+    UML_REQUIRE(ad->W && ad->m && (a->kind == 3 || ad->v) && ad->Z && ad->dZ, "sweep_adapter_run: null adapter buffer");
+    UML_REQUIRE(ad->adapter_stride >= static_cast<int64_t>(a->dim) * ad->img_dim && ad->adapter_stride % 4 == 0 &&
+                    aligned16(ad->W) && aligned16(ad->m) && aligned16(ad->v),
+                "sweep_adapter_run: adapter slabs must be 16-byte aligned, adapter_stride >= dim * img_dim, a multiple of 4");
+    UML_REQUIRE(ad->ldz >= a->dim && ad->ldz % 4 == 0 && ad->max_img_rows >= 1 && aligned16(ad->Z) && aligned16(ad->dZ),
+                "sweep_adapter_run: Z / dZ must be 16-byte aligned with ldz >= dim, a multiple of 4");
+  }
+  if (temps)
+    UML_REQUIRE(ad->scale_m && (a->kind == 3 || ad->scale_v) && ad->row_dscale,
+                "sweep_adapter_run: learnable temperatures need scale_m, scale_v and row_dscale");
+  cudaStream_t st = as_stream(stream);
+  SweepDev p;
+  memset(&p, 0, sizeof(p));
+  uint32_t mask = 0;
+  for (int k = 0; k < K; ++k) {
+    if (!a->active[k]) continue;
+    mask |= 1u << k;
+    for (int s = 0; s < 2; ++s) p.perm[s][k] = a->perm[s][k];
+    p.alpha[k] = a->alpha[k];
+    p.wd[k] = a->weight_decay[k];
+  }
+  if (mask == 0 || n_steps == 0) return 0;
+  for (int s = 0; s < 2; ++s) {
+    p.bank[s] = a->bank[s];
+    p.labels[s] = a->labels[s];
+    p.ld[s] = a->bank_ld[s];
+    p.scale[s] = a->scale[s];
+  }
+  p.W = a->W;
+  p.m = a->m;
+  p.v = a->v;
+  p.head_stride = a->head_stride;
+  p.G = a->G;
+  p.ldg = a->ldg;
+  p.g_stride = a->max_rows * a->ldg;
+  p.row_loss = a->row_loss;
+  p.row_correct = a->row_correct;
+  p.row_stride = a->max_rows;
+  p.dim = a->dim;
+  p.n_classes = a->n_classes;
+  p.active_mask = mask;
+  p.vec_rows = 1;
+  p.kind = a->kind;
+  p.beta1 = a->beta1;
+  p.beta2 = a->beta2;
+  p.eps = a->eps;
+  p.momentum = a->momentum;
+  if (temps) {
+    p.scale_dev = ad->scale_param;
+    p.scale_m = ad->scale_m;
+    p.scale_v = ad->scale_v;
+    p.row_dscale = ad->row_dscale;
+  }
+  if (adapter) {
+    p.zrows = ad->Z;
+    p.z_ld = ad->ldz;
+    p.z_stride = ad->max_img_rows * ad->ldz;
+  }
+  static const cudaError_t attr = [] {
+    cudaError_t e = cudaFuncSetAttribute(sweep_logits_tc_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, kTcLgSmemBytes);
+    if (e == cudaSuccess)
+      e = cudaFuncSetAttribute(sweep_logits_tc_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, kTcLgSmemBytes);
+    if (e == cudaSuccess)
+      e = cudaFuncSetAttribute(sweep_dw_update_tc_kernel<512>, cudaFuncAttributeMaxDynamicSharedMemorySize, kTcDwSmemBytes);
+    if (e == cudaSuccess) e = cudaFuncSetAttribute(sweep_dz_tc_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, kTcDzSmemBytes);
+    return e;
+  }();
+  UML_CUDA(attr);
+  // [K][rows][dim] views of the slabs for the dW kernel's slot ring: the head (C x D) and the adapter (D x Dv)
+  CUtensorMap tm_w, tm_m, tm_v, tma_w, tma_m, tma_v;
+  memset(&tm_v, 0, sizeof(tm_v));
+  memset(&tma_w, 0, sizeof(tma_w));
+  memset(&tma_m, 0, sizeof(tma_m));
+  memset(&tma_v, 0, sizeof(tma_v));
+  {
+    const uint64_t d = static_cast<uint64_t>(a->dim), c = static_cast<uint64_t>(a->n_classes), k = static_cast<uint64_t>(K);
+    const uint64_t hs = static_cast<uint64_t>(a->head_stride) * 4;
+    if (make_tmap_3d(&tm_w, a->W, CU_TENSOR_MAP_DATA_TYPE_FLOAT32, d, c, k, d * 4, hs, 128, 16, 1)) return 1;
+    if (make_tmap_3d(&tm_m, a->m, CU_TENSOR_MAP_DATA_TYPE_FLOAT32, d, c, k, d * 4, hs, 128, 16, 1)) return 1;
+    if (a->kind != 3 && make_tmap_3d(&tm_v, a->v, CU_TENSOR_MAP_DATA_TYPE_FLOAT32, d, c, k, d * 4, hs, 128, 16, 1)) return 1;
+    if (adapter) {
+      const uint64_t dv = static_cast<uint64_t>(ad->img_dim), as = static_cast<uint64_t>(ad->adapter_stride) * 4;
+      if (make_tmap_3d(&tma_w, ad->W, CU_TENSOR_MAP_DATA_TYPE_FLOAT32, dv, d, k, dv * 4, as, 128, 16, 1)) return 1;
+      if (make_tmap_3d(&tma_m, ad->m, CU_TENSOR_MAP_DATA_TYPE_FLOAT32, dv, d, k, dv * 4, as, 128, 16, 1)) return 1;
+      if (a->kind != 3 && make_tmap_3d(&tma_v, ad->v, CU_TENSOR_MAP_DATA_TYPE_FLOAT32, dv, d, k, dv * 4, as, 128, 16, 1))
+        return 1;
+    }
+  }
+  const int n_act = __builtin_popcount(mask);
+  int64_t pos[2] = {a->pos[0], a->pos[1]};
+  for (int i = 0; i < n_steps; ++i) {
+    const int64_t n0 = rows[2 * i], n1 = rows[2 * i + 1], R = n0 + n1;
+    UML_REQUIRE(n0 >= 0 && n1 >= 0 && R > 0 && R <= a->max_rows, "sweep_adapter_run: step %d has %lld rows (capacity %lld)", i,
+                static_cast<long long>(R), static_cast<long long>(a->max_rows));
+    UML_REQUIRE(!adapter || n0 <= ad->max_img_rows, "sweep_adapter_run: step %d has %lld image rows (Z holds %lld)", i,
+                static_cast<long long>(n0), static_cast<long long>(ad->max_img_rows));
+    for (int s = 0; s < 2; ++s) {
+      const int64_t n = s ? n1 : n0;
+      if (n == 0) continue;
+      UML_REQUIRE(a->bank[s] && a->labels[s] && pos[s] >= 0 && pos[s] + n <= a->perm_len[s],
+                  "sweep_adapter_run: step %d runs past the end of permutation %d", i, s);
+      for (int k = 0; k < K; ++k)
+        UML_REQUIRE(!((mask >> k) & 1u) || a->perm[s][k], "sweep_adapter_run: head %d has no permutation %d", k, s);
+    }
+    p.n0 = n0;
+    p.n1 = n1;
+    p.pos[0] = pos[0];
+    p.pos[1] = pos[1];
+    p.stats = a->stats + static_cast<int64_t>(i) * K * 2;
+    const double t = static_cast<double>(a->step + i);
+    const double bc1 = 1.0 - pow(static_cast<double>(a->beta1), t);
+    const double bc2 = 1.0 - pow(static_cast<double>(a->beta2), t);
+    p.bc2_sqrt_inv = static_cast<float>(1.0 / sqrt(bc2));
+    p.first_step = (a->step + i) <= 1;
+    for (int k = 0; k < K; ++k) {
+      const float l = lr[static_cast<int64_t>(i) * K + k];
+      p.lr[k] = l;
+      p.step_size[k] = static_cast<float>(static_cast<double>(l) / bc1);
+      p.decay[k] = static_cast<float>(1.0 - static_cast<double>(l) * static_cast<double>(a->weight_decay[k]));
+    }
+    const bool timed = i == n_steps - 1;
+    auto mark = [&](int e) -> int {
+      if (timed && ad->ev[e]) UML_CUDA(cudaEventRecord(static_cast<cudaEvent_t>(ad->ev[e]), st));
+      return 0;
+    };
+    const bool with_adapter = adapter && n0 > 0;
+    // the adapter's side of the step: its rows are the image rows, its "classes" the head's input dims
+    SweepDev pa = p;
+    pa.zrows = nullptr;
+    pa.scale_dev = nullptr;
+    pa.n1 = 0;
+    pa.bank[1] = nullptr;
+    pa.dim = ad->img_dim;
+    pa.n_classes = a->dim;
+    pa.W = ad->W;
+    pa.m = ad->m;
+    pa.v = ad->v;
+    pa.head_stride = ad->adapter_stride;
+    pa.stats = nullptr;
+    if (mark(0)) return 1;
+    if (with_adapter) {  // Z_k = X_img Wp_k^T: the logits kernel without softmax, the adapter as its weight
+      pa.G = ad->Z;
+      pa.ldg = ad->ldz;
+      pa.g_stride = ad->max_img_rows * ad->ldz;
+      sweep_logits_tc_kernel<false><<<dim3(static_cast<unsigned>((a->dim + 127) / 128), 1, K), 256, kTcLgSmemBytes, st>>>(pa);
+      UML_CUDA(cudaGetLastError());
+      ++g_sweep_launches;
+    }
+    if (mark(1) || mark(2)) return 1;
+    const unsigned n_ctile = static_cast<unsigned>((a->n_classes + 127) / 128);
+    UML_CUDA(launch_kernel(sweep_logits_tc_kernel<true>, dim3(n_ctile, 1, K), dim3(256), kTcLgSmemBytes, st,
+                           static_cast<int>(n_ctile), 0, p));
+    ++g_sweep_launches;
+    if (mark(3) || mark(4)) return 1;
+    if (with_adapter) {  // dZ from the head's weights before their update
+      sweep_dz_tc_kernel<<<dim3(static_cast<unsigned>((a->dim + 127) / 128), K), 256, kTcDzSmemBytes, st>>>(p, ad->dZ, ad->ldz,
+                                                                                                        ad->max_img_rows * ad->ldz);
+      UML_CUDA(cudaGetLastError());
+      ++g_sweep_launches;
+    }
+    if (mark(5) || mark(6)) return 1;
+    {
+      const int64_t units = static_cast<int64_t>(n_act) * ((a->dim + 127) / 128) * ((a->n_classes + 63) / 64);
+      const unsigned g = static_cast<unsigned>(std::min<int64_t>(units, sm_count()));
+      sweep_dw_update_tc_kernel<512><<<g, 512 + 64, kTcDwSmemBytes, st>>>(p, tm_w, tm_m, tm_v);
+      UML_CUDA(cudaGetLastError());
+      ++g_sweep_launches;
+    }
+    if (mark(7) || mark(8)) return 1;
+    if (with_adapter) {  // dWp_k = dZ_k^T X_img with the update; the statistics warp is off (pa.stats == NULL)
+      pa.G = ad->dZ;
+      pa.ldg = ad->ldz;
+      pa.g_stride = ad->max_img_rows * ad->ldz;
+      const int64_t units = static_cast<int64_t>(n_act) * ((ad->img_dim + 127) / 128) * ((a->dim + 63) / 64);
+      const unsigned g = static_cast<unsigned>(std::min<int64_t>(units, sm_count()));
+      sweep_dw_update_tc_kernel<512><<<g, 512 + 64, kTcDwSmemBytes, st>>>(pa, tma_w, tma_m, tma_v);
+      UML_CUDA(cudaGetLastError());
+      ++g_sweep_launches;
+    }
+    if (mark(9)) return 1;
     pos[0] += n0;
     pos[1] += n1;
   }

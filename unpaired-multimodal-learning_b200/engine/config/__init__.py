@@ -59,3 +59,6 @@ _add("--precision", type=str, default="auto", choices=["auto", "fp32", "bf16"],
 _add("--sweep-batched", action="store_true", default=False,
      help="train the hyper-parameter combinations of the sweep in lock step on one GPU (one step of all heads = four "
           "launches) instead of one after the other; every combination gets its own seeded sampler stream")
+_add("--sweep-batched-adapter", action="store_true", default=False,
+     help="--sweep-batched, and the combinations whose heads have an image adapter or learnable temperatures (preset "
+          "'linear') also train in lock step (five launches per step of all heads) instead of one after the other")

@@ -14,7 +14,7 @@ from typing import List, Optional, Sequence
 import torch
 
 from .. import _lib
-from .._lib import SWEEP_MAX_HEADS, SweepArgs, check
+from .._lib import SWEEP_MAX_HEADS, SweepAdapterArgs, SweepArgs, check
 from ..ops import UPDATE_KINDS
 
 MAX_HEADS = SWEEP_MAX_HEADS
@@ -52,6 +52,53 @@ def group_blockers(models, optimizers, image_loaders, text_loaders) -> List[str]
     return why
 
 
+ADAPTER_MAX_ROWS = 64  # rows per step of uml_sweep_adapter_run (one feature tile of its tensor-core kernels)
+ADAPTER_MAX_CLASSES = 1024  # softmax / CE in the logits epilogue
+
+
+def adapter_group_blockers(models, optimizers, image_loaders, text_loaders) -> List[str]:
+    """Why these runs cannot share an AdapterHeadGroup (empty list: they can): UML heads with an image adapter and / or
+    learnable temperatures, the runs of preset ``linear``."""
+    why = []
+    m0, o0 = models[0], optimizers[0]
+    if len(models) > MAX_HEADS:
+        why.append(f"more than {MAX_HEADS} heads")
+    if not all(hasattr(m, "img_scale") for m in models):
+        why.append("only UML heads (image adapter, per-modality temperatures) are batched with adapters")
+        return why
+    adapters = [m.img_proj is not None for m in models]
+    if any(adapters) and not all(adapters):
+        why.append("heads mix adapter and non-adapter variants")
+    if any(m.num_classes != m0.num_classes or m.shared_dim != m0.shared_dim or m.img_indim != m0.img_indim for m in models):
+        why.append("heads differ in shape")
+    if any(bool(m.learnable_temp) != bool(m0.learnable_temp) for m in models):
+        why.append("heads differ in learnable_temp")
+    elif not m0.learnable_temp and any(tuple(float(s) for s in m.scales()) != tuple(float(s) for s in m0.scales())
+                                       for m in models):
+        why.append("heads differ in logit scale")
+    if m0.num_classes > ADAPTER_MAX_CLASSES:
+        why.append(f"more than {ADAPTER_MAX_CLASSES} classes")
+    if m0.shared_dim % 4 or (m0.img_proj is not None and m0.img_indim % 4):
+        why.append("feature widths must be multiples of 4")
+    rows = sum(ls[0].batch_size for ls in (image_loaders, text_loaders) if ls and ls[0] is not None)
+    if rows > ADAPTER_MAX_ROWS:
+        why.append(f"more than {ADAPTER_MAX_ROWS} rows per step")
+    if any(o.name != o0.name or o.defaults["betas"] != o0.defaults["betas"] or o.defaults["eps"] != o0.defaults["eps"]
+           or o.defaults["momentum"] != o0.defaults["momentum"] for o in optimizers):
+        why.append("optimizers differ in kind / betas / eps / momentum")
+    for loaders in (image_loaders, text_loaders):
+        live = [l for l in loaders if l is not None]
+        if live and len(live) != len(loaders):
+            why.append("runs differ in modality")
+        elif live:
+            l0 = live[0]
+            if any(l.bank is not l0.bank or l.batch_size != l0.batch_size or l.drop_last != l0.drop_last
+                   or not l.shuffle or l.generator is not None or l.shard_of is not None or l.upload != "epoch"
+                   for l in live):
+                why.append("loaders must share bank, batch size and protocol (shuffled, upload='epoch', no generator)")
+    return why
+
+
 class HeadGroup:
     def __init__(self, models: Sequence, optimizers: Sequence, image_bank, text_bank, max_img_rows: int,
                  max_txt_rows: int, device, log_slots: int = 128):
@@ -68,9 +115,9 @@ class HeadGroup:
         if self.kind == 0:
             raise ValueError("HeadGroup needs an optimizer")
         self.banks = (image_bank, text_bank)
-        for b in self.banks:
-            if b is not None and (b.features.dtype != torch.float32 or b.dim != self.D or not b.features.is_contiguous()):
-                raise ValueError("HeadGroup: banks must be contiguous fp32 [N, shared_dim]")
+        for b, width in zip(self.banks, self._row_widths(m0)):
+            if b is not None and (b.features.dtype != torch.float32 or b.dim != width or not b.features.is_contiguous()):
+                raise ValueError("HeadGroup: banks must be contiguous fp32 [N, row width]")
         self.max_rows = int(max_img_rows) + int(max_txt_rows)
         n = self.C * self.D
         self.stride = (n + 3) // 4 * 4
@@ -151,13 +198,25 @@ class HeadGroup:
         rows_c = (C.c_int64 * (2 * n))(*[int(x) for r in rows for x in r])
         lr_c = (C.c_float * (n * K))(*[float(x) for l in lrs for x in l])
         l0 = _lib.load().uml_sweep_launch_count()
-        check(_lib.load().uml_sweep_run(C.byref(a), n, rows_c, lr_c, torch.cuda.current_stream().cuda_stream))
-        launched = (_lib.load().uml_sweep_launch_count() - l0) & 0x7FFFFFFF  # two to four kernels per step (csrc/sweep.cu)
+        check(self._enqueue(n, rows_c, lr_c))
+        launched = (_lib.load().uml_sweep_launch_count() - l0) & 0x7FFFFFFF  # two to five kernels per step (csrc/sweep.cu)
         self.launches += launched
         _lib.LAUNCH_COUNT[0] += launched
         for k in range(K):
             if active[k]:
-                self.opts[k].slot(self.models[k].head.weight)["step"] += n
+                for p in self._trained(self.models[k]):
+                    self.opts[k].slot(p)["step"] += n
+
+    def _row_widths(self, m0):
+        """Widths of the image and text bank rows."""
+        return self.D, self.D
+
+    def _trained(self, model):
+        """The parameters of a head that one step updates."""
+        return [model.head.weight]
+
+    def _enqueue(self, n, rows_c, lr_c):
+        return _lib.load().uml_sweep_run(C.byref(self.args), n, rows_c, lr_c, torch.cuda.current_stream().cuda_stream)
 
     KERNELS = ("sweep_logits", "sweep_softmax_ce", "sweep_dw_update", "sweep_stats")
 
@@ -190,3 +249,98 @@ class HeadGroup:
                 out[name_l] = raw[idx, :, s, 0].tolist()
                 out[name_a] = (ints[idx, :, s, 2] / ints[idx, :, s, 3].clip(min=1)).tolist()
         return out
+
+
+class AdapterHeadGroup(HeadGroup):
+    """HeadGroup for UML heads with an image adapter (``img_proj``, Dv -> D) and / or learnable temperatures
+    (``img_scale``, ``txt_scale``): one step of all K heads is five launches (``uml_sweep_adapter_run``) - Z = X Wp^T,
+    logits + softmax / CE over [Z; X_txt] (+ per-row d loss / d scale), dZ = G W, head dW + update + statistics +
+    temperature update, adapter dWp + update; two without an adapter.  Besides the head's slabs, the adapters and
+    their optimizer state live in ``[K, D*Dv]`` slabs and the temperatures in ``[K, 2]`` ones; every module's
+    parameters and optimizer state become views into them."""
+
+    KERNELS = ("sweep_adapter_z", "sweep_logits", "sweep_adapter_dz", "sweep_dw_update", "sweep_adapter_dw_update")
+
+    def __init__(self, models: Sequence, optimizers: Sequence, image_bank, text_bank, max_img_rows: int,
+                 max_txt_rows: int, device, log_slots: int = 128):
+        super().__init__(models, optimizers, image_bank, text_bank, max_img_rows, max_txt_rows, device, log_slots)
+        if self.max_rows > ADAPTER_MAX_ROWS:
+            raise ValueError(f"AdapterHeadGroup: at most {ADAPTER_MAX_ROWS} rows per step")
+        K, D, m0 = self.K, self.D, models[0]
+        self.Dv = int(m0.img_indim) if m0.img_proj is not None else 0
+        self.learnable = bool(m0.learnable_temp)
+        sgd = optimizers[0].name == "sgd"
+        ad = self.adapter_args = SweepAdapterArgs()
+
+        def adopt(slabs, k, p, shape, opt):
+            """p.data and its optimizer state become views of row k of the (param, m, v) slabs."""
+            n = p.numel()
+            view = slabs[0][k, :n].view(shape)
+            view.copy_(p.data)
+            p.data = view
+            st = opt.slot(p)
+            if st["step"] != 0:
+                raise ValueError("AdapterHeadGroup: optimizers must be fresh")
+            st["m"] = slabs[1][k, :n].view(shape)
+            if slabs[2] is not None:
+                st["v"] = slabs[2][k, :n].view(shape)
+
+        if self.Dv:
+            self.a_stride = (D * self.Dv + 3) // 4 * 4
+            self.Wp = torch.empty((K, self.a_stride), device=self.device)
+            self.mp = torch.zeros((K, self.a_stride), device=self.device)
+            self.vp = None if sgd else torch.zeros((K, self.a_stride), device=self.device)
+            for k, (model, opt) in enumerate(zip(models, optimizers)):
+                adopt((self.Wp, self.mp, self.vp), k, model.img_proj.weight, (D, self.Dv), opt)
+            self.ldz = D
+            self.Z = torch.empty((K, max(int(max_img_rows), 1), D), device=self.device)
+            self.dZ = torch.empty_like(self.Z)
+            ad.img_dim, ad.adapter_stride = self.Dv, self.a_stride
+            ad.W, ad.m = self.Wp.data_ptr(), self.mp.data_ptr()
+            ad.v = self.vp.data_ptr() if self.vp is not None else None
+            ad.Z, ad.dZ, ad.ldz, ad.max_img_rows = self.Z.data_ptr(), self.dZ.data_ptr(), self.ldz, self.Z.shape[1]
+        if self.learnable:
+            self.T = torch.empty((K, 2), device=self.device)
+            self.Tm = torch.zeros((K, 2), device=self.device)
+            self.Tv = None if sgd else torch.zeros((K, 2), device=self.device)
+            for k, (model, opt) in enumerate(zip(models, optimizers)):
+                for j, p in enumerate((model.img_scale, model.txt_scale)):
+                    adopt((self.T[:, j:j + 1], self.Tm[:, j:j + 1], self.Tv[:, j:j + 1] if self.Tv is not None else None),
+                          k, p, (), opt)
+            self.row_dscale = torch.empty((K, self.max_rows), device=self.device)
+            ad.scale_param, ad.scale_m = self.T.data_ptr(), self.Tm.data_ptr()
+            ad.scale_v = self.Tv.data_ptr() if self.Tv is not None else None
+            ad.row_dscale = self.row_dscale.data_ptr()
+
+    def _row_widths(self, m0):
+        return (int(m0.img_indim) if m0.img_proj is not None else self.D), self.D
+
+    def _trained(self, model):
+        ps = [model.head.weight]
+        if model.img_proj is not None:
+            ps.append(model.img_proj.weight)
+        if model.learnable_temp:
+            ps += [model.img_scale, model.txt_scale]
+        return ps
+
+    def _enqueue(self, n, rows_c, lr_c):
+        return _lib.load().uml_sweep_adapter_run(C.byref(self.args), C.byref(self.adapter_args), n, rows_c, lr_c,
+                                                 torch.cuda.current_stream().cuda_stream)
+
+    def image_scales(self):
+        """Every head's image-run temperature, one read-back (what evaluation multiplies the logits by)."""
+        if self.learnable:
+            return self.T[:, 0].tolist()
+        return [float(m.scales()[0]) for m in self.models]
+
+    def time_last_step(self, enable: bool = True):
+        """Bracket the five launch sites of the LAST step of every following ``run`` with CUDA events (a skipped site
+        spans nothing)."""
+        n = 2 * len(self.KERNELS)
+        self._ev = [torch.cuda.Event(enable_timing=True) for _ in range(n)] if enable else []
+        for i in range(n):
+            if enable:
+                self._ev[i].record()
+                self.adapter_args.ev[i] = self._ev[i].cuda_event
+            else:
+                self.adapter_args.ev[i] = None

@@ -104,14 +104,15 @@ def _dbg(msg):
         print(f"[train] {msg}", file=sys.stderr, flush=True)
 
 
-def validate_enqueue(model, val_loader):
+def validate_enqueue(model, val_loader, s_img=None):
     """Launches the evaluation of ``validate`` and returns ``(loss, hits, n_rows)`` - two one-element DEVICE tensors
-    and the row count - without synchronising; callers that evaluate many heads read them back together."""
+    and the row count - without synchronising; callers that evaluate many heads read them back together.  ``s_img``:
+    the model's image temperature when the caller has already read it (a learnable one lives on the device)."""
     iter(val_loader)  # a DataLoader iterator draws a base seed from the global RNG; keep the stream aligned
     bank, bs = val_loader.bank, val_loader.batch_size
     n = len(bank)
     dev = bank.device
-    s_img = float(model.scales()[0])
+    s_img = float(model.scales()[0]) if s_img is None else float(s_img)
     row_loss = torch.empty(n, device=dev)
     row_pred = torch.empty(n, device=dev, dtype=torch.int32)
     W = model.head.weight.data
@@ -398,7 +399,9 @@ def train(model, image_loader, text_loader, val_loader, test_loader, optimizer, 
 def train_group(models, image_loaders, text_loaders, val_loaders, test_loaders, optimizers, schedulers, device="cuda",
                 max_iters=1000, alphas=1.0, eval_freq=EVAL_FREQ, patience=5, loggers=None, traces=None, tags=None):
     """K runs of ``train`` advanced in lock step over shared banks (sweep-level batching, SURVEY §8 f-1): one step of all
-    K heads is two launches (``engine/sweep.py``, ``csrc/sweep.cu``) instead of K latency-bound steps.
+    K heads is two launches (``engine/sweep.py``, ``csrc/sweep.cu``) instead of K latency-bound steps.  When every head
+    has an image adapter or learnable temperatures (preset ``linear``) the heads form an ``AdapterHeadGroup`` instead
+    (up to five launches per step) and are evaluated head by head with ``validate_enqueue``.
 
     Every argument that ``train`` takes once is a list with one entry per head (``max_iters``, ``alphas`` and
     ``patience`` may be scalars); returns the list of ``train``'s result dicts.  Head k follows exactly the loop of
@@ -407,7 +410,7 @@ def train_group(models, image_loaders, text_loaders, val_loaders, test_loaders, 
     run draws them from the global generator, so head k reproduces ``torch.manual_seed(s); train(...)`` when its
     generator was seeded with ``s``.  (The reference's sequential sweep lets one global stream run through all
     combinations; the order inside each run is the same, the seeds differ.)"""
-    from .engine.sweep import HeadGroup, group_blockers
+    from .engine import sweep as sweep_mod
 
     K = len(models)
     as_list = lambda x: list(x) if isinstance(x, (list, tuple)) else [x] * K
@@ -418,7 +421,9 @@ def train_group(models, image_loaders, text_loaders, val_loaders, test_loaders, 
     loggers = as_list(loggers) if loggers is not None else [None] * K
     traces = as_list(traces) if traces is not None else [None] * K
     tags = as_list(tags) if tags is not None else [f"head {k}" for k in range(K)]
-    why = group_blockers(models, optimizers, image_loaders, text_loaders)
+    adapter = all(m.img_proj is not None or getattr(m, "learnable_temp", False) for m in models)
+    blockers = sweep_mod.adapter_group_blockers if adapter else sweep_mod.group_blockers
+    why = blockers(models, optimizers, image_loaders, text_loaders)
     if _dist()[1] > 1:
         why.append("data-parallel runs are not batched")
     if why:
@@ -429,8 +434,9 @@ def train_group(models, image_loaders, text_loaders, val_loaders, test_loaders, 
     for m in models:
         m.train()
     log_slots = min(max(int(eval_freq), 1), int(max(max_iters))) + 1
-    group = HeadGroup(models, optimizers, il0.bank if has_img else None, tl0.bank if has_txt else None,
-                      il0.batch_size if has_img else 0, tl0.batch_size if has_txt else 0, device, log_slots=log_slots)
+    group = (sweep_mod.AdapterHeadGroup if adapter else sweep_mod.HeadGroup)(
+        models, optimizers, il0.bank if has_img else None, tl0.bank if has_txt else None,
+        il0.batch_size if has_img else 0, tl0.batch_size if has_txt else 0, device, log_slots=log_slots)
     outs = [{"iter": None, "val_acc": None, "model": None, "val_classwise": None, "val_loss": None, "model_records": []}
             for _ in range(K)]
     for tr in traces:
@@ -539,11 +545,17 @@ def train_group(models, image_loaders, text_loaders, val_loaders, test_loaders, 
             heads = [k for k in range(K) if running[k]]
             # every head's evaluation is enqueued before anything is read back: one synchronisation per round
             # the same draw order per head as the sequential loop (val, then test): each head has its own generator
-            results = validate_group_enqueue(group, models, heads, lambda k: val_loaders[k])
             with_test = [k for k in heads if test_loaders[k] is not None]
-            t_res = dict(zip(with_test, validate_group_enqueue(group, models, with_test, lambda k: test_loaders[k]))) if with_test else {}
+            if adapter:  # head by head (the adapter runs in fp32 inside validate_enqueue), all enqueued before one read-back
+                s_img = group.image_scales()
+                results = [validate_enqueue(models[k], val_loaders[k], s_img[k]) for k in heads]
+                t_res = {k: validate_enqueue(models[k], test_loaders[k], s_img[k]) for k in with_test}
+                snaps = None
+            else:
+                results = validate_group_enqueue(group, models, heads, lambda k: val_loaders[k])
+                t_res = dict(zip(with_test, validate_group_enqueue(group, models, with_test, lambda k: test_loaders[k]))) if with_test else {}
+                snaps = group.W.clone()
             tests = [t_res.get(k) for k in heads]
-            snaps = group.W.clone()
             losses = torch.cat([r[0] for r in results]).cpu().tolist()
             hits = torch.cat([r[1] for r in results]).cpu().tolist()
             for h, k in enumerate(heads):
@@ -552,8 +564,11 @@ def train_group(models, image_loaders, text_loaders, val_loaders, test_loaders, 
                 if tests[h] is not None:
                     testlog = f" | Test Acc: {int(tests[h][1].item()) / tests[h][2]:.4f}"
                 if outs[k]["val_acc"] is None or val_acc > outs[k]["val_acc"]:
-                    w = snaps[k, :group.C * group.D].view(group.C, group.D).cpu()
-                    outs[k].update(iter=last_step, val_acc=val_acc, val_loss=val_loss, model={"head.weight": w})
+                    if snaps is None:  # every state-dict key: head.weight, img_proj.weight, img_scale, txt_scale
+                        best = {n_: v.detach().cpu().clone() for n_, v in models[k].state_dict().items()}
+                    else:
+                        best = {"head.weight": snaps[k, :group.C * group.D].view(group.C, group.D).cpu()}
+                    outs[k].update(iter=last_step, val_acc=val_acc, val_loss=val_loss, model=best)
                     no_improve[k] = 0
                 else:
                     no_improve[k] += 1
@@ -703,11 +718,21 @@ def setup_group(datasets, combos, args, positions=None):
     differ in --alpha and therefore in ``savepath``).  Run k's loaders draw from their own generator seeded
     ``run_seed(args_k, positions[k])`` (``positions``: each combination's index in the preset's grid, default
     0, 1, ...) - or from the global stream when ``args.seed < 0``."""
-    from .engine.sweep import MAX_HEADS, group_blockers
+    from .engine.sweep import MAX_HEADS, adapter_group_blockers, group_blockers
 
     per_run = list(args) if isinstance(args, (list, tuple)) else [args] * len(combos)
     positions = list(positions) if positions is not None else list(range(len(combos)))
     args = per_run[0]
+    with_adapters = bool(getattr(args, "sweep_batched_adapter", False))
+
+    def blockers(cand):
+        """--sweep-batched-adapter: runs with an image adapter or learnable temperatures form AdapterHeadGroups."""
+        ms = [ctxs[c]["model"] for c in cand]
+        adapter = with_adapters and any(m.img_proj is not None or getattr(m, "learnable_temp", False) for m in ms)
+        return (adapter_group_blockers if adapter else group_blockers)(
+            ms, [ctxs[c]["optimizer"] for c in cand], [ctxs[c]["image_loader"] for c in cand],
+            [ctxs[c]["text_loader"] for c in cand])
+
     results = [None] * len(combos)
     ctxs = {}
     for n, hp in enumerate(combos):
@@ -728,11 +753,9 @@ def setup_group(datasets, combos, args, positions=None):
             if len(members) >= MAX_HEADS:
                 break
             cand = members + [n]
-            if not group_blockers([ctxs[c]["model"] for c in cand], [ctxs[c]["optimizer"] for c in cand],
-                                  [ctxs[c]["image_loader"] for c in cand], [ctxs[c]["text_loader"] for c in cand]):
+            if not blockers(cand):
                 members = cand
-        solo = group_blockers([ctxs[first]["model"]], [ctxs[first]["optimizer"]], [ctxs[first]["image_loader"]],
-                              [ctxs[first]["text_loader"]]) or _dist()[1] > 1
+        solo = blockers([first]) or _dist()[1] > 1
         todo = [n for n in todo if n not in members]
         col = lambda key: [ctxs[c][key] for c in members]
         if solo:  # not batchable at all (adapter, learnable temperature, data parallel): the plain loop, same loaders
@@ -793,7 +816,7 @@ def _collect(hps, outcomes, args):
 
 def sweep(datasets, hyperparams, args):
     hps = _grid(hyperparams)
-    if getattr(args, "sweep_batched", False):
+    if getattr(args, "sweep_batched", False) or getattr(args, "sweep_batched_adapter", False):
         # --sweep-batched: the combinations train in lock step on one GPU (setup_group) instead of one after the other
         return _collect(hps, setup_group(datasets, hps, args), args)
     return _collect(hps, [lambda hp=hp: setup(datasets, hp, args) for hp in hps], args)
@@ -830,6 +853,8 @@ def main(args, alphas=None):
         os.environ.setdefault("MASTER_ADDR", "127.0.0.1")
         torch.distributed.init_process_group("nccl", device_id=torch.device(args.device))
     args.use_clip = args.vision_model == "" and args.language_model == ""
+    if getattr(args, "sweep_batched_adapter", False):
+        args.sweep_batched = True
     encoder_name = args.clip_encoder if args.use_clip else f"{args.vision_model}-{args.language_model}"
     alpha_list = [float(a) for a in alphas] if alphas else [args.alpha]
     savepaths = [savedir(args.result_dir, args.dataset, encoder_name, args.train_shot, args.seed, args.text_type,
@@ -929,7 +954,8 @@ def cli(argv=None):
     jobs = []
     for c in combos:
         rest_ = {k: v for k, v in c.items() if k != "alpha"}
-        mate = next((j for j in jobs if c.get("sweep_batched") and j[0] == rest_ and "alpha" in c), None)
+        batched = c.get("sweep_batched") or c.get("sweep_batched_adapter")
+        mate = next((j for j in jobs if batched and j[0] == rest_ and "alpha" in c), None)
         if mate is not None:
             mate[1].append(c["alpha"])
         else:
