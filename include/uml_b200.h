@@ -193,17 +193,6 @@ int uml_head_fwd_ce_bf16(const uint16_t* X, int64_t n_rows, int32_t dim, const u
 int uml_fwd_x_failed(const float* tile_ws);
 /* per-run {mean loss, dscale, hits, rows} from the forward kernel's per-tile partials (fixed order)     */
 int uml_reduce_tile_stats(const float* tile_ws, int64_t n_rows, int32_t nseg, uml_seg_stats* stats, void* stream);
-/* The same forward without its fix-up pass: G receives the unnormalised bf16 exp(l - m_running) and tile_ws the
- * per-row normalisation factors; only valid as the producer of uml_head_bwd_dw_fix_bf16, which applies
- * `G = G~ * factor - onehot * coef` to every operand stage in shared memory (the "softmax-minus-onehot term fused
- * into the dW prologue") and reduces the per-run statistics into `stats` with an otherwise idle warp.        */
-int uml_head_fwd_ce_deferred_bf16(const uint16_t* X, int64_t n_rows, int32_t dim, const uint16_t* W, int32_t n_classes,
-                                  const int32_t* labels, const uml_tc_segments* segs /*host*/, uint16_t* G, int64_t ldg,
-                                  float* tile_ws, void* stream);
-int uml_head_bwd_dw_fix_bf16(const uint16_t* G, int64_t ldg, const uint16_t* X, int64_t n_rows, int32_t dim,
-                             int32_t n_classes, float* partials, int32_t n_splits,
-                             const uml_tc_segments* segs /*host; NULL: G is already final (plain dW)*/,
-                             const int32_t* labels, const float* tile_ws, uml_seg_stats* stats /*nullable*/, void* stream);
 /* dW_partial[s] = (G^T X) over the s-th K split; partials: [n_splits, n_classes, dim] fp32.       */
 int uml_head_bwd_dw_bf16(const uint16_t* G, int64_t ldg, const uint16_t* X, int64_t n_rows, int32_t dim,
                          int32_t n_classes, float* partials, int32_t n_splits, void* stream);
@@ -258,8 +247,8 @@ typedef struct {
    * does not use) on a side stream while step i's GEMMs run                                                  */
   uint16_t*     X16_alt;  int32_t* labels32_alt;
   int64_t       g_capacity_rows;            /* rows the G workspace has room for (fp32 path: split-K planes); 0 = rows */
-  /* optional third operand buffers: the gather then runs two steps ahead, and no forward kernel waits for an event
-   * of the side stream that is signalled at the last moment (UML_PREFETCH_DEPTH=1 keeps one step ahead)              */
+  /* optional third operand buffers: the gather then runs two steps ahead (when a call has more than two steps), and
+   * no forward kernel waits for an event of the side stream that is signalled at the last moment                     */
   uint16_t*     X16_alt2;  int32_t* labels32_alt2;
   /* optional cudaEvent_t after which every index batch of the call is valid in device memory (recorded by whoever
    * uploaded them).  With it - and the three operand buffers - uml_linear_run keeps its gather pipeline running through

@@ -422,36 +422,6 @@ def test_grad_diagnostics_match_autograd():
     assert torch.equal(model.head.weight.detach().cpu(), w)  # a probe: nothing was updated
 
 
-@pytest.mark.parametrize("n_img,n_txt,d,c", [(300, 212, 256, 1000), (2048, 1500, 768, 1000), (129, 0, 512, 397), (1000, 1000, 512, 101),
-                                             (4736, 4736, 768, 1000)])
-def test_dw_prologue_fixup_matches_the_default_forward(n_img, n_txt, d, c):
-    """The deferred softmax normalisation applied to the dW operand stages in shared memory (tc_gemm kFix, an
-    experiment kept behind UML_FUSE_FIX=1) against the default path - the exchange forward kernel, whose G is final -
-    + plain dW: the same partial sums up to the bf16 rounding of G (the two paths round the rescaled probabilities
-    differently), the same hit counts, the same per-run statistics."""
-    xi, yi, xt, yt, w, g = _mk(n_img + d + c, max(n_img, 1), max(n_txt, 1), d, d, c)
-    x = torch.cat([xi[:n_img], xt[:n_txt]]).to(DEV)
-    y = torch.cat([yi[:n_img], yt[:n_txt]]).to(DEV).to(torch.int32)
-    n = n_img + n_txt
-    x16, w16 = ops.cast_bf16(x), ops.cast_bf16(w.to(DEV))
-    rows = [k for k in (n_img, n_txt) if k]
-    segs = ops.tc_segments(rows, [30.0] * len(rows), [1.0, 0.5][:len(rows)])
-    splits = max(1, ops.tc_dw_splits(n, d, c))
-    ws_a, ws_b = ops.HeadWorkspace(n, c, DEV, bf16=True), ops.HeadWorkspace(n, c, DEV, bf16=True)
-    pa, pb = torch.zeros(splits, c, d, device=DEV), torch.zeros(splits, c, d, device=DEV)
-    st_a, st_b = torch.zeros(2, 4, device=DEV), torch.zeros(2, 4, device=DEV)
-    # (row_dscale asks the exchange kernel for d loss / d scale, which it otherwise only computes for a learnable temperature)
-    ops.head_fwd_ce_bf16(x16, w16, y, segs, ws_a, None, n_rows=n, stats=st_a, row_dscale=ws_a.row_dscale)
-    ops.head_bwd_dw_bf16(ws_a.G, ws_a.ldg, x16, n, c, pa, splits)
-    ops.head_fwd_ce_deferred_bf16(x16, w16, y, segs, ws_b, n_rows=n)
-    ops.head_bwd_dw_fix_bf16(ws_b, x16, n, c, pb, splits, segs, y, stats=st_b)
-    torch.cuda.synchronize()
-    assert (pa.sum(0) - pb.sum(0)).abs().max().item() <= 2e-3 * pa.sum(0).abs().max().item()
-    k = len(rows)
-    assert torch.equal(st_a.view(torch.int32)[:k, 2:], st_b.view(torch.int32)[:k, 2:])       # hits, rows
-    torch.testing.assert_close(st_a[:k, :2], st_b[:k, :2], rtol=2e-4, atol=2e-5)             # mean loss, dscale
-
-
 def test_full_size_step_properties():
     """BASELINE.json's throughput shape (2 x 18944 rows, D=768, C=1000) is too big for the CPU oracle in a unit test;
     check size-independent properties of the tensor-core step instead:

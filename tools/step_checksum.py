@@ -1,5 +1,5 @@
-"""Prints a checksum of the head weights and the per-step stats after 9 bf16 steps of a fixed scenario - run it under
-different launcher settings (UML_OVERLAP_FIXUP, UML_PREFETCH, UML_PREFETCH_AT, UML_FUSE_FIX) to check they are bit-identical."""
+"""Prints a checksum of the head weights and the per-step stats after 9 bf16 steps of a fixed scenario - run it against
+two builds of the library (UML_LIB_PATH selects one) to check that they compute bit-identical results."""
 import hashlib
 import os
 import sys

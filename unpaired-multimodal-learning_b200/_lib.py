@@ -112,9 +112,6 @@ PROTOTYPES = {
     "uml_head_fwd_ce_bf16": [c_vp, c_i64, c_i32, c_vp, c_i32, c_vp, C.POINTER(TcSegments), c_vp, c_i64, c_vp, c_vp,
                              c_vp, c_vp, c_vp, c_vp, c_vp],
     "uml_head_bwd_dw_bf16": [c_vp, c_i64, c_vp, c_i64, c_i32, c_i32, c_vp, c_i32, c_vp],
-    "uml_head_fwd_ce_deferred_bf16": [c_vp, c_i64, c_i32, c_vp, c_i32, c_vp, C.POINTER(TcSegments), c_vp, c_i64, c_vp, c_vp],
-    "uml_head_bwd_dw_fix_bf16": [c_vp, c_i64, c_vp, c_i64, c_i32, c_i32, c_vp, c_i32, C.POINTER(TcSegments), c_vp, c_vp, c_vp,
-                                 c_vp],
     "uml_tc_dw_splits": [c_i64, c_i32, c_i32],
     "uml_gemm_bf16": [c_vp, c_i64, c_i32, c_vp, c_i64, c_i32, c_i64, c_i64, c_i64, c_vp, c_i64, c_i32, c_i32, c_vp],
     "uml_gemm_bf16_splits": [c_i64, c_i64, c_i64],
@@ -160,7 +157,7 @@ _lib = None
 # kernels launched per C-ABI call (bench.py reports the sum as "gpu_launches")
 KERNELS_PER_CALL = {
     "uml_gather_rows_f32": 1, "uml_gather_rows_bf16": 1, "uml_gather_labels_i32": 1, "uml_cast_f32_to_bf16": 1,
-    "uml_gather_rows_labels_bf16": 1, "uml_gather2_rows_bf16": 1, "uml_gather2_rows_bf16_light": 1, "uml_gauss_step": 2, "uml_gauss_eval": 2, "uml_head_fwd_ce_deferred_bf16": 1, "uml_head_bwd_dw_fix_bf16": 1,
+    "uml_gather_rows_labels_bf16": 1, "uml_gather2_rows_bf16": 1, "uml_gather2_rows_bf16_light": 1, "uml_gauss_step": 2, "uml_gauss_eval": 2,
     "uml_head_fwd_ce_f32": 3, "uml_head_bwd_dw_f32": 1, "uml_gemm_nt_f32": 1, "uml_gemm_nn_f32": 1,
     "uml_gemm_tn_f32": 1, "uml_adamw_step": 1, "uml_sgd_step": 1, "uml_eval_f32": 1, "uml_eval_reduce": 1, "uml_eval_group_f32": 1, "uml_eval_reduce_group": 1, "uml_cka_linear_f32": 3, "uml_mutual_knn_f32": 4, "uml_gauss_embed": 1,
     "uml_grad_diag": 2, "uml_head_fwd_ce_bf16": 2, "uml_reduce_tile_stats": 1, "uml_head_bwd_dw_bf16": 1, "uml_gemm_bf16": 1, "uml_adamw_step_partials": 1,

@@ -45,37 +45,24 @@ void set_error(const char* fmt, ...);
 inline cudaStream_t as_stream(void* s) { return reinterpret_cast<cudaStream_t>(s); }
 
 int sm_count();  // cached multiprocessor count of the current device
-// Programmatic dependent launch between the kernels of a step: a launch site takes part when its bit is set in the mask
-// (env UML_PDL, default kPdlDefault): the dependent's CTAs may become resident - and run their prologue up to
-// griddepcontrol.wait - while the kernel before it drains.
-enum : int { kPdlFwd = 1, kPdlDw = 2, kPdlUpdate = 4, kPdlGather = 8, kPdlStats = 16, kPdlFwdOld = 32 };
-int pdl_mask();
 
-// Launch with optional thread-block cluster and programmatic stream serialization (PDL).  A kernel launched
-// with `pdl` MUST execute pdl_wait() before touching anything an earlier kernel on the stream produced (or
-// overwriting anything it reads) - and must execute it even if it needs nothing, so that completion stays
-// transitive along the stream.
+// Launch with an optional thread-block cluster of cluster_x CTAs along x.
 template <typename... KArgs, typename... Args>
 inline cudaError_t launch_kernel(void (*kern)(KArgs...), dim3 grid, dim3 block, size_t smem, cudaStream_t st, int cluster_x,
-                                 int pdl_site, Args... args) {
+                                 Args... args) {
   cudaLaunchConfig_t cfg;
   memset(&cfg, 0, sizeof(cfg));
   cfg.gridDim = grid;
   cfg.blockDim = block;
   cfg.dynamicSmemBytes = smem;
   cfg.stream = st;
-  cudaLaunchAttribute attr[2];
+  cudaLaunchAttribute attr[1];
   unsigned na = 0;
   if (cluster_x > 1) {
     attr[na].id = cudaLaunchAttributeClusterDimension;
     attr[na].val.clusterDim.x = static_cast<unsigned>(cluster_x);
     attr[na].val.clusterDim.y = 1;
     attr[na].val.clusterDim.z = 1;
-    ++na;
-  }
-  if (pdl_site & pdl_mask()) {
-    attr[na].id = cudaLaunchAttributeProgrammaticStreamSerialization;
-    attr[na].val.programmaticStreamSerializationAllowed = 1;
     ++na;
   }
   cfg.attrs = attr;
@@ -102,12 +89,6 @@ __device__ __forceinline__ uint32_t smem_u32(const void* p) {
 }
 
 __device__ __forceinline__ uint32_t lane_id() { return threadIdx.x & 31u; }
-
-// ---- programmatic dependent launch --------------------------------------------------------------
-// pdl_trigger: the next kernel on the stream may start launching (its prologue overlaps our run / tail).
-// pdl_wait   : blocks until every kernel this one depends on has completed and its writes are visible.
-__device__ __forceinline__ void pdl_trigger() { asm volatile("griddepcontrol.launch_dependents;" ::: "memory"); }
-__device__ __forceinline__ void pdl_wait() { asm volatile("griddepcontrol.wait;" ::: "memory"); }
 
 __device__ __forceinline__ bool elect_one() {
   uint32_t pred = 0;

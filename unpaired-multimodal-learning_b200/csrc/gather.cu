@@ -10,12 +10,17 @@
 // (this is the A operand of the tcgen05 head GEMM).  Stages are ring-buffered so several hundred KB
 // are in flight per SM, which is what an HBM-latency-bound gather needs.
 #include <algorithm>
-#include <cstdlib>
 
 #include "common.cuh"
-#include "gather.cuh"
 
 namespace uml {
+
+struct CopySeg {
+  const unsigned char* bank;   // row-major, row_bytes per row
+  const int64_t* idx;          // gather indices (required)
+  const int64_t* labels;       // bank labels (int64) or nullptr
+  int64_t n;
+};
 
 constexpr int kGatherStages = 3;
 constexpr int kGatherStageBytes = 48 * 1024;
@@ -102,12 +107,10 @@ __global__ void gather_labels_kernel(const int64_t* __restrict__ labels, const i
 
 // Row copy for banks that already hold the operand type (the bf16 shadow of a feature bank): both runs of a
 // step - image rows then text rows - in ONE launch, bytes moved by the TMA engine only (bulk global->shared,
-// bulk shared->global), no thread ever touches the data.  4-stage ring: the stage refilled at iteration `it`
-// is the one whose stores were committed at `it - 1`, so one store group may stay in flight.
-constexpr int kCopyStagesFull = 4;   // stand-alone launch: 4 x 48 KB
-constexpr int kCopyStagesLight = 3;  // side-stream launch next to a GEMM CTA: 3 x <= 9 KB
+// bulk shared->global), no thread ever touches the data.  4-stage ring of up to 48 KB each: the stage refilled at
+// iteration `it` is the one whose stores were committed at `it - 1`, so one store group may stay in flight.
+constexpr int kCopyStages = 4;
 
-template <int kCopyStages>
 __global__ void __launch_bounds__(32)
     gather_copy2_kernel(CopySeg s0, CopySeg s1, uint32_t row_bytes, int rows_per_stage, unsigned char* __restrict__ out,
                         int64_t out_pitch, int32_t* __restrict__ out_labels) {
@@ -122,8 +125,6 @@ __global__ void __launch_bounds__(32)
     fence_barrier_init();
   }
   __syncwarp();
-  pdl_trigger();
-  pdl_wait();  // the previous step's dW still reads the operand buffer this kernel overwrites
 
   auto issue = [&](int64_t it) {
     const int64_t g = blockIdx.x + it * gridDim.x;
@@ -212,7 +213,29 @@ __global__ void __launch_bounds__(256)
                           int32_t* __restrict__ out_labels) {
   const int64_t warp = (blockIdx.x * static_cast<int64_t>(blockDim.x) + threadIdx.x) >> 5;
   const int64_t n_warps = (static_cast<int64_t>(gridDim.x) * blockDim.x) >> 5;
-  gather_rows_by_warp(s0, s1, vec_per_row, out, out_pitch_vec, out_labels, warp, n_warps);
+  const int64_t n = s0.n + s1.n;
+  const int lane = threadIdx.x & 31;
+  for (int64_t r = warp; r < n; r += n_warps) {
+    const bool second = r >= s0.n;
+    const CopySeg& sg = second ? s1 : s0;
+    const int64_t src = __ldg(sg.idx + (second ? r - s0.n : r));
+    const uint4* row = reinterpret_cast<const uint4*>(sg.bank) + src * vec_per_row;
+    uint4* dst = out + r * out_pitch_vec;
+    if (lane == 0 && out_labels) out_labels[r] = static_cast<int32_t>(__ldg(sg.labels + src));
+    for (int v0 = 0; v0 < vec_per_row; v0 += 128) {
+      uint4 x[4];
+#pragma unroll
+      for (int j = 0; j < 4; ++j) {
+        const int v = v0 + j * 32 + lane;
+        if (v < vec_per_row) x[j] = __ldcs(row + v);  // streamed: a bank row is read once per epoch
+      }
+#pragma unroll
+      for (int j = 0; j < 4; ++j) {
+        const int v = v0 + j * 32 + lane;
+        if (v < vec_per_row) __stcs(dst + v, x[j]);  // read again a step or two later, after 0.5 GB of other traffic: not worth L2
+      }
+    }
+  }
 }
 
 template <bool kBf16>
@@ -287,18 +310,18 @@ int uml_gather2_rows_bf16(const uint16_t* bank0, const int64_t* labels0, const i
               "gather2: pointers must be 16B aligned");
   int rows = static_cast<int>(48 * 1024 / row_bytes);
   if (rows > 32) rows = 32;
-  const size_t smem = static_cast<size_t>(kCopyStagesFull) * rows * row_bytes;
+  const size_t smem = static_cast<size_t>(kCopyStages) * rows * row_bytes;
   static bool attr_set = false;
   if (!attr_set) {
-    UML_CUDA(cudaFuncSetAttribute(gather_copy2_kernel<kCopyStagesFull>, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                                  kCopyStagesFull * 48 * 1024));
+    UML_CUDA(cudaFuncSetAttribute(gather_copy2_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                                  kCopyStages * 48 * 1024));
     attr_set = true;
   }
   const int64_t groups = (n0 + n1 + rows - 1) / rows;
   const int grid = static_cast<int>(std::min<int64_t>(groups, sm_count()));
   CopySeg a{reinterpret_cast<const unsigned char*>(bank0), idx0, labels0, n0};
   CopySeg b{reinterpret_cast<const unsigned char*>(bank1), idx1, labels1, n1};
-  UML_CUDA(launch_kernel(gather_copy2_kernel<kCopyStagesFull>, dim3(grid), dim3(32), smem, as_stream(stream), 1, kPdlGather, a, b,
+  UML_CUDA(launch_kernel(gather_copy2_kernel, dim3(grid), dim3(32), smem, as_stream(stream), 1, a, b,
                          row_bytes, rows, reinterpret_cast<unsigned char*>(out), ld_out * 2, out_labels));
   return 0;
 }
@@ -316,25 +339,6 @@ int uml_gather2_rows_bf16_light(const uint16_t* bank0, const int64_t* labels0, c
               "gather2_light: pointers must be 16B aligned");
   CopySeg a{reinterpret_cast<const unsigned char*>(bank0), idx0, labels0, n0};
   CopySeg b{reinterpret_cast<const unsigned char*>(bank1), idx1, labels1, n1};
-  // Default: the register-copy kernel.  UML_LIGHT_GATHER=tma selects TMA copies through a 27 KB ring (one warp per
-  // SM, fits beside a dW CTA) - measured slower on B200: too few bytes in flight, the dW kernel it overlaps went
-  // from 66 us to 88 us (0.207 vs 0.184 ms/step).
-  static int mode = -1;
-  if (mode < 0) {
-    const char* e = getenv("UML_LIGHT_GATHER");
-    mode = (e && e[0] == 't') ? 0 : 1;
-  }
-  const uint32_t row_bytes = static_cast<uint32_t>(dim) * 2u;
-  if (mode == 0 && row_bytes <= 9 * 1024) {
-    const int rows = std::max(1, std::min<int>(32, 9 * 1024 / row_bytes));
-    const size_t smem = static_cast<size_t>(kCopyStagesLight) * rows * row_bytes;
-    const int64_t groups = (n0 + n1 + rows - 1) / rows;
-    const int grid = static_cast<int>(std::min<int64_t>(groups, sm_count()));
-    gather_copy2_kernel<kCopyStagesLight><<<grid, 32, smem, as_stream(stream)>>>(a, b, row_bytes, rows, reinterpret_cast<unsigned char*>(out),
-                                                                                 ld_out * 2, out_labels);
-    UML_CUDA(cudaGetLastError());
-    return 0;
-  }
   const int64_t blocks = std::min<int64_t>((n0 + n1 + 7) / 8, static_cast<int64_t>(sm_count()) * 4);
   gather_direct2_kernel<<<static_cast<unsigned>(blocks), 256, 0, as_stream(stream)>>>(a, b, dim / 8, reinterpret_cast<uint4*>(out),
                                                                                       ld_out / 8, out_labels);

@@ -1,7 +1,6 @@
 // Library plumbing: error string, device check, tensor-map encoding through the driver entry point
 // (so the .so links against libcudart only and loads on a host without libcuda).
 #include <cstdarg>
-#include <cstdlib>
 
 #include "common.cuh"
 
@@ -26,17 +25,6 @@ int sm_count() {
     cached[dev] = n;
   }
   return cached[dev];
-}
-
-int pdl_mask() {
-  static int cached = -1;
-  if (cached < 0) {
-    // Round 1 measured "every site on" as SLOWER (0.266 vs 0.214 ms/step: early-resident dependents compete with the
-    // running kernel) and the end-to-end arm hung; the sites are now selectable one by one (UML_PDL=<bit mask>).
-    const char* e = getenv("UML_PDL");
-    cached = e ? atoi(e) : 0;
-  }
-  return cached;
 }
 
 typedef CUresult (*encode_tiled_fn)(CUtensorMap*, CUtensorMapDataType, cuuint32_t, void*, const cuuint64_t*,

@@ -22,8 +22,6 @@ __global__ void __launch_bounds__(256)
                 AdamArgs a, __nv_bfloat16* __restrict__ shadow, float* __restrict__ g_out) {
   const int64_t tid = blockIdx.x * static_cast<int64_t>(blockDim.x) + threadIdx.x;
   const int64_t nthreads = static_cast<int64_t>(gridDim.x) * blockDim.x;
-  pdl_trigger();
-  pdl_wait();
   if (kVec) {
     const int64_t nv = n >> 2;
     for (int64_t i = tid; i < nv; i += nthreads) {
@@ -113,10 +111,10 @@ static int launch_adam(float* p, const float* parts, int n_parts, int64_t stride
   const int grid = static_cast<int>(std::min<int64_t>((work + 255) / 256, static_cast<int64_t>(sm_count()) * ctas_per_sm));
   __nv_bfloat16* sh = reinterpret_cast<__nv_bfloat16*>(shadow);
   if (vec)
-    UML_CUDA(launch_kernel(adam_kernel<true>, dim3(grid), dim3(256), 0, st, 1, kPdlUpdate, p, parts, n_parts, stride, g2, w2, m, v, n,
+    UML_CUDA(launch_kernel(adam_kernel<true>, dim3(grid), dim3(256), 0, st, 1, p, parts, n_parts, stride, g2, w2, m, v, n,
                            a, sh, g_out));
   else
-    UML_CUDA(launch_kernel(adam_kernel<false>, dim3(grid), dim3(256), 0, st, 1, kPdlUpdate, p, parts, n_parts, stride, g2, w2, m, v, n,
+    UML_CUDA(launch_kernel(adam_kernel<false>, dim3(grid), dim3(256), 0, st, 1, p, parts, n_parts, stride, g2, w2, m, v, n,
                            a, sh, g_out));
   return 0;
 }

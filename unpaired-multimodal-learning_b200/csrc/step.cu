@@ -2,25 +2,16 @@
 // (reference loop body, vision_language/finetune.py:163-195) without returning to Python in between.
 // At the reference's batch sizes the step is launch-latency bound, at throughput batch sizes the host
 // must stay ahead of a ~150 us GPU step - either way per-kernel Python dispatch is what limits it.
-#include <cstdlib>
-
 #include "common.cuh"
-#include "optim.cuh"
-#include "gather.cuh"
 
 namespace {
 inline void rec(void* ev, void* stream) {
   if (ev) cudaEventRecord(static_cast<cudaEvent_t>(ev), uml::as_stream(stream));
 }
 
-bool overlap_fixup();
-
 // Side stream + events for the gather prefetch of uml_linear_run (one set per device, created on first use).
 struct Pipe {
   cudaStream_t aux = nullptr;
-  cudaStream_t aux2 = nullptr;          // the dW GEMM when it overlaps the fix-up launch
-  cudaEvent_t dw_done = nullptr, fwd_done = nullptr;
-  unsigned* split_done = nullptr;       // [8] fix-up CTAs finished per dW split, then one int: watchdog flag
   cudaEvent_t ready[3] = {nullptr, nullptr, nullptr}, freed[3] = {nullptr, nullptr, nullptr}, start = nullptr, mid = nullptr;
   // the pipeline of uml_linear_run survives the call boundary when the caller vouches for its index batches (idx_ready):
   bool warm = false;                    // freed[] / fwd_mid[] describe the last steps of the previous call
@@ -48,14 +39,10 @@ Pipe* get_pipe() {
   Pipe& p = pipes[dev];
   if (!tried[dev]) {
     tried[dev] = true;
-    const char* e = getenv("UML_PREFETCH");
-    if (e && e[0] == '0') return nullptr;
     int lo = 0, hi = 0;
     if (cudaDeviceGetStreamPriorityRange(&lo, &hi) != cudaSuccess) return nullptr;
     // lowest priority: the prefetch must never delay a kernel of the step it hides under
-    const char* pe = getenv("UML_AUX_PRIORITY");  // experiments: "hi" = the GEMMs' priority class and above
-    const int aux_prio = (pe && pe[0] == 'h') ? hi : lo;
-    if (cudaStreamCreateWithPriority(&p.aux, cudaStreamNonBlocking, aux_prio) != cudaSuccess) return nullptr;
+    if (cudaStreamCreateWithPriority(&p.aux, cudaStreamNonBlocking, lo) != cudaSuccess) return nullptr;
     bool good = true;
     for (int i = 0; i < 3; ++i) {
       good = good && cudaEventCreateWithFlags(&p.ready[i], cudaEventDisableTiming) == cudaSuccess;
@@ -64,75 +51,9 @@ Pipe* get_pipe() {
     good = good && cudaEventCreateWithFlags(&p.start, cudaEventDisableTiming) == cudaSuccess;
     for (int i = 0; i < 2; ++i) good = good && cudaEventCreateWithFlags(&p.fwd_mid[i], cudaEventDisableTiming) == cudaSuccess;
     good = good && cudaEventCreateWithFlags(&p.mid, cudaEventDisableTiming) == cudaSuccess;
-    good = good && cudaEventCreateWithFlags(&p.dw_done, cudaEventDisableTiming) == cudaSuccess;
-    good = good && cudaEventCreateWithFlags(&p.fwd_done, cudaEventDisableTiming) == cudaSuccess;
-    good = good && cudaStreamCreateWithPriority(&p.aux2, cudaStreamNonBlocking, hi) == cudaSuccess;
-    if (overlap_fixup())  // (a device allocation synchronises: only when the experiment is switched on)
-      good = good && cudaMalloc(&p.split_done, 64) == cudaSuccess && cudaMemset(p.split_done, 0, 64) == cudaSuccess;
     p.ok = good;
   }
   return p.ok ? &p : nullptr;
-}
-
-// Where in step i the gather of step i+1 is enqueued.  Measured on B200 (cfg3, 2 x 18944 rows): at the START of the
-// step (it then shares the machine with the forward and, mostly, the bandwidth-bound fix-up) 0.1925 ms/step;
-// AFTER forward + fix-up (sharing with the dW GEMM, which streams both operands from HBM) 0.237 ms/step - slower
-// than no prefetch at all (0.207); right AFTER THE FORWARD KERNEL (sharing with fix-up, dW, update) 0.189 ms/step
-// with the forward kernel running undisturbed (67.5 us instead of 84 us).  UML_PREFETCH_AT = 0 | 1 | 2 selects
-// start / after fix-up / after the forward kernel (default 2).  Placement 3 needs no side stream: the copy of step
-// i+1's rows rides in step i's fix-up launch as extra, interleaved CTAs - measured 0.1936 ms/step against 0.1862 for
-// placement 2 (two bandwidth-bound jobs in one launch just add up: 49.7 us for the launch instead of 24.5 us).
-// Placement 4: after the dW GEMM, i.e. under the step's data-parallel tail (that kernel waits on NVLink most of the time).
-static bool g_dp_step = false;  // set by linear_run for the step being enqueued
-// UML_UPDATE_IN_DW=1: the split-K sum and AdamW run in the tail of the dW GEMM instead of a launch of their own.
-// Measured on B200 (cfg3, 73 728 rows): 0.2376 ms/step against 0.2319 with the separate launch - every CTA waits for the
-// slowest split of its tile with the whole SM in hand, and its share of the update (21 rows x 256 columns, nine
-// arrays) is latency-bound, while the separate kernel spreads the same bytes over 750 CTAs.  Off by default.
-bool update_in_dw_enabled() {
-  static int on = -1;
-  if (on < 0) {
-    const char* e = getenv("UML_UPDATE_IN_DW");
-    on = (e && e[0] == '1') ? 1 : 0;
-  }
-  return on == 1;
-}
-
-int prefetch_placement() {
-  static int cached = -2;
-  if (cached == -2) {
-    const char* e = getenv("UML_PREFETCH_AT");
-    cached = (e && e[0] >= '0' && e[0] <= '4') ? e[0] - '0' : -1;
-  }
-  if (cached >= 0) return cached;
-  (void)g_dp_step;  // measured on 2 B200s: placement 4 0.1627 ms/step, placement 2 0.1618 - no gain, 2 stays the default
-  return 2;
-}
-
-// UML_FUSE_FIX=1: the deferred softmax normalisation is applied in the dW prologue (tc_gemm kFix: each G stage is
-// rescaled in shared memory between the TMA arrival and the MMA) instead of by a fix-up pass over G after the
-// forward kernel.  Bit-identical results, but measured SLOWER on B200 (cfg3): 0.231 vs 0.189 ms/step - the dW
-// GEMM with two MN-major operands already moves ~100 KB through shared memory per 950-cycle stage, the transform's
-// extra 32 KB per stage makes it shared-memory bound.  Default: the fix-up kernel.
-bool fuse_fix() {
-  static int cached = -1;
-  if (cached < 0) {
-    const char* e = getenv("UML_FUSE_FIX");
-    cached = (e && e[0] == '1') ? 1 : 0;
-  }
-  return cached == 1;
-}
-
-// UML_OVERLAP_FIXUP=1: the dW GEMM is launched on a second stream as soon as the forward kernel ends and each of its K
-// splits starts when the fix-up CTAs of ITS rows are done (per-split counters), instead of the whole GEMM waiting for
-// the whole fix-up pass.  Bit-identical, but measured SLOWER on B200 (cfg3): 0.205 vs 0.185 ms/step - the resident,
-// waiting GEMM CTAs plus the prefetching gather leave the fix-up CTAs almost no registers to run in.  Default: off.
-bool overlap_fixup() {
-  static int cached = -1;
-  if (cached < 0) {
-    const char* e = getenv("UML_OVERLAP_FIXUP");
-    cached = (e && e[0] == '1') ? 1 : 0;
-  }
-  return cached == 1;
 }
 
 // true when every non-empty run of the step can be gathered from bf16 shadow banks by one copy launch
@@ -144,8 +65,8 @@ bool shadow_gatherable(const uml_linear_step_args* a) {
   return true;
 }
 
-// both runs' rows + labels -> (X16, labels32) by one launch of the TMA copy kernel (or its small-footprint twin)
-int shadow_gather(const uml_linear_step_args* a, uint16_t* X16, int32_t* labels32, bool light, void* stream) {
+// both runs' rows + labels -> (X16, labels32) by one launch of the register-copy kernel
+int shadow_gather(const uml_linear_step_args* a, uint16_t* X16, int32_t* labels32, void* stream) {
   const uml_segment* g[2] = {nullptr, nullptr};
   int ng = 0;
   for (int i = 0; i < a->nseg; ++i)
@@ -153,31 +74,27 @@ int shadow_gather(const uml_linear_step_args* a, uint16_t* X16, int32_t* labels3
   if (ng == 0) return 0;
   // The register-copy kernel is also the faster one stand-alone (ncu, cfg3: 17.8 us = 6.5 TB/s, the measured copy
   // peak, against 30 us for the TMA ring kernel), so it serves both the prefetch and the in-line gather.
-  (void)light;
-  auto fn = uml_gather2_rows_bf16_light;
-  return fn(g[0]->rows16, g[0]->labels, g[0]->idx, g[0]->n, ng > 1 ? g[1]->rows16 : nullptr, ng > 1 ? g[1]->labels : nullptr,
-            ng > 1 ? g[1]->idx : nullptr, ng > 1 ? g[1]->n : 0, a->dim, X16, a->dim, labels32, stream);
+  return uml_gather2_rows_bf16_light(g[0]->rows16, g[0]->labels, g[0]->idx, g[0]->n, ng > 1 ? g[1]->rows16 : nullptr,
+                                     ng > 1 ? g[1]->labels : nullptr, ng > 1 ? g[1]->idx : nullptr, ng > 1 ? g[1]->n : 0,
+                                     a->dim, X16, a->dim, labels32, stream);
 }
 }  // namespace
 
-// `mid` (optional) runs on the host right after the forward + fix-up launches were enqueued: the place where
-// uml_linear_run enqueues the next step's gather, so that it overlaps dW / update but not the bandwidth-bound fix-up
+// `mid` (optional) runs on the host right after the forward launches were enqueued: where uml_linear_run enqueues a
+// later step's gather, ordered after the forward KERNEL (`after_fwd_kernel`).  The gather then shares the machine with
+// the dW GEMM and the update but not with the forward kernel, which it slowed from 67.5 to 84 us on B200 (cfg3).
 struct StepHooks {
   bool pregathered = false;
   cudaEvent_t operand_free = nullptr;
   int (*mid)(void*) = nullptr;
   void* mid_arg = nullptr;
-  cudaEvent_t after_fwd_kernel = nullptr;  // placement 2: recorded between the forward kernel and its fix-up
-  const uml::GatherJob* merged = nullptr;  // placement 3: the fix-up launch also copies the NEXT step's rows
+  cudaEvent_t after_fwd_kernel = nullptr;
 };
 static int linear_step_impl(const uml_linear_step_args* a, void* stream, const StepHooks& hooks);
 int uml_head_fwd_ce_bf16_ev(const uint16_t* X, int64_t n_rows, int32_t dim, const uint16_t* W, int32_t n_classes,
                             const int32_t* labels, const uml_tc_segments* segs, uint16_t* G, int64_t ldg, float* row_loss,
                             int32_t* row_pred, int32_t* row_correct, float* row_dscale, float* tile_ws, uml_seg_stats* stats,
-                            void* ev_after_fwd, void* stream, int defer_fixup, void* ev_after_fwd2 = nullptr,
-                            const uml::GatherJob* job = nullptr, const uml::FixupSignal* sig = nullptr);  // tc_fwd.cu
-int uml_head_bwd_dw_gated_bf16(const uint16_t* G, int64_t ldg, const uint16_t* X, int64_t n_rows, int32_t dim, int32_t n_classes,
-                               float* partials, int32_t n_splits, const unsigned* done, int* failed, void* stream);  // tc_gemm.cu
+                            void* ev_after_fwd, void* stream, void* ev_after_fwd2 = nullptr);  // tc_fwd.cu
 
 // tc_fwd2.cu / tc_gemm.cu: exchange forward kernel (G final after one pass) and the dW GEMM that reduces its statistics
 bool uml_fwd_x_eligible(int64_t n_rows, int32_t n_classes);
@@ -185,11 +102,6 @@ void uml_fwd_x_partials(float* tile_ws, int64_t n_rows, int32_t n_classes, const
 int uml_head_bwd_dw_stats_bf16(const uint16_t* G, int64_t ldg, const uint16_t* X, int64_t n_rows, int32_t dim, int32_t n_classes,
                                float* partials, int32_t n_splits, const float* part, int64_t part_entries, int32_t nseg,
                                uml_seg_stats* stats, void* stream);
-
-int uml_head_bwd_dw_update_bf16(const uint16_t* G, int64_t ldg, const uint16_t* X, int64_t n_rows, int32_t dim, int32_t n_classes,
-                                float* partials, int32_t n_splits, const float* part, int64_t part_entries, int32_t nseg,
-                                uml_seg_stats* stats, float* W, float* m, float* v, uint16_t* W16, const uml::AdamArgs* adam,
-                                unsigned* failed, void* stream);
 
 float* uml_dp_p2p_input(int64_t n);   // dp.cu: this rank's exchange buffers of the peer-memory all-reduce (or NULL)
 float* uml_dp_p2p_output(int64_t n);
@@ -230,16 +142,6 @@ static int dp_reduce_and_update(const uml_linear_step_args* a, int64_t np, void*
                         a->upd.eps, a->upd.weight_decay, a->upd.step, a->upd.kind == 1, shadow, stream);
   rec(a->ev[7], stream);
   return rc;
-}
-
-
-static bool continuous_enabled() {
-  static int on = -1;
-  if (on < 0) {
-    const char* e = getenv("UML_PREFETCH_CONTINUOUS");
-    on = (e && e[0] == '0') ? 0 : 1;
-  }
-  return on == 1;
 }
 
 static int linear_run_continuous(const uml_linear_step_args* base, const uml_run_step* steps, int32_t n_steps, void* stream,
@@ -285,7 +187,7 @@ static int linear_run_continuous(const uml_linear_step_args* base, const uml_run
     UML_CUDA(cudaStreamWaitEvent(pipe->aux, (t >= kNb || warm) ? pipe->freed[tb] : pipe->start, 0));
     if (after_fwd) UML_CUDA(cudaStreamWaitEvent(pipe->aux, after_fwd, 0));
     rec(g.ev[0], pipe->aux);
-    const int rc = shadow_gather(&g, xbuf[tb], lbuf[tb], true, pipe->aux);
+    const int rc = shadow_gather(&g, xbuf[tb], lbuf[tb], pipe->aux);
     if (rc) return rc;
     rec(g.ev[1], pipe->aux);
     UML_CUDA(cudaEventRecord(pipe->ready[tb], pipe->aux));
@@ -298,7 +200,6 @@ static int linear_run_continuous(const uml_linear_step_args* base, const uml_run
     if (rc) return rc;
   }
 
-  g_dp_step = base->dp_allreduce != 0;
   for (int i = 0; i < n_steps; ++i) {
     patch(a, steps[i]);
     if (i > 0) a.w16_valid = 1;  // the optimizer kernel of the previous step refreshed the shadow
@@ -310,8 +211,7 @@ static int linear_run_continuous(const uml_linear_step_args* base, const uml_run
       decltype(launch_gather)* launch;
       int t;
       cudaEvent_t mid;
-      cudaStream_t main_st;
-    } next{&launch_gather, i + kDepth < n_steps ? i + kDepth : -1, pipe->fwd_mid[(g0 + i) & 1u], main_st};
+    } next{&launch_gather, i + kDepth < n_steps ? i + kDepth : -1, pipe->fwd_mid[(g0 + i) & 1u]};
     StepHooks hooks;
     hooks.pregathered = true;
     hooks.operand_free = pipe->freed[b];
@@ -371,7 +271,7 @@ int uml_linear_run(const uml_linear_step_args* base, const uml_run_step* steps, 
   // step they would have followed inside one long call - when the host is a chunk ahead of the GPU (it normally is) they
   // run beside the previous call's last steps, and a call costs no gather on the main stream at all.
   if (a.precision == 1 && base->X16_alt && base->labels32_alt && base->X16_alt2 && base->labels32_alt2 && base->idx_ready &&
-      n_steps >= 1 && prefetch_placement() == 2 && !fuse_fix() && continuous_enabled()) {
+      n_steps >= 1) {
     bool all = true;
     for (int i = 0; i < n_steps && all; ++i) {
       uml_linear_step_args t = a;
@@ -386,18 +286,13 @@ int uml_linear_run(const uml_linear_step_args* base, const uml_run_step* steps, 
   // update run and may spill into step i + 1 - no forward kernel ever waits for an event that is signalled at the last
   // moment (one step ahead, the gather of step i + 1 ended about when the update did, and the cross-stream hand-over
   // put ~9 us between the update and the next forward kernel).
-  int nb = 2;
-  if (pipe && base->X16_alt2 && base->labels32_alt2 && n_steps > 2 && prefetch_placement() != 3) {
-    const char* e = getenv("UML_PREFETCH_DEPTH");
-    if (!(e && e[0] == '1')) nb = 3;
-  }
+  const int nb = (pipe && base->X16_alt2 && base->labels32_alt2 && n_steps > 2) ? 3 : 2;
   const int depth = nb - 1;
   uint16_t* xbuf[3] = {base->X16, base->X16_alt, base->X16_alt2};
   int32_t* lbuf[3] = {base->labels32, base->labels32_alt, base->labels32_alt2};
   cudaStream_t main_st = as_stream(stream);
   if (pipe) UML_CUDA(cudaEventRecord(pipe->start, main_st));  // everything enqueued so far may still read the other buffers
 
-  g_dp_step = base->dp_allreduce != 0;
   for (int i = 0; i < n_steps; ++i) {
     patch(a, steps[i]);
     if (i > 0 && a.precision == 1) a.w16_valid = 1;  // the optimizer kernel of the previous step refreshed the shadow
@@ -414,10 +309,10 @@ int uml_linear_run(const uml_linear_step_args* base, const uml_run_step* steps, 
       // starts BOTH the second and the third step's gathers: beside the first forward kernel a gather would only have
       // the SMs that kernel leaves free (4 of 148) and hold up the second step
       rec(a.ev[0], stream);
-      const int rc0 = shadow_gather(&a, xbuf[0], lbuf[0], false, stream);
+      const int rc0 = shadow_gather(&a, xbuf[0], lbuf[0], stream);
       if (rc0) return rc0;
       rec(a.ev[1], stream);
-    } else if (prefetch_placement() != 3 || fuse_fix()) {
+    } else {
       UML_CUDA(cudaStreamWaitEvent(main_st, pipe->ready[b], 0));
     }
     struct Job {
@@ -430,15 +325,10 @@ int uml_linear_run(const uml_linear_step_args* base, const uml_run_step* steps, 
       Pipe* pipe;
       Job job[2];
       int n_jobs;
-      cudaEvent_t wait_b;
-      cudaStream_t main_st;
-      bool have, record_mid;
+      bool have;
     } next;
     next.pipe = pipe;
     next.n_jobs = 0;
-    next.record_mid = prefetch_placement() != 2;
-    next.wait_b = pipe->mid;
-    next.main_st = main_st;
     // step i's hook starts the gather of step i + depth (the first step's: of every step up to `depth`)
     for (int t = (i == 0 ? 1 : i + depth); t <= i + depth && t < n_steps; ++t) {
       const int tb = t % nb;  // last read by the dW kernel of step t - nb (never, when that is before this call)
@@ -454,44 +344,17 @@ int uml_linear_run(const uml_linear_step_args* base, const uml_run_step* steps, 
     StepHooks hooks;
     hooks.pregathered = true;
     hooks.operand_free = pipe->freed[b];
-    GatherJob gjob;
-    memset(&gjob, 0, sizeof(gjob));
-    const bool merged = prefetch_placement() == 3 && !fuse_fix();
-    if (merged) {
-      if (next.have) {
-        const uml_segment* g[2] = {nullptr, nullptr};
-        int ng = 0;
-        for (int k = 0; k < next.job[0].nx.nseg; ++k)
-          if (next.job[0].nx.seg[k].n > 0) g[ng++] = &next.job[0].nx.seg[k];
-        if (ng > 0) {
-          gjob.s0 = CopySeg{reinterpret_cast<const unsigned char*>(g[0]->rows16), g[0]->idx, g[0]->labels, g[0]->n};
-          if (ng > 1) gjob.s1 = CopySeg{reinterpret_cast<const unsigned char*>(g[1]->rows16), g[1]->idx, g[1]->labels, g[1]->n};
-          gjob.vec_per_row = a.dim / 8;
-          gjob.out = reinterpret_cast<uint4*>(next.job[0].x);
-          gjob.out_pitch_vec = a.dim / 8;
-          gjob.out_labels = next.job[0].l;
-          gjob.blocks = 4 * sm_count();
-          hooks.merged = &gjob;
-        }
-      }
-      if (next.have) {  // (the merged copy has no launch of its own to bracket)
-        rec(next.job[0].nx.ev[0], stream);
-        rec(next.job[0].nx.ev[1], stream);
-      }
-      next.have = false;  // nothing for the side stream to do
-    }
     hooks.mid_arg = &next;
-    hooks.after_fwd_kernel = (prefetch_placement() == 2 && next.have) ? pipe->mid : nullptr;
+    hooks.after_fwd_kernel = next.have ? pipe->mid : nullptr;
     hooks.mid = [](void* p) -> int {
       Next* n = static_cast<Next*>(p);
       if (!n->have) return 0;
-      if (n->record_mid) UML_CUDA(cudaEventRecord(n->pipe->mid, n->main_st));
       for (int k = 0; k < n->n_jobs; ++k) {
         Job& j = n->job[k];
         UML_CUDA(cudaStreamWaitEvent(n->pipe->aux, j.wait_a, 0));
-        UML_CUDA(cudaStreamWaitEvent(n->pipe->aux, n->wait_b, 0));
+        UML_CUDA(cudaStreamWaitEvent(n->pipe->aux, n->pipe->mid, 0));
         rec(j.nx.ev[0], n->pipe->aux);  // ev[0]..ev[1] bracket the gather where it really runs: on the side stream
-        const int rc = shadow_gather(&j.nx, j.x, j.l, true, n->pipe->aux);
+        const int rc = shadow_gather(&j.nx, j.x, j.l, n->pipe->aux);
         if (rc) return rc;
         rec(j.nx.ev[1], n->pipe->aux);
         UML_CUDA(cudaEventRecord(j.ready, n->pipe->aux));
@@ -521,7 +384,6 @@ static int linear_step_impl(const uml_linear_step_args* a, void* stream, const S
   using namespace uml;
   const bool pregathered = hooks.pregathered;
   const cudaEvent_t operand_free = hooks.operand_free;
-  Pipe* opipe = nullptr;  // set when this step's dW runs on the second stream, overlapping the fix-up launch
   bool stats_in_dw = false;  // the forward's per-run statistics are reduced inside the dW kernel
   UML_REQUIRE(a != nullptr, "linear_step: null args");
   UML_REQUIRE(a->nseg >= 1 && a->nseg <= UML_MAX_SEGMENTS, "linear_step: 1..2 segments");
@@ -567,7 +429,7 @@ static int linear_step_impl(const uml_linear_step_args* a, void* stream, const S
     if (!pregathered) rec(a->ev[0], stream);  // (a pre-gathered step's ev[0]..ev[1] were recorded around its gather)
     const bool shadow = pregathered || shadow_gatherable(a);
     if (shadow && !pregathered) {
-      rc = shadow_gather(a, a->X16, a->labels32, false, stream);
+      rc = shadow_gather(a, a->X16, a->labels32, stream);
       if (rc) return rc;
     }
     for (int i = 0; i < a->nseg; ++i) {
@@ -598,58 +460,19 @@ static int linear_step_impl(const uml_linear_step_args* a, void* stream, const S
       off += s.n;
     }
     if (!pregathered) rec(a->ev[1], stream);
-    if (hooks.mid && prefetch_placement() == 0) {
-      rc = hooks.mid(hooks.mid_arg);
-      if (rc) return rc;
-    }
     if (total > 0) {
-      // fix-up / dW overlap: counters zeroed before the forward kernel, dW launched on aux2 right after it
-      int splits_o = uml_tc_dw_splits(total, a->dim, a->n_classes);
-      if (splits_o > a->max_splits) splits_o = a->max_splits;
-      opipe = (overlap_fixup() && !fuse_fix() && splits_o >= 1 && splits_o <= 8) ? get_pipe() : nullptr;
-      FixupSignal sig;
-      memset(&sig, 0, sizeof(sig));
-      cudaEvent_t after_fwd = hooks.after_fwd_kernel;
-      if (opipe) {
-        UML_CUDA(cudaMemsetAsync(opipe->split_done, 0, 64, as_stream(stream)));
-        sig.done = opipe->split_done;
-        sig.n_splits = splits_o;
-        sig.num_kb = (total + 63) / 64;
-        if (!after_fwd) after_fwd = opipe->fwd_done;
-      }
       rec(a->ev[2], stream);
-      // ev[2]..ev[3] bracket the tensor-core kernel alone.  Exchange kernel (default): G is final when it ends and the
-      // per-run statistics are reduced by an idle warp of the dW GEMM - unless a learnable temperature needs them
-      // before that (then a small reduction launch follows the forward).  Chunk-sequential kernel (UML_FWD_IMPL=old):
-      // the fix-up launch, which also reduces the statistics, follows it.
-      stats_in_dw = !fuse_fix() && !opipe && uml_fwd_x_eligible(total, a->n_classes) && !a->scale_param[0] &&
-                    !a->scale_param[1];
+      // ev[2]..ev[3] bracket the tensor-core kernel alone.  Exchange kernel (the default above 128 rows): G is final when it ends
+      // and the per-run statistics are reduced by an idle warp of the dW GEMM - unless a learnable temperature needs them
+      // before that (then a small reduction launch follows the forward).  Chunk-sequential kernel: the fix-up launch,
+      // which also reduces the statistics, follows it.
+      stats_in_dw = uml_fwd_x_eligible(total, a->n_classes) && !a->scale_param[0] && !a->scale_param[1];
       rc = uml_head_fwd_ce_bf16_ev(a->X16, total, a->dim, a->W16, a->n_classes, a->labels32, &ts,
                                    static_cast<uint16_t*>(a->G), a->ldg, nullptr, nullptr, nullptr, nullptr, a->tile_ws,
-                                   stats_in_dw ? nullptr : a->stats, a->ev[3], stream, fuse_fix() ? 1 : 0, after_fwd,
-                                   fuse_fix() ? nullptr : hooks.merged, opipe ? &sig : nullptr);
-      if (rc) return rc;
-      if (opipe) {
-        // the GEMM goes to the second stream behind "forward kernel done"; the fix-up launch just enqueued on the main
-        // stream runs concurrently and releases the GEMM's splits one by one
-        cudaStream_t s2 = opipe->aux2;
-        UML_CUDA(cudaStreamWaitEvent(s2, after_fwd, 0));
-        rec(a->ev[4], s2);
-        rc = uml_head_bwd_dw_gated_bf16(static_cast<const uint16_t*>(a->G), a->ldg, a->X16, total, a->dim, a->n_classes,
-                                        a->partials, splits_o, opipe->split_done, reinterpret_cast<int*>(opipe->split_done + 8), s2);
-        if (rc) return rc;
-        rec(a->ev[5], s2);
-        UML_CUDA(cudaEventRecord(opipe->dw_done, s2));
-      }
-    } else if (hooks.merged) {
-      // no rows on this rank this step, hence no fix-up launch to ride in: copy the next step's rows directly
-      const GatherJob& j = *hooks.merged;
-      rc = uml_gather2_rows_bf16_light(reinterpret_cast<const uint16_t*>(j.s0.bank), j.s0.labels, j.s0.idx, j.s0.n,
-                                       reinterpret_cast<const uint16_t*>(j.s1.bank), j.s1.labels, j.s1.idx, j.s1.n, a->dim,
-                                       reinterpret_cast<uint16_t*>(j.out), a->dim, j.out_labels, stream);
+                                   stats_in_dw ? nullptr : a->stats, a->ev[3], stream, hooks.after_fwd_kernel);
       if (rc) return rc;
     }
-    if (hooks.mid && prefetch_placement() != 0 && prefetch_placement() != 4) {
+    if (hooks.mid) {
       rc = hooks.mid(hooks.mid_arg);
       if (rc) return rc;
     }
@@ -674,10 +497,6 @@ static int linear_step_impl(const uml_linear_step_args* a, void* stream, const S
   }
 
   const int64_t np_all = static_cast<int64_t>(a->n_classes) * a->dim;
-  if (total == 0 && a->precision == 1 && hooks.mid && prefetch_placement() == 4) {  // (no dW launch to follow on this rank)
-    rc = hooks.mid(hooks.mid_arg);
-    if (rc) return rc;
-  }
   if (total == 0 && !dp) return 0;
   if (total == 0) {  // a rank without rows still takes part in the all-reduce, contributing zeros
     UML_CUDA(cudaMemsetAsync(dp_local_sum_target(a, np_all), 0, np_all * sizeof(float), as_stream(stream)));
@@ -695,40 +514,8 @@ static int linear_step_impl(const uml_linear_step_args* a, void* stream, const S
   }
   int splits = uml_tc_dw_splits(total, a->dim, a->n_classes);
   if (splits > a->max_splits) splits = a->max_splits;
-  const bool update_in_dw = fused && !dp && a->upd.kind != 3 && a->W16 && splits <= 8 && a->dim % 4 == 0 && update_in_dw_enabled();
-  if (opipe) {
-    UML_CUDA(cudaStreamWaitEvent(as_stream(stream), opipe->dw_done, 0));  // the GEMM was launched with the forward
-    rc = 0;
-  } else {
   rec(a->ev[4], stream);
-  if (fuse_fix()) {
-    // the forward skipped its fix-up pass: the dW prologue normalises every G stage in shared memory
-    uml_tc_segments ts2;
-    memset(&ts2, 0, sizeof(ts2));
-    for (int i = 0; i < a->nseg; ++i) {
-      const uml_segment& sg = a->seg[i];
-      if (sg.n == 0) continue;
-      ts2.seg_rows[ts2.nseg] = sg.n;
-      ts2.scale[ts2.nseg] = sg.scale;
-      ts2.loss_weight[ts2.nseg] = sg.loss_weight;
-      ts2.scale_dev[ts2.nseg] = sg.scale_dev;
-      ts2.nseg++;
-    }
-    rc = uml_head_bwd_dw_fix_bf16(static_cast<const uint16_t*>(a->G), a->ldg, a->X16, total, a->dim, a->n_classes,
-                                  a->partials, splits, &ts2, a->labels32, a->tile_ws, a->stats, stream);
-  } else if (stats_in_dw && update_in_dw) {
-    // single GPU, AdamW: statistics, split-K sum and the update all run inside the dW launch (no update launch)
-    const float* part = nullptr;
-    int64_t entries = 0;
-    uml_fwd_x_partials(a->tile_ws, total, a->n_classes, &part, &entries);
-    int nseg_live = 0;
-    for (int i = 0; i < a->nseg; ++i) nseg_live += a->seg[i].n > 0 ? 1 : 0;
-    const uml::AdamArgs adam = uml::make_adam(a->upd.lr, a->upd.beta1, a->upd.beta2, a->upd.eps, a->upd.weight_decay, a->upd.step,
-                                              a->upd.kind == 1);
-    rc = uml_head_bwd_dw_update_bf16(static_cast<const uint16_t*>(a->G), a->ldg, a->X16, total, a->dim, a->n_classes,
-                                     a->partials, splits, part, entries, nseg_live, a->stats, a->W, a->upd.m, a->upd.v, a->W16,
-                                     &adam, reinterpret_cast<unsigned*>(a->tile_ws) + 2, stream);
-  } else if (stats_in_dw) {
+  if (stats_in_dw) {
     const float* part = nullptr;
     int64_t entries = 0;
     uml_fwd_x_partials(a->tile_ws, total, a->n_classes, &part, &entries);
@@ -742,18 +529,8 @@ static int linear_step_impl(const uml_linear_step_args* a, void* stream, const S
   }
   if (rc) return rc;
   rec(a->ev[5], stream);
-  }
   if (operand_free) UML_CUDA(cudaEventRecord(operand_free, as_stream(stream)));  // X16 / labels32 may be overwritten
-  if (a->precision == 1 && hooks.mid && prefetch_placement() == 4) {  // the next step's gather starts when dW has finished
-    rc = hooks.mid(hooks.mid_arg);
-    if (rc) return rc;
-  }
   const int64_t np = static_cast<int64_t>(a->n_classes) * a->dim;
-  if (stats_in_dw && update_in_dw) {  // (the events of the update bracket nothing: it ran inside the dW kernel)
-    rec(a->ev[6], stream);
-    rec(a->ev[7], stream);
-    return 0;
-  }
   if (!fused) {
     if (dp && a->upd.kind != 3 && uml_dp_p2p_input(np)) {
       // data parallel over NVLink peer memory: split-K sum + exchange + Adam in ONE kernel per rank

@@ -1615,7 +1615,7 @@ int uml_sweep_run(const uml_sweep_args* a, int32_t n_steps, const int64_t* rows,
     const bool fuse_softmax = use_tc && want_fused_softmax && n_ctile <= 8;
     if (fuse_softmax)
       UML_CUDA(launch_kernel(sweep_logits_tc_kernel<true>, dim3(n_ctile, rt, K), dim3(256), kTcLgSmemBytes, st,
-                             static_cast<int>(n_ctile), 0, p));
+                             static_cast<int>(n_ctile), p));
     else if (use_tc)
       sweep_logits_tc_kernel<false><<<dim3(n_ctile, rt, K), 256, kTcLgSmemBytes, st>>>(p);
     else if (use_async)
@@ -1834,7 +1834,7 @@ int uml_sweep_adapter_run(const uml_sweep_args* a, const uml_sweep_adapter_args*
     if (mark(1) || mark(2)) return 1;
     const unsigned n_ctile = static_cast<unsigned>((a->n_classes + 127) / 128);
     UML_CUDA(launch_kernel(sweep_logits_tc_kernel<true>, dim3(n_ctile, 1, K), dim3(256), kTcLgSmemBytes, st,
-                           static_cast<int>(n_ctile), 0, p));
+                           static_cast<int>(n_ctile), p));
     ++g_sweep_launches;
     if (mark(3) || mark(4)) return 1;
     if (with_adapter) {  // dZ from the head's weights before their update

@@ -22,13 +22,12 @@
 // max / sum: the normalisation is DEFERRED - per row and 64-column group the factor exp(m_group - m_final) / sum *
 // coef goes to a small side array and g_fixup_kernel (below) applies it, together with the one-hot term, in one
 // coalesced pass over G while it is still in L2.  (Alternatives measured: normaliser warps inside this kernel - slower;
-// the same transform applied to the dW kernel's operand stages - bit-identical but shared-memory bound, see tc_gemm.cu.)
+// the same transform applied to the dW kernel's operand stages - bit-identical but shared-memory bound, see DESIGN.md.)
 // Logits never exist in HBM in fp32 and nothing is recomputed.
 #include <cstdlib>
 #include <type_traits>
 
 #include "common.cuh"
-#include "gather.cuh"
 
 namespace uml {
 
@@ -143,8 +142,6 @@ __global__ void __launch_bounds__(kFwdThreads, 1)
   else __syncthreads();
   tc_fence_after();
   const uint32_t tmem_base = *tmem_slot;
-  pdl_trigger();
-  pdl_wait();  // barriers, TMEM and descriptors were set up while the gather kernel was still draining
 
   if (warp == kWarpTma) {
     // ------------------------------------------------ TMA producer ------------------------------
@@ -519,36 +516,20 @@ __device__ void tile_stats_block(const float* __restrict__ tile_part, int64_t n_
 }
 
 // Second half of the deferred softmax normalisation: G[b,c] = G[b,c] * fac[b][c / 64] - [c == y_b] * coef_b.
-// One warp per row, 16-byte vectors, all loads of a row in flight at once; fully coalesced.  The last `nseg`
+// One warp per row, 16-byte vectors, all loads of a row in flight at once; fully coalesced.  The first `stat_blocks`
 // CTAs of the grid reduce the forward kernel's per-tile partials into the per-run statistics instead (what
 // used to be a launch of its own).
 __global__ void __launch_bounds__(256)
     g_fixup_kernel(__nv_bfloat16* __restrict__ G, int64_t ldg, int64_t n_rows, const int32_t* __restrict__ labels,
                    const float* __restrict__ fac, FwdSegs segs, const float* __restrict__ tile_part, int64_t n_tiles,
-                   int row_blocks, int stat_blocks, uml_seg_stats* __restrict__ stats, GatherJob job, FixupSignal sig) {
-  pdl_trigger();
-  pdl_wait();
-  // CTA roles: [0, stat_blocks) reduce the statistics; the rest are fix-up CTAs with, every (R+1)-th, a CTA that
-  // copies rows of the NEXT step's operand (job.blocks of them, interleaved so both kinds run from the start)
+                   int stat_blocks, uml_seg_stats* __restrict__ stats) {
   if (static_cast<int>(blockIdx.x) < stat_blocks) {
     tile_stats_block(tile_part, n_tiles, static_cast<int>(blockIdx.x), stats);
     return;
   }
-  int j = static_cast<int>(blockIdx.x) - stat_blocks;
-  if (job.blocks > 0) {
-    const int R = row_blocks / job.blocks > 0 ? row_blocks / job.blocks : 1;
-    const int k = j / (R + 1), r = j - k * (R + 1);
-    if (r == R && k < job.blocks) {
-      gather_rows_by_warp(job.s0, job.s1, job.vec_per_row, job.out, job.out_pitch_vec, job.out_labels,
-                          static_cast<int64_t>(k) * 8 + (threadIdx.x >> 5), static_cast<int64_t>(job.blocks) * 8);
-      return;
-    }
-    j -= k < job.blocks ? k : job.blocks;
-  }
-  if (j >= row_blocks) return;
-  const int64_t row = static_cast<int64_t>(j) * 8 + (threadIdx.x >> 5);
+  const int64_t row = static_cast<int64_t>(static_cast<int>(blockIdx.x) - stat_blocks) * 8 + (threadIdx.x >> 5);
   const int lane = threadIdx.x & 31;
-  if (row < n_rows) {
+  if (row >= n_rows) return;
   const int label = labels[row];
   const bool sg = row >= segs.n0;
   const float* sdev = sg ? segs.scale_dev[1] : segs.scale_dev[0];
@@ -584,17 +565,6 @@ __global__ void __launch_bounds__(256)
       *reinterpret_cast<uint4*>(g + c) = make_uint4(w[0], w[1], w[2], w[3]);
     }
   }
-  }  // row < n_rows
-  if (sig.done) {  // this CTA's 8 rows are final: count it for the dW split they belong to
-    __threadfence();
-    __syncthreads();
-    if (threadIdx.x == 0) {
-      const int64_t kb = (static_cast<int64_t>(j) * 8) / 64;
-      int sp = sig.n_splits - 1;
-      while (sp > 0 && (sig.num_kb * sp) / sig.n_splits > kb) --sp;
-      atomicAdd(sig.done + sp, 1u);
-    }
-  }
 }
 
 static int fwd_cta_group(int64_t n_rows) {
@@ -610,8 +580,6 @@ static int fwd_cta_group(int64_t n_rows) {
 // stand-alone version for forward passes that write no G (evaluation) and therefore launch no fix-up kernel
 __global__ void __launch_bounds__(1024)
     tile_stats_kernel(const float* __restrict__ tile_part, int64_t n_tiles, int nseg, uml_seg_stats* __restrict__ out) {
-  pdl_trigger();
-  pdl_wait();
   tile_stats_block(tile_part, n_tiles, blockIdx.x, out);
   (void)nseg;
 }
@@ -623,9 +591,7 @@ __global__ void __launch_bounds__(1024)
 int uml_head_fwd_ce_bf16_ev(const uint16_t* X, int64_t n_rows, int32_t dim, const uint16_t* W, int32_t n_classes,
                             const int32_t* labels, const uml_tc_segments* segs, uint16_t* G, int64_t ldg, float* row_loss,
                             int32_t* row_pred, int32_t* row_correct, float* row_dscale, float* tile_ws, uml_seg_stats* stats,
-                            void* ev_after_fwd, void* stream, int defer_fixup = 0, void* ev_after_fwd2 = nullptr,
-                            const uml::GatherJob* job = nullptr, const uml::FixupSignal* sig = nullptr);
-int64_t uml_fwd_tiles(int64_t n_rows);
+                            void* ev_after_fwd, void* stream, void* ev_after_fwd2 = nullptr);
 // tc_fwd2.cu: the exchange kernel (class chunks of a row tile on different CTA pairs, G final after one pass)
 bool uml_fwd_x_eligible(int64_t n_rows, int32_t n_classes);
 int uml_head_fwd_ce_x_bf16(const uint16_t* X, int64_t n_rows, int32_t dim, const uint16_t* W, int32_t n_classes,
@@ -659,8 +625,7 @@ int uml_head_fwd_ce_bf16(const uint16_t* X, int64_t n_rows, int32_t dim, const u
 int uml_head_fwd_ce_bf16_ev(const uint16_t* X, int64_t n_rows, int32_t dim, const uint16_t* W, int32_t n_classes,
                             const int32_t* labels, const uml_tc_segments* segs, uint16_t* G, int64_t ldg, float* row_loss,
                             int32_t* row_pred, int32_t* row_correct, float* row_dscale, float* tile_ws, uml_seg_stats* stats,
-                            void* ev_after_fwd, void* stream, int defer_fixup, void* ev_after_fwd2, const uml::GatherJob* job,
-                            const uml::FixupSignal* sig) {
+                            void* ev_after_fwd, void* stream, void* ev_after_fwd2) {
   using namespace uml;
   UML_REQUIRE(X && W && labels && segs && n_rows >= 0 && dim > 0 && n_classes > 0, "head_fwd_ce_bf16: bad arguments");
   UML_REQUIRE(dim % 8 == 0, "head_fwd_ce_bf16: dim (%d) must be a multiple of 8 (16-byte bf16 rows for TMA)", dim);
@@ -669,18 +634,14 @@ int uml_head_fwd_ce_bf16_ev(const uint16_t* X, int64_t n_rows, int32_t dim, cons
               "head_fwd_ce_bf16: ldg must be a multiple of 64 and >= n_classes");
   UML_REQUIRE(segs->nseg >= 1 && segs->nseg <= UML_MAX_SEGMENTS, "head_fwd_ce_bf16: 1..2 segments");
   if (n_rows == 0) return 0;
-  if (!defer_fixup && !sig && tile_ws && uml_fwd_x_eligible(n_rows, n_classes)) {
+  if (tile_ws && uml_fwd_x_eligible(n_rows, n_classes)) {
     // default for anything larger than one 128-row tile: one kernel, G final, no fix-up launch
     int rc = uml_head_fwd_ce_x_bf16(X, n_rows, dim, W, n_classes, labels, segs, G, ldg, row_loss, row_pred, row_correct,
                                     row_dscale, tile_ws, stats, stream);
     if (rc) return rc;
     if (ev_after_fwd) UML_CUDA(cudaEventRecord(static_cast<cudaEvent_t>(ev_after_fwd), uml::as_stream(stream)));
     if (ev_after_fwd2) UML_CUDA(cudaEventRecord(static_cast<cudaEvent_t>(ev_after_fwd2), uml::as_stream(stream)));
-    if (job && job->blocks > 0)  // (prefetch placement 3 rode in the fix-up launch: copy the rows directly instead)
-      rc = uml_gather2_rows_bf16_light(reinterpret_cast<const uint16_t*>(job->s0.bank), job->s0.labels, job->s0.idx, job->s0.n,
-                                       reinterpret_cast<const uint16_t*>(job->s1.bank), job->s1.labels, job->s1.idx, job->s1.n,
-                                       dim, reinterpret_cast<uint16_t*>(job->out), dim, job->out_labels, stream);
-    return rc;
+    return 0;
   }
   const int64_t n0 = segs->seg_rows[0], n1 = segs->nseg > 1 ? segs->seg_rows[1] : 0;
   UML_REQUIRE(n0 + n1 == n_rows, "head_fwd_ce_bf16: segment rows (%lld+%lld) != n_rows (%lld)", (long long)n0,
@@ -724,46 +685,23 @@ int uml_head_fwd_ce_bf16_ev(const uint16_t* X, int64_t n_rows, int32_t dim, cons
   // workspace layout: per-tile partial sums, then the per-row normalisation factors
   float* fac = tile_ws ? tile_ws + units * cg * 32 : nullptr;
   const dim3 grid(static_cast<unsigned>((units < max_clusters ? units : max_clusters) * cg));
-  UML_CUDA(launch_kernel(kern, grid, dim3(kFwdThreads), kFwdSmemBytes, as_stream(stream), cg, kPdlFwdOld, tx, tw, tg, n_rows,
+  UML_CUDA(launch_kernel(kern, grid, dim3(kFwdThreads), kFwdSmemBytes, as_stream(stream), cg, tx, tw, tg, n_rows,
                          static_cast<int>(dim), static_cast<int>(n_classes), labels, fs, reinterpret_cast<__nv_bfloat16*>(G), ldg,
                          row_loss, row_pred, row_correct, row_dscale, tile_ws, fac));
   if (ev_after_fwd) UML_CUDA(cudaEventRecord(static_cast<cudaEvent_t>(ev_after_fwd), as_stream(stream)));
   if (ev_after_fwd2) UML_CUDA(cudaEventRecord(static_cast<cudaEvent_t>(ev_after_fwd2), as_stream(stream)));
-  if (G && !defer_fixup) {
+  if (G) {
     const int row_blocks = static_cast<int>((n_rows + 7) / 8);
     const int stat_blocks = stats ? segs->nseg : 0;
-    GatherJob gj;
-    memset(&gj, 0, sizeof(gj));
-    if (job) gj = *job;
-    if (gj.blocks > row_blocks) gj.blocks = row_blocks;
-    FixupSignal fsig;
-    memset(&fsig, 0, sizeof(fsig));
-    if (sig) fsig = *sig;
-    UML_CUDA(launch_kernel(g_fixup_kernel, dim3(static_cast<unsigned>(row_blocks + stat_blocks + gj.blocks)), dim3(256), 0,
-                           as_stream(stream), 1, kPdlFwdOld, reinterpret_cast<__nv_bfloat16*>(G), ldg, n_rows, labels,
-                           static_cast<const float*>(fac), fs, static_cast<const float*>(tile_ws), units * cg, row_blocks,
-                           stat_blocks, stats, gj, fsig));
+    UML_CUDA(launch_kernel(g_fixup_kernel, dim3(static_cast<unsigned>(row_blocks + stat_blocks)), dim3(256), 0,
+                           as_stream(stream), 1, reinterpret_cast<__nv_bfloat16*>(G), ldg, n_rows, labels,
+                           static_cast<const float*>(fac), fs, static_cast<const float*>(tile_ws), units * cg, stat_blocks,
+                           stats));
   }
   return 0;
 }
 
-// 128-row tiles the forward kernel writes per-tile partials for (its work units are pairs of tiles in CTA-pair mode)
-int64_t uml_fwd_tiles(int64_t n_rows) {
-  const int cg = uml::fwd_cta_group(n_rows);
-  return ((n_rows + uml::kFwdBlockM * cg - 1) / (uml::kFwdBlockM * cg)) * cg;
-}
-
 extern "C" {
-
-// Forward WITHOUT the fix-up pass: G receives the unnormalised exp(l - m_running) and tile_ws the per-row factors;
-// uml_head_bwd_dw_fix_bf16 finishes the normalisation in its prologue (and reduces the statistics).
-int uml_head_fwd_ce_deferred_bf16(const uint16_t* X, int64_t n_rows, int32_t dim, const uint16_t* W, int32_t n_classes,
-                                  const int32_t* labels, const uml_tc_segments* segs, uint16_t* G, int64_t ldg,
-                                  float* tile_ws, void* stream) {
-  UML_REQUIRE(G && tile_ws, "head_fwd_ce_deferred_bf16: G and tile_ws are required");
-  return uml_head_fwd_ce_bf16_ev(X, n_rows, dim, W, n_classes, labels, segs, G, ldg, nullptr, nullptr, nullptr, nullptr,
-                                 tile_ws, nullptr, nullptr, stream, 1);
-}
 
 int uml_reduce_tile_stats(const float* tile_ws, int64_t n_rows, int32_t nseg, uml_seg_stats* stats, void* stream) {
   using namespace uml;
@@ -771,7 +709,7 @@ int uml_reduce_tile_stats(const float* tile_ws, int64_t n_rows, int32_t nseg, um
   if (uml_fwd_x_eligible(n_rows, 1)) return uml_fwd_x_reduce_stats(const_cast<float*>(tile_ws), n_rows, nseg, stats, stream);
   const int cg = fwd_cta_group(n_rows);
   const int64_t tiles = ((n_rows + kFwdBlockM * cg - 1) / (kFwdBlockM * cg)) * cg;  // tiles the forward kernel wrote
-  UML_CUDA(launch_kernel(tile_stats_kernel, dim3(nseg), dim3(1024), 0, as_stream(stream), 1, kPdlStats, tile_ws, tiles,
+  UML_CUDA(launch_kernel(tile_stats_kernel, dim3(nseg), dim3(1024), 0, as_stream(stream), 1, tile_ws, tiles,
                          static_cast<int>(nseg), stats));
   return 0;
 }

@@ -31,7 +31,6 @@
 //     the next kernel of the step (the dW GEMM's idle warp) or uml_reduce_tile_stats adds them in a fixed order.
 // All CTAs of the grid (<= one per SM) are co-resident, which the flag exchange relies on; a watchdog turns a
 // missing peer into an error flag (uml_fwd_x_failed) instead of a hang.
-#include <cstdlib>
 #include <type_traits>
 
 #include "common.cuh"
@@ -288,8 +287,6 @@ __global__ void __launch_bounds__(kXThreads, 1)
   cluster_sync_all();  // the peer's barriers exist before anything signals them
   tc_fence_after();
   const uint32_t tmem_base = *tmem_slot;
-  pdl_trigger();
-  pdl_wait();
   if (threadIdx.x < 2) run_scale[threadIdx.x] = segs.scale_dev[threadIdx.x] ? __ldg(segs.scale_dev[threadIdx.x]) : segs.scale[threadIdx.x];
   if (threadIdx.x == 0) {
     *epoch_slot = *reinterpret_cast<volatile unsigned*>(wk.ctrl) + 1u;
@@ -889,8 +886,6 @@ __global__ void __launch_bounds__(kXThreads, 1)
 // per-run statistics from the per-(tile, chunk, warp) partials, summed in a fixed order; one CTA per run
 __global__ void __launch_bounds__(1024)
     x_tile_stats_kernel(const float* __restrict__ tile_part, int64_t n_entries, uml_seg_stats* __restrict__ out) {
-  pdl_trigger();
-  pdl_wait();
   __shared__ float sh[4][32];
   const int s = blockIdx.x;
   float acc[4] = {0.f, 0.f, 0.f, 0.f};
@@ -919,8 +914,6 @@ __global__ void __launch_bounds__(1024)
 // the same with the number of partial records read from the workspace (uml_reduce_tile_stats knows no class count)
 __global__ void __launch_bounds__(1024)
     x_tile_stats_dev_kernel(const float* __restrict__ tile_part, const unsigned* __restrict__ ctrl, uml_seg_stats* __restrict__ out) {
-  pdl_trigger();
-  pdl_wait();
   __shared__ float sh[4][32];
   const int s = blockIdx.x;
   const int64_t n_entries = ctrl[3];
@@ -972,12 +965,7 @@ static XLayout x_layout(float* tile_ws, int64_t n_rows, int n_classes) {
 
 // true when the exchange kernel serves this shape (else tc_fwd.cu's chunk-sequential kernel runs)
 bool uml_fwd_x_eligible(int64_t n_rows, int32_t n_classes) {
-  static int mode = -1;
-  if (mode < 0) {
-    const char* e = getenv("UML_FWD_IMPL");
-    mode = (e && e[0] == 'o') ? 0 : 1;  // UML_FWD_IMPL=old keeps the chunk-sequential kernel + fix-up pass
-  }
-  return mode == 1 && n_rows > 128 && n_classes <= uml::kXMaxChunks * 256;
+  return n_rows > 128 && n_classes <= uml::kXMaxChunks * 256;
 }
 
 // where the per-(tile, chunk, warp) partials of the exchange kernel live and how many there are per run
@@ -1044,11 +1032,11 @@ int uml_head_fwd_ce_x_bf16(const uint16_t* X, int64_t n_rows, int32_t dim, const
   wk.recs = l.recs;
   wk.ctrl = l.ctrl;
   const dim3 grid(static_cast<unsigned>(n_groups * n_chunks * 2));
-  UML_CUDA(launch_kernel(kerns[slot], grid, dim3(kXThreads), kXSmemBytes, as_stream(stream), 2, kPdlFwd, tx, tw, tg, n_rows,
+  UML_CUDA(launch_kernel(kerns[slot], grid, dim3(kXThreads), kXSmemBytes, as_stream(stream), 2, tx, tw, tg, n_rows,
                          static_cast<int>(dim), static_cast<int>(n_classes), static_cast<int>(n_groups), labels, fs, G, ldg,
                          row_loss, row_pred, row_correct, row_dscale, wk));
   if (stats)
-    UML_CUDA(launch_kernel(x_tile_stats_kernel, dim3(segs->nseg), dim3(1024), 0, as_stream(stream), 1, kPdlStats,
+    UML_CUDA(launch_kernel(x_tile_stats_kernel, dim3(segs->nseg), dim3(1024), 0, as_stream(stream), 1,
                            static_cast<const float*>(l.tile_part), l.part_entries, stats));
   return 0;
 }
@@ -1057,7 +1045,7 @@ int uml_head_fwd_ce_x_bf16(const uint16_t* X, int64_t n_rows, int32_t dim, const
 int uml_fwd_x_reduce_stats(float* tile_ws, int64_t n_rows, int32_t nseg, uml_seg_stats* stats, void* stream) {
   using namespace uml;
   const XLayout l = x_layout(tile_ws, n_rows, 1);  // (the offsets do not depend on the class count)
-  UML_CUDA(launch_kernel(x_tile_stats_dev_kernel, dim3(nseg), dim3(1024), 0, as_stream(stream), 1, kPdlStats,
+  UML_CUDA(launch_kernel(x_tile_stats_dev_kernel, dim3(nseg), dim3(1024), 0, as_stream(stream), 1,
                          static_cast<const float*>(l.tile_part), static_cast<const unsigned*>(l.ctrl), stats));
   return 0;
 }

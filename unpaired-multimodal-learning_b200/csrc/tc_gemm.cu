@@ -19,23 +19,13 @@
 #include <cstdlib>
 
 #include "common.cuh"
-#include "optim.cuh"
 
-// order in which a split walks the contraction (plain kernel only; the kFix prologue keeps contiguous ascending):
-//   0 contiguous slice per split, ascending   1 contiguous, descending   2 k-blocks split, split + S, ... descending
-// The dW GEMM contracts over the batch rows, and the forward kernel has just written G in ascending row order: the
-// newest rows are the ones still in L2.
-// Measured on B200 inside the cfg3 step (73 728 rows, 6 splits): 0.2246-0.2270 ms/step with order 0, the same with 1,
-// 0.2228-0.2232 with 2 - every CTA then reads neighbouring k-blocks at the same time (the 3 + 8 CTAs that share a block
-// of G or X meet in L2) and the sweep starts where G is still resident.
-#ifndef UML_DW_KORDER
-#define UML_DW_KORDER 2
-#endif
-#ifndef UML_DW_UPD_UNROLL
-#define UML_DW_UPD_UNROLL 1  // float4 elements per thread and trip of the fused update (registers: 32 per element)
-#endif
-
-int64_t uml_fwd_tiles(int64_t n_rows);  // tc_fwd.cu: 128-row tiles the forward kernel writes partials for
+// Order in which a split walks the contraction: k-blocks split, split + S, split + 2S, ..., newest first.  The dW GEMM
+// contracts over the batch rows, and the forward kernel has just written G in ascending row order: the newest rows are
+// the ones still in L2.
+// Measured on B200 inside the cfg3 step (73 728 rows, 6 splits): 0.2246-0.2270 ms/step with a contiguous slice per split
+// (ascending or descending), 0.2228-0.2232 with this order - every CTA then reads neighbouring k-blocks at the same time
+// (the 3 + 8 CTAs that share a block of G or X meet in L2) and the sweep starts where G is still resident.
 
 namespace uml {
 
@@ -56,53 +46,19 @@ struct GemmCfg {
   static constexpr int kSmemBytes = kStages * kStageBytes + 1024 + 256;
 };
 
-// dW prologue (kFix): the A operand is the forward kernel's UNNORMALISED bf16 exp(l - m_running); the deferred
-// softmax normalisation and the one-hot term are applied to each A stage in shared memory, between the TMA
-// arrival and the MMA, by the four warps that are idle until the epilogue:
-//   G[b, c] = A[b, c] * fac[b][c / 64] - [c == y_b] * gcoef_b          (what g_fixup_kernel did in a pass over HBM/L2)
-struct FixArgs {
-  const float* fac;         // [rows, 16] per-row, per-64-class factors written by the forward kernel
-  const int32_t* labels;    // [rows]
-  int64_t n0;               // rows >= n0 belong to the second run
-  float gcoef[2];           // loss_weight / n * scale per run ...
-  float dcoef[2];           // ... or loss_weight / n, multiplied by *scale_dev[run] when that is set
-  const float* scale_dev[2];
-  const float* tile_part;   // forward kernel's per-tile partial statistics (reduced here by one idle warp)
-  int64_t n_tiles;
-  int nseg;
-  uml_seg_stats* stats;
-  // any instantiation: let split z start only when wait_done[z] >= wait_expected[z] (fix-up CTAs of its rows finished)
-  const unsigned* wait_done;
-  unsigned wait_expected[8];
-  int* wait_failed;
-  // any instantiation: the exchange forward kernel's per-(tile, chunk, warp) partials (tc_fwd2.cu), reduced into
-  // `stats` by an idle warp of the first CTA - the forward's statistics cost no launch of their own
+// the dW GEMM's side job: the exchange forward kernel's per-(tile, chunk, warp) partials (tc_fwd2.cu), reduced into
+// `stats` by an idle warp of the first CTA - the forward's statistics cost no launch of their own
+struct DwStatsJob {
   const float* part;
   int64_t part_entries;
-  // fp32 split-K output only (single-GPU step): when upd_p is set the kernel also finishes the step - every CTA signals
-  // its partial tile, waits for the tile's other splits (all CTAs of the grid are co-resident or become so without
-  // anybody's help) and then sums ITS share of the tile's rows over the splits, in split order, and applies AdamW to
-  // them: W, m, v and the bf16 shadow of W leave this kernel final, no update launch follows (ldo == N: the output
-  // tile is laid out like W)
-  float* upd_p;
-  float* upd_m;
-  float* upd_v;
-  __nv_bfloat16* upd_shadow;
-  AdamArgs upd;
-  unsigned* upd_cnt;     // [2 per CTA tile]: arrived, departed (both 0 between launches)
-  unsigned* upd_failed;  // set when a split never arrived (the update of that tile is then skipped)
+  int nseg;
+  uml_seg_stats* stats;
 };
 
-__device__ __forceinline__ unsigned ld_acquire_u32(const unsigned* p) {
-  unsigned v;
-  asm volatile("ld.acquire.gpu.global.u32 %0, [%1];" : "=r"(v) : "l"(p) : "memory");
-  return v;
-}
-
-template <bool kAMn, bool kBMn, bool kOutBf16, int kCG, bool kFix = false, bool kUpd = false>
+template <bool kAMn, bool kBMn, bool kOutBf16, int kCG>
 __global__ void __launch_bounds__(256, 1)
     tc_gemm_kernel(const __grid_constant__ CUtensorMap tmap_a, const __grid_constant__ CUtensorMap tmap_b, int64_t M,
-                   int64_t N, int64_t K, int n_splits, void* __restrict__ out_v, int64_t ldo, FixArgs fix) {
+                   int64_t N, int64_t K, int n_splits, void* __restrict__ out_v, int64_t ldo, DwStatsJob job) {
   using Cfg = GemmCfg<kCG>;
   constexpr int kGStages = Cfg::kStages;
   extern __shared__ unsigned char smem_raw[];
@@ -110,8 +66,7 @@ __global__ void __launch_bounds__(256, 1)
   uint64_t* full_bar = reinterpret_cast<uint64_t*>(smem + kGStages * Cfg::kStageBytes);
   uint64_t* empty_bar = full_bar + kGStages;
   uint64_t* tfull_bar = empty_bar + kGStages;
-  uint64_t* ready_bar = tfull_bar + 1;  // kFix: stage transformed in BOTH CTAs of the pair (lives on the leader)
-  uint32_t* tmem_slot = reinterpret_cast<uint32_t*>(ready_bar + kGStages);
+  uint32_t* tmem_slot = reinterpret_cast<uint32_t*>(tfull_bar + 1);
 
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
   const uint32_t rank = (kCG == 2) ? cluster_ctarank() : 0u;
@@ -120,11 +75,8 @@ __global__ void __launch_bounds__(256, 1)
   const int64_t m_cta = static_cast<int64_t>(m_tile) * Cfg::kTileM + rank * 128;   // first output row of this CTA
   const int64_t n_cta = static_cast<int64_t>(n_tile) * Cfg::kTileN + rank * Cfg::kCtaN;  // first B column staged here
   const int num_kb = static_cast<int>((K + kGBlockK - 1) / kGBlockK);
-  constexpr int kOrder = kFix ? 0 : UML_DW_KORDER;
-  // (kOrder 2: kb_lo .. kb_hi only count this split's k-blocks; block j of the walk is split + n_splits * (count - 1 - j))
-  const int kb_lo = kOrder == 2 ? 0 : static_cast<int>((static_cast<int64_t>(num_kb) * split) / n_splits);
-  const int kb_hi = kOrder == 2 ? (num_kb - split + n_splits - 1) / n_splits
-                                : static_cast<int>((static_cast<int64_t>(num_kb) * (split + 1)) / n_splits);
+  // this split's k-blocks; block j of the walk is split + n_splits * (kb_hi - 1 - j)
+  const int kb_hi = (num_kb - split + n_splits - 1) / n_splits;
 
   if (warp == 0 && lane == 0) {
     tma_prefetch_desc(&tmap_a);
@@ -132,11 +84,8 @@ __global__ void __launch_bounds__(256, 1)
   }
   if (warp == 1 && lane == 0) {
     for (int s = 0; s < kGStages; ++s) {
-      // plain: one arrival per producer of the pair, tx bytes counted on the leader.  kFix: every CTA tracks its
-      // OWN loads (its transform warps must know when its stage landed) and the MMA waits on ready_bar instead
-      mbar_init(&full_bar[s], kFix ? 1 : kCG);
+      mbar_init(&full_bar[s], kCG);  // one arrival per producer of the pair; tx bytes are counted on the leader
       mbar_init(&empty_bar[s], 1);
-      mbar_init(&ready_bar[s], 4 * kCG);
     }
     mbar_init(tfull_bar, 1);
     fence_barrier_init();
@@ -150,37 +99,18 @@ __global__ void __launch_bounds__(256, 1)
   else __syncthreads();
   tc_fence_after();
   const uint32_t tmem_base = *tmem_slot;
-  pdl_trigger();
-  pdl_wait();  // everything above (barriers, TMEM, descriptor prefetch) overlapped the previous kernel's tail
 
   if (warp == 0) {
     // ------------------------------------------------ TMA producer (every CTA) -------------------
     if (lane == 0) {
-      if (fix.wait_done) {
-        // the A operand of this split is still being finalised by the concurrently running fix-up launch
-        const unsigned need = fix.wait_expected[split];
-        const long long t0 = clock64();
-        for (;;) {
-          unsigned v;
-          asm volatile("ld.acquire.gpu.global.u32 %0, [%1];" : "=r"(v) : "l"(fix.wait_done + split) : "memory");
-          if (v >= need) break;
-          if (clock64() - t0 > 400000000ll) {  // ~0.2 s: never hang the GPU; the caller checks the flag
-            *fix.wait_failed = 1;
-            break;
-          }
-          __nanosleep(100);
-        }
-        asm volatile("fence.proxy.async;" ::: "memory");  // generic-proxy writes of G -> this thread's TMA reads
-      }
       uint32_t it = 0;
-      for (int kb = kb_lo; kb < kb_hi; ++kb, ++it) {
+      for (int kb = 0; kb < kb_hi; ++kb, ++it) {
         const uint32_t s = it % kGStages, ph = (it / kGStages) & 1;
         mbar_wait(&empty_bar[s], ph ^ 1);
         unsigned char* a = smem + s * Cfg::kStageBytes;
         unsigned char* b = a + Cfg::kABytes;
-        const int kbe = kOrder == 0 ? kb : kOrder == 1 ? kb_hi - 1 - (kb - kb_lo) : split + n_splits * (kb_hi - 1 - kb);
-        const int32_t k0 = kbe * kGBlockK;
-        if (kCG == 1 || kFix) {
+        const int32_t k0 = (split + n_splits * (kb_hi - 1 - kb)) * kGBlockK;
+        if (kCG == 1) {
           mbar_arrive_expect_tx(&full_bar[s], Cfg::kStageBytes);
           if (kAMn) {
             tma_load_2d(a, &tmap_a, &full_bar[s], static_cast<int32_t>(m_cta), k0);
@@ -221,9 +151,9 @@ __global__ void __launch_bounds__(256, 1)
     if (lane == 0 && leader) {
       constexpr uint32_t idesc = make_idesc_bf16(Cfg::kTileM, Cfg::kTileN, kAMn ? 1 : 0, kBMn ? 1 : 0);
       uint32_t it = 0;
-      for (int kb = kb_lo; kb < kb_hi; ++kb, ++it) {
+      for (int kb = 0; kb < kb_hi; ++kb, ++it) {
         const uint32_t s = it % kGStages, ph = (it / kGStages) & 1;
-        mbar_wait(kFix ? &ready_bar[s] : &full_bar[s], ph);
+        mbar_wait(&full_bar[s], ph);
         tc_fence_after();
         const uint32_t a_addr = smem_u32(smem + s * Cfg::kStageBytes);
         const uint32_t b_addr = a_addr + Cfg::kABytes;
@@ -246,17 +176,17 @@ __global__ void __launch_bounds__(256, 1)
       else umma_commit(tfull_bar);
     }
     __syncwarp();
-  } else if (!kFix && warp == 3) {
+  } else if (warp == 3) {
     // ------------------------------------------------ per-run statistics of the exchange forward kernel -------
-    if (blockIdx.x == 0 && blockIdx.y == 0 && blockIdx.z == 0 && fix.stats && fix.part) {
-      for (int sgi = 0; sgi < fix.nseg; ++sgi) {
+    if (blockIdx.x == 0 && blockIdx.y == 0 && blockIdx.z == 0 && job.stats && job.part) {
+      for (int sgi = 0; sgi < job.nseg; ++sgi) {
         float acc[4] = {0.f, 0.f, 0.f, 0.f};
-        for (int64_t i0 = 0; i0 < fix.part_entries; i0 += 128) {  // four independent 16-byte loads in flight per lane
+        for (int64_t i0 = 0; i0 < job.part_entries; i0 += 128) {  // four independent 16-byte loads in flight per lane
           float4 v[4];
 #pragma unroll
           for (int u = 0; u < 4; ++u) {
             const int64_t i = i0 + u * 32 + lane;
-            v[u] = i < fix.part_entries ? __ldcg(reinterpret_cast<const float4*>(fix.part) + i * 2 + sgi)
+            v[u] = i < job.part_entries ? __ldcg(reinterpret_cast<const float4*>(job.part) + i * 2 + sgi)
                                         : make_float4(0.f, 0.f, 0.f, 0.f);
           }
 #pragma unroll
@@ -265,105 +195,18 @@ __global__ void __launch_bounds__(256, 1)
 #pragma unroll
         for (int k = 0; k < 4; ++k) acc[k] = warp_sum(acc[k]);
         if (lane == 0) {
-          fix.stats[sgi].loss_mean = acc[3] > 0.f ? acc[0] / acc[3] : 0.f;
-          fix.stats[sgi].dscale = acc[1];
-          fix.stats[sgi].correct = static_cast<int32_t>(acc[2] + 0.5f);
-          fix.stats[sgi].n = static_cast<int32_t>(acc[3] + 0.5f);
-        }
-      }
-    }
-  } else if (kFix && warp == 3) {
-    // ------------------------------------------------ per-run statistics (one idle warp of one CTA) ---------
-    if (blockIdx.x == 0 && blockIdx.y == 0 && blockIdx.z == 0 && fix.stats) {
-      for (int sgi = 0; sgi < fix.nseg; ++sgi) {
-        float acc[4] = {0.f, 0.f, 0.f, 0.f};
-        for (int64_t i = lane; i < fix.n_tiles * 4; i += 32) {
-          const float* p = fix.tile_part + (i * 2 + sgi) * 4;
-#pragma unroll
-          for (int k = 0; k < 4; ++k) acc[k] += p[k];
-        }
-#pragma unroll
-        for (int k = 0; k < 4; ++k) acc[k] = warp_sum(acc[k]);
-        if (lane == 0) {
-          fix.stats[sgi].loss_mean = acc[3] > 0.f ? acc[0] / acc[3] : 0.f;
-          fix.stats[sgi].dscale = acc[1];
-          fix.stats[sgi].correct = static_cast<int32_t>(acc[2] + 0.5f);
-          fix.stats[sgi].n = static_cast<int32_t>(acc[3] + 0.5f);
+          job.stats[sgi].loss_mean = acc[3] > 0.f ? acc[0] / acc[3] : 0.f;
+          job.stats[sgi].dscale = acc[1];
+          job.stats[sgi].correct = static_cast<int32_t>(acc[2] + 0.5f);
+          job.stats[sgi].n = static_cast<int32_t>(acc[3] + 0.5f);
         }
       }
     }
   } else if (warp >= 4) {
-    if (kFix) {
-      // ---------------------------------------------- A-stage transform (see FixArgs) -----------------------
-      // thread -> (k row r of the stage, 64-class box b); a row is 128 B = 8 chunks of 16 B, chunk c of row r sits
-      // at physical chunk c ^ (r & 7) (SWIZZLE_128B): a quarter warp touches all 32 banks exactly once
-      const int t = threadIdx.x - 128, r = t & 63, b = t >> 6;
-      const int grp = static_cast<int>(m_cta / 64) + b;
-      const uint32_t lead_ready = kCG == 2 ? mapa_cta(smem_u32(&ready_bar[0]), 0) : 0u;
-      // per-row metadata (factor, one-hot coefficient, label position) is fetched ONE k-block ahead: an L2 round
-      // trip per stage on the transform's critical path made the whole GEMM twice as slow
-      auto load_meta = [&](int kb, float& f, float& gc, int& lc) {
-        const int64_t row = static_cast<int64_t>(kb) * kGBlockK + r;
-        f = 0.f; gc = 0.f; lc = -1;
-        if (kb < kb_hi && row < K) {
-          f = __ldg(fix.fac + row * 16 + grp);
-          const bool sg = row >= fix.n0;
-          const float* sd = sg ? fix.scale_dev[1] : fix.scale_dev[0];
-          gc = sd ? (sg ? fix.dcoef[1] : fix.dcoef[0]) * __ldg(sd) : (sg ? fix.gcoef[1] : fix.gcoef[0]);
-          lc = __ldg(fix.labels + row) - grp * 64;
-        }
-      };
-      float f_nx, gc_nx;
-      int lc_nx;
-      load_meta(kb_lo, f_nx, gc_nx, lc_nx);
-      uint32_t it = 0;
-      for (int kb = kb_lo; kb < kb_hi; ++kb, ++it) {
-        const uint32_t s = it % kGStages, ph = (it / kGStages) & 1;
-        const bool live = static_cast<int64_t>(kb) * kGBlockK + r < K;
-        const float f = f_nx, gc = gc_nx;
-        const int lc = lc_nx;
-        load_meta(kb + 1, f_nx, gc_nx, lc_nx);
-        mbar_wait(&full_bar[s], ph);
-        if (live) {
-          unsigned char* rowp = smem + s * Cfg::kStageBytes + b * kGBoxBytes + r * 128;
-          uint4 v[8];
-#pragma unroll
-          for (int c = 0; c < 8; ++c) v[c] = *reinterpret_cast<const uint4*>(rowp + ((c ^ (r & 7)) << 4));
-#pragma unroll
-          for (int c = 0; c < 8; ++c) {
-            uint32_t w[4] = {v[c].x, v[c].y, v[c].z, v[c].w};
-#pragma unroll
-            for (int i = 0; i < 4; ++i) {
-              float2 p = __bfloat1622float2(*reinterpret_cast<__nv_bfloat162*>(&w[i]));
-              p.x *= f;
-              p.y *= f;
-              __nv_bfloat162 h = __floats2bfloat162_rn(p.x, p.y);
-              w[i] = *reinterpret_cast<uint32_t*>(&h);
-            }
-            *reinterpret_cast<uint4*>(rowp + ((c ^ (r & 7)) << 4)) = make_uint4(w[0], w[1], w[2], w[3]);
-          }
-          if (lc >= 0 && lc < 64) {
-            // the one-hot term: G = G~ * f - coef, recomputed from the ORIGINAL element so that the rounding is the
-            // fix-up kernel's (multiply, subtract, one rounding)
-            const int c = lc >> 3, e = lc & 7;
-            const uint32_t word = (&v[c].x)[e >> 1];
-            const float2 p = __bfloat1622float2(*reinterpret_cast<const __nv_bfloat162*>(&word));
-            const float val = ((e & 1) ? p.y : p.x) * f - gc;
-            reinterpret_cast<__nv_bfloat16*>(rowp + ((c ^ (r & 7)) << 4))[e] = __float2bfloat16_rn(val);
-          }
-        }
-        fence_proxy_async();  // generic-proxy writes -> visible to the tensor core's async-proxy reads
-        __syncwarp();
-        if (lane == 0) {
-          if (kCG == 2 && !leader) mbar_arrive_remote(lead_ready + s * 8);
-          else mbar_arrive(&ready_bar[s]);
-        }
-      }
-    }
     // ------------------------------------------------ epilogue (every CTA: its own 128 rows) ------
     const int q = warp - 4;
     const int64_t m = m_cta + q * 32 + lane;
-    const bool have = kb_hi > kb_lo;
+    const bool have = kb_hi > 0;
     if (have) {
       mbar_wait(tfull_bar, 0);
       tc_fence_after();
@@ -422,89 +265,6 @@ __global__ void __launch_bounds__(256, 1)
     if (kCG == 2) tmem_dealloc_cg2(tmem_base, 256);
     else tmem_dealloc(tmem_base, 256);
   }
-  if constexpr (kUpd && !kOutBf16) {
-    if (fix.upd_p != nullptr) {
-      // ------------------------------------------------ split-K sum + AdamW of this CTA's share of its tile ----------
-      __shared__ int upd_ok;
-      unsigned* arrived = fix.upd_cnt + 2 * (blockIdx.x * gridDim.y + blockIdx.y);
-      __threadfence();  // the epilogue warps' partial rows are visible device-wide before the arrival below
-      __syncthreads();
-      if (threadIdx.x == 0) {
-        atomicAdd(arrived, 1u);
-        bool ok = true;
-        for (unsigned polls = 0; ld_acquire_u32(arrived) < static_cast<unsigned>(n_splits); ++polls) {
-          if (polls > (1u << 22)) {  // ~ a second: never hang the GPU; the host checks the flag
-            atomicExch(fix.upd_failed, 1u);
-            ok = false;
-            break;
-          }
-        }
-        upd_ok = ok ? 1 : 0;
-      }
-      __syncthreads();
-      if (upd_ok) {
-        const float* parts = static_cast<const float*>(out_v);
-        const int64_t plane = M * ldo;
-        const int r_lo = (128 * split) / n_splits, r_hi = (128 * (split + 1)) / n_splits;
-        const int64_t n_base = static_cast<int64_t>(n_tile) * Cfg::kTileN;
-        const int cols4 = static_cast<int>(((N - n_base < Cfg::kTileN ? N - n_base : Cfg::kTileN) + 3) / 4);
-        const int total4 = (r_hi - r_lo) * cols4;
-        constexpr int kU = UML_DW_UPD_UNROLL, kMaxSplits = 8;
-#pragma unroll 1
-        for (int e0 = threadIdx.x; e0 < total4; e0 += 256 * kU) {
-          float4 q[kMaxSplits][kU], w[kU], mm[kU], vv[kU];
-          int64_t off[kU];
-          bool on[kU];
-#pragma unroll
-          for (int u = 0; u < kU; ++u) {
-            const int e = e0 + u * 256, r = e / cols4;
-            const int64_t m = m_cta + r_lo + r;
-            on[u] = e < total4 && m < M;
-            off[u] = m * ldo + n_base + (e - r * cols4) * 4;
-          }
-#pragma unroll
-          for (int sp = 0; sp < kMaxSplits; ++sp) {
-#pragma unroll
-            for (int u = 0; u < kU; ++u)
-              if (sp < n_splits && on[u]) q[sp][u] = __ldcg(reinterpret_cast<const float4*>(parts + sp * plane + off[u]));
-          }
-#pragma unroll
-          for (int u = 0; u < kU; ++u) {
-            if (on[u]) {
-              w[u] = *reinterpret_cast<const float4*>(fix.upd_p + off[u]);
-              mm[u] = *reinterpret_cast<const float4*>(fix.upd_m + off[u]);
-              vv[u] = *reinterpret_cast<const float4*>(fix.upd_v + off[u]);
-            }
-          }
-#pragma unroll
-          for (int u = 0; u < kU; ++u) {
-            if (!on[u]) continue;
-            float4 g = q[0][u];
-#pragma unroll
-            for (int sp = 1; sp < kMaxSplits; ++sp) {
-              if (sp < n_splits) { g.x += q[sp][u].x; g.y += q[sp][u].y; g.z += q[sp][u].z; g.w += q[sp][u].w; }
-            }
-            float4 o = w[u];
-            o.x = adam_one(fix.upd, o.x, g.x, mm[u].x, vv[u].x);
-            o.y = adam_one(fix.upd, o.y, g.y, mm[u].y, vv[u].y);
-            o.z = adam_one(fix.upd, o.z, g.z, mm[u].z, vv[u].z);
-            o.w = adam_one(fix.upd, o.w, g.w, mm[u].w, vv[u].w);
-            *reinterpret_cast<float4*>(fix.upd_p + off[u]) = o;
-            *reinterpret_cast<float4*>(fix.upd_m + off[u]) = mm[u];
-            *reinterpret_cast<float4*>(fix.upd_v + off[u]) = vv[u];
-            if (fix.upd_shadow) *reinterpret_cast<uint2*>(fix.upd_shadow + off[u]) = pack_bf16x4(o);
-          }
-        }
-      }
-      if (threadIdx.x == 0) {  // the last split to leave puts the tile's counters back to zero for the next launch
-        const unsigned d = atomicAdd(arrived + 1, 1u);
-        if (d == static_cast<unsigned>(n_splits) - 1u) {
-          atomicExch(arrived, 0u);
-          atomicExch(arrived + 1, 0u);
-        }
-      }
-    }
-  }
 }
 
 static int cta_group_for(int64_t M) {
@@ -526,11 +286,11 @@ static int gemm_splits(int64_t M, int64_t N, int64_t K, int cg) {
   return static_cast<int>(s);
 }
 
-template <bool kAMn, bool kBMn, bool kOutBf16, int kCG, bool kFix = false, bool kUpd = false>
+template <bool kAMn, bool kBMn, bool kOutBf16, int kCG>
 static int launch_tc_gemm(const CUtensorMap& ta, const CUtensorMap& tb, int64_t M, int64_t N, int64_t K, int n_splits,
-                          void* out, int64_t ldo, cudaStream_t st, const FixArgs& fix = FixArgs()) {
+                          void* out, int64_t ldo, cudaStream_t st, const DwStatsJob& job = DwStatsJob()) {
   using Cfg = GemmCfg<kCG>;
-  auto kern = tc_gemm_kernel<kAMn, kBMn, kOutBf16, kCG, kFix, kUpd>;
+  auto kern = tc_gemm_kernel<kAMn, kBMn, kOutBf16, kCG>;
   static bool attr_set = false;
   if (!attr_set) {
     UML_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, Cfg::kSmemBytes));
@@ -538,13 +298,13 @@ static int launch_tc_gemm(const CUtensorMap& ta, const CUtensorMap& tb, int64_t 
   }
   const dim3 grid(static_cast<unsigned>((M + Cfg::kTileM - 1) / Cfg::kTileM) * kCG,
                   static_cast<unsigned>((N + Cfg::kTileN - 1) / Cfg::kTileN), static_cast<unsigned>(n_splits));
-  UML_CUDA(launch_kernel(kern, grid, dim3(256), Cfg::kSmemBytes, st, kCG, kPdlDw, ta, tb, M, N, K, n_splits, out, ldo, fix));
+  UML_CUDA(launch_kernel(kern, grid, dim3(256), Cfg::kSmemBytes, st, kCG, ta, tb, M, N, K, n_splits, out, ldo, job));
   return 0;
 }
 
 static int tc_gemm(const uint16_t* A, int64_t lda, bool a_mn, const uint16_t* B, int64_t ldb, bool b_mn, int64_t M,
                    int64_t N, int64_t K, void* out, int64_t ldo, bool out_bf16, int n_splits, cudaStream_t st,
-                   const FixArgs* fix = nullptr) {
+                   const DwStatsJob* job = nullptr) {
   UML_REQUIRE(A && B && out && M > 0 && N > 0 && K > 0 && n_splits >= 1, "tc_gemm: bad arguments");
   UML_REQUIRE(lda % 8 == 0 && ldb % 8 == 0, "tc_gemm: leading dimensions must be multiples of 8 (16-byte bf16 rows)");
   UML_REQUIRE(!out_bf16 || n_splits == 1, "tc_gemm: split-K needs the fp32 partial output");
@@ -564,26 +324,10 @@ static int tc_gemm(const uint16_t* A, int64_t lda, bool a_mn, const uint16_t* B,
   } else {
     if (make_tmap_2d(&tb, B, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 2, K, N, ldb * 2, kGBlockK, 256 / cg, CU_TENSOR_MAP_SWIZZLE_128B)) return 1;
   }
-  if (fix && !fix->fac && !fix->wait_done && fix->upd_p) {  // dW kernel with the update in its tail (an instantiation of its own:
-    UML_REQUIRE(a_mn && b_mn && !out_bf16 && ldo == N, "tc_gemm: the fused update is wired for the dW layout only");  // its registers)
-    return cg == 2 ? launch_tc_gemm<true, true, false, 2, false, true>(ta, tb, M, N, K, n_splits, out, ldo, st, *fix)
-                   : launch_tc_gemm<true, true, false, 1, false, true>(ta, tb, M, N, K, n_splits, out, ldo, st, *fix);
-  }
-  if (fix && !fix->fac && !fix->wait_done) {  // statistics job only: plain dW kernel
+  if (job) {  // statistics job: the dW kernel
     UML_REQUIRE(a_mn && b_mn && !out_bf16, "tc_gemm: the statistics job is wired for the dW layout only");
-    return cg == 2 ? launch_tc_gemm<true, true, false, 2, false>(ta, tb, M, N, K, n_splits, out, ldo, st, *fix)
-                   : launch_tc_gemm<true, true, false, 1, false>(ta, tb, M, N, K, n_splits, out, ldo, st, *fix);
-  }
-  if (fix && !fix->fac) {  // wait-only: plain dW kernel whose splits are gated by the fix-up counters
-    UML_REQUIRE(UML_DW_KORDER == 0, "tc_gemm: split gating needs every split to own a contiguous row range");
-    UML_REQUIRE(a_mn && b_mn && !out_bf16, "tc_gemm: split gating is wired for the dW layout only");
-    return cg == 2 ? launch_tc_gemm<true, true, false, 2, false>(ta, tb, M, N, K, n_splits, out, ldo, st, *fix)
-                   : launch_tc_gemm<true, true, false, 1, false>(ta, tb, M, N, K, n_splits, out, ldo, st, *fix);
-  }
-  if (fix) {
-    UML_REQUIRE(a_mn && b_mn && !out_bf16, "tc_gemm: the A-stage transform is instantiated for the dW layout only");
-    return cg == 2 ? launch_tc_gemm<true, true, false, 2, true>(ta, tb, M, N, K, n_splits, out, ldo, st, *fix)
-                   : launch_tc_gemm<true, true, false, 1, true>(ta, tb, M, N, K, n_splits, out, ldo, st, *fix);
+    return cg == 2 ? launch_tc_gemm<true, true, false, 2>(ta, tb, M, N, K, n_splits, out, ldo, st, *job)
+                   : launch_tc_gemm<true, true, false, 1>(ta, tb, M, N, K, n_splits, out, ldo, st, *job);
   }
 #define UML_GEMM_CASE(AM, BM, OB)                                                                              \
   if (a_mn == AM && b_mn == BM && out_bf16 == OB)                                                              \
@@ -600,24 +344,6 @@ static int tc_gemm(const uint16_t* A, int64_t lda, bool a_mn, const uint16_t* B,
 
 }  // namespace uml
 
-// dW whose K splits wait for the fix-up launch's per-split counters (see FixupSignal); library-internal
-int uml_head_bwd_dw_gated_bf16(const uint16_t* G, int64_t ldg, const uint16_t* X, int64_t n_rows, int32_t dim, int32_t n_classes,
-                               float* partials, int32_t n_splits, const unsigned* done, int* failed, void* stream) {
-  using namespace uml;
-  UML_REQUIRE(G && X && partials && done && failed && n_rows > 0 && n_splits >= 1 && n_splits <= 8, "dw_gated: bad arguments");
-  FixArgs fx;
-  memset(&fx, 0, sizeof(fx));
-  fx.wait_done = done;
-  fx.wait_failed = failed;
-  const int64_t num_kb = (n_rows + kGBlockK - 1) / kGBlockK;
-  for (int sp = 0; sp < n_splits; ++sp) {
-    const int64_t r_lo = (num_kb * sp / n_splits) * kGBlockK, r_hi_raw = (num_kb * (sp + 1) / n_splits) * kGBlockK;
-    const int64_t r_hi = r_hi_raw < n_rows ? r_hi_raw : n_rows;
-    fx.wait_expected[sp] = r_hi > r_lo ? static_cast<unsigned>((r_hi - r_lo + 7) / 8) : 0u;
-  }
-  return tc_gemm(G, ldg, true, X, dim, true, n_classes, dim, n_rows, partials, dim, false, n_splits, as_stream(stream), &fx);
-}
-
 // dW that also reduces the exchange forward kernel's partial statistics (library-internal, step.cu)
 int uml_head_bwd_dw_stats_bf16(const uint16_t* G, int64_t ldg, const uint16_t* X, int64_t n_rows, int32_t dim, int32_t n_classes,
                                float* partials, int32_t n_splits, const float* part, int64_t part_entries, int32_t nseg,
@@ -626,51 +352,8 @@ int uml_head_bwd_dw_stats_bf16(const uint16_t* G, int64_t ldg, const uint16_t* X
   UML_REQUIRE(G && X && partials && n_rows > 0 && n_splits >= 1 && part && stats && nseg >= 1 && nseg <= UML_MAX_SEGMENTS,
               "dw_stats: bad arguments");
   UML_REQUIRE(dim % 8 == 0 && ldg % 64 == 0 && ldg >= n_classes, "dw_stats: dim must be a multiple of 8 and ldg of 64");
-  FixArgs fx;
-  memset(&fx, 0, sizeof(fx));
-  fx.part = part;
-  fx.part_entries = part_entries;
-  fx.nseg = nseg;
-  fx.stats = stats;
-  return tc_gemm(G, ldg, true, X, dim, true, n_classes, dim, n_rows, partials, dim, false, n_splits, as_stream(stream), &fx);
-}
-
-// dW + forward statistics + split-K sum + AdamW in one launch (library-internal, step.cu; single-GPU bf16 step)
-int uml_head_bwd_dw_update_bf16(const uint16_t* G, int64_t ldg, const uint16_t* X, int64_t n_rows, int32_t dim, int32_t n_classes,
-                                float* partials, int32_t n_splits, const float* part, int64_t part_entries, int32_t nseg,
-                                uml_seg_stats* stats, float* W, float* m, float* v, uint16_t* W16, const uml::AdamArgs* adam,
-                                unsigned* failed, void* stream) {
-  using namespace uml;
-  UML_REQUIRE(G && X && partials && n_rows > 0 && n_splits >= 1 && n_splits <= 8 && W && m && v && adam && failed,
-              "dw_update: bad arguments");
-  UML_REQUIRE(dim % 8 == 0 && ldg % 64 == 0 && ldg >= n_classes, "dw_update: dim must be a multiple of 8 and ldg of 64");
-  // counters of the tiles' splits: one small device buffer per device, zero between launches (the kernel resets them)
-  static unsigned* cnt[64] = {nullptr};
-  int dev = 0;
-  UML_CUDA(cudaGetDevice(&dev));
-  UML_REQUIRE(dev >= 0 && dev < 64, "dw_update: device index");
-  constexpr int kCntWords = 2 * 1024;
-  if (!cnt[dev]) {
-    UML_CUDA(cudaMalloc(&cnt[dev], kCntWords * sizeof(unsigned)));
-    UML_CUDA(cudaMemset(cnt[dev], 0, kCntWords * sizeof(unsigned)));
-  }
-  const int cg = cta_group_for(n_classes);
-  const int64_t tiles = ((n_classes + 128 * cg - 1) / (128 * cg)) * cg * ((dim + 255) / 256);
-  UML_REQUIRE(tiles * 2 <= kCntWords, "dw_update: too many output tiles (%lld)", (long long)tiles);
-  FixArgs fx;
-  memset(&fx, 0, sizeof(fx));
-  fx.part = part;
-  fx.part_entries = part_entries;
-  fx.nseg = nseg;
-  fx.stats = part ? stats : nullptr;
-  fx.upd_p = W;
-  fx.upd_m = m;
-  fx.upd_v = v;
-  fx.upd_shadow = reinterpret_cast<__nv_bfloat16*>(W16);
-  fx.upd = *adam;
-  fx.upd_cnt = cnt[dev];
-  fx.upd_failed = failed;
-  return tc_gemm(G, ldg, true, X, dim, true, n_classes, dim, n_rows, partials, dim, false, n_splits, as_stream(stream), &fx);
+  const DwStatsJob job{part, part_entries, nseg, stats};
+  return tc_gemm(G, ldg, true, X, dim, true, n_classes, dim, n_rows, partials, dim, false, n_splits, as_stream(stream), &job);
 }
 
 extern "C" {
@@ -692,13 +375,6 @@ int uml_tc_dw_splits(int64_t n_rows, int32_t dim, int32_t n_classes) {
 
 int uml_head_bwd_dw_bf16(const uint16_t* G, int64_t ldg, const uint16_t* X, int64_t n_rows, int32_t dim,
                          int32_t n_classes, float* partials, int32_t n_splits, void* stream) {
-  return uml_head_bwd_dw_fix_bf16(G, ldg, X, n_rows, dim, n_classes, partials, n_splits, nullptr, nullptr, nullptr, nullptr,
-                                  stream);
-}
-
-int uml_head_bwd_dw_fix_bf16(const uint16_t* G, int64_t ldg, const uint16_t* X, int64_t n_rows, int32_t dim,
-                             int32_t n_classes, float* partials, int32_t n_splits, const uml_tc_segments* segs,
-                             const int32_t* labels, const float* tile_ws, uml_seg_stats* stats, void* stream) {
   using namespace uml;
   UML_REQUIRE(G && X && partials && n_rows > 0 && dim > 0 && n_classes > 0 && n_splits >= 1,
               "head_bwd_dw_bf16: bad arguments");
@@ -706,28 +382,7 @@ int uml_head_bwd_dw_fix_bf16(const uint16_t* G, int64_t ldg, const uint16_t* X, 
               "head_bwd_dw_bf16: dim must be a multiple of 8 and ldg a multiple of 64 >= n_classes");
   UML_REQUIRE((reinterpret_cast<uintptr_t>(partials) & 15u) == 0, "head_bwd_dw_bf16: partials must be 16B aligned");
   // dW[c,d] = sum_b G[b,c] X[b,d]: A = G stored [K=b, M=c], B = X stored [K=b, N=d]
-  if (!segs)
-    return tc_gemm(G, ldg, true, X, dim, true, n_classes, dim, n_rows, partials, dim, false, n_splits, as_stream(stream));
-  // G holds the forward kernel's unnormalised probabilities (defer_fixup): finish them in the prologue
-  UML_REQUIRE(labels && tile_ws && segs->nseg >= 1 && segs->nseg <= UML_MAX_SEGMENTS, "head_bwd_dw_fix_bf16: bad arguments");
-  const int64_t tiles = uml_fwd_tiles(n_rows);
-  FixArgs fx;
-  memset(&fx, 0, sizeof(fx));
-  fx.tile_part = tile_ws;
-  fx.fac = tile_ws + tiles * 32;
-  fx.labels = labels;
-  fx.n_tiles = tiles;
-  fx.nseg = segs->nseg;
-  fx.stats = stats;
-  fx.n0 = segs->nseg > 1 ? segs->seg_rows[0] : INT64_MAX;
-  for (int i = 0; i < 2; ++i) {
-    const int j = i < segs->nseg ? i : 0;
-    const double n = static_cast<double>(segs->seg_rows[j] > 0 ? segs->seg_rows[j] : 1);
-    fx.dcoef[i] = static_cast<float>(static_cast<double>(segs->loss_weight[j]) / n);
-    fx.gcoef[i] = fx.dcoef[i] * segs->scale[j];
-    fx.scale_dev[i] = segs->scale_dev[j];
-  }
-  return tc_gemm(G, ldg, true, X, dim, true, n_classes, dim, n_rows, partials, dim, false, n_splits, as_stream(stream), &fx);
+  return tc_gemm(G, ldg, true, X, dim, true, n_classes, dim, n_rows, partials, dim, false, n_splits, as_stream(stream));
 }
 
 }  // extern "C"

@@ -26,9 +26,6 @@ import torch
 from .. import ops
 from .datasets.utils import IndexBatch, local_slice as _local_slice
 
-import os as _os
-
-_FUSE_FIX = _os.environ.get("UML_FUSE_FIX", "0") == "1"  # mirrors csrc/step.cu: fix-up fused into the dW prologue
 BF16_MIN_ROWS = 1024  # below this the step is launch-bound and the exact fp32 path is used
 
 
@@ -319,7 +316,7 @@ class StepEngine:
         return a, k, scale_params
 
     def _kernels_per_step(self, k, bf16):
-        n = ((1 if self.shadow_banks else k) + (3 if _FUSE_FIX else 4) + (0 if self._w16_valid else 1)) if bf16 else 4
+        n = ((1 if self.shadow_banks else k) + 4 + (0 if self._w16_valid else 1)) if bf16 else 4
         # data parallel: the fused peer-memory tail replaces the update launch; over NCCL: + split sum + all-reduce
         return n + (k if self.learnable else 0) + (0 if self.world == 1 or _P2P_FLOATS else 2)
 

@@ -376,28 +376,6 @@ def head_fwd_ce_bf16(X, W_bf16, labels_i32, segs: TcSegments, ws: Optional[HeadW
                                            _ptr(stats) if ws is not None else None, _stream()))
 
 
-def head_fwd_ce_deferred_bf16(X, W_bf16, labels_i32, segs: TcSegments, ws: HeadWorkspace, n_rows: Optional[int] = None):
-    """Forward without the fix-up pass: ws.G <- unnormalised exp(l - m_running), ws.fac <- per-row factors.  Only
-    valid as the producer of head_bwd_dw_fix_bf16."""
-    _need(X, torch.bfloat16, "X")
-    _need(W_bf16, torch.bfloat16, "W")
-    _need(labels_i32, torch.int32, "labels")
-    n_rows = X.shape[0] if n_rows is None else n_rows
-    check(_lib.load().uml_head_fwd_ce_deferred_bf16(X.data_ptr(), n_rows, X.shape[1], W_bf16.data_ptr(), W_bf16.shape[0],
-                                                    labels_i32.data_ptr(), C.byref(segs), ws.G.data_ptr(), ws.ldg,
-                                                    ws.fac.data_ptr(), _stream()))
-
-
-def head_bwd_dw_fix_bf16(ws: HeadWorkspace, X, n_rows, n_classes, partials, n_splits, segs: TcSegments, labels_i32, stats=None):
-    """dW partials from the deferred forward's G: the softmax normalisation and the one-hot term are applied to each
-    operand stage in shared memory inside the GEMM; ``stats`` ([nseg, 4] fp32) receives the per-run statistics."""
-    _need(X, torch.bfloat16, "X")
-    _need(partials, torch.float32, "partials")
-    check(_lib.load().uml_head_bwd_dw_fix_bf16(ws.G.data_ptr(), ws.ldg, X.data_ptr(), n_rows, X.shape[1], n_classes,
-                                               partials.data_ptr(), n_splits, C.byref(segs), labels_i32.data_ptr(),
-                                               ws.fac.data_ptr(), _ptr(stats), _stream()))
-
-
 def tc_dw_splits(n_rows: int, dim: int, n_classes: int) -> int:
     return int(_lib.load().uml_tc_dw_splits(n_rows, dim, n_classes))
 
