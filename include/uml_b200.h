@@ -231,7 +231,12 @@ typedef struct {
   void*         G;                          /* [rows, ldg] workspace: fp32 (precision 0) / bf16 (1)    */
   int64_t       ldg;
   float*        row_loss;  int32_t* row_correct;  float* row_dscale;   /* [rows] workspaces            */
-  uml_seg_stats* stats;                     /* [nseg] per-run results of THIS step                     */
+  uml_seg_stats* stats;                     /* [nseg] per-run results of THIS step, stats[i] for seg[i] on
+                                               both paths; a run with n == 0 gets {0, 0, 0, 0}, and its
+                                               learnable temperature (scale_param[i]) is left untouched -
+                                               no step, no decay, m and v kept - as torch.optim skips a
+                                               parameter without a gradient (data-parallel mode excepted:
+                                               there the zero record still joins the all-reduce)          */
   uint16_t*     X16;  uint16_t* W16;  int32_t* labels32;  float* partials;   /* bf16 path workspaces   */
   float*        tile_ws;                    /* [UML_TILE_WS_FLOATS(rows)], bf16 path                   */
   int32_t       max_splits;  int32_t w16_valid;

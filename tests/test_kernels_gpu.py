@@ -53,23 +53,37 @@ def test_gather_rows(n_bank, dim, n):
     assert torch.equal(lab32[:n].cpu().long(), labels[idx])
 
 
-@pytest.mark.parametrize("n0,n1,dim", [(32, 32, 512), (1000, 517, 768), (0, 77, 768), (77, 0, 3200), (16384, 10996, 768),
-                                        (1, 1, 8), (0, 0, 768)])
-def test_gather2_rows_bf16(n0, n1, dim):
-    """Both runs of a step from bf16 shadow banks in one launch: byte-exact rows, int64 -> int32 labels."""
+@pytest.mark.parametrize("n0,n1,dim,ld,labels", [
+    (32, 32, 512, 512, True), (1000, 517, 768, 768, True), (0, 77, 768, 768, True), (77, 0, 3200, 3200, True),
+    (16384, 10996, 768, 768, True), (1, 1, 8, 8, True), (0, 0, 768, 768, True),
+    (300, 211, 1032, 1032, True),    # 129 16-byte vectors per row: the light kernel's second pass over a row moves one
+    (150, 90, 3200, 3200, True),     # OpenLLaMA width
+    (4000, 1700, 256, 256, True),    # more rows than the light kernel's grid has warps (148 * 4 * 8 = 4736)
+    (500, 300, 768, 776, True),      # ld_out > dim: the padding between rows stays untouched
+    (700, 400, 512, 512, False),     # out_labels = NULL
+])
+@pytest.mark.parametrize("light", [False, True], ids=["tma", "light"])
+def test_gather2_rows_bf16(n0, n1, dim, ld, labels, light):
+    """Both runs of a step from bf16 shadow banks in one launch, through the TMA ring kernel and through the
+    register-copy kernel the training step calls: byte-exact rows, int64 -> int32 labels."""
     g = torch.Generator().manual_seed(n0 * 7 + n1 + dim)
     b0 = torch.randn(3000, dim, generator=g).to(torch.bfloat16)
     b1 = torch.randn(700, dim, generator=g).to(torch.bfloat16)
     l0, l1 = torch.randint(0, 1000, (3000,), generator=g), torch.randint(0, 1000, (700,), generator=g)
     i0, i1 = torch.randint(0, 3000, (n0,), generator=g), torch.randint(0, 700, (n1,), generator=g)
-    out = torch.full((n0 + n1 + 3, dim), 7.0, dtype=torch.bfloat16, device=DEV)
+    buf = torch.full((n0 + n1 + 3, ld), 7.0, dtype=torch.bfloat16, device=DEV)
+    out = buf[:, :dim]
     lab = torch.full((n0 + n1 + 3,), -5, dtype=torch.int32, device=DEV)
     ops.gather2_rows_bf16(b0.to(DEV) if n0 else None, l0.to(DEV) if n0 else None, i0.to(DEV) if n0 else None,
-                          b1.to(DEV) if n1 else None, l1.to(DEV) if n1 else None, i1.to(DEV) if n1 else None, out, lab)
+                          b1.to(DEV) if n1 else None, l1.to(DEV) if n1 else None, i1.to(DEV) if n1 else None, out,
+                          lab if labels else None, light=light)
     want = torch.cat([b0[i0], b1[i1]])
     assert torch.equal(out[:n0 + n1].cpu(), want)
-    assert torch.equal(lab[:n0 + n1].cpu().long(), torch.cat([l0[i0], l1[i1]]))
-    assert bool((out[n0 + n1:] == 7.0).all()) and bool((lab[n0 + n1:] == -5).all())  # nothing written past the end
+    if labels:
+        assert torch.equal(lab[:n0 + n1].cpu().long(), torch.cat([l0[i0], l1[i1]]))
+    assert bool((lab == -5).all()) if not labels else bool((lab[n0 + n1:] == -5).all())
+    assert bool((out[n0 + n1:] == 7.0).all())  # nothing written past the end
+    assert bool((buf[:, dim:] == 7.0).all())   # nor into the padding between rows
 
 
 def test_cast_bf16():

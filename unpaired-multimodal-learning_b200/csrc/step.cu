@@ -386,6 +386,8 @@ static int linear_step_impl(const uml_linear_step_args* a, void* stream, const S
   const cudaEvent_t operand_free = hooks.operand_free;
   bool stats_in_dw = false;  // the forward's per-run statistics are reduced inside the dW kernel
   UML_REQUIRE(a != nullptr, "linear_step: null args");
+  // bf16 path: the kernels write one record per run WITH rows, in order, starting here (stats[i] belongs to seg[i])
+  uml_seg_stats* live_stats = a->stats;
   UML_REQUIRE(a->nseg >= 1 && a->nseg <= UML_MAX_SEGMENTS, "linear_step: 1..2 segments");
   UML_REQUIRE(a->W && a->G && a->row_loss && a->row_correct && a->stats, "linear_step: null buffers");
   const int64_t n0 = a->seg[0].n, n1 = a->nseg > 1 ? a->seg[1].n : 0, total = n0 + n1;
@@ -393,6 +395,7 @@ static int linear_step_impl(const uml_linear_step_args* a, void* stream, const S
   UML_REQUIRE(!dp || a->dW_out, "linear_step: data-parallel mode needs dW_out");
   const bool fused = a->dW_out == nullptr;
   int rc;
+  bool w_done = false;  // the fp32 fused kernel took the whole step of W: only the temperatures are left
 
   if (a->precision == 0) {
     // ------------------------------------------------------------------ fp32 exact path (one fused launch, else 3 + 1)
@@ -407,13 +410,15 @@ static int linear_step_impl(const uml_linear_step_args* a, void* stream, const S
         rec(a->ev[3], stream);
         rec(a->ev[4], stream);
         rec(a->ev[5], stream);
-        return 0;
+        w_done = true;
       }
     }
-    rc = uml_head_fwd_ce_f32(a->seg, a->nseg, a->dim, a->W, a->n_classes, static_cast<float*>(a->G), a->ldg,
-                             a->row_loss, a->row_correct, a->row_dscale, a->stats, a->g_capacity_rows, stream);
-    if (rc) return rc;
-    rec(a->ev[3], stream);
+    if (!w_done) {
+      rc = uml_head_fwd_ce_f32(a->seg, a->nseg, a->dim, a->W, a->n_classes, static_cast<float*>(a->G), a->ldg,
+                               a->row_loss, a->row_correct, a->row_dscale, a->stats, a->g_capacity_rows, stream);
+      if (rc) return rc;
+      rec(a->ev[3], stream);
+    }
   } else {
     // ------------------------------------------------------------------ bf16 tensor-core path
     UML_REQUIRE(a->X16 && a->W16 && a->labels32 && a->partials && a->tile_ws && a->max_splits >= 1,
@@ -434,7 +439,11 @@ static int linear_step_impl(const uml_linear_step_args* a, void* stream, const S
     }
     for (int i = 0; i < a->nseg; ++i) {
       const uml_segment& s = a->seg[i];
-      if (s.n == 0) continue;
+      if (s.n == 0) {  // the kernels see only the runs with rows: an empty run's record is zeroed here
+        UML_CUDA(cudaMemsetAsync(&a->stats[i], 0, sizeof(uml_seg_stats), as_stream(stream)));
+        continue;
+      }
+      if (ts.nseg == 0) live_stats = &a->stats[i];
       if (!shadow) {
         const float* rows = static_cast<const float*>(s.rows);
         UML_REQUIRE(s.ld == a->dim, "linear_step: bf16 path needs dense bank rows (ld == dim)");
@@ -469,7 +478,7 @@ static int linear_step_impl(const uml_linear_step_args* a, void* stream, const S
       stats_in_dw = uml_fwd_x_eligible(total, a->n_classes) && !a->scale_param[0] && !a->scale_param[1];
       rc = uml_head_fwd_ce_bf16_ev(a->X16, total, a->dim, a->W16, a->n_classes, a->labels32, &ts,
                                    static_cast<uint16_t*>(a->G), a->ldg, nullptr, nullptr, nullptr, nullptr, a->tile_ws,
-                                   stats_in_dw ? nullptr : a->stats, a->ev[3], stream, hooks.after_fwd_kernel);
+                                   stats_in_dw ? nullptr : live_stats, a->ev[3], stream, hooks.after_fwd_kernel);
       if (rc) return rc;
     }
     if (hooks.mid) {
@@ -478,9 +487,11 @@ static int linear_step_impl(const uml_linear_step_args* a, void* stream, const S
     }
   }
 
-  // learnable temperatures: scalar Adam(W) steps fed straight from the stats record on the device
+  // learnable temperatures: scalar Adam(W) steps fed straight from the stats record on the device.  A run without rows
+  // gives its temperature no gradient, and it is skipped as torch.optim skips a parameter whose .grad is None; in
+  // data-parallel mode this rank's empty run still takes part in the all-reduce (its record is zero).
   for (int i = 0; i < a->nseg; ++i) {
-    if (!a->scale_param[i]) continue;
+    if (!a->scale_param[i] || (!dp && a->seg[i].n == 0)) continue;
     float* g = &a->stats[i].dscale;
     if (dp) {  // the temperature gradient is a sum over the global batch as well
       rc = uml_dp_allreduce_f32(g, 1, stream);
@@ -497,7 +508,7 @@ static int linear_step_impl(const uml_linear_step_args* a, void* stream, const S
   }
 
   const int64_t np_all = static_cast<int64_t>(a->n_classes) * a->dim;
-  if (total == 0 && !dp) return 0;
+  if (w_done || (total == 0 && !dp)) return 0;
   if (total == 0) {  // a rank without rows still takes part in the all-reduce, contributing zeros
     UML_CUDA(cudaMemsetAsync(dp_local_sum_target(a, np_all), 0, np_all * sizeof(float), as_stream(stream)));
     return dp_reduce_and_update(a, np_all, stream);
@@ -522,7 +533,7 @@ static int linear_step_impl(const uml_linear_step_args* a, void* stream, const S
     int nseg_live = 0;
     for (int i = 0; i < a->nseg; ++i) nseg_live += a->seg[i].n > 0 ? 1 : 0;
     rc = uml_head_bwd_dw_stats_bf16(static_cast<const uint16_t*>(a->G), a->ldg, a->X16, total, a->dim, a->n_classes,
-                                    a->partials, splits, part, entries, nseg_live, a->stats, stream);
+                                    a->partials, splits, part, entries, nseg_live, live_stats, stream);
   } else {
     rc = uml_head_bwd_dw_bf16(static_cast<const uint16_t*>(a->G), a->ldg, a->X16, total, a->dim, a->n_classes, a->partials,
                               splits, stream);

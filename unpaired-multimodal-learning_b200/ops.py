@@ -107,9 +107,10 @@ def gather_rows_labels(bank, labels, idx, out16, out_labels32):
                                                   _stream()))
 
 
-def gather2_rows_bf16(bank0, labels0, idx0, bank1, labels1, idx1, out16, out_labels32=None):
+def gather2_rows_bf16(bank0, labels0, idx0, bank1, labels1, idx1, out16, out_labels32=None, light=False):
     """Both runs of a step copied from bf16 shadow banks into one operand (rows of run 0, then run 1) with their
-    labels, in one launch of the TMA copy kernel.  Either run may be None."""
+    labels, in one launch of the TMA copy kernel (``light``: of the register-copy kernel the training step uses).
+    Either run may be None."""
     d = out16.shape[1]
     args = []
     for bank, labels, idx, nm in ((bank0, labels0, idx0, "0"), (bank1, labels1, idx1, "1")):
@@ -126,7 +127,8 @@ def gather2_rows_bf16(bank0, labels0, idx0, bank1, labels1, idx1, out16, out_lab
     _need(out16, torch.bfloat16, "out16", contiguous=False)
     if args[3] + args[7] > out16.shape[0]:
         raise ValueError("gather2_rows_bf16: output too small")
-    check(_lib.load().uml_gather2_rows_bf16(*args, d, out16.data_ptr(), out16.stride(0), _ptr(out_labels32), _stream()))
+    fn = _lib.load().uml_gather2_rows_bf16_light if light else _lib.load().uml_gather2_rows_bf16
+    check(fn(*args, d, out16.data_ptr(), out16.stride(0), _ptr(out_labels32), _stream()))
     return out16
 
 
