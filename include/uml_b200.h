@@ -394,8 +394,9 @@ typedef struct {
  * the last batch of an epoch is short) with learning rates lr[i*n_heads + k] (host array).                      */
 int uml_sweep_run(const uml_sweep_args* args /*host*/, int32_t n_steps, const int64_t* rows /*host*/,
                   const float* lr /*host*/, void* stream);
-/* kernels launched by uml_sweep_run and uml_sweep_adapter_run in this process so far (modulo 2^31): three per step when
- * the tensor-core dW launch carries the statistics warp, four otherwise; see uml_sweep_adapter_run for its count */
+/* kernels launched by uml_sweep_run, uml_sweep_adapter_run and uml_sweep_run_diag in this process so far (modulo 2^31):
+ * three per step when the tensor-core dW launch carries the statistics warp, four otherwise; see uml_sweep_adapter_run
+ * for its count; uml_sweep_run_diag adds two per step */
 int uml_sweep_launch_count(void);
 
 /* The same lock-step sweep for UML heads with an image adapter and / or learnable temperatures (head.py:39-98: the
@@ -427,6 +428,26 @@ typedef struct {
 } uml_sweep_adapter_args;
 int uml_sweep_adapter_run(const uml_sweep_args* args /*host*/, const uml_sweep_adapter_args* adapter /*host*/,
                           int32_t n_steps, const int64_t* rows /*host*/, const float* lr /*host*/, void* stream);
+
+/* uml_sweep_run (adapter == NULL) or uml_sweep_adapter_run with the reference's per-step gradient probes
+ * (finetune.py:190-206, a-13): for every running head and step, at the step's weights before its update,
+ *   A = d image_loss / d W_k,  B = d text_loss / d W_k  (plain mean cross-entropies: B carries no alpha),
+ * reduced on the device to out[step][head] = {sum A.B, sum A^2, sum B^2, #(sign A == sign B)} (torch.sign: 0 equals
+ * only 0) - two more launches per step (a tensor-core pass over G and the step's rows, a fixed-order finish), no
+ * [C, D] gradient in HBM, no host synchronisation.  They only read, so the training results are bit-identical to the
+ * same call without diagnostics.  Contract, checked before anything touches the device: dim % 4 == 0, 16-byte aligned
+ * slabs, G, banks and Z; alpha > 0 for every running head when there is a text bank; scratch_floats >=
+ * uml_sweep_diag_scratch_floats(n_heads, dim, n_classes).                                                        */
+typedef struct {
+  float*   out;             /* [n_steps][n_heads][4] (rows of stopped heads are not written)                      */
+  float*   scratch;         /* per-unit partial sums                                                               */
+  int64_t  scratch_floats;
+  void*    ev[2];           /* optional cudaEvent_t pair around the diagnostics launches of the LAST step         */
+} uml_sweep_diag;
+int64_t uml_sweep_diag_scratch_floats(int32_t n_heads, int32_t dim, int32_t n_classes); /* a COUNT, not a status */
+int uml_sweep_run_diag(const uml_sweep_args* args /*host*/, const uml_sweep_adapter_args* adapter /*host, NULL: linear heads*/,
+                       const uml_sweep_diag* diag /*host*/, int32_t n_steps, const int64_t* rows /*host*/,
+                       const float* lr /*host*/, void* stream);
 
 /* ---- sampler: the epoch permutation on the host, bit-exact with torch.randperm(n, generator=
  * torch.Generator().manual_seed(seed)) on the CPU - what RandomSampler draws once per epoch for the

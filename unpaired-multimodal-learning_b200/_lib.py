@@ -76,6 +76,11 @@ class SweepAdapterArgs(C.Structure):
                 ("scale_v", c_vp), ("row_dscale", c_vp), ("ev", c_vp * 10)]
 
 
+class SweepDiag(C.Structure):
+    """uml_sweep_diag"""
+    _fields_ = [("out", c_vp), ("scratch", c_vp), ("scratch_floats", c_i64), ("ev", c_vp * 2)]
+
+
 # name -> argtypes; every function returns int except uml_last_error
 PROTOTYPES = {
     "uml_abi_version": [],
@@ -144,6 +149,8 @@ PROTOTYPES = {
     "uml_gauss_eval": [c_vp, c_i32, c_i32, c_i32, c_vp, c_vp, c_i64, c_vp, c_vp, c_vp],
     "uml_sweep_run": [C.POINTER(SweepArgs), c_i32, c_vp, c_vp, c_vp],
     "uml_sweep_adapter_run": [C.POINTER(SweepArgs), C.POINTER(SweepAdapterArgs), c_i32, c_vp, c_vp, c_vp],
+    "uml_sweep_diag_scratch_floats": [c_i32, c_i32, c_i32],
+    "uml_sweep_run_diag": [C.POINTER(SweepArgs), C.POINTER(SweepAdapterArgs), C.POINTER(SweepDiag), c_i32, c_vp, c_vp, c_vp],
     "uml_randperm_i64": [C.c_uint64, c_i64, c_vp],
     "uml_randperm_begin": [c_vp, C.c_uint64, c_i64, c_vp],
     "uml_randperm_advance": [c_vp, c_i64],
@@ -200,6 +207,7 @@ def load() -> C.CDLL:
         fn.argtypes = args
         if name in KERNELS_PER_CALL:
             setattr(lib, name, _Counted(fn, KERNELS_PER_CALL[name]))
+    lib.uml_sweep_diag_scratch_floats.restype = c_i64
     if lib.uml_abi_version() != 1:
         raise UmlLibraryError("libuml_b200.so ABI version mismatch")
     _lib = lib

@@ -997,6 +997,56 @@ __device__ __forceinline__ float lds_f32(uint32_t a) {
 }
 __device__ __forceinline__ void sts_f32(uint32_t a, float v) { asm volatile("st.shared.f32 [%0], %1;" ::"r"(a), "f"(v) : "memory"); }
 
+// Operand staging of the X^T . G contractions (the dW kernel below and sweep_grad_diag_tc_kernel): 64 rows are the K
+// dimension, both tiles MN-major in SWIZZLE_128B_BASE32B boxes of 32 columns x 64 rows (8 KB).  Feature tile: rowp[64]
+// rows x 128 dims from d0 (four boxes, a warp per row); G tile: `rows` rows x 64 classes from c0 (two boxes).  Missing
+// rows and dims are zero-filled.  The tf32 split writes hi in place and lo one tile further (X: +32 KB, G: +16 KB).
+template <int kWarps>
+__device__ __forceinline__ void x_tile_issue(unsigned char* xs, const float* const* rowp, int d0, int D, const void* dummy) {
+  const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
+#pragma unroll
+  for (int i = 0; i < 64 / kWarps; ++i) {
+    const int row = warp + kWarps * i, box = lane >> 3;
+    const float* rp = rowp[row];
+    const bool ok = rp != nullptr && d0 + lane * 4 < D;
+    cp_async16(xs + box * 8192 + sw128_b32(row, lane & 7), ok ? rp + d0 + lane * 4 : dummy, ok);
+  }
+}
+template <int kWarps>
+__device__ __forceinline__ void x_tile_split(unsigned char* xs) {  // a thread splits its own chunks (visible to it after the wait)
+  const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
+#pragma unroll
+  for (int i = 0; i < 64 / kWarps; ++i) {
+    const int row = warp + kWarps * i, box = lane >> 3;
+    unsigned char* a = xs + box * 8192 + sw128_b32(row, lane & 7);
+    float4 hi, lo;
+    split_tf32(*reinterpret_cast<const float4*>(a), hi, lo);
+    *reinterpret_cast<float4*>(a) = hi;
+    *reinterpret_cast<float4*>(a + 32768) = lo;
+  }
+}
+template <int kNT>
+__device__ __forceinline__ void g_tile_issue(unsigned char* gs, const float* G, int64_t ldg, int64_t rows, int c0, int C) {
+#pragma unroll
+  for (int i = 0; i < 1024 / kNT; ++i) {
+    const int f = threadIdx.x + kNT * i, row = f >> 4, chg = f & 15, box = chg >> 3;
+    const bool ok = row < rows && c0 + chg * 4 < C;  // ldg % 4 == 0 and ldg >= C: the 16 bytes stay inside the row
+    cp_async16(gs + box * 8192 + sw128_b32(row, chg & 7), ok ? G + row * ldg + c0 + chg * 4 : G, ok);
+  }
+}
+template <int kNT>
+__device__ __forceinline__ void g_tile_split(unsigned char* gs) {
+#pragma unroll
+  for (int i = 0; i < 1024 / kNT; ++i) {
+    const int f = threadIdx.x + kNT * i, row = f >> 4, chg = f & 15, box = chg >> 3;
+    unsigned char* b = gs + box * 8192 + sw128_b32(row, chg & 7);
+    float4 hi, lo;
+    split_tf32(*reinterpret_cast<const float4*>(b), hi, lo);
+    *reinterpret_cast<float4*>(b) = hi;
+    *reinterpret_cast<float4*>(b + 16384) = lo;
+  }
+}
+
 template <int kNT>
 __global__ void __launch_bounds__(kNT + 64, 1)
     sweep_dw_update_tc_kernel(const __grid_constant__ SweepDev p, const __grid_constant__ CUtensorMap tm_w,
@@ -1141,49 +1191,10 @@ __global__ void __launch_bounds__(kNT + 64, 1)
     // ------------------------------------------------ update warps: operand staging, MMA issue, read-back --------------
     auto sync_update_warps = [&]() { asm volatile("bar.sync 1, %0;" ::"n"(kNT) : "memory"); };
     // feature tile: 64 rows x 32 chunks (a warp per row); G tile: 64 rows x 16 chunks
-    auto x_issue = [&](int d0) {
-#pragma unroll
-      for (int i = 0; i < kR / kWarps; ++i) {
-        const int row = warp + kWarps * i, box = lane >> 3;
-        const float* rp = rowp[row];
-        const bool ok = rp != nullptr && d0 + lane * 4 < D;
-        cp_async16(smem + box * 8192 + sw128_b32(row, lane & 7), ok ? rp + d0 + lane * 4 : p.G, ok);
-      }
-    };
-    auto x_split = [&]() {  // a thread splits its own chunks (its cp.async writes are visible to it after the wait)
-#pragma unroll
-      for (int i = 0; i < kR / kWarps; ++i) {
-        const int row = warp + kWarps * i, box = lane >> 3;
-        unsigned char* a = smem + box * 8192 + sw128_b32(row, lane & 7);
-        float4 hi, lo;
-        split_tf32(*reinterpret_cast<const float4*>(a), hi, lo);
-        *reinterpret_cast<float4*>(a) = hi;
-        *reinterpret_cast<float4*>(a + 32768) = lo;
-      }
-    };
-    auto g_issue = [&](const DwUnit& un) {
-      unsigned char* gb = smem + 65536;
-      const float* __restrict__ G = p.G + un.head * p.g_stride;
-      const int c0 = un.ct * BN;
-#pragma unroll
-      for (int i = 0; i < 1024 / kNT; ++i) {
-        const int f = t + kNT * i, row = f >> 4, chg = f & 15, box = chg >> 3;
-        const bool ok = row < R && c0 + chg * 4 < C;  // ldg % 4 == 0 and ldg >= C: the 16 bytes stay inside the row
-        cp_async16(gb + box * 8192 + sw128_b32(row, chg & 7), ok ? G + row * p.ldg + c0 + chg * 4 : G, ok);
-      }
-    };
-    auto g_split = [&]() {
-      unsigned char* gb = smem + 65536;
-#pragma unroll
-      for (int i = 0; i < 1024 / kNT; ++i) {
-        const int f = t + kNT * i, row = f >> 4, chg = f & 15, box = chg >> 3;
-        unsigned char* b = gb + box * 8192 + sw128_b32(row, chg & 7);
-        float4 hi, lo;
-        split_tf32(*reinterpret_cast<const float4*>(b), hi, lo);
-        *reinterpret_cast<float4*>(b) = hi;
-        *reinterpret_cast<float4*>(b + 16384) = lo;
-      }
-    };
+    auto x_issue = [&](int d0) { x_tile_issue<kWarps>(smem, rowp, d0, D, p.G); };
+    auto x_split = [&]() { x_tile_split<kWarps>(smem); };
+    auto g_issue = [&](const DwUnit& un) { g_tile_issue<kNT>(smem + 65536, p.G + un.head * p.g_stride, p.ldg, R, un.ct * BN, C); };
+    auto g_split = [&]() { g_tile_split<kNT>(smem + 65536); };
     constexpr uint32_t idesc = make_idesc_tf32(BM, BN, 1, 1);
     const uint32_t a_hi = smem_u32(smem), a_lo = a_hi + 32768, b_hi = a_hi + 65536, b_lo = b_hi + 16384;
     auto mma_unit = [&](int n) {  // one thread; accumulators of local unit n in TMEM region n & 1
@@ -1423,6 +1434,204 @@ __global__ void __launch_bounds__(256, 2)
   if (warp == 1) tmem_dealloc(tmem_base, 64);
 }
 
+// 6t. gradient diagnostics (the reference's per-step probes, finetune.py:190-206): per running head the image-loss and
+//     text-loss gradients of the head weights, A = X_img^T G[image rows] and B = X_txt^T G[text rows] (both [D, C]
+//     transposed), reduced without being stored to {sum A.B, sum A^2, sum B^2, #(sign A == sign B)}.
+//     Persistent over the dW kernel's (head, 128-dim tile, 64-class tile) units with its operand staging and 3xTF32 MMAs;
+//     the rows are the K dimension, 64 per k-tile, accumulated in TMEM - any step size.  Two accumulators per unit
+//     (columns [0, 64) image, [64, 128) text): the G tile is split twice, each copy with the other modality's rows zero,
+//     so a k-step of 8 rows that crosses n0 adds only its own rows to each.  A unit's sums go to its own slot of `part`
+//     ([K][dim tiles][class tiles][4], by head index), finished in a fixed order by sweep_grad_diag_finish_kernel: no
+//     float atomics, so a head's figures depend neither on its slot nor on its neighbours.  Reads G and rows only.
+constexpr int kTcDiagSmemBytes = 128 * 1024 + 1024 + 64;  // X hi | X lo (32 KB each) | G image hi | lo | G text hi | lo (16 KB each)
+
+__global__ void __launch_bounds__(256, 1) sweep_grad_diag_tc_kernel(const __grid_constant__ SweepDev p, float* __restrict__ part) {
+  constexpr int BM = 128, BN = 64, kR = 64, kNT = 256, kWarps = kNT / 32;
+  const int D = p.dim, C = p.n_classes;
+  const int n_dt = (D + BM - 1) / BM, n_ct = (C + BN - 1) / BN, per_head = n_dt * n_ct;
+  const int n_units = __popc(p.active_mask) * per_head;
+  const int u_lo = static_cast<int>(static_cast<int64_t>(n_units) * blockIdx.x / gridDim.x);
+  const int u_hi = static_cast<int>(static_cast<int64_t>(n_units) * (blockIdx.x + 1) / gridDim.x);
+  if (u_lo >= u_hi) return;
+  extern __shared__ unsigned char tc_smem_raw[];
+  unsigned char* smem = reinterpret_cast<unsigned char*>((reinterpret_cast<uintptr_t>(tc_smem_raw) + 1023) & ~uintptr_t(1023));
+  unsigned char* gs = smem + 65536;
+  uint64_t* mma_bar = reinterpret_cast<uint64_t*>(smem + 128 * 1024);
+  uint32_t* tmem_slot = reinterpret_cast<uint32_t*>(mma_bar + 1);
+  __shared__ const float* rowp[kR];
+  __shared__ float red[kWarps][3];
+  __shared__ int red_n[kWarps];
+  const int t = threadIdx.x, warp = t >> 5, lane = t & 31;
+  const int64_t n0 = p.n0, R = p.n0 + p.n1;
+  const bool has_img = p.n0 > 0, has_txt = p.n1 > 0;
+  if (t == 0) {
+    mbar_init(mma_bar, 1);
+    fence_barrier_init();
+  }
+  if (warp == 1) tmem_alloc(tmem_slot, 128);
+  tc_fence_before();
+  __syncthreads();
+  tc_fence_after();
+  const uint32_t tmem_base = *tmem_slot;
+  constexpr uint32_t idesc = make_idesc_tf32(BM, BN, 1, 1);
+  const uint32_t a_hi = smem_u32(smem), a_lo = a_hi + 32768, gi_hi = smem_u32(gs), gi_lo = gi_hi + 16384,
+                 gt_hi = gi_hi + 32768, gt_lo = gi_hi + 49152;
+
+  int head, dt, ct;
+  {
+    const int a = u_lo / per_head, r = u_lo - a * per_head;
+    head = __fns(p.active_mask, 0, a + 1);  // the a-th running head
+    dt = r / n_ct;
+    ct = r - dt * n_ct;
+  }
+  int x_head = -1, x_dt = -1;  // the feature tile in shared memory (steps of at most 64 rows keep it across class tiles)
+  uint32_t phase = 0;
+#pragma unroll 1
+  for (int u = u_lo; u < u_hi; ++u) {
+    const float* __restrict__ G = p.G + head * p.g_stride;
+    const int d0 = dt * BM, c0 = ct * BN;
+    uint32_t acc_img = 0, acc_txt = 0;  // MMAs issued into each accumulator (thread 0)
+#pragma unroll 1
+    for (int64_t r0 = 0; r0 < R; r0 += kR) {
+      const int64_t rows = min(static_cast<int64_t>(kR), R - r0);
+      const bool new_x = R > kR || head != x_head || dt != x_dt;
+      if (new_x) {
+        if (t < kR) rowp[t] = (t < rows) ? row_ptr(p, head, r0 + t) : nullptr;
+        __syncthreads();
+        x_tile_issue<kWarps>(smem, rowp, d0, D, G);
+        x_head = head;
+        x_dt = dt;
+      }
+      g_tile_issue<kNT>(gs, G + r0 * p.ldg, p.ldg, rows, c0, C);
+      cp_async_commit();
+      cp_async_wait<0>();
+      if (new_x) x_tile_split<kWarps>(smem);
+#pragma unroll
+      for (int i = 0; i < 1024 / kNT; ++i) {  // G split twice: image rows only | text rows only
+        const int f = t + kNT * i, row = f >> 4, chg = f & 15, box = chg >> 3;
+        unsigned char* b = gs + box * 8192 + sw128_b32(row, chg & 7);
+        float4 hi, lo;
+        split_tf32(*reinterpret_cast<const float4*>(b), hi, lo);
+        const float4 z = make_float4(0.f, 0.f, 0.f, 0.f);
+        const bool img = r0 + row < n0;
+        *reinterpret_cast<float4*>(b) = img ? hi : z;
+        *reinterpret_cast<float4*>(b + 16384) = img ? lo : z;
+        *reinterpret_cast<float4*>(b + 32768) = img ? z : hi;
+        *reinterpret_cast<float4*>(b + 49152) = img ? z : lo;
+      }
+      fence_proxy_async();  // generic-proxy stores -> the tensor core's async-proxy reads
+      tc_fence_before();    // (the previous unit's TMEM read-back is complete)
+      __syncthreads();
+      if (t == 0) {
+        tc_fence_after();
+#pragma unroll 1
+        for (int k = 0; k < kR / 8 && r0 + 8 * k < R; ++k) {  // 8 rows = two 4-row atoms (SBO 512 B); next 32 columns 8 KB further
+          const int64_t rb = r0 + 8 * k;
+          const uint64_t dah = make_smem_desc(a_hi + k * 1024, 8192, 512, kLayoutSw128Base32);
+          const uint64_t dal = make_smem_desc(a_lo + k * 1024, 8192, 512, kLayoutSw128Base32);
+          if (rb < n0) {
+            const uint64_t dbh = make_smem_desc(gi_hi + k * 1024, 8192, 512, kLayoutSw128Base32);
+            const uint64_t dbl = make_smem_desc(gi_lo + k * 1024, 8192, 512, kLayoutSw128Base32);
+            umma_tf32(tmem_base, dal, dbh, idesc, acc_img != 0);
+            umma_tf32(tmem_base, dah, dbl, idesc, 1);
+            umma_tf32(tmem_base, dah, dbh, idesc, 1);
+            ++acc_img;
+          }
+          if (has_txt && rb + 8 > n0) {
+            const uint64_t dbh = make_smem_desc(gt_hi + k * 1024, 8192, 512, kLayoutSw128Base32);
+            const uint64_t dbl = make_smem_desc(gt_lo + k * 1024, 8192, 512, kLayoutSw128Base32);
+            umma_tf32(tmem_base + BN, dal, dbh, idesc, acc_txt != 0);
+            umma_tf32(tmem_base + BN, dah, dbl, idesc, 1);
+            umma_tf32(tmem_base + BN, dah, dbh, idesc, 1);
+            ++acc_txt;
+          }
+        }
+        umma_commit(mma_bar);
+      }
+      mbar_wait_or_trap(mma_bar, phase);  // the MMAs have read the tiles and written TMEM
+      phase ^= 1u;
+      tc_fence_after();
+    }
+
+    // read-back: TMEM lane = dim, column = class; warp w reads lane quadrant w % 4, classes 32 (w / 4) ..
+    const int q = warp & 3, h = warp >> 2;
+    uint32_t va[32], vb[32];
+    tmem_ld32(tmem_base + (static_cast<uint32_t>(q * 32) << 16) + h * 32, va);
+    tmem_ld32(tmem_base + (static_cast<uint32_t>(q * 32) << 16) + BN + h * 32, vb);
+    tmem_ld_wait();
+    float dot = 0.f, aa = 0.f, bb = 0.f;
+    int agree = 0;
+    if (d0 + q * 32 + lane < D) {
+#pragma unroll
+      for (int i = 0; i < 32; ++i) {
+        if (c0 + h * 32 + i >= C) break;
+        const float x = has_img ? __uint_as_float(va[i]) : 0.f, y = has_txt ? __uint_as_float(vb[i]) : 0.f;
+        dot = fmaf(x, y, dot);
+        aa = fmaf(x, x, aa);
+        bb = fmaf(y, y, bb);
+        agree += ((x > 0.f) - (x < 0.f)) == ((y > 0.f) - (y < 0.f));  // torch.sign: 0 only equals 0
+      }
+    }
+    dot = warp_sum(dot);
+    aa = warp_sum(aa);
+    bb = warp_sum(bb);
+    agree = warp_sum_i(agree);
+    if (lane == 0) {
+      red[warp][0] = dot;
+      red[warp][1] = aa;
+      red[warp][2] = bb;
+      red_n[warp] = agree;
+    }
+    __syncthreads();
+    if (t == 0) {
+      float s0 = 0.f, s1 = 0.f, s2 = 0.f;
+      int n = 0;
+      for (int w = 0; w < kWarps; ++w) {
+        s0 += red[w][0];
+        s1 += red[w][1];
+        s2 += red[w][2];
+        n += red_n[w];
+      }
+      float* o = part + (static_cast<int64_t>(head) * per_head + dt * n_ct + ct) * 4;
+      o[0] = s0;
+      o[1] = s1;
+      o[2] = s2;
+      o[3] = static_cast<float>(n);  // at most 128 x 64: exact
+    }
+    if (++ct == n_ct) {
+      ct = 0;
+      if (++dt == n_dt) {
+        dt = 0;
+        if (u + 1 < u_hi) head = __ffs(p.active_mask >> (head + 1)) + head;  // the next running head
+      }
+    }
+  }
+  tc_fence_before();
+  __syncthreads();
+  if (warp == 1) tmem_dealloc(tmem_base, 128);
+}
+
+// out[head] = the unit sums of each running head in unit order (double), the text side divided by alpha / alpha^2 (G's
+// text rows carry the loss weight; the figures describe the plain text loss)        grid (K), 32 threads
+__global__ void __launch_bounds__(32) sweep_grad_diag_finish_kernel(const __grid_constant__ SweepDev p, const float* __restrict__ part,
+                                                                    int units_per_head, float* __restrict__ out) {
+  const int head = blockIdx.x, j = threadIdx.x;
+  if (!head_active(p, head) || j >= 4) return;
+  const float* ph = part + static_cast<int64_t>(head) * units_per_head * 4;
+  double s = 0.0;
+  if (j == 3) {
+    long long n = 0;
+    for (int u = 0; u < units_per_head; ++u) n += static_cast<long long>(ph[4 * u + 3]);
+    s = static_cast<double>(n);
+  } else {
+    for (int u = 0; u < units_per_head; ++u) s += static_cast<double>(ph[4 * u + j]);
+    const double al = p.alpha[head];  // > 0 whenever there are text rows (launcher)
+    if (j == 0 && p.n1 > 0) s /= al;
+    if (j == 2 && p.n1 > 0) s /= al * al;
+  }
+  out[4 * head + j] = static_cast<float>(s);
+}
+
 // ---------------------------------------------------------------------------------------------------------------
 // 4. per-head, per-run {mean loss, hits, rows} in a fixed summation order   grid (2, K)
 // ---------------------------------------------------------------------------------------------------------------
@@ -1459,7 +1668,36 @@ extern "C" {
 
 int uml_sweep_launch_count(void) { return static_cast<int>(g_sweep_launches & 0x7fffffff); }
 
-int uml_sweep_run(const uml_sweep_args* a, int32_t n_steps, const int64_t* rows, const float* lr, void* stream) {
+static bool aligned16(const void* ptr) { return (reinterpret_cast<uintptr_t>(ptr) & 15) == 0; }
+
+int64_t uml_sweep_diag_scratch_floats(int32_t n_heads, int32_t dim, int32_t n_classes) {
+  if (n_heads < 1 || dim < 1 || n_classes < 1) return 0;
+  return static_cast<int64_t>(n_heads) * ((dim + 127) / 128) * ((n_classes + 63) / 64) * 4;
+}
+
+// Step i's gradient diagnostics (uml_sweep_run_diag): enqueued after the step's last update launch and before the next
+// step's first launch, so G and the rows (bank rows or Z) are still the step's own.
+static int launch_grad_diag(const uml::sweep::SweepDev& p, const uml_sweep_diag* dg, int K, int i, bool timed, cudaStream_t st) {
+  using namespace uml;
+  using namespace uml::sweep;
+  static const cudaError_t attr =
+      cudaFuncSetAttribute(sweep_grad_diag_tc_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, kTcDiagSmemBytes);
+  UML_CUDA(attr);
+  const int per_head = ((p.dim + 127) / 128) * ((p.n_classes + 63) / 64);
+  const int64_t units = static_cast<int64_t>(__builtin_popcount(p.active_mask)) * per_head;
+  const unsigned g = static_cast<unsigned>(std::min<int64_t>(units, sm_count()));
+  if (timed && dg->ev[0]) UML_CUDA(cudaEventRecord(static_cast<cudaEvent_t>(dg->ev[0]), st));
+  sweep_grad_diag_tc_kernel<<<g, 256, kTcDiagSmemBytes, st>>>(p, dg->scratch);
+  UML_CUDA(cudaGetLastError());
+  sweep_grad_diag_finish_kernel<<<K, 32, 0, st>>>(p, dg->scratch, per_head, dg->out + static_cast<int64_t>(i) * K * 4);
+  UML_CUDA(cudaGetLastError());
+  g_sweep_launches += 2;
+  if (timed && dg->ev[1]) UML_CUDA(cudaEventRecord(static_cast<cudaEvent_t>(dg->ev[1]), st));
+  return 0;
+}
+
+static int sweep_run_impl(const uml_sweep_args* a, const uml_sweep_diag* dg, int32_t n_steps, const int64_t* rows,
+                          const float* lr, void* stream) {
   using namespace uml;
   using namespace uml::sweep;
   UML_REQUIRE(a && rows && lr && n_steps >= 0, "sweep_run: null argument");
@@ -1650,16 +1888,19 @@ int uml_sweep_run(const uml_sweep_args* a, int32_t n_steps, const int64_t* rows,
       ++g_sweep_launches;
     }
     if (mark(7)) return 1;
+    if (dg && launch_grad_diag(p, dg, K, i, timed, st)) return 1;
     pos[0] += n0;
     pos[1] += n1;
   }
   return 0;
 }
 
-static bool aligned16(const void* ptr) { return (reinterpret_cast<uintptr_t>(ptr) & 15) == 0; }
+int uml_sweep_run(const uml_sweep_args* a, int32_t n_steps, const int64_t* rows, const float* lr, void* stream) {
+  return sweep_run_impl(a, nullptr, n_steps, rows, lr, stream);
+}
 
-int uml_sweep_adapter_run(const uml_sweep_args* a, const uml_sweep_adapter_args* ad, int32_t n_steps, const int64_t* rows,
-                          const float* lr, void* stream) {
+static int sweep_adapter_run_impl(const uml_sweep_args* a, const uml_sweep_adapter_args* ad, const uml_sweep_diag* dg,
+                                  int32_t n_steps, const int64_t* rows, const float* lr, void* stream) {
   using namespace uml;
   using namespace uml::sweep;
   UML_REQUIRE(a && ad && rows && lr && n_steps >= 0, "sweep_adapter_run: null argument");
@@ -1863,10 +2104,42 @@ int uml_sweep_adapter_run(const uml_sweep_args* a, const uml_sweep_adapter_args*
       ++g_sweep_launches;
     }
     if (mark(9)) return 1;
+    if (dg && launch_grad_diag(p, dg, K, i, timed, st)) return 1;  // (Z is overwritten by the next step's first launch)
     pos[0] += n0;
     pos[1] += n1;
   }
   return 0;
+}
+
+int uml_sweep_adapter_run(const uml_sweep_args* a, const uml_sweep_adapter_args* ad, int32_t n_steps, const int64_t* rows,
+                          const float* lr, void* stream) {
+  return sweep_adapter_run_impl(a, ad, nullptr, n_steps, rows, lr, stream);
+}
+
+int uml_sweep_run_diag(const uml_sweep_args* a, const uml_sweep_adapter_args* ad, const uml_sweep_diag* dg, int32_t n_steps,
+                       const int64_t* rows, const float* lr, void* stream) {
+  using namespace uml::sweep;
+  UML_REQUIRE(a && dg && rows && lr && n_steps >= 0, "sweep_run_diag: null argument");
+  const int K = a->n_heads;
+  UML_REQUIRE(K >= 1 && K <= kMaxHeads, "sweep_run_diag: 1..%d heads", kMaxHeads);
+  UML_REQUIRE(dg->out && dg->scratch, "sweep_run_diag: null diagnostics buffer");
+  UML_REQUIRE(a->dim > 0 && a->dim % 4 == 0 && a->n_classes > 0, "sweep_run_diag: dim must be a multiple of 4");
+  UML_REQUIRE(aligned16(a->W) && aligned16(a->m) && aligned16(a->v) && a->head_stride % 4 == 0 && aligned16(a->G) &&
+                  a->ldg % 4 == 0,
+              "sweep_run_diag: W, m, v, G must be 16-byte aligned with strides that are multiples of 4");
+  for (int s = 0; s < 2; ++s)
+    UML_REQUIRE(!a->bank[s] || (aligned16(a->bank[s]) && a->bank_ld[s] % 4 == 0),
+                "sweep_run_diag: bank %d rows must be 16-byte aligned", s);
+  if (ad && ad->img_dim > 0)
+    UML_REQUIRE(aligned16(ad->Z) && ad->ldz % 4 == 0, "sweep_run_diag: Z must be 16-byte aligned with ldz a multiple of 4");
+  for (int k = 0; k < K; ++k)  // G's text rows carry alpha: the plain text-loss gradient is G / alpha
+    UML_REQUIRE(!a->active[k] || !a->bank[1] || a->alpha[k] > 0.f,
+                "sweep_run_diag: head %d has alpha %g <= 0, its text-loss gradient cannot be recovered", k,
+                static_cast<double>(a->alpha[k]));
+  const int64_t need = uml_sweep_diag_scratch_floats(K, a->dim, a->n_classes);
+  UML_REQUIRE(dg->scratch_floats >= need, "sweep_run_diag: scratch holds %lld floats, %lld needed",
+              static_cast<long long>(dg->scratch_floats), static_cast<long long>(need));
+  return ad ? sweep_adapter_run_impl(a, ad, dg, n_steps, rows, lr, stream) : sweep_run_impl(a, dg, n_steps, rows, lr, stream);
 }
 
 }  // extern "C"

@@ -62,3 +62,6 @@ _add("--sweep-batched", action="store_true", default=False,
 _add("--sweep-batched-adapter", action="store_true", default=False,
      help="--sweep-batched, and the combinations whose heads have an image adapter or learnable temperatures (preset "
           "'linear') also train in lock step (five launches per step of all heads) instead of one after the other")
+_add("--grad-diagnostics", action="store_true", default=False,
+     help="log the reference's gradient probes (train/grad_direction_sim, img_grad_norm, txt_grad_norm, "
+          "grad_agreement_rate): every step for batched sweep groups, at evaluation cadence for single runs")

@@ -14,8 +14,8 @@ from typing import List, Optional, Sequence
 import torch
 
 from .. import _lib
-from .._lib import SWEEP_MAX_HEADS, SweepAdapterArgs, SweepArgs, check
-from ..ops import UPDATE_KINDS
+from .._lib import SWEEP_MAX_HEADS, SweepAdapterArgs, SweepArgs, SweepDiag, check
+from ..ops import UPDATE_KINDS, grad_diag_record
 
 MAX_HEADS = SWEEP_MAX_HEADS
 
@@ -49,6 +49,17 @@ def group_blockers(models, optimizers, image_loaders, text_loaders) -> List[str]
                    or not l.shuffle or l.generator is not None or l.shard_of is not None or l.upload != "epoch"
                    for l in live):
                 why.append("loaders must share bank, batch size and protocol (shuffled, upload='epoch', no generator)")
+    return why
+
+
+def diag_blockers(models, alphas, text_loaders) -> List[str]:
+    """Why these runs cannot log per-step gradient diagnostics as one group (``uml_sweep_run_diag``): the text-loss
+    gradient is recovered from G, whose text rows carry alpha, and the tensor-core pass needs 16-byte rows."""
+    why = []
+    if any(l is not None for l in text_loaders) and any(float(a) <= 0 for a in alphas):
+        why.append("gradient diagnostics need alpha > 0 when there are text rows")
+    if any(int(m.shared_dim) % 4 for m in models):
+        why.append("gradient diagnostics need feature widths that are multiples of 4")
     return why
 
 
@@ -100,8 +111,10 @@ def adapter_group_blockers(models, optimizers, image_loaders, text_loaders) -> L
 
 
 class HeadGroup:
+    diag = diag_log = None  # uml_sweep_diag and its [log_slots, K, 4] device log (grad_diagnostics)
+
     def __init__(self, models: Sequence, optimizers: Sequence, image_bank, text_bank, max_img_rows: int,
-                 max_txt_rows: int, device, log_slots: int = 128):
+                 max_txt_rows: int, device, log_slots: int = 128, grad_diagnostics: bool = False):
         self.K = K = len(models)
         if not 1 <= K <= MAX_HEADS:
             raise ValueError(f"a HeadGroup holds 1..{MAX_HEADS} heads")
@@ -143,6 +156,13 @@ class HeadGroup:
         self.row_correct = torch.empty((K, self.max_rows), device=self.device, dtype=torch.int32)
         self.log_slots = int(log_slots)
         self.stats_log = torch.zeros((self.log_slots, K, 2, 4), device=self.device)
+        # grad_diagnostics: the reference's per-step gradient probes of every head, four sums per step and head
+        if grad_diagnostics:
+            self.diag_log = torch.zeros((self.log_slots, K, 4), device=self.device)
+            n = _lib.load().uml_sweep_diag_scratch_floats(K, self.D, self.C)
+            self._diag_scratch = torch.empty(n, device=self.device)
+            self.diag = SweepDiag()
+            self.diag.scratch, self.diag.scratch_floats = self._diag_scratch.data_ptr(), n
         self.launches = 0
         s_i, s_t = (float(s) for s in m0.scales())
         a = self.args = SweepArgs()
@@ -195,11 +215,13 @@ class HeadGroup:
                     raise ValueError("HeadGroup.run: active heads must have taken the same number of steps")
         a.step = step + 1
         a.stats = self.stats_log[s0].data_ptr()
+        if self.diag is not None:
+            self.diag.out = self.diag_log[s0].data_ptr()
         rows_c = (C.c_int64 * (2 * n))(*[int(x) for r in rows for x in r])
         lr_c = (C.c_float * (n * K))(*[float(x) for l in lrs for x in l])
         l0 = _lib.load().uml_sweep_launch_count()
         check(self._enqueue(n, rows_c, lr_c))
-        launched = (_lib.load().uml_sweep_launch_count() - l0) & 0x7FFFFFFF  # two to five kernels per step (csrc/sweep.cu)
+        launched = (_lib.load().uml_sweep_launch_count() - l0) & 0x7FFFFFFF  # two to seven kernels per step (csrc/sweep.cu)
         self.launches += launched
         _lib.LAUNCH_COUNT[0] += launched
         for k in range(K):
@@ -216,7 +238,10 @@ class HeadGroup:
         return [model.head.weight]
 
     def _enqueue(self, n, rows_c, lr_c):
-        return _lib.load().uml_sweep_run(C.byref(self.args), n, rows_c, lr_c, torch.cuda.current_stream().cuda_stream)
+        st = torch.cuda.current_stream().cuda_stream
+        if self.diag is not None:
+            return _lib.load().uml_sweep_run_diag(C.byref(self.args), None, C.byref(self.diag), n, rows_c, lr_c, st)
+        return _lib.load().uml_sweep_run(C.byref(self.args), n, rows_c, lr_c, st)
 
     KERNELS = ("sweep_logits", "sweep_softmax_ce", "sweep_dw_update", "sweep_stats")
 
@@ -230,24 +255,50 @@ class HeadGroup:
                 self.args.ev[i] = self._ev[i].cuda_event
             else:
                 self.args.ev[i] = None
+        self._time_diag(enable)
 
     def kernel_times_ms(self):
-        """Device time of each launch of the last timed step (call after a synchronize)."""
+        """Device time of each launch of the last timed step (call after a synchronize); with gradient diagnostics also
+        ``sweep_grad_diag`` (its two launches)."""
         ev = getattr(self, "_ev", [])
-        return {name: ev[2 * i].elapsed_time(ev[2 * i + 1]) for i, name in enumerate(self.KERNELS)} if ev else {}
+        out = {name: ev[2 * i].elapsed_time(ev[2 * i + 1]) for i, name in enumerate(self.KERNELS)} if ev else {}
+        dev = getattr(self, "_diag_ev", [])
+        if dev:
+            out["sweep_grad_diag"] = dev[0].elapsed_time(dev[1])
+        return out
+
+    def _time_diag(self, enable):
+        """The event pair around the diagnostics launches of the last step of every following ``run``."""
+        if self.diag is None:
+            return
+        self._diag_ev = [torch.cuda.Event(enable_timing=True) for _ in range(2)] if enable else []
+        for i in range(2):
+            if enable:
+                self._diag_ev[i].record()
+            self.diag.ev[i] = self._diag_ev[i].cuda_event if enable else None
 
     def read_log(self, slots: Sequence[int], has_img: bool, has_txt: bool):
         """Per-step stats of the given log slots as ``{name: [len(slots)][K] nested lists}`` for image_loss, text_loss,
-        img_acc, text_acc (zeros for an absent modality); one synchronising D2H copy of the log."""
-        raw = self.stats_log.cpu().numpy()
+        img_acc, text_acc (zeros for an absent modality) and, with gradient diagnostics, ``grad_diag``: the reference's
+        four gradient-probe keys per step and head (``ops.grad_diag_record``); one synchronising D2H copy of the log."""
+        L = self.log_slots
+        if self.diag_log is None:
+            raw = self.stats_log.cpu().numpy()
+        else:  # both logs in one copy
+            both = torch.cat((self.stats_log.view(L, -1), self.diag_log.view(L, -1)), 1).cpu().numpy()
+            raw, diag = both[:, :self.K * 8].reshape(L, self.K, 2, 4), both[:, self.K * 8:].reshape(L, self.K, 4)
         ints = raw.view("int32")
-        idx = [s % self.log_slots for s in slots]
+        idx = [s % L for s in slots]
         zeros = [[0.0] * self.K for _ in idx]
         out = {"image_loss": zeros, "text_loss": zeros, "img_acc": zeros, "text_acc": zeros}
         for name_l, name_a, s, present in (("image_loss", "img_acc", 0, has_img), ("text_loss", "text_acc", 1, has_txt)):
             if present:
                 out[name_l] = raw[idx, :, s, 0].tolist()
                 out[name_a] = (ints[idx, :, s, 2] / ints[idx, :, s, 3].clip(min=1)).tolist()
+        if self.diag_log is not None:
+            numel, two = self.C * self.D, has_img and has_txt
+            out["grad_diag"] = [[grad_diag_record(*(float(x) for x in diag[i, k]), numel, two) for k in range(self.K)]
+                                for i in idx]
         return out
 
 
@@ -262,8 +313,9 @@ class AdapterHeadGroup(HeadGroup):
     KERNELS = ("sweep_adapter_z", "sweep_logits", "sweep_adapter_dz", "sweep_dw_update", "sweep_adapter_dw_update")
 
     def __init__(self, models: Sequence, optimizers: Sequence, image_bank, text_bank, max_img_rows: int,
-                 max_txt_rows: int, device, log_slots: int = 128):
-        super().__init__(models, optimizers, image_bank, text_bank, max_img_rows, max_txt_rows, device, log_slots)
+                 max_txt_rows: int, device, log_slots: int = 128, grad_diagnostics: bool = False):
+        super().__init__(models, optimizers, image_bank, text_bank, max_img_rows, max_txt_rows, device, log_slots,
+                         grad_diagnostics)
         if self.max_rows > ADAPTER_MAX_ROWS:
             raise ValueError(f"AdapterHeadGroup: at most {ADAPTER_MAX_ROWS} rows per step")
         K, D, m0 = self.K, self.D, models[0]
@@ -324,8 +376,11 @@ class AdapterHeadGroup(HeadGroup):
         return ps
 
     def _enqueue(self, n, rows_c, lr_c):
-        return _lib.load().uml_sweep_adapter_run(C.byref(self.args), C.byref(self.adapter_args), n, rows_c, lr_c,
-                                                 torch.cuda.current_stream().cuda_stream)
+        st = torch.cuda.current_stream().cuda_stream
+        if self.diag is not None:
+            return _lib.load().uml_sweep_run_diag(C.byref(self.args), C.byref(self.adapter_args), C.byref(self.diag), n,
+                                                  rows_c, lr_c, st)
+        return _lib.load().uml_sweep_adapter_run(C.byref(self.args), C.byref(self.adapter_args), n, rows_c, lr_c, st)
 
     def image_scales(self):
         """Every head's image-run temperature, one read-back (what evaluation multiplies the logits by)."""
@@ -344,3 +399,4 @@ class AdapterHeadGroup(HeadGroup):
                 self.adapter_args.ev[i] = self._ev[i].cuda_event
             else:
                 self.adapter_args.ev[i] = None
+        self._time_diag(enable)

@@ -713,11 +713,7 @@ class StepEngine:
             ops.head_bwd_dw_f32(run, W, ws, dW=g)
         both = img is not None and txt is not None and img.n > 0 and txt.n > 0
         ops.grad_diag(g_img, g_txt, scratch, out4)
-        dot, aa, bb, agree = out4.tolist()
-        ni, nt = aa ** 0.5, bb ** 0.5
-        return {"train/grad_direction_sim": dot / (ni * nt) if both and ni > 0 and nt > 0 else 0.0,
-                "train/img_grad_norm": ni, "train/txt_grad_norm": nt,
-                "train/grad_agreement_rate": agree / W.numel() if both else 0.0}
+        return ops.grad_diag_record(*out4.tolist(), W.numel(), both)
 
     # ------------------------------------------------------------------------------------ readback
     def copy_slot_to_host(self, slot):

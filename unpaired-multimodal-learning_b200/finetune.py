@@ -271,6 +271,10 @@ def train(model, image_loader, text_loader, val_loader, test_loader, optimizer, 
     # call per chunk instead of a Python round trip per kernel; the loaders are advanced in the reference's order
     # (image batch, then text batch, per step) so the sampler stream is unchanged.
     grad_diag = bool(getattr(args, "grad_diagnostics", False) or (trace is not None and trace.get("grad_diagnostics")))
+    if grad_diag and engine.adapter:  # StepEngine.grad_diagnostics covers the linear head only
+        print("=> --grad-diagnostics: no gradient probes for a single run of a head with an image adapter (batched "
+              "sweeps with --sweep-batched-adapter log them); training continues without them")
+        grad_diag = False
     per_step = trace is not None and bool(trace.get("record_weights"))
     # small chunks: the host prepares chunk c+1 (sampler draws, index uploads) while the GPU runs chunk c
     max_chunk = 1 if per_step else 16
@@ -397,7 +401,8 @@ def train(model, image_loader, text_loader, val_loader, test_loader, optimizer, 
 
 
 def train_group(models, image_loaders, text_loaders, val_loaders, test_loaders, optimizers, schedulers, device="cuda",
-                max_iters=1000, alphas=1.0, eval_freq=EVAL_FREQ, patience=5, loggers=None, traces=None, tags=None):
+                max_iters=1000, alphas=1.0, eval_freq=EVAL_FREQ, patience=5, loggers=None, traces=None, tags=None,
+                args=None):
     """K runs of ``train`` advanced in lock step over shared banks (sweep-level batching, SURVEY §8 f-1): one step of all
     K heads is two launches (``engine/sweep.py``, ``csrc/sweep.cu``) instead of K latency-bound steps.  When every head
     has an image adapter or learnable temperatures (preset ``linear``) the heads form an ``AdapterHeadGroup`` instead
@@ -409,7 +414,11 @@ def train_group(models, image_loaders, text_loaders, val_loaders, test_loaders, 
     its own sampler stream: its loaders draw their seeds from their own ``rng`` generator in the order a stand-alone
     run draws them from the global generator, so head k reproduces ``torch.manual_seed(s); train(...)`` when its
     generator was seeded with ``s``.  (The reference's sequential sweep lets one global stream run through all
-    combinations; the order inside each run is the same, the seeds differ.)"""
+    combinations; the order inside each run is the same, the seeds differ.)
+
+    ``args.grad_diagnostics`` (or ``traces[k]["grad_diagnostics"]``): the reference's four gradient probes of every
+    step of every running head, at the step's weights before its update, logged next to the step's ``train/*`` record
+    and appended as ``(step, dict)`` to ``traces[k]["grad_diag"]``."""
     from .engine import sweep as sweep_mod
 
     K = len(models)
@@ -424,6 +433,10 @@ def train_group(models, image_loaders, text_loaders, val_loaders, test_loaders, 
     adapter = all(m.img_proj is not None or getattr(m, "learnable_temp", False) for m in models)
     blockers = sweep_mod.adapter_group_blockers if adapter else sweep_mod.group_blockers
     why = blockers(models, optimizers, image_loaders, text_loaders)
+    grad_diag = bool(getattr(args, "grad_diagnostics", False) or any(tr is not None and tr.get("grad_diagnostics")
+                                                                      for tr in traces))
+    if grad_diag:
+        why += sweep_mod.diag_blockers(models, alphas, text_loaders)
     if _dist()[1] > 1:
         why.append("data-parallel runs are not batched")
     if why:
@@ -436,7 +449,8 @@ def train_group(models, image_loaders, text_loaders, val_loaders, test_loaders, 
     log_slots = min(max(int(eval_freq), 1), int(max(max_iters))) + 1
     group = (sweep_mod.AdapterHeadGroup if adapter else sweep_mod.HeadGroup)(
         models, optimizers, il0.bank if has_img else None, tl0.bank if has_txt else None,
-        il0.batch_size if has_img else 0, tl0.batch_size if has_txt else 0, device, log_slots=log_slots)
+        il0.batch_size if has_img else 0, tl0.batch_size if has_txt else 0, device, log_slots=log_slots,
+        **({"grad_diagnostics": True} if grad_diag else {}))
     outs = [{"iter": None, "val_acc": None, "model": None, "val_classwise": None, "val_loss": None, "model_records": []}
             for _ in range(K)]
     for tr in traces:
@@ -459,18 +473,22 @@ def train_group(models, image_loaders, text_loaders, val_loaders, test_loaders, 
         if not pending:
             return
         cols = group.read_log([s for s, _, _ in pending], has_img, has_txt)
-        for j, (_, lrs, act) in enumerate(pending):
+        for j, (step, lrs, act) in enumerate(pending):
             for k in range(K):
                 if not act[k] or (traces[k] is None and loggers[k] is None):
                     continue
                 rec = {"image_loss": cols["image_loss"][j][k], "text_loss": cols["text_loss"][j][k],
                        "img_acc": cols["img_acc"][j][k], "text_acc": cols["text_acc"][j][k]}
+                diag = cols["grad_diag"][j][k] if grad_diag else {}
                 if traces[k] is not None:
                     traces[k].setdefault("stats", []).append(dict(rec, lr=lrs[k]))
+                    if grad_diag:
+                        traces[k].setdefault("grad_diag", []).append((step, diag))
                 if loggers[k] is not None:
                     loggers[k].log({"train/image_loss": rec["image_loss"], "train/text_loss": rec["text_loss"],
-                                    "train/image_acc": rec["img_acc"], "train/text_acc": rec["text_acc"], "train/lr": lrs[k]})
-        last = {name: col[-1] for name, col in cols.items()}
+                                    "train/image_acc": rec["img_acc"], "train/text_acc": rec["text_acc"], "train/lr": lrs[k],
+                                    **diag})
+        last = {name: col[-1] for name, col in cols.items() if name != "grad_diag"}
         pending.clear()
 
     def take(loaders, its, k, n):
@@ -718,7 +736,7 @@ def setup_group(datasets, combos, args, positions=None):
     differ in --alpha and therefore in ``savepath``).  Run k's loaders draw from their own generator seeded
     ``run_seed(args_k, positions[k])`` (``positions``: each combination's index in the preset's grid, default
     0, 1, ...) - or from the global stream when ``args.seed < 0``."""
-    from .engine.sweep import MAX_HEADS, adapter_group_blockers, group_blockers
+    from .engine.sweep import MAX_HEADS, adapter_group_blockers, diag_blockers, group_blockers
 
     per_run = list(args) if isinstance(args, (list, tuple)) else [args] * len(combos)
     positions = list(positions) if positions is not None else list(range(len(combos)))
@@ -729,9 +747,12 @@ def setup_group(datasets, combos, args, positions=None):
         """--sweep-batched-adapter: runs with an image adapter or learnable temperatures form AdapterHeadGroups."""
         ms = [ctxs[c]["model"] for c in cand]
         adapter = with_adapters and any(m.img_proj is not None or getattr(m, "learnable_temp", False) for m in ms)
-        return (adapter_group_blockers if adapter else group_blockers)(
+        why = (adapter_group_blockers if adapter else group_blockers)(
             ms, [ctxs[c]["optimizer"] for c in cand], [ctxs[c]["image_loader"] for c in cand],
             [ctxs[c]["text_loader"] for c in cand])
+        if getattr(args, "grad_diagnostics", False):  # --grad-diagnostics: per-step probes on the device
+            why += diag_blockers(ms, [ctxs[c]["args"].alpha for c in cand], [ctxs[c]["text_loader"] for c in cand])
+        return why
 
     results = [None] * len(combos)
     ctxs = {}
@@ -771,7 +792,7 @@ def setup_group(datasets, combos, args, positions=None):
                                device=args.device, max_iters=[ctxs[c]["hparams"]["max_iter"] for c in members],
                                alphas=[ctxs[c]["args"].alpha for c in members], eval_freq=EVAL_FREQ,
                                patience=[ctxs[c]["hparams"]["patience"] for c in members], loggers=col("logger"),
-                               tags=[f"run {c + 1}" for c in members])
+                               tags=[f"run {c + 1}" for c in members], args=args)
         for c, out in zip(members, outs):
             ctx = ctxs.pop(c)
             results[c] = _finish(ctx, out, ctx["args"])

@@ -345,6 +345,16 @@ def grad_diag(a, b, workspace, out4):
                                     _stream()))
 
 
+def grad_diag_record(dot: float, aa: float, bb: float, agree: float, numel: int, both: bool) -> dict:
+    """The reference's gradient-probe logger keys (finetune.py:200-206) from the four sums of ``grad_diag`` /
+    ``uml_sweep_run_diag`` over the image-loss gradient A and the text-loss gradient B of the head weights (``numel``
+    elements each); ``both``: the step had rows of both modalities (else the cosine and agreement are 0)."""
+    ni, nt = float(aa) ** 0.5, float(bb) ** 0.5
+    return {"train/grad_direction_sim": float(dot) / (ni * nt) if both and ni > 0 and nt > 0 else 0.0,
+            "train/img_grad_norm": ni, "train/txt_grad_norm": nt,
+            "train/grad_agreement_rate": float(agree) / numel if both else 0.0}
+
+
 # ------------------------------------------------------------------------------------------ tensor-core head
 
 def tc_segments(rows: Sequence[int], scales: Sequence[float], weights: Sequence[float],
