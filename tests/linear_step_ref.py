@@ -14,6 +14,10 @@ temperature is left untouched, as torch.optim skips a parameter whose .grad is N
 
 ``bf16_operands=True`` rounds X and W to bf16 first, as the tensor-core step's operands are; everything after that is
 float64.  Large steps are processed in row blocks, so the benchmark's 73728 x 1000 logits never exist at once.
+
+``adapter_step`` adds the image adapter Wp [D, Dv] of a UML head (preset ``linear``): the image run's rows become
+Z = X_img Wp^T, then dZ = G_img W with W taken before its update, dWp = dZ^T X_img, and Wp takes the same rule as W
+(one parameter group).  A step without image rows leaves Wp, its m, v and step count untouched.
 """
 from __future__ import annotations
 
@@ -157,4 +161,38 @@ def linear_step(W: torch.Tensor, runs: List[RunIn], hp: Hyper, step: int, m: tor
         g = torch.tensor(st["dscale"], dtype=torch.float64, device=r.temp.value.device)
         temps.append(apply_update(hp, r.temp.value, g, r.temp.m, r.temp.v, r.temp.step))
     out["temps"] = temps
+    return out
+
+
+@dataclass
+class Adapter:
+    """The image adapter Wp [D, Dv] with its optimizer state and step count (steps taken so far)."""
+    Wp: torch.Tensor
+    m: torch.Tensor
+    v: Optional[torch.Tensor]
+    step: int
+
+
+def adapter_step(W: torch.Tensor, ad: Adapter, img: Optional[RunIn], txt: Optional[RunIn], hp: Hyper, step: int,
+                 m: torch.Tensor, v: Optional[torch.Tensor]):
+    """One step of a head with an image adapter.  ``img.x`` holds the image features X_img [n_img, Dv] (not Z);
+    ``step`` is W's 1-based step.  Returns linear_step's dict over the runs [image (rows Z), text] that have rows, plus
+    Z [n_img, D], dZ, dWp (None without image rows) and Wp, Wp_m, Wp_v, Wp_step after the step."""
+    W64 = W.double()
+    runs, Z = [], None
+    if img is not None and img.n:
+        Z = img.x.double() @ ad.Wp.double().t()
+        runs.append(RunIn(Z, img.labels, img.scale, img.loss_weight, img.temp))
+    if txt is not None and txt.n:
+        runs.append(txt)
+    out = linear_step(W64, runs, hp, step, m, v, keep_g=True)
+    out["Z"], out["dZ"], out["dWp"] = Z, None, None
+    out["Wp"], out["Wp_m"] = ad.Wp.double(), ad.m.double()
+    out["Wp_v"] = ad.v.double() if ad.v is not None else None
+    out["Wp_step"] = ad.step
+    if Z is not None:
+        out["dZ"] = out["G"][:img.n] @ W64
+        out["dWp"] = out["dZ"].t() @ img.x.double()
+        out["Wp_step"] = ad.step + 1
+        out["Wp"], out["Wp_m"], out["Wp_v"] = apply_update(hp, ad.Wp, out["dWp"], ad.m, ad.v, out["Wp_step"])
     return out

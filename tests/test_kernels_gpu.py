@@ -212,23 +212,88 @@ def test_learnable_scale_gradient_f32():
     assert math.isclose(got[1]["dscale"], float(grads["txt_scale"]), rel_tol=1e-4, abs_tol=1e-6)
 
 
+# (rows b, Dv, D, C, alpha, optimizer rule fused into gemm_tn or None, padding of gemm_tn's ldc)
+ADAPTER_GEMMS = {"toy": (37, 96, 160, 50, 2.0, None, 0), "toy_sgd": (37, 96, 160, 50, 1.0, "sgd", 3),
+                 "preset_linear_adamw": (32, 1536, 3200, 1000, 1.0, "adamw", 0),
+                 "preset_linear_adam": (32, 1536, 3200, 1000, 0.5, "adam", 5)}
+
+
 def test_adapter_gemms_f32():
-    g = torch.Generator().manual_seed(5)
-    b, dv, d, c = 37, 96, 160, 50
-    bank = torch.randn(100, dv, generator=g)
-    idx = torch.randint(0, 100, (b,), generator=g)
-    wp = torch.randn(d, dv, generator=g) * 0.1
-    w = torch.randn(c, d, generator=g) * 0.1
-    gm = torch.randn(b, c, generator=g)
-    z = torch.empty(b, d, device=DEV)
-    ops.gemm_nt(bank.to(DEV), wp.to(DEV), z, a_row_idx=idx.to(DEV))
-    np.testing.assert_allclose(z.cpu().numpy(), (bank[idx] @ wp.t()).numpy(), rtol=1e-4, atol=1e-5)
-    dz = torch.empty(b, d, device=DEV)
-    ops.gemm_nn(gm.to(DEV), w.to(DEV), dz, alpha=2.0)
-    np.testing.assert_allclose(dz.cpu().numpy(), (2.0 * gm @ w).numpy(), rtol=1e-4, atol=1e-5)
-    dwp = torch.empty(d, dv, device=DEV)
-    ops.gemm_tn(dz, bank.to(DEV), dwp, k=b, m=d, n=dv, b_row_idx=idx.to(DEV))
-    np.testing.assert_allclose(dwp.cpu().numpy(), ((2.0 * gm @ w).t() @ bank[idx]).numpy(), rtol=1e-4, atol=1e-4)
+    """The three GEMMs of the adapter's exact step (engine/trainer.py _step_fp32) against float64 on their own fp32
+    operands, with the worst-case bound k u sum|a b| of an FMA chain of k terms: gemm_nt (Z = X[idx] Wp^T) and gemm_nn
+    (dZ = G W over k = C < ldg) with m below the output's rows, whose rows past m stay untouched; gemm_tn (dWp = dZ^T
+    X[idx]) with the optimizer update fused into its epilogue, on 32 x 32 tiles (toy) and 64 x 64 tiles (3200 x 1536),
+    into a padded ldc whose padding stays untouched.  The fused update is judged by the gradient recovered from m.
+    Every case of ADAPTER_GEMMS runs."""
+    for case in ADAPTER_GEMMS:
+        _check_adapter_gemms(case)
+
+
+def _check_adapter_gemms(case):
+    from linear_step_case import U, check_update, recover_grad
+    from linear_step_ref import Hyper, apply_update
+    b, dv, d, c, alpha, kind, pad = ADAPTER_GEMMS[case]
+    g = torch.Generator(device=DEV).manual_seed(b + dv + d + c + pad)
+    bank = torch.randn(b + 60, dv, device=DEV, generator=g) / math.sqrt(dv)
+    idx = torch.randint(0, b + 60, (b,), device=DEV, generator=g)
+    wp = torch.randn(d, dv, device=DEV, generator=g) / math.sqrt(dv)
+    w = torch.randn(c, d, device=DEV, generator=g) / math.sqrt(d)
+    ldg = (c + 63) // 64 * 64
+    gm = torch.randn(b + 7, ldg, device=DEV, generator=g) / c   # G's rows past the image rows and its padding columns
+    x64, wp64, w64, g64 = bank[idx].double(), wp.double(), w.double(), gm[:b, :c].double()
+
+    def close(got, want, bound, what):
+        r = float(((got.double() - want).abs() / (bound + 1e-30)).max())
+        assert r <= 1.0, (what, r)
+        return r
+
+    z = torch.full((b + 5, d), float("nan"), device=DEV)
+    ops.gemm_nt(bank, wp, z, alpha=alpha, a_row_idx=idx, m=b)
+    rz = close(z[:b], alpha * x64 @ wp64.t(), abs(alpha) * dv * U * (x64.abs() @ wp64.abs().t()), "gemm_nt")
+    assert bool(z[b:].isnan().all()), "gemm_nt wrote past m"
+    dz = torch.full((b + 5, d), float("nan"), device=DEV)
+    ops.gemm_nn(gm, w, dz, alpha=alpha, m=b, k=c)
+    rdz = close(dz[:b], alpha * g64 @ w64, abs(alpha) * c * U * (g64.abs() @ w64.abs()), "gemm_nn")
+    assert bool(dz[b:].isnan().all()), "gemm_nn wrote past m"
+    dz64 = dz[:b].double()
+    want = alpha * dz64.t() @ x64
+    bound = abs(alpha) * b * U * (dz64.abs().t() @ x64.abs())
+    if kind is None:
+        dwp = torch.full((d, dv + pad), float("nan"), device=DEV)
+        ops.gemm_tn(dz, bank, dwp, k=b, m=d, n=dv, alpha=alpha, b_row_idx=idx)
+        rtn = close(dwp[:, :dv], want, bound, "gemm_tn")
+        assert bool(dwp[:, dv:].isnan().all()), "gemm_tn wrote into the padding"
+        print(f"\n[{case}] nt {rz:.2e}, nn {rdz:.2e}, tn {rtn:.2e} of the bounds")
+        return
+    # the update fused into gemm_tn, from a warm state; P, m and v padded like a strided parameter view
+    hp = Hyper(kind, lr=1e-2, weight_decay=0.05).as_f32()
+    store = lambda t: torch.cat([t, torch.full((d, pad), 7.0, device=DEV)], 1)
+    P0 = torch.randn(d, dv, device=DEV, generator=g) / math.sqrt(dv)
+    m0 = want.float() * (torch.rand(d, dv, device=DEV, generator=g) * 3 - 1)
+    v0 = (want.float() ** 2 + (0.05 * float(want.abs().max())) ** 2) * (torch.rand(d, dv, device=DEV, generator=g) + 0.5)
+    P, M, V = store(P0), store(m0), store(v0)
+    upd = ops.make_update(kind, hp.lr, 5, M, V if kind != "sgd" else None, weight_decay=hp.weight_decay,
+                          betas=(hp.beta1, hp.beta2), eps=hp.eps, momentum=hp.momentum)
+    ops.gemm_tn(dz, bank, None, k=b, m=d, n=dv, alpha=alpha, b_row_idx=idx, P=P, update=upd, ldc=dv + pad)
+    torch.cuda.synchronize()
+    for t, nm in ((P, "P"), (M, "m"), (V, "v")):
+        assert bool((t[:, dv:] == 7.0).all()), nm + ": the padding was written"
+    grad, rec = recover_grad(kind, hp, m0, M[:, :dv], P0)
+    rtn = close(grad, want, bound + rec, "gemm_tn recovered gradient")
+    pw, mw, vw = apply_update(hp, P0, grad, m0, v0 if kind != "sgd" else None, 5)
+    ru = check_update(P[:, :dv], pw, "P")
+    check_update(M[:, :dv], mw, "m")
+    if kind != "sgd":
+        check_update(V[:, :dv], vw, "v", atol=1e-12)
+    else:
+        assert torch.equal(V, store(v0)), "SGD has no v"
+    # a missing weight decay would stand out: wd |p| (Adam, SGD) or lr wd |p| (AdamW) against the bound it would break
+    p0 = P0.double().abs()
+    decay = (hp.lr * hp.weight_decay * p0 / (2e-7 + 2e-6 * pw.abs()) if kind == "adamw"
+             else hp.weight_decay * p0 / (bound + rec))
+    assert float(decay.median()) >= 10.0, float(decay.median())
+    print(f"\n[{case}] nt {rz:.2e}, nn {rdz:.2e}, tn gradient {rtn:.2e}, update {ru:.2e} of the bounds; "
+          f"weight decay {float(decay.median()):.0f}x its bound")
 
 
 # ------------------------------------------------------------------------------------------ K7

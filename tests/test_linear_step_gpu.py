@@ -20,144 +20,18 @@ Observed on an NVIDIA B200 (the cfg3 case, 70144 + 3584 rows): gradient relative
 (128 rows, chunk-sequential forward) and 0.04.
 """
 import ctypes
-import math
-from dataclasses import dataclass
-from typing import List, Optional
 
 import pytest
 import torch
 
-from linear_step_ref import Hyper, RunIn, Temperature, apply_update, forward_backward
+from linear_step_case import (DEV, OPT_STEP, Run, Workspace, call, check_stats, check_update, stats_rec, stream,
+                              temp_state)
+from linear_step_ref import Hyper, apply_update, forward_backward
 
 pytestmark = pytest.mark.gpu
 
 if torch.cuda.is_available():
-    import uml_b200  # noqa: F401
-    from uml_b200 import _lib, ops
-
-DEV = "cuda:0"
-OPT_STEP = 5   # a warm Adam state: at step 1 AdamW takes lr * sign(g), which flips for near-zero gradients
-
-
-def _stream():
-    return torch.cuda.current_stream().cuda_stream
-
-
-def _call(fn, *args):
-    _lib.check(fn(*args))
-
-
-# ------------------------------------------------------------------------------------------ one run of a step
-@dataclass
-class Run:
-    """One run of rows as the step reads it, and what its gather must produce."""
-    n: int
-    rows: torch.Tensor                   # fp32 bank (or the dense rows when idx is None)
-    labels: torch.Tensor                 # int64 bank labels (dense labels when neither idx nor label_idx)
-    idx: Optional[torch.Tensor]
-    rows16: Optional[torch.Tensor] = None
-    label_idx: Optional[torch.Tensor] = None
-    scale: float = 1.0
-    loss_weight: float = 1.0
-    temp: Optional[dict] = None          # {"value", "m", "v"} 0-dim fp32 device tensors + "step"
-
-    def segment(self):
-        sd = self.temp["value"].data_ptr() if self.temp else None
-        return _lib.Segment(self.rows.data_ptr(), self.idx.data_ptr() if self.idx is not None else None,
-                            self.labels.data_ptr(), self.n, self.rows.stride(0), self.scale, self.loss_weight,
-                            self.label_idx.data_ptr() if self.label_idx is not None else None, sd,
-                            self.rows16.data_ptr() if self.rows16 is not None else None)
-
-    def x16(self):
-        """The rows the step must gather, in bf16."""
-        x = self.rows[self.idx[:self.n]] if self.idx is not None else self.rows[:self.n]
-        return x.to(torch.bfloat16)
-
-    def y(self):
-        sel = self.label_idx if self.label_idx is not None else self.idx
-        return (self.labels[sel[:self.n]] if sel is not None else self.labels[:self.n]).to(torch.int32)
-
-    def ref_in(self, x16):
-        t = None
-        if self.temp:
-            t = Temperature(self.temp["value"].double(), self.temp["m"].double(), self.temp["v"].double()
-                            if self.temp["v"] is not None else None, self.temp["step"])
-        return RunIn(x16, self.y(), self.scale, self.loss_weight, t)
-
-
-class Workspace:
-    """Caller-owned buffers of the step (the library never allocates)."""
-
-    def __init__(self, D, C, rows, n_buffers=1, precision=1):
-        self.D, self.C, self.rows = D, C, rows
-        self.ldg = (C + 63) // 64 * 64
-        self.G = torch.empty((rows, self.ldg), device=DEV, dtype=torch.bfloat16 if precision else torch.float32)
-        self.row_loss = torch.empty(rows, device=DEV)
-        self.row_correct = torch.empty(rows, device=DEV, dtype=torch.int32)
-        self.row_dscale = torch.empty(rows, device=DEV)
-        self.X16 = [torch.empty((rows, D), device=DEV, dtype=torch.bfloat16) for _ in range(n_buffers)]
-        self.labels32 = [torch.empty(rows, device=DEV, dtype=torch.int32) for _ in range(n_buffers)]
-        self.W16 = torch.empty((C, D), device=DEV, dtype=torch.bfloat16)
-        self.max_splits = max(1, ops.tc_dw_splits(rows, D, C))
-        self.partials = torch.empty((self.max_splits, C, D), device=DEV)
-        self.tile_ws = torch.zeros(16 + (rows + 255) // 256 * 264 + rows * 32, device=DEV)  # UML_TILE_WS_FLOATS
-        self.dW = torch.empty((C, D), device=DEV)
-
-    def args(self, runs: List[Run], W, m, v, hp: Hyper, opt_step, stats, *, dW_out=None, dW_scratch=None,
-             w16_valid=1, max_splits=None, precision=1):
-        a = _lib.LinearStepArgs()
-        a.dim, a.n_classes, a.nseg, a.precision = self.D, self.C, len(runs), precision
-        for k, r in enumerate(runs):
-            a.seg[k] = r.segment()
-            if r.temp:
-                a.scale_param[k], a.scale_m[k] = r.temp["value"].data_ptr(), r.temp["m"].data_ptr()
-                a.scale_v[k] = r.temp["v"].data_ptr() if r.temp["v"] is not None else None
-                a.scale_step[k] = r.temp["step"]
-        a.W = W.data_ptr()
-        a.upd = ops.make_update(hp.kind, hp.lr, opt_step, m, v if hp.kind != "sgd" else None,
-                                weight_decay=hp.weight_decay, betas=(hp.beta1, hp.beta2), eps=hp.eps, momentum=hp.momentum)
-        a.G, a.ldg, a.g_capacity_rows = self.G.data_ptr(), self.ldg, self.rows
-        a.row_loss, a.row_correct, a.row_dscale = (self.row_loss.data_ptr(), self.row_correct.data_ptr(),
-                                                   self.row_dscale.data_ptr())
-        a.stats = stats.data_ptr()
-        if precision:
-            a.X16, a.labels32, a.W16 = self.X16[0].data_ptr(), self.labels32[0].data_ptr(), self.W16.data_ptr()
-            a.partials, a.tile_ws = self.partials.data_ptr(), self.tile_ws.data_ptr()
-            a.max_splits = self.max_splits if max_splits is None else max_splits
-            a.w16_valid = w16_valid
-        a.dW_out = dW_out.data_ptr() if dW_out is not None else None
-        a.dW_scratch = dW_scratch.data_ptr() if dW_scratch is not None else None
-        return a
-
-
-def _stats_rec(stats, k):
-    f, i = stats[k].cpu(), stats[k].cpu().view(torch.int32)
-    return dict(loss_mean=float(f[0]), dscale=float(f[1]), correct=int(i[2]), n=int(i[3]))
-
-
-def _check_stats(stats, ref_stats, where="", dscale=True):
-    """dscale is d loss / d scale for a learnable temperature: with fixed scales the bf16 step need not compute it."""
-    for k, r in enumerate(ref_stats):
-        got = _stats_rec(stats, k)
-        assert got["n"] == r["n"], (where, k, got, r)
-        assert math.isclose(got["loss_mean"], r["loss_mean"], rel_tol=2e-4, abs_tol=1e-6), (where, k, got, r)
-        if dscale:
-            assert math.isclose(got["dscale"], r["dscale"], rel_tol=2e-3, abs_tol=1e-6), (where, k, got, r)
-        assert abs(got["correct"] - r["correct"]) <= r["near_ties"], (where, k, got, r)
-
-
-def _check_update(got, want, what, rtol=2e-6, atol=2e-7):
-    """max |got - want| / (atol + rtol |want|) <= 1; returns that ratio."""
-    ratio = float(((got.double() - want).abs() / (atol + rtol * want.abs())).max())
-    assert ratio <= 1.0, (what, ratio)
-    return ratio
-
-
-def _temp(value, g, kind):
-    """A learnable temperature at OPT_STEP with a seeded optimizer state."""
-    return dict(value=torch.tensor(value, device=DEV), m=torch.tensor(float(torch.randn(1, generator=g)) * 0.3, device=DEV),
-                v=None if kind == "sgd" else torch.tensor(0.05 + float(torch.rand(1, generator=g)) * 0.1, device=DEV),
-                step=OPT_STEP)
+    from uml_b200 import _lib
 
 
 # ------------------------------------------------------------------------------------------ (a) one step vs float64
@@ -197,7 +71,7 @@ def _make_runs(cfg, g):
             if k == 0:
                 r.rows, r.idx = rows[:n].contiguous(), None
         if cfg.get("learnable"):
-            r.temp = _temp(r.scale, torch.Generator().manual_seed(k), cfg["kind"])
+            r.temp = temp_state(r.scale, torch.Generator().manual_seed(k), cfg["kind"])
         runs.append(r)
     return runs
 
@@ -230,7 +104,7 @@ def test_step_matches_the_float64_reference(case):
         ws.G.fill_(float("nan"))
         stats = torch.full((2, 4), float("nan"), device=DEV)
         a = ws.args(runs, W, m, v, hp, OPT_STEP, stats, w16_valid=w16_valid, max_splits=max_splits, **kw)
-        _call(_lib.load().uml_linear_step, ctypes.byref(a), _stream())
+        call(_lib.load().uml_linear_step, ctypes.byref(a), stream())
         torch.cuda.synchronize()
         return stats
 
@@ -251,7 +125,7 @@ def test_step_matches_the_float64_reference(case):
     assert bool((G[:, C:] == 0).all()), "G's padding columns must be zero"
     gmax = float(ref["G"].abs().max())
     assert float((G[:, :C].double() - ref["G"]).abs().max()) <= 6e-3 * gmax
-    _check_stats(stats, ref["stats"], case, dscale=bool(cfg.get("learnable")))
+    check_stats(stats, ref["stats"], case, dscale=bool(cfg.get("learnable")))
     dW_ref = ref["dW"]
     rel = float((grad.double() - dW_ref).norm() / dW_ref.norm())
     mx = float((grad.double() - dW_ref).abs().max()) / float(dW_ref.abs().max())
@@ -262,13 +136,13 @@ def test_step_matches_the_float64_reference(case):
         for k, (r, t0) in enumerate(zip(runs, temps0)):
             if not t0:
                 continue
-            ds = torch.tensor(_stats_rec(stats, k)["dscale"], dtype=torch.float64)
+            ds = torch.tensor(stats_rec(stats, k)["dscale"], dtype=torch.float64)
             want = apply_update(hp, t0["value"].cpu(), ds, t0["m"].cpu(), t0["v"].cpu() if t0["v"] is not None else None,
                                 t0["step"])
-            _check_update(r.temp["value"].cpu(), want[0], where + " temperature")
-            _check_update(r.temp["m"].cpu(), want[1], where + " temperature m")
+            check_update(r.temp["value"].cpu(), want[0], where + " temperature")
+            check_update(r.temp["m"].cpu(), want[1], where + " temperature m")
             if want[2] is not None:
-                _check_update(r.temp["v"].cpu(), want[2], where + " temperature v")
+                check_update(r.temp["v"].cpu(), want[2], where + " temperature v")
 
     check_temps("dW_out")
     # ---- fused: the update from a warm state (m != 0, v > 0), judged on the kernel's own gradient ----------------
@@ -282,10 +156,10 @@ def test_step_matches_the_float64_reference(case):
     if scratch is not None:
         assert torch.equal(scratch, grad), "dW_scratch holds the gradient dW_out held"
     Ww, mw, vw = apply_update(hp, W0, grad, m0, v0 if kind != "sgd" else None, OPT_STEP)
-    worst = _check_update(W, Ww, "W")
-    _check_update(m, mw, "m")
+    worst = check_update(W, Ww, "W")
+    check_update(m, mw, "m")
     if kind != "sgd":
-        _check_update(v, vw, "v", atol=1e-12)
+        check_update(v, vw, "v", atol=1e-12)
     assert torch.equal(ws.W16, W.to(torch.bfloat16)), "the bf16 shadow is the updated W"
     print(f"[{case}] update: largest W error {worst:.2f} of the bound (rtol 2e-6, atol 2e-7)")
     check_temps("fused")
@@ -319,7 +193,7 @@ def pipeline_case():
         before.append(W.clone())
         hp = Hyper(**{**case["hp"].__dict__, "lr": lrs[i]})
         a = ws.args(_pipeline_runs(case, i), W, m, v, hp, i + 1, stats[i])
-        _call(_lib.load().uml_linear_step, ctypes.byref(a), _stream())
+        call(_lib.load().uml_linear_step, ctypes.byref(a), stream())
     torch.cuda.synchronize()
     case["chain"] = dict(W=W, m=m, v=v, W16=ws.W16.clone(), stats=stats, before=before)
     return case
@@ -335,7 +209,7 @@ def test_chain_stats_match_the_float64_reference(pipeline_case):
     for i in range(P_STEPS):
         runs = _pipeline_runs(c, i)
         ref = forward_backward(c["chain"]["before"][i].to(torch.bfloat16), [r.ref_in(r.x16()) for r in runs], keep_g=False)
-        _check_stats(c["chain"]["stats"][i], ref["stats"], f"step {i}", dscale=False)
+        check_stats(c["chain"]["stats"][i], ref["stats"], f"step {i}", dscale=False)
 
 
 @pytest.mark.parametrize("n_buffers", [1, 2, 3])
@@ -346,7 +220,7 @@ def test_run_is_bit_identical_to_a_chain_of_single_steps(pipeline_case, n_buffer
     uml_linear_step (the next run must start cold), steps 7-11 in calls again, the last one short."""
     c = pipeline_case
     lib = _lib.load()
-    _call(lib.uml_linear_run_reset)
+    call(lib.uml_linear_run_reset)
     W, m, v = c["W0"].clone(), torch.zeros_like(c["W0"]), torch.zeros_like(c["W0"])
     ws = Workspace(P_D, P_C, 500, n_buffers=n_buffers)
     ws.W16.copy_(W.to(torch.bfloat16))
@@ -370,11 +244,11 @@ def test_run_is_bit_identical_to_a_chain_of_single_steps(pipeline_case, n_buffer
                     s.idx[k], s.n[k], s.loss_weight[k] = ix.data_ptr(), len(ix), (1.0, 0.5)[k]
                 s.lr, s.opt_step, s.stats = c["lrs"][i], i + 1, stats[i].data_ptr()
             keep.append(steps)
-            _call(lib.uml_linear_run, ctypes.byref(base), steps, hi - lo, _stream())
+            call(lib.uml_linear_run, ctypes.byref(base), steps, hi - lo, stream())
 
     run_calls(0, 6)
     a = ws.args(_pipeline_runs(c, 6), W, m, v, Hyper(**{**hp0.__dict__, "lr": c["lrs"][6]}), 7, stats[6])
-    _call(lib.uml_linear_step, ctypes.byref(a), _stream())
+    call(lib.uml_linear_step, ctypes.byref(a), stream())
     run_calls(7, P_STEPS)
     torch.cuda.synchronize()
     ch = c["chain"]
@@ -402,7 +276,7 @@ def test_empty_run(precision, empty, learnable, n_live):
                 torch.randperm(400, device=DEV, generator=g)[:max(n, 1)], rows16=rows.to(torch.bfloat16) if precision else None,
                 scale=(20.0, 8.0)[k], loss_weight=(1.0, 0.5)[k])
         if learnable:
-            r.temp = _temp(r.scale, torch.Generator().manual_seed(k + 7), "adamw")
+            r.temp = temp_state(r.scale, torch.Generator().manual_seed(k + 7), "adamw")
         runs.append(r)
     temps0 = [{key: (val.clone() if torch.is_tensor(val) else val) for key, val in r.temp.items()} if learnable else None
               for r in runs]
@@ -420,17 +294,17 @@ def test_empty_run(precision, empty, learnable, n_live):
     x = r.x16() if precision else r.rows[r.idx[:r.n]]
     ref = forward_backward(W0, [r.ref_in(x)], bf16_operands=bool(precision), keep_g=False)
     a = ws.args(runs, W, m, v, hp, 1, stats, precision=precision)
-    _call(_lib.load().uml_linear_step, ctypes.byref(a), _stream())
+    call(_lib.load().uml_linear_step, ctypes.byref(a), stream())
     torch.cuda.synchronize()
     assert bool((stats[empty].view(torch.int32) == 0).all()), ("the empty run's record", stats[empty])
-    got = _stats_rec(stats, live)
-    _check_stats(stats[live:live + 1], ref["stats"], "live run", dscale=learnable or precision == 0)
+    got = stats_rec(stats, live)
+    check_stats(stats[live:live + 1], ref["stats"], "live run", dscale=learnable or precision == 0)
     if learnable:
         t0 = temps0[live]
         want = apply_update(hp, t0["value"].cpu(), torch.tensor(got["dscale"], dtype=torch.float64), t0["m"].cpu(),
                             t0["v"].cpu(), t0["step"])
-        _check_update(runs[live].temp["value"].cpu(), want[0], "live temperature")
-        _check_update(runs[live].temp["m"].cpu(), want[1], "live temperature m")
-        _check_update(runs[live].temp["v"].cpu(), want[2], "live temperature v")
+        check_update(runs[live].temp["value"].cpu(), want[0], "live temperature")
+        check_update(runs[live].temp["m"].cpu(), want[1], "live temperature m")
+        check_update(runs[live].temp["v"].cpu(), want[2], "live temperature v")
         for key in ("value", "m", "v"):
             assert torch.equal(runs[empty].temp[key], temps0[empty][key]), ("the empty run's temperature " + key)

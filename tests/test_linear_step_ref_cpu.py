@@ -6,7 +6,7 @@ import math
 import pytest
 import torch
 
-from linear_step_ref import Hyper, RunIn, Temperature, apply_update, linear_step
+from linear_step_ref import Adapter, Hyper, RunIn, Temperature, adapter_step, apply_update, linear_step
 from oracle import uml_oracle as O
 
 # (n_img, n_txt, D, C): one run, two runs, ragged and tiny shapes
@@ -72,6 +72,71 @@ def test_reference_step_matches_the_oracle(shape, kind, learnable):
                 k += 1
     # G of the last step: rows of a softmax-minus-onehot sum to zero
     assert float(out["G"].sum(1).abs().max()) <= 1e-12
+
+
+@pytest.mark.parametrize("shape", [(6, 5, 12, 16, 7), (9, 0, 10, 8, 5), (0, 7, 10, 8, 5)],
+                         ids=["both_runs", "image_only", "text_only"])
+@pytest.mark.parametrize("kind", ["adamw", "adam", "sgd"])
+@pytest.mark.parametrize("learnable", [False, True])
+def test_adapter_reference_matches_the_oracle(shape, kind, learnable):
+    """adapter_step against uml_step_grads with HeadState.img_proj and OracleOptimizer over three steps: a step with
+    both runs (or one modality) first, then a step with the other modality missing, then both again - Wp, its moments
+    and its step count only move on steps with image rows, as the oracle skips a parameter without a gradient."""
+    ni, nt, dv, d, c = shape
+    g = torch.Generator().manual_seed(ni * 100 + nt * 10 + dv + d + c)
+    Wp0, W0 = torch.randn(d, dv, generator=g) / math.sqrt(dv), torch.randn(c, d, generator=g) / math.sqrt(d)
+    s_img, s_txt, alpha, wd, lr = 1.3, 0.8, 0.5, 0.02, 1e-2
+    st = O.HeadState(head=W0.clone(), img_proj=Wp0.clone(), img_scale=s_img, txt_scale=s_txt, learnable_temp=learnable)
+    opt = O.OracleOptimizer(st.param_dict(), kind, lr, wd)
+    hp = Hyper(kind, lr=lr, weight_decay=wd)
+    z = lambda t: torch.zeros_like(t, dtype=torch.float64)
+    W, m, v = W0.double(), z(W0), z(W0)
+    ad = Adapter(Wp0.double(), z(Wp0), z(Wp0), 0)
+    temps = [Temperature(torch.tensor(s, dtype=torch.float64), torch.tensor(0.0, dtype=torch.float64),
+                         torch.tensor(0.0, dtype=torch.float64), 0) for s in (s_img, s_txt)]
+    # the second step drops one modality: the image run when the first step had both or only text rows
+    plan = [(ni, nt), (0, nt) if nt else (ni, 0), (ni, nt)] if ni and nt else [(ni, nt), (ni or 4, nt or 3), (ni, nt)]
+    for step, (si, sn) in enumerate(plan, start=1):
+        xi, yi = torch.randn(si, dv, generator=g), torch.randint(0, c, (si,), generator=g)
+        xt, yt = torch.randn(sn, d, generator=g), torch.randint(0, c, (sn,), generator=g)
+        ostats, ograds = O.uml_step_grads(st, xi if si else None, yi if si else None, xt if sn else None,
+                                          yt if sn else None, alpha)
+        opt.step(ograds)
+        for n, t in ((si, temps[0]), (sn, temps[1])):
+            if n and learnable:
+                t.step += 1
+        img = RunIn(xi, yi, s_img, 1.0, temps[0] if learnable else None) if si else None
+        txt = RunIn(xt, yt, s_txt, alpha, temps[1] if learnable else None) if sn else None
+        wp_before = ad.Wp.clone()
+        out = adapter_step(W, ad, img, txt, hp, step, m, v)
+        k = 0
+        for n, lk, ak in ((si, "image_loss", "img_acc"), (sn, "text_loss", "text_acc")):
+            if n:
+                assert math.isclose(out["stats"][k]["loss_mean"], ostats[lk], rel_tol=2e-5, abs_tol=1e-6)
+                assert out["stats"][k]["correct"] == round(ostats[ak] * n)
+                k += 1
+        _close(out["dW"], ograds["head.weight"])
+        _close(out["W"], st.head)
+        if si:
+            _close(out["Z"], xi.double() @ wp_before.t())
+            _close(out["dWp"], ograds["img_proj.weight"])
+            assert out["Wp_step"] == ad.step + 1
+        else:
+            assert out["dWp"] is None and out["Wp_step"] == ad.step
+            assert torch.equal(out["Wp"], ad.Wp) and torch.equal(out["Wp_m"], ad.m)
+        _close(out["Wp"], st.img_proj)
+        W, m, v = out["W"], out["m"], out["v"]
+        ad = Adapter(out["Wp"], out["Wp_m"], out["Wp_v"], out["Wp_step"])
+        if learnable:
+            k = 0
+            for n, t, key in ((si, temps[0], "img_scale"), (sn, temps[1], "txt_scale")):
+                if not n:
+                    continue
+                tv, tm, tvv = out["temps"][k]
+                assert math.isclose(float(tv), float(st.scales[key]), rel_tol=2e-6, abs_tol=1e-7)
+                t.value, t.m, t.v = tv, tm, tvv
+                k += 1
+    assert ad.step == sum(1 for si, _ in plan if si)
 
 
 @pytest.mark.parametrize("kind", ["adamw", "adam", "sgd"])
