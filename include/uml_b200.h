@@ -335,6 +335,57 @@ int uml_gauss_eval(const float* params, int32_t dim_obs, int32_t dim_common, int
                    const float* data_y, int64_t n_rows, float* workspace /* >= 2*ceil(n_rows/16) floats */,
                    float* loss_out, void* stream);
 
+/* ---- a-14 grid: K runs of the Gaussian experiment (one model shape, one dataset, one batch size) in lock step --------
+ * The combinations of the reference's YAML grid (main.py) trained together: run k has its own parameters and Adam
+ * moments (row k of the [n_runs][param_stride] slabs), index batch per step, mode, alpha_x, alpha_y, lr and active
+ * flag; betas, eps and the Adam step count are shared.  One step of all runs is two launches (the run is a grid
+ * dimension of both kernels), and run k computes exactly what uml_gauss_run computes for it alone, bit for bit.
+ * A run with active[k] == 0 is not touched: parameters, moments and its rows of both logs stay as they are.
+ * Probes (eval_every > 0): after the update of the call's step i with (eval_phase + i + 1) % eval_every == 0, every
+ * active run's {val_loss_x, val_loss_y, linear CKA, mutual top-k NN} of its validation rows (what uml_gauss_eval,
+ * uml_gauss_embed, uml_cka_linear_f32 and uml_mutual_knn_f32 return for those weights, bit for bit) goes to the next
+ * row of eval_log - on the device, without a host synchronisation.
+ * Contract, checked before anything touches the device: 1..32 runs; non-null data, slabs, loss_log and workspace
+ * (16-byte aligned, workspace_bytes >= uml_gauss_group_workspace_bytes(n_runs, dims, batch, n_val, topk), n_val = 0
+ * without probes); param_stride >= uml_gauss_param_count; mode_xy 0 or 1; with probes: validation rows of every
+ * active run, eval_log, 2 <= n_val, 1 <= topk <= 64, topk < n_val.                                            */
+#define UML_GAUSS_GROUP_MAX_RUNS 32
+typedef struct {
+  int32_t      n_runs, dim_obs, dim_common, dim_latent;
+  const float* data_x;          /* [n_x, dim_obs] rows shared by every run (UnpairedDataset)                   */
+  int64_t      n_x;
+  const float* data_y;          /* [n_y, dim_obs]                                                              */
+  int64_t      n_y;
+  int64_t      batch;           /* rows per index batch (the same for every run)                               */
+  float*       params;          /* [n_runs][param_stride] flat parameters, uml_gauss_step's layout per run     */
+  float*       adam_m;          /* same layout                                                                  */
+  float*       adam_v;
+  int64_t      param_stride;
+  double       beta1, beta2, eps;
+  int64_t      first_step;      /* 1-based Adam step of the call's first step (all runs alike)                 */
+  int32_t      mode_xy[UML_GAUSS_GROUP_MAX_RUNS];   /* 1: alpha_x MSE(x) + alpha_y MSE(y); 0: MSE(x) alone      */
+  float        alpha_x[UML_GAUSS_GROUP_MAX_RUNS];
+  float        alpha_y[UML_GAUSS_GROUP_MAX_RUNS];
+  double       lr[UML_GAUSS_GROUP_MAX_RUNS];
+  uint8_t      active[UML_GAUSS_GROUP_MAX_RUNS];
+  float*       loss_log;        /* out [n_steps][n_runs][2]: {loss_x, loss_y} of every step                    */
+  int32_t      eval_every;      /* 0: no probes                                                                 */
+  int32_t      topk;            /* neighbours of the mutual-kNN probe (the reference: 10)                      */
+  int64_t      eval_phase;      /* steps of the evaluation schedule before the call's first step               */
+  int64_t      n_val;           /* validation rows of every run                                                 */
+  const float* val_x[UML_GAUSS_GROUP_MAX_RUNS];     /* [n_val, dim_obs] validation rows of run k               */
+  const float* val_y[UML_GAUSS_GROUP_MAX_RUNS];
+  float*       eval_log;        /* out [evaluations of the call][n_runs][4]: {val_x, val_y, cka, mknn}          */
+  void*        workspace;       /* scratch: gradient slots, per-tile losses, the runs' validation embeddings
+                                   ([n_runs][n_val][dim_latent] x 2), CKA Gram partials, neighbour lists        */
+  int64_t      workspace_bytes;
+} uml_gauss_group_args;
+int64_t uml_gauss_group_workspace_bytes(int32_t n_runs, int32_t dim_obs, int32_t dim_common, int32_t dim_latent,
+                                        int64_t batch, int64_t n_val, int32_t topk);   /* a COUNT, not a status */
+/* n_steps steps: idx is a HOST array [n_steps][n_runs] of device index batches (entries of inactive runs unused) */
+int uml_gauss_group_run(const uml_gauss_group_args* args /*host*/, int32_t n_steps, const int64_t* const* idx /*host*/,
+                        void* stream);
+
 /* ---- f-3  alignment probes (diagnostics logged beside the loops: metrics.py:55-119,252-285 of the reference, called at
  * Gaussian_experiment/main.py:67-84 and vision_language/finetune.py:209-233) --------------------------------------
  * uml_cka_linear_f32: out[0] = linear CKA with the biased HSIC estimator of A [n, da] and B [n, db] (row pitches lda /

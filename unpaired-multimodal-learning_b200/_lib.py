@@ -81,6 +81,22 @@ class SweepDiag(C.Structure):
     _fields_ = [("out", c_vp), ("scratch", c_vp), ("scratch_floats", c_i64), ("ev", c_vp * 2)]
 
 
+GAUSS_GROUP_MAX_RUNS = 32
+
+
+class GaussGroupArgs(C.Structure):
+    """uml_gauss_group_args"""
+    _fields_ = [("n_runs", c_i32), ("dim_obs", c_i32), ("dim_common", c_i32), ("dim_latent", c_i32),
+                ("data_x", c_vp), ("n_x", c_i64), ("data_y", c_vp), ("n_y", c_i64), ("batch", c_i64),
+                ("params", c_vp), ("adam_m", c_vp), ("adam_v", c_vp), ("param_stride", c_i64),
+                ("beta1", c_f64), ("beta2", c_f64), ("eps", c_f64), ("first_step", c_i64),
+                ("mode_xy", c_i32 * GAUSS_GROUP_MAX_RUNS), ("alpha_x", c_f32 * GAUSS_GROUP_MAX_RUNS),
+                ("alpha_y", c_f32 * GAUSS_GROUP_MAX_RUNS), ("lr", c_f64 * GAUSS_GROUP_MAX_RUNS),
+                ("active", C.c_uint8 * GAUSS_GROUP_MAX_RUNS), ("loss_log", c_vp), ("eval_every", c_i32), ("topk", c_i32),
+                ("eval_phase", c_i64), ("n_val", c_i64), ("val_x", c_vp * GAUSS_GROUP_MAX_RUNS),
+                ("val_y", c_vp * GAUSS_GROUP_MAX_RUNS), ("eval_log", c_vp), ("workspace", c_vp), ("workspace_bytes", c_i64)]
+
+
 # name -> argtypes; every function returns int except uml_last_error
 PROTOTYPES = {
     "uml_abi_version": [],
@@ -147,6 +163,8 @@ PROTOTYPES = {
     "uml_gauss_run": [c_vp, c_vp, c_vp, c_i32, c_i32, c_i32, c_vp, c_i64, c_vp, c_i64, c_vp, c_i32, c_i64, c_i32, c_f32, c_f32,
                       c_f64, c_f64, c_f64, c_f64, c_i64, c_vp, c_vp, c_vp],
     "uml_gauss_eval": [c_vp, c_i32, c_i32, c_i32, c_vp, c_vp, c_i64, c_vp, c_vp, c_vp],
+    "uml_gauss_group_workspace_bytes": [c_i32, c_i32, c_i32, c_i32, c_i64, c_i64, c_i32],
+    "uml_gauss_group_run": [C.POINTER(GaussGroupArgs), c_i32, c_vp, c_vp],
     "uml_sweep_run": [C.POINTER(SweepArgs), c_i32, c_vp, c_vp, c_vp],
     "uml_sweep_adapter_run": [C.POINTER(SweepArgs), C.POINTER(SweepAdapterArgs), c_i32, c_vp, c_vp, c_vp],
     "uml_sweep_diag_scratch_floats": [c_i32, c_i32, c_i32],
@@ -208,6 +226,7 @@ def load() -> C.CDLL:
         if name in KERNELS_PER_CALL:
             setattr(lib, name, _Counted(fn, KERNELS_PER_CALL[name]))
     lib.uml_sweep_diag_scratch_floats.restype = c_i64
+    lib.uml_gauss_group_workspace_bytes.restype = c_i64
     if lib.uml_abi_version() != 1:
         raise UmlLibraryError("libuml_b200.so ABI version mismatch")
     _lib = lib

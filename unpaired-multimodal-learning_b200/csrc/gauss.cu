@@ -136,11 +136,13 @@ struct GaussData {
   float dscale[2];        // alpha_m * 2 / (B * obs); 0 => no gradient for that modality (forward + loss only)
 };
 
-__global__ void __launch_bounds__(kGaussThreads)
-    gauss_fwd_bwd_kernel(const float* __restrict__ P, GaussLayout L, GaussData D, float* __restrict__ partial,
-                         float* __restrict__ loss_part) {
+// One CTA of the step: modality m, rows [tile * 16, tile * 16 + 16) of the batch.  `partial` and `loss_part` are the
+// run's own buffers.  The single-run kernel and the group kernel both run this body, so a run of a group computes
+// exactly what it computes alone.
+__device__ __forceinline__ void gauss_fwd_bwd_cta(const float* __restrict__ P, const GaussLayout& L, const GaussData& D,
+                                                  float* __restrict__ partial, float* __restrict__ loss_part, int m,
+                                                  int tile, int n_tiles) {
   extern __shared__ __align__(16) float sm[];
-  const int m = blockIdx.y, tile = blockIdx.x, n_tiles = gridDim.x;
   const int obs = L.obs, com = L.com, lat = L.lat;
   constexpr int R = kGaussRows;
   // ---- carve shared memory
@@ -229,14 +231,22 @@ __global__ void __launch_bounds__(kGaussThreads)
   dense_bwd_weight(dA, v, obs, com, g + L.in_w[m], g + L.in_b[m]);
 }
 
+__global__ void __launch_bounds__(kGaussThreads)
+    gauss_fwd_bwd_kernel(const float* __restrict__ P, GaussLayout L, GaussData D, float* __restrict__ partial,
+                         float* __restrict__ loss_part) {
+  gauss_fwd_bwd_cta(P, L, D, partial, loss_part, blockIdx.y, blockIdx.x, gridDim.x);
+}
+
 struct GaussAdam {
   float beta1, beta2, one_m_b1, one_m_b2, eps, step_size, bc2_sqrt_inv;
 };
 
-__global__ void __launch_bounds__(256)
-    gauss_update_kernel(float* __restrict__ P, float* __restrict__ M, float* __restrict__ V, GaussLayout L,
-                        const float* __restrict__ partial, int n_tiles, int grad_x, int grad_y, GaussAdam A,
-                        const float* __restrict__ loss_part, float inv_count, float* __restrict__ loss_out) {
+// Parameter i of one run (and, in block 0, the run's {loss_x, loss_y} record); shared by the single-run and group kernels
+__device__ __forceinline__ void gauss_update_elem(float* __restrict__ P, float* __restrict__ M, float* __restrict__ V,
+                                                  const GaussLayout& L, const float* __restrict__ partial, int n_tiles,
+                                                  int grad_x, int grad_y, const GaussAdam& A,
+                                                  const float* __restrict__ loss_part, float inv_count,
+                                                  float* __restrict__ loss_out) {
   const int i = blockIdx.x * blockDim.x + threadIdx.x;
   if (blockIdx.x == 0 && threadIdx.x < 2 && loss_out) {  // {loss_x, loss_y} of this step, fixed summation order
     float t = 0.f;
@@ -263,6 +273,13 @@ __global__ void __launch_bounds__(256)
   P[i] = P[i] - A.step_size * (mm / (sqrtf(vv) * A.bc2_sqrt_inv + A.eps));
 }
 
+__global__ void __launch_bounds__(256)
+    gauss_update_kernel(float* __restrict__ P, float* __restrict__ M, float* __restrict__ V, GaussLayout L,
+                        const float* __restrict__ partial, int n_tiles, int grad_x, int grad_y, GaussAdam A,
+                        const float* __restrict__ loss_part, float inv_count, float* __restrict__ loss_out) {
+  gauss_update_elem(P, M, V, L, partial, n_tiles, grad_x, grad_y, A, loss_part, inv_count, loss_out);
+}
+
 static size_t gauss_smem_bytes(const GaussLayout& L) {
   const int obs = L.obs, com = L.com, lat = L.lat, R = kGaussRows;
   size_t f = static_cast<size_t>(com) * (obs + 1) + com + static_cast<size_t>(lat) * (com + 1) + lat +
@@ -270,6 +287,26 @@ static size_t gauss_smem_bytes(const GaussLayout& L) {
              static_cast<size_t>(obs) * (com + 1) + obs;
   f += static_cast<size_t>(R + 4) * (2 * obs + 3 * com + 7 * lat) + 4 * 32;  // + alignment slack of the carve
   return f * sizeof(float);
+}
+
+// gradient scale of each modality's MSE; "x" mode: loss = loss_x (no alpha), the y branch only reports its loss
+// (main.py:52-54)
+static void gauss_dscale(int32_t mode_xy, float alpha_x, float alpha_y, double cnt, float* dscale) {
+  dscale[0] = static_cast<float>((mode_xy ? alpha_x : 1.0) * 2.0 / cnt);
+  dscale[1] = mode_xy ? static_cast<float>(alpha_y * 2.0 / cnt) : 0.f;
+}
+
+static GaussAdam gauss_adam(double lr, double beta1, double beta2, double eps, int64_t step) {
+  GaussAdam A;
+  const double t = static_cast<double>(step);
+  A.beta1 = static_cast<float>(beta1);
+  A.beta2 = static_cast<float>(beta2);
+  A.one_m_b1 = static_cast<float>(1.0 - beta1);
+  A.one_m_b2 = static_cast<float>(1.0 - beta2);
+  A.eps = static_cast<float>(eps);
+  A.step_size = static_cast<float>(lr / (1.0 - std::pow(beta1, t)));
+  A.bc2_sqrt_inv = static_cast<float>(1.0 / std::sqrt(1.0 - std::pow(beta2, t)));
+  return A;
 }
 
 static int gauss_launch_fwd_bwd(const float* P, const GaussLayout& L, const GaussData& D, float* partial, float* loss_part,
@@ -286,6 +323,84 @@ static int gauss_launch_fwd_bwd(const float* P, const GaussLayout& L, const Gaus
   UML_CUDA(cudaGetLastError());
   return 0;
 }
+
+// ---- lock-step group of runs (uml_gauss_group_run): the run is grid dimension z of the forward/backward launch and y of
+// the update launch; each CTA runs the single-run body on its run's slab row, batch and buffers.
+constexpr int kGaussMaxRuns = UML_GAUSS_GROUP_MAX_RUNS;
+
+struct GaussGroupLaunch {
+  GaussData d[kGaussMaxRuns];      // run k: rows, index batch (nullptr: dense validation rows), gradient scales
+  float step_size[kGaussMaxRuns];  // Adam lr / (1 - beta1^t) of run k
+  int32_t slot[kGaussMaxRuns];     // grid index -> run (active runs only)
+};
+
+__global__ void __launch_bounds__(kGaussThreads)
+    gauss_group_fwd_bwd_kernel(const float* __restrict__ P, int64_t stride, GaussLayout L, GaussGroupLaunch G,
+                               float* __restrict__ partial, float* __restrict__ loss_part) {
+  const int k = G.slot[blockIdx.z];
+  const int64_t n_tiles = gridDim.x;
+  const GaussData D = G.d[k];
+  gauss_fwd_bwd_cta(P + k * stride, L, D, partial ? partial + k * 2 * n_tiles * L.total : nullptr,
+                    loss_part + k * 2 * n_tiles, blockIdx.y, blockIdx.x, gridDim.x);
+}
+
+// P == nullptr: losses only (validation); run k's {loss_x, loss_y} go to loss_out + k * loss_stride
+__global__ void __launch_bounds__(256)
+    gauss_group_update_kernel(float* __restrict__ P, float* __restrict__ M, float* __restrict__ V, int64_t stride,
+                              GaussLayout L, const float* __restrict__ partial, int n_tiles, GaussGroupLaunch G,
+                              GaussAdam A, const float* __restrict__ loss_part, float inv_count,
+                              float* __restrict__ loss_out, int loss_stride) {
+  const int k = G.slot[blockIdx.y];
+  A.step_size = G.step_size[k];
+  const int64_t w = P ? k * stride : 0;
+  gauss_update_elem(P ? P + w : nullptr, M ? M + w : nullptr, V ? V + w : nullptr, L,
+                    partial ? partial + static_cast<int64_t>(k) * 2 * n_tiles * L.total : nullptr, n_tiles,
+                    G.d[k].dscale[0] != 0.f, G.d[k].dscale[1] != 0.f, A, loss_part + k * 2 * n_tiles, inv_count,
+                    loss_out + k * loss_stride);
+}
+
+static int gauss_group_launch_fwd_bwd(const float* P, int64_t stride, const GaussLayout& L, const GaussGroupLaunch& G,
+                                      int n_active, int64_t rows, float* partial, float* loss_part, cudaStream_t st) {
+  const size_t smem = gauss_smem_bytes(L);
+  static size_t attr = 0;
+  if (smem > attr) {
+    UML_CUDA(cudaFuncSetAttribute(gauss_group_fwd_bwd_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                                  static_cast<int>(smem)));
+    attr = smem;
+  }
+  const int tiles = static_cast<int>((rows + kGaussRows - 1) / kGaussRows);
+  gauss_group_fwd_bwd_kernel<<<dim3(tiles, 2, n_active), kGaussThreads, smem, st>>>(P, stride, L, G, partial, loss_part);
+  UML_CUDA(cudaGetLastError());
+  return 0;
+}
+
+// byte offsets of the pieces of a group's workspace (each 256-byte aligned); n_val = 0: no probe scratch
+struct GaussGroupWs {
+  int64_t partial, loss_part, val_part, emb_x, emb_y, cka, knn, totals, total;
+};
+
+static GaussGroupWs gauss_group_ws(int n_runs, const GaussLayout& L, int64_t batch, int64_t n_val, int topk) {
+  GaussGroupWs W;
+  int64_t o = 0;
+  auto take = [&](int64_t bytes) { const int64_t r = o; o += (bytes + 255) & ~int64_t(255); return r; };
+  const int64_t K = n_runs, tiles = (batch + kGaussRows - 1) / kGaussRows, vtiles = (n_val + kGaussRows - 1) / kGaussRows;
+  const int64_t d2 = 2 * static_cast<int64_t>(L.lat);
+  W.partial = take(K * 2 * tiles * L.total * 4);
+  W.loss_part = take(K * 2 * tiles * 4);
+  W.val_part = take(K * 2 * vtiles * 4);
+  W.emb_x = take(K * n_val * L.lat * 4);
+  W.emb_y = take(K * n_val * L.lat * 4);
+  W.cka = take(n_val ? K * (d2 + 8 * d2 * d2) * 8 : 0);
+  W.knn = take(K * 2 * n_val * topk * 4);
+  W.totals = take(n_val ? K * 4 : 0);
+  W.total = o;
+  return W;
+}
+
+int gauss_group_alignment(const float* params, int64_t stride, int dim_obs, int dim_common, int dim_latent,
+                          const float* const* val_x, const float* const* val_y, int64_t n, int topk, const int32_t* slots,
+                          int n_active, int n_runs, float* emb_x, float* emb_y, double* cka_ws, int32_t* knn_ws,
+                          int32_t* totals, float* out, cudaStream_t st);  // probes.cu
 
 }  // namespace uml
 
@@ -317,20 +432,10 @@ int uml_gauss_step(float* params, float* adam_m, float* adam_v, int32_t dim_obs,
   D.idx = idx;
   D.B = batch;
   const double cnt = static_cast<double>(batch) * dim_obs;
-  // "x" mode: loss = loss_x (no alpha), the y branch only reports its loss (main.py:52-54)
-  D.dscale[0] = static_cast<float>((mode_xy ? alpha_x : 1.0) * 2.0 / cnt);
-  D.dscale[1] = mode_xy ? static_cast<float>(alpha_y * 2.0 / cnt) : 0.f;
+  gauss_dscale(mode_xy, alpha_x, alpha_y, cnt, D.dscale);
   int rc = gauss_launch_fwd_bwd(params, L, D, partial, loss_part, as_stream(stream));
   if (rc) return rc;
-  GaussAdam A;
-  const double t = static_cast<double>(step);
-  A.beta1 = static_cast<float>(beta1);
-  A.beta2 = static_cast<float>(beta2);
-  A.one_m_b1 = static_cast<float>(1.0 - beta1);
-  A.one_m_b2 = static_cast<float>(1.0 - beta2);
-  A.eps = static_cast<float>(eps);
-  A.step_size = static_cast<float>(lr / (1.0 - std::pow(beta1, t)));
-  A.bc2_sqrt_inv = static_cast<float>(1.0 / std::sqrt(1.0 - std::pow(beta2, t)));
+  const GaussAdam A = gauss_adam(lr, beta1, beta2, eps, step);
   gauss_update_kernel<<<(L.total + 255) / 256, 256, 0, as_stream(stream)>>>(
       params, adam_m, adam_v, L, partial, tiles, D.dscale[0] != 0.f, D.dscale[1] != 0.f, A, loss_part,
       static_cast<float>(1.0 / cnt), loss_out);
@@ -376,6 +481,110 @@ int uml_gauss_eval(const float* params, int32_t dim_obs, int32_t dim_common, int
                                                          static_cast<float>(1.0 / (static_cast<double>(n_rows) * dim_obs)),
                                                          loss_out);
   UML_CUDA(cudaGetLastError());
+  return 0;
+}
+
+int64_t uml_gauss_group_workspace_bytes(int32_t n_runs, int32_t dim_obs, int32_t dim_common, int32_t dim_latent,
+                                        int64_t batch, int64_t n_val, int32_t topk) {
+  return uml::gauss_group_ws(n_runs, uml::make_layout(dim_obs, dim_common, dim_latent), batch, n_val, topk).total;
+}
+
+int uml_gauss_group_run(const uml_gauss_group_args* a, int32_t n_steps, const int64_t* const* idx, void* stream) {
+  using namespace uml;
+  UML_REQUIRE(a && idx && n_steps >= 0, "gauss_group_run: null argument");
+  const int K = a->n_runs;
+  UML_REQUIRE(K >= 1 && K <= kGaussMaxRuns, "gauss_group_run: 1..%d runs (got %d)", kGaussMaxRuns, K);
+  UML_REQUIRE(a->dim_obs > 0 && a->dim_common > 0 && a->dim_latent > 0 && a->batch > 0 && a->n_x > 0 && a->n_y > 0,
+              "gauss_group_run: bad shape");
+  UML_REQUIRE(a->data_x && a->data_y && a->params && a->adam_m && a->adam_v && a->loss_log && a->workspace,
+              "gauss_group_run: null buffer");
+  const GaussLayout L = make_layout(a->dim_obs, a->dim_common, a->dim_latent);
+  UML_REQUIRE(a->param_stride >= L.total, "gauss_group_run: param_stride %lld is below the %d parameters of a run",
+              static_cast<long long>(a->param_stride), L.total);
+  UML_REQUIRE(a->first_step >= 1, "gauss_group_run: first_step must be >= 1");
+  UML_REQUIRE(a->eval_every >= 0 && a->eval_phase >= 0, "gauss_group_run: eval_every and eval_phase must be >= 0");
+  const size_t smem = gauss_smem_bytes(L);
+  UML_REQUIRE(smem <= 220 * 1024, "gauss_group_run: model too wide for the shared-memory resident kernel (%zu B)", smem);
+  const bool probes = a->eval_every > 0;
+  int32_t slots[kGaussMaxRuns];
+  int n_active = 0;
+  for (int k = 0; k < K; ++k) {
+    UML_REQUIRE(a->mode_xy[k] == 0 || a->mode_xy[k] == 1, "gauss_group_run: run %d: mode_xy must be 0 or 1", k);
+    if (!a->active[k]) continue;
+    slots[n_active++] = k;
+    if (probes)
+      UML_REQUIRE(a->val_x[k] && a->val_y[k], "gauss_group_run: run %d has no validation rows", k);
+  }
+  if (probes) {
+    UML_REQUIRE(a->eval_log, "gauss_group_run: null eval_log");
+    UML_REQUIRE(a->n_val >= 2 && a->topk >= 1 && a->topk <= 64 && a->topk < a->n_val,
+                "gauss_group_run: probes need n_val >= 2 and 1 <= topk <= min(64, n_val - 1)");
+    UML_REQUIRE((static_cast<size_t>(a->n_val) + a->dim_latent) * sizeof(float) <= 200 * 1024,
+                "gauss_group_run: at most ~50 000 validation rows (a row's similarities live in shared memory)");
+    UML_REQUIRE(128 * static_cast<size_t>(a->dim_common + a->dim_latent) * sizeof(float) <= 200 * 1024,
+                "gauss_group_run: dim_common + dim_latent too large for the embedding kernel's per-thread scratch");
+  }
+  const GaussGroupWs W = gauss_group_ws(K, L, a->batch, probes ? a->n_val : 0, probes ? a->topk : 0);
+  UML_REQUIRE(a->workspace_bytes >= W.total, "gauss_group_run: workspace holds %lld bytes, %lld needed",
+              static_cast<long long>(a->workspace_bytes), static_cast<long long>(W.total));
+  UML_REQUIRE((reinterpret_cast<uintptr_t>(a->workspace) & 15) == 0, "gauss_group_run: workspace must be 16-byte aligned");
+  for (int i = 0; i < n_steps; ++i)
+    for (int z = 0; z < n_active; ++z)
+      UML_REQUIRE(idx[static_cast<int64_t>(i) * K + slots[z]], "gauss_group_run: step %d has no index batch for run %d", i,
+                  slots[z]);
+  if (n_active == 0 || n_steps == 0) return 0;
+
+  cudaStream_t st = as_stream(stream);
+  char* ws = static_cast<char*>(a->workspace);
+  float* partial = reinterpret_cast<float*>(ws + W.partial);
+  float* loss_part = reinterpret_cast<float*>(ws + W.loss_part);
+  const int tiles = static_cast<int>((a->batch + kGaussRows - 1) / kGaussRows);
+  const double cnt = static_cast<double>(a->batch) * a->dim_obs;
+  GaussGroupLaunch G, V;
+  memset(&G, 0, sizeof(G));
+  memset(&V, 0, sizeof(V));
+  for (int k = 0; k < K; ++k) {
+    G.d[k].data[0] = a->data_x; G.d[k].data[1] = a->data_y;
+    G.d[k].n[0] = a->n_x; G.d[k].n[1] = a->n_y;
+    G.d[k].B = a->batch;
+    gauss_dscale(a->mode_xy[k], a->alpha_x[k], a->alpha_y[k], cnt, G.d[k].dscale);
+    V.d[k].data[0] = a->val_x[k]; V.d[k].data[1] = a->val_y[k];
+    V.d[k].n[0] = V.d[k].n[1] = a->n_val;
+    V.d[k].B = a->n_val;  // idx nullptr, dscale 0: forward + MSE over dense rows (uml_gauss_eval)
+  }
+  for (int z = 0; z < n_active; ++z) G.slot[z] = V.slot[z] = slots[z];
+  const int64_t stride = a->param_stride;
+  int64_t evals = 0;
+  for (int i = 0; i < n_steps; ++i) {
+    const GaussAdam A = gauss_adam(a->lr[0], a->beta1, a->beta2, a->eps, a->first_step + i);
+    for (int k = 0; k < K; ++k) {
+      G.d[k].idx = a->active[k] ? idx[static_cast<int64_t>(i) * K + k] : nullptr;
+      G.step_size[k] = gauss_adam(a->lr[k], a->beta1, a->beta2, a->eps, a->first_step + i).step_size;
+    }
+    int rc = gauss_group_launch_fwd_bwd(a->params, stride, L, G, n_active, a->batch, partial, loss_part, st);
+    if (rc) return rc;
+    gauss_group_update_kernel<<<dim3((L.total + 255) / 256, n_active), 256, 0, st>>>(
+        a->params, a->adam_m, a->adam_v, stride, L, partial, tiles, G, A, loss_part, static_cast<float>(1.0 / cnt),
+        a->loss_log + static_cast<int64_t>(i) * K * 2, 2);
+    UML_CUDA(cudaGetLastError());
+    if (!probes || (a->eval_phase + i + 1) % a->eval_every != 0) continue;
+    // probes of the weights after this step's update: validation losses, then the alignment of the embeddings
+    float* out = a->eval_log + evals++ * K * 4;
+    float* val_part = reinterpret_cast<float*>(ws + W.val_part);
+    rc = gauss_group_launch_fwd_bwd(a->params, stride, L, V, n_active, a->n_val, nullptr, val_part, st);
+    if (rc) return rc;
+    GaussAdam none;
+    memset(&none, 0, sizeof(none));
+    gauss_group_update_kernel<<<dim3(1, n_active), 256, 0, st>>>(
+        nullptr, nullptr, nullptr, stride, L, nullptr, static_cast<int>((a->n_val + kGaussRows - 1) / kGaussRows), V, none,
+        val_part, static_cast<float>(1.0 / (static_cast<double>(a->n_val) * a->dim_obs)), out, 4);
+    UML_CUDA(cudaGetLastError());
+    rc = gauss_group_alignment(a->params, stride, a->dim_obs, a->dim_common, a->dim_latent, a->val_x, a->val_y, a->n_val,
+                               a->topk, slots, n_active, K, reinterpret_cast<float*>(ws + W.emb_x),
+                               reinterpret_cast<float*>(ws + W.emb_y), reinterpret_cast<double*>(ws + W.cka),
+                               reinterpret_cast<int32_t*>(ws + W.knn), reinterpret_cast<int32_t*>(ws + W.totals), out, st);
+    if (rc) return rc;
+  }
   return 0;
 }
 

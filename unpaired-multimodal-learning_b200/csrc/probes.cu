@@ -22,11 +22,11 @@ namespace uml {
 
 constexpr int kProbeSplits = 8;   // row splits of the Gram accumulation (fp64 partials, summed in split order)
 
-__global__ void __launch_bounds__(256)
-    probe_col_mean_kernel(const float* __restrict__ A, int64_t lda, int da, const float* __restrict__ B, int64_t ldb, int db,
-                          int64_t n, double* __restrict__ mean) {
+// Every probe kernel's body is a device function of its CTA coordinates: the single-call kernels below and the group
+// kernels (one more grid dimension over the runs of a Gaussian group) run the same code in the same order.
+__device__ __forceinline__ void col_mean_cta(const float* __restrict__ A, int64_t lda, int da, const float* __restrict__ B,
+                                             int64_t ldb, int db, int64_t n, double* __restrict__ mean, int c) {
   __shared__ double sh[256];
-  const int c = blockIdx.x;
   const float* X = c < da ? A + c : B + (c - da);
   const int64_t ld = c < da ? lda : ldb;
   double s = 0.0;
@@ -40,14 +40,20 @@ __global__ void __launch_bounds__(256)
   if (threadIdx.x == 0) mean[c] = sh[0] / static_cast<double>(n);
 }
 
-// Z = [A | B] (d = da + db columns), centred: part[split][i][j] = sum over the split's rows of Zc[r][i] * Zc[r][j]
 __global__ void __launch_bounds__(256)
-    probe_gram_kernel(const float* __restrict__ A, int64_t lda, int da, const float* __restrict__ B, int64_t ldb, int db,
-                      int64_t n, const double* __restrict__ mean, double* __restrict__ part) {
+    probe_col_mean_kernel(const float* __restrict__ A, int64_t lda, int da, const float* __restrict__ B, int64_t ldb, int db,
+                          int64_t n, double* __restrict__ mean) {
+  col_mean_cta(A, lda, da, B, ldb, db, n, mean, blockIdx.x);
+}
+
+// Z = [A | B] (d = da + db columns), centred: part[split][i][j] = sum over the split's rows of Zc[r][i] * Zc[r][j]
+__device__ __forceinline__ void gram_tile_cta(const float* __restrict__ A, int64_t lda, int da, const float* __restrict__ B,
+                                              int64_t ldb, int db, int64_t n, const double* __restrict__ mean,
+                                              double* __restrict__ part, int tile_i, int tile_j, int split) {
   constexpr int T = 16, R = 64;
   __shared__ float zi[R][T + 1], zj[R][T + 1];
   const int d = da + db;
-  const int i0 = blockIdx.x * T, j0 = blockIdx.y * T, split = blockIdx.z;
+  const int i0 = tile_i * T, j0 = tile_j * T;
   if (j0 + T <= i0) return;  // the Gram matrix is symmetric: only tiles that touch the upper triangle are computed
   const int tx = threadIdx.x & 15, ty = threadIdx.x >> 4;
   const int64_t per = (n + kProbeSplits - 1) / kProbeSplits, r_lo = per * split, r_hi = r_lo + per < n ? r_lo + per : n;
@@ -74,9 +80,14 @@ __global__ void __launch_bounds__(256)
   if (i < d && j < d) part[(static_cast<int64_t>(split) * d + i) * d + j] = acc;
 }
 
+__global__ void __launch_bounds__(256)
+    probe_gram_kernel(const float* __restrict__ A, int64_t lda, int da, const float* __restrict__ B, int64_t ldb, int db,
+                      int64_t n, const double* __restrict__ mean, double* __restrict__ part) {
+  gram_tile_cta(A, lda, da, B, ldb, db, n, mean, part, blockIdx.x, blockIdx.y, blockIdx.z);
+}
+
 // kl = sum G_ab^2, kk = sum G_aa^2, ll = sum G_bb^2 (fixed order) -> out[0] = kl / (sqrt(kk * ll) + 1e-6)
-__global__ void __launch_bounds__(1024)
-    probe_cka_finish_kernel(const double* __restrict__ part, int da, int db, float* __restrict__ out) {
+__device__ __forceinline__ void cka_finish_cta(const double* __restrict__ part, int da, int db, float* __restrict__ out) {
   __shared__ double sh[3][1024];
   const int d = da + db;
   double kk = 0.0, ll = 0.0, kl = 0.0;
@@ -109,14 +120,18 @@ __global__ void __launch_bounds__(1024)
   if (threadIdx.x == 0) out[0] = static_cast<float>(sh[2][0] / (sqrt(sh[0][0] * sh[1][0]) + 1e-6));
 }
 
-// top-k inner-product neighbours of row blockIdx.x (self excluded the reference's way: its similarity is set to -1e8)
-__global__ void __launch_bounds__(256)
-    probe_knn_kernel(const float* __restrict__ X, int64_t ld, int d, int64_t n, int k, int32_t* __restrict__ idx_out) {
+__global__ void __launch_bounds__(1024)
+    probe_cka_finish_kernel(const double* __restrict__ part, int da, int db, float* __restrict__ out) {
+  cka_finish_cta(part, da, db, out);
+}
+
+// top-k inner-product neighbours of row i (self excluded the reference's way: its similarity is set to -1e8)
+__device__ __forceinline__ void knn_row_cta(const float* __restrict__ X, int64_t ld, int d, int64_t n, int k,
+                                            int32_t* __restrict__ idx_out, int64_t i) {
   extern __shared__ float sims[];  // [n] then the row itself [d]
   float* xi = sims + n;
   __shared__ float bv[8];
   __shared__ int bi[8];
-  const int64_t i = blockIdx.x;
   for (int c = threadIdx.x; c < d; c += blockDim.x) xi[c] = X[i * ld + c];
   __syncthreads();
   for (int64_t j = threadIdx.x; j < n; j += blockDim.x) {
@@ -152,7 +167,12 @@ __global__ void __launch_bounds__(256)
 }
 
 __global__ void __launch_bounds__(256)
-    probe_knn_count_kernel(const int32_t* __restrict__ ka, const int32_t* __restrict__ kb, int64_t n, int k, int32_t* __restrict__ total) {
+    probe_knn_kernel(const float* __restrict__ X, int64_t ld, int d, int64_t n, int k, int32_t* __restrict__ idx_out) {
+  knn_row_cta(X, ld, d, n, k, idx_out, blockIdx.x);
+}
+
+__device__ __forceinline__ void knn_count_block(const int32_t* __restrict__ ka, const int32_t* __restrict__ kb, int64_t n,
+                                                int k, int32_t* __restrict__ total) {
   const int64_t i = blockIdx.x * static_cast<int64_t>(blockDim.x) + threadIdx.x;
   int c = 0;
   if (i < n) {
@@ -165,17 +185,26 @@ __global__ void __launch_bounds__(256)
   if ((threadIdx.x & 31) == 0 && c) atomicAdd(total, c);  // integer sum: order does not matter
 }
 
+__global__ void __launch_bounds__(256)
+    probe_knn_count_kernel(const int32_t* __restrict__ ka, const int32_t* __restrict__ kb, int64_t n, int k, int32_t* __restrict__ total) {
+  knn_count_block(ka, kb, n, k, total);
+}
+
+__device__ __forceinline__ float knn_mean(int32_t total, int64_t n, int k) {
+  return static_cast<float>(static_cast<double>(total) / (static_cast<double>(n) * k));
+}
+
 __global__ void probe_knn_finish_kernel(const int32_t* __restrict__ total, int64_t n, int k, float* __restrict__ out) {
-  out[0] = static_cast<float>(static_cast<double>(total[0]) / (static_cast<double>(n) * k));
+  out[0] = knn_mean(total[0], n, k);
 }
 
 // latent = shared_encoder(in_head(row)) for both modalities of the Gaussian experiment (model.py:51-60): one thread per row
-__global__ void __launch_bounds__(128)
-    gauss_embed_kernel(const float* __restrict__ params, int dim_obs, int dim_common, int dim_latent, const float* __restrict__ data_x,
-                       const float* __restrict__ data_y, int64_t n_rows, float* __restrict__ emb_x, float* __restrict__ emb_y) {
+__device__ __forceinline__ void gauss_embed_row(const float* __restrict__ params, int dim_obs, int dim_common, int dim_latent,
+                                                const float* __restrict__ data_x, const float* __restrict__ data_y,
+                                                int64_t n_rows, float* __restrict__ emb_x, float* __restrict__ emb_y,
+                                                int mod /* 0: x, 1: y */) {
   extern __shared__ float scratch[];  // per thread: dim_common + dim_latent floats
   const int64_t row = blockIdx.x * static_cast<int64_t>(blockDim.x) + threadIdx.x;
-  const int mod = blockIdx.y;  // 0: x, 1: y
   const float* data = mod == 0 ? data_x : data_y;
   float* emb = mod == 0 ? emb_x : emb_y;
   if (!data || !emb || row >= n_rows) return;
@@ -207,13 +236,124 @@ __global__ void __launch_bounds__(128)
   }
 }
 
+__global__ void __launch_bounds__(128)
+    gauss_embed_kernel(const float* __restrict__ params, int dim_obs, int dim_common, int dim_latent, const float* __restrict__ data_x,
+                       const float* __restrict__ data_y, int64_t n_rows, float* __restrict__ emb_x, float* __restrict__ emb_y) {
+  gauss_embed_row(params, dim_obs, dim_common, dim_latent, data_x, data_y, n_rows, emb_x, emb_y, blockIdx.y);
+}
+
+// ---- the same probes for the runs of a Gaussian group (uml_gauss_group_run): the run is one more grid dimension and
+// every buffer has a run stride.  Run k's embeddings are emb_x / emb_y + k n d, its CKA scratch cka_ws + k (d2 + 8 d2^2)
+// with d2 = 2 d, its neighbour lists knn_ws + k 2 n topk (x, then y) and its neighbour count totals[k].
+__host__ __device__ __forceinline__ int64_t cka_ws_doubles(int64_t d) { return d + kProbeSplits * d * d; }
+
+struct GaussProbeRuns {
+  const float* val_x[UML_GAUSS_GROUP_MAX_RUNS];
+  const float* val_y[UML_GAUSS_GROUP_MAX_RUNS];
+  int32_t slot[UML_GAUSS_GROUP_MAX_RUNS];  // grid index -> run
+};
+
+__global__ void __launch_bounds__(128)
+    gauss_group_embed_kernel(const float* __restrict__ params, int64_t stride, int dim_obs, int dim_common, int dim_latent,
+                             GaussProbeRuns R, int64_t n, float* __restrict__ emb_x, float* __restrict__ emb_y) {
+  const int k = R.slot[blockIdx.z];
+  const int64_t e = static_cast<int64_t>(k) * n * dim_latent;
+  gauss_embed_row(params + k * stride, dim_obs, dim_common, dim_latent, R.val_x[k], R.val_y[k], n, emb_x + e, emb_y + e,
+                  blockIdx.y);
+}
+
+__global__ void __launch_bounds__(256)
+    probe_group_col_mean_kernel(const float* __restrict__ emb_x, const float* __restrict__ emb_y, int d, int64_t n,
+                                double* __restrict__ cka_ws, GaussProbeRuns R) {
+  const int k = R.slot[blockIdx.y];
+  const int64_t e = static_cast<int64_t>(k) * n * d;
+  col_mean_cta(emb_x + e, d, d, emb_y + e, d, d, n, cka_ws + k * cka_ws_doubles(2 * d), blockIdx.x);
+}
+
+__global__ void __launch_bounds__(256)
+    probe_group_gram_kernel(const float* __restrict__ emb_x, const float* __restrict__ emb_y, int d, int64_t n,
+                            double* __restrict__ cka_ws, GaussProbeRuns R) {
+  const int k = R.slot[blockIdx.z / kProbeSplits];
+  const int64_t e = static_cast<int64_t>(k) * n * d;
+  double* ws = cka_ws + k * cka_ws_doubles(2 * d);
+  gram_tile_cta(emb_x + e, d, d, emb_y + e, d, d, n, ws, ws + 2 * d, blockIdx.x, blockIdx.y, blockIdx.z % kProbeSplits);
+}
+
+__global__ void __launch_bounds__(256)
+    probe_group_knn_kernel(const float* __restrict__ emb_x, const float* __restrict__ emb_y, int d, int64_t n, int topk,
+                           int32_t* __restrict__ knn_ws, GaussProbeRuns R) {
+  const int k = R.slot[blockIdx.z];
+  const int64_t e = static_cast<int64_t>(k) * n * d;
+  knn_row_cta((blockIdx.y == 0 ? emb_x : emb_y) + e, d, d, n, topk, knn_ws + (2 * static_cast<int64_t>(k) + blockIdx.y) * n * topk,
+              blockIdx.x);
+}
+
+__global__ void __launch_bounds__(256)
+    probe_group_knn_count_kernel(const int32_t* __restrict__ knn_ws, int64_t n, int topk, int32_t* __restrict__ totals,
+                                 GaussProbeRuns R) {
+  const int k = R.slot[blockIdx.y];
+  const int32_t* ka = knn_ws + 2 * static_cast<int64_t>(k) * n * topk;
+  knn_count_block(ka, ka + n * topk, n, topk, totals + k);
+}
+
+// out[k][2] = CKA, out[k][3] = mutual kNN of run k (out[k][0..1] hold its validation losses)
+__global__ void __launch_bounds__(1024)
+    probe_group_finish_kernel(const double* __restrict__ cka_ws, int d, const int32_t* __restrict__ totals, int64_t n,
+                              int topk, float* __restrict__ out, GaussProbeRuns R) {
+  const int k = R.slot[blockIdx.x];
+  cka_finish_cta(cka_ws + k * cka_ws_doubles(2 * d) + 2 * d, d, d, out + 4 * k + 2);
+  if (threadIdx.x == 0) out[4 * k + 3] = knn_mean(totals[k], n, topk);
+}
+
+// Embeddings, CKA and mutual kNN of the validation rows of the active runs `slots[0..n_active)` of a Gaussian group
+// (arguments checked by the caller): five launches and a memset for all runs.
+int gauss_group_alignment(const float* params, int64_t stride, int dim_obs, int dim_common, int dim_latent,
+                          const float* const* val_x, const float* const* val_y, int64_t n, int topk, const int32_t* slots,
+                          int n_active, int n_runs, float* emb_x, float* emb_y, double* cka_ws, int32_t* knn_ws,
+                          int32_t* totals, float* out, cudaStream_t st) {
+  GaussProbeRuns R;
+  memset(&R, 0, sizeof(R));
+  for (int k = 0; k < UML_GAUSS_GROUP_MAX_RUNS; ++k) { R.val_x[k] = val_x[k]; R.val_y[k] = val_y[k]; }
+  for (int z = 0; z < n_active; ++z) R.slot[z] = slots[z];
+  const unsigned na = static_cast<unsigned>(n_active);
+  const size_t embed_smem = 128 * static_cast<size_t>(dim_common + dim_latent) * sizeof(float);
+  static size_t embed_attr = 0;
+  if (embed_smem > 48 * 1024 && embed_smem > embed_attr) {
+    UML_CUDA(cudaFuncSetAttribute(gauss_group_embed_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024));
+    embed_attr = 200 * 1024;
+  }
+  gauss_group_embed_kernel<<<dim3(static_cast<unsigned>((n + 127) / 128), 2, na), 128, embed_smem, st>>>(
+      params, stride, dim_obs, dim_common, dim_latent, R, n, emb_x, emb_y);
+  UML_CUDA(cudaGetLastError());
+  const int d2 = 2 * dim_latent;
+  probe_group_col_mean_kernel<<<dim3(d2, na), 256, 0, st>>>(emb_x, emb_y, dim_latent, n, cka_ws, R);
+  UML_CUDA(cudaGetLastError());
+  const unsigned tiles = static_cast<unsigned>((d2 + 15) / 16);
+  probe_group_gram_kernel<<<dim3(tiles, tiles, kProbeSplits * na), 256, 0, st>>>(emb_x, emb_y, dim_latent, n, cka_ws, R);
+  UML_CUDA(cudaGetLastError());
+  const size_t knn_smem = (static_cast<size_t>(n) + dim_latent) * sizeof(float);
+  static size_t knn_attr = 0;
+  if (knn_smem > 48 * 1024 && knn_smem > knn_attr) {
+    UML_CUDA(cudaFuncSetAttribute(probe_group_knn_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024));
+    knn_attr = 200 * 1024;
+  }
+  UML_CUDA(cudaMemsetAsync(totals, 0, n_runs * sizeof(int32_t), st));
+  probe_group_knn_kernel<<<dim3(static_cast<unsigned>(n), 2, na), 256, knn_smem, st>>>(emb_x, emb_y, dim_latent, n, topk,
+                                                                                      knn_ws, R);
+  UML_CUDA(cudaGetLastError());
+  probe_group_knn_count_kernel<<<dim3(static_cast<unsigned>((n + 255) / 256), na), 256, 0, st>>>(knn_ws, n, topk, totals, R);
+  UML_CUDA(cudaGetLastError());
+  probe_group_finish_kernel<<<na, 1024, 0, st>>>(cka_ws, dim_latent, totals, n, topk, out, R);
+  UML_CUDA(cudaGetLastError());
+  return 0;
+}
+
 }  // namespace uml
 
 extern "C" {
 
 int64_t uml_cka_workspace_doubles(int32_t da, int32_t db) {
-  const int64_t d = static_cast<int64_t>(da) + db;
-  return d + uml::kProbeSplits * d * d;
+  return uml::cka_ws_doubles(static_cast<int64_t>(da) + db);
 }
 
 int uml_cka_linear_f32(const float* A, int64_t lda, int32_t da, const float* B, int64_t ldb, int32_t db, int64_t n, double* ws,
