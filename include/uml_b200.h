@@ -282,6 +282,36 @@ typedef struct {
 int uml_linear_run(const uml_linear_step_args* base /*host*/, const uml_run_step* steps /*host*/, int32_t n_steps,
                    void* stream);
 
+/* Per-step gradient diagnostics of a single run (the reference's probes, finetune.py:190-206): the image-loss and the
+ * text-loss gradients of the head weights, A = X_img^T G[image rows] and B = X_txt^T G[text rows] / alpha, reduced on
+ * the device to out = {sum A.B, sum A^2, sum B^2, #(sign A == sign B)} (torch.sign: 0 equals only 0), from the step's
+ * own G and rows, i.e. at the weights before its update.  They only read, so the training results are bit-identical
+ * to the same call without diagnostics.
+ *   precision 0: G and the rows (seg[].rows / idx, dense when idx == NULL) through the sweep's 3xTF32 tensor-core
+ *                diagnostics pass and its fixed-order finish: two launches after the step's last launch;
+ *   precision 1: two split-K bf16 dW GEMMs over the image and the text rows of X16 and G into scratch, one launch that
+ *                sums each side's partials in split order and reduces them into per-block slots, one fixed-order finish
+ *                (up to four launches), after the step's dW launch and before its operand buffer is handed back to the
+ *                gather pipeline of uml_linear_run.
+ * The image run is seg[0] when has_img, the text run the remaining one; the image run's loss weight must be 1 (no
+ * data parallelism).  Contract, checked before anything touches the device: dim % 4 == 0 (precision 1: % 8), 16-byte
+ * aligned G and rows (X16 on precision 1) with leading dimensions that are multiples of 4 (ldg: 64 on precision 1),
+ * loss weight (alpha) > 0 when there are text rows, no data-parallel all-reduce, scratch_floats >=
+ * uml_linear_diag_scratch_floats(precision, rows of the largest step, dim, n_classes).                              */
+typedef struct {
+  float*   scratch;         /* device workspace                                                                  */
+  int64_t  scratch_floats;
+  int32_t  has_img;         /* seg[0] is the image run                                                           */
+} uml_linear_diag;
+int64_t uml_linear_diag_scratch_floats(int32_t precision, int64_t max_rows, int32_t dim, int32_t n_classes); /* a COUNT */
+/* uml_linear_run with step i's diagnostics written to out[i] (device float[4])                                    */
+int uml_linear_run_diag(const uml_linear_step_args* base /*host*/, const uml_run_step* steps /*host*/, int32_t n_steps,
+                        const uml_linear_diag* diag /*host*/, float* const* out /*host [n_steps]*/, void* stream);
+/* the diagnostics alone, of the step `args` describes whose G and rows (X16) are still in place: for the steps the
+ * host dispatches kernel by kernel (adapter heads: seg[0].rows is the fp32 adapter output Z, or bf16 Z in X16)       */
+int uml_linear_grad_diag(const uml_linear_step_args* args /*host*/, const uml_linear_diag* diag /*host*/, float* out,
+                         void* stream);
+
 /* ---- data parallel: NCCL all-reduce of the head gradient issued from inside the step --------------
  * uml_dp_unique_id fills a 128-byte NCCL id on one rank; every rank then calls uml_dp_init with it.
  * With args->dp_allreduce != 0 the step sums dW over the ranks (ncclAllReduce on `stream`) between the

@@ -81,6 +81,11 @@ class SweepDiag(C.Structure):
     _fields_ = [("out", c_vp), ("scratch", c_vp), ("scratch_floats", c_i64), ("ev", c_vp * 2)]
 
 
+class LinearDiag(C.Structure):
+    """uml_linear_diag"""
+    _fields_ = [("scratch", c_vp), ("scratch_floats", c_i64), ("has_img", c_i32)]
+
+
 GAUSS_GROUP_MAX_RUNS = 32
 
 
@@ -169,6 +174,9 @@ PROTOTYPES = {
     "uml_sweep_adapter_run": [C.POINTER(SweepArgs), C.POINTER(SweepAdapterArgs), c_i32, c_vp, c_vp, c_vp],
     "uml_sweep_diag_scratch_floats": [c_i32, c_i32, c_i32],
     "uml_sweep_run_diag": [C.POINTER(SweepArgs), C.POINTER(SweepAdapterArgs), C.POINTER(SweepDiag), c_i32, c_vp, c_vp, c_vp],
+    "uml_linear_diag_scratch_floats": [c_i32, c_i64, c_i32, c_i32],
+    "uml_linear_run_diag": [C.POINTER(LinearStepArgs), C.POINTER(RunStep), c_i32, C.POINTER(LinearDiag), c_vp, c_vp],
+    "uml_linear_grad_diag": [C.POINTER(LinearStepArgs), C.POINTER(LinearDiag), c_vp, c_vp],
     "uml_randperm_i64": [C.c_uint64, c_i64, c_vp],
     "uml_randperm_begin": [c_vp, C.c_uint64, c_i64, c_vp],
     "uml_randperm_advance": [c_vp, c_i64],
@@ -226,6 +234,7 @@ def load() -> C.CDLL:
         if name in KERNELS_PER_CALL:
             setattr(lib, name, _Counted(fn, KERNELS_PER_CALL[name]))
     lib.uml_sweep_diag_scratch_floats.restype = c_i64
+    lib.uml_linear_diag_scratch_floats.restype = c_i64
     lib.uml_gauss_group_workspace_bytes.restype = c_i64
     if lib.uml_abi_version() != 1:
         raise UmlLibraryError("libuml_b200.so ABI version mismatch")

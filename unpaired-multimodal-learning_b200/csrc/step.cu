@@ -2,7 +2,10 @@
 // (reference loop body, vision_language/finetune.py:163-195) without returning to Python in between.
 // At the reference's batch sizes the step is launch-latency bound, at throughput batch sizes the host
 // must stay ahead of a ~150 us GPU step - either way per-kernel Python dispatch is what limits it.
+#include <algorithm>
+
 #include "common.cuh"
+#include "grad_diag.cuh"
 
 namespace {
 inline void rec(void* ev, void* stream) {
@@ -89,8 +92,12 @@ struct StepHooks {
   int (*mid)(void*) = nullptr;
   void* mid_arg = nullptr;
   cudaEvent_t after_fwd_kernel = nullptr;
+  const uml_linear_diag* diag = nullptr;  // uml_linear_run_diag: the step's gradient diagnostics go to diag_out
+  float* diag_out = nullptr;
 };
 static int linear_step_impl(const uml_linear_step_args* a, void* stream, const StepHooks& hooks);
+static int linear_grad_diag(const uml_linear_step_args* a, const uml_linear_diag* d, float* out, cudaStream_t st);
+static int check_linear_diag(const uml_linear_step_args* a, const uml_linear_diag* d, const float* out);
 int uml_head_fwd_ce_bf16_ev(const uint16_t* X, int64_t n_rows, int32_t dim, const uint16_t* W, int32_t n_classes,
                             const int32_t* labels, const uml_tc_segments* segs, uint16_t* G, int64_t ldg, float* row_loss,
                             int32_t* row_pred, int32_t* row_correct, float* row_dscale, float* tile_ws, uml_seg_stats* stats,
@@ -145,7 +152,7 @@ static int dp_reduce_and_update(const uml_linear_step_args* a, int64_t np, void*
 }
 
 static int linear_run_continuous(const uml_linear_step_args* base, const uml_run_step* steps, int32_t n_steps, void* stream,
-                                 Pipe* pipe) {
+                                 Pipe* pipe, const uml_linear_diag* diag, float* const* diag_out) {
   using namespace uml;
   constexpr int kNb = 3, kDepth = 2;
   uml_linear_step_args a = *base;
@@ -217,6 +224,8 @@ static int linear_run_continuous(const uml_linear_step_args* base, const uml_run
     hooks.operand_free = pipe->freed[b];
     hooks.mid_arg = &next;
     hooks.after_fwd_kernel = next.mid;  // recorded right after the forward kernel, also for the next call's first gathers
+    hooks.diag = diag;
+    hooks.diag_out = diag ? diag_out[i] : nullptr;
     hooks.mid = [](void* p) -> int {
       Next* n = static_cast<Next*>(p);
       return n->t >= 0 ? (*n->launch)(n->t, n->mid) : 0;
@@ -233,11 +242,9 @@ static int linear_run_continuous(const uml_linear_step_args* base, const uml_run
   return 0;
 }
 
-extern "C" {
-
-int uml_linear_run(const uml_linear_step_args* base, const uml_run_step* steps, int32_t n_steps, void* stream) {
+static int linear_run_impl(const uml_linear_step_args* base, const uml_run_step* steps, int32_t n_steps,
+                           const uml_linear_diag* diag, float* const* diag_out, void* stream) {
   using namespace uml;
-  UML_REQUIRE(base && steps && n_steps >= 0, "linear_run: bad arguments");
   uml_linear_step_args a = *base;
   auto patch = [&](uml_linear_step_args& t, const uml_run_step& s) {
     for (int k = 0; k < t.nseg; ++k) {
@@ -279,7 +286,7 @@ int uml_linear_run(const uml_linear_step_args* base, const uml_run_step* steps, 
       all = shadow_gatherable(&t);
     }
     Pipe* cp = all ? get_pipe() : nullptr;
-    if (cp) return linear_run_continuous(base, steps, n_steps, stream, cp);
+    if (cp) return linear_run_continuous(base, steps, n_steps, stream, cp, diag, diag_out);
   }
   pipe_invalidate();
   // With a third operand buffer the gather runs TWO steps ahead: step i + 2's rows are copied while step i's dW and
@@ -297,7 +304,11 @@ int uml_linear_run(const uml_linear_step_args* base, const uml_run_step* steps, 
     patch(a, steps[i]);
     if (i > 0 && a.precision == 1) a.w16_valid = 1;  // the optimizer kernel of the previous step refreshed the shadow
     if (!pipe) {
-      const int rc = uml_linear_step(&a, stream);
+      StepHooks plain;  // (uml_linear_step)
+      plain.diag = diag;
+      plain.diag_out = diag ? diag_out[i] : nullptr;
+      pipe_invalidate();
+      const int rc = linear_step_impl(&a, stream, plain);
       if (rc) return rc;
       continue;
     }
@@ -346,6 +357,8 @@ int uml_linear_run(const uml_linear_step_args* base, const uml_run_step* steps, 
     hooks.operand_free = pipe->freed[b];
     hooks.mid_arg = &next;
     hooks.after_fwd_kernel = next.have ? pipe->mid : nullptr;
+    hooks.diag = diag;
+    hooks.diag_out = diag ? diag_out[i] : nullptr;
     hooks.mid = [](void* p) -> int {
       Next* n = static_cast<Next*>(p);
       if (!n->have) return 0;
@@ -367,6 +380,42 @@ int uml_linear_run(const uml_linear_step_args* base, const uml_run_step* steps, 
   return 0;
 }
 
+extern "C" {
+
+int uml_linear_run(const uml_linear_step_args* base, const uml_run_step* steps, int32_t n_steps, void* stream) {
+  UML_REQUIRE(base && steps && n_steps >= 0, "linear_run: bad arguments");
+  return linear_run_impl(base, steps, n_steps, nullptr, nullptr, stream);
+}
+
+int64_t uml_linear_diag_scratch_floats(int32_t precision, int64_t max_rows, int32_t dim, int32_t n_classes) {
+  if (max_rows < 1 || dim < 1 || n_classes < 1) return 0;
+  if (precision == 0) return static_cast<int64_t>((dim + 127) / 128) * ((n_classes + 63) / 64) * 4;
+  // bf16: per-block slots, then the split-K partials of A and of B (as many splits as a step of max_rows takes)
+  const int64_t splits = std::max(1, uml_tc_dw_splits(max_rows, dim, n_classes));
+  return 4 * static_cast<int64_t>(uml::grad_diag_partial_slots()) + 2 * splits * n_classes * static_cast<int64_t>(dim);
+}
+
+int uml_linear_run_diag(const uml_linear_step_args* base, const uml_run_step* steps, int32_t n_steps,
+                        const uml_linear_diag* diag, float* const* out, void* stream) {
+  UML_REQUIRE(base && steps && n_steps >= 0 && diag && (out || n_steps == 0), "linear_run_diag: bad arguments");
+  for (int i = 0; i < n_steps; ++i) {  // every step's contract before anything is enqueued
+    uml_linear_step_args t = *base;
+    for (int k = 0; k < t.nseg; ++k) {
+      t.seg[k].idx = steps[i].idx[k];
+      t.seg[k].n = steps[i].n[k];
+      t.seg[k].loss_weight = steps[i].loss_weight[k];
+    }
+    if (check_linear_diag(&t, diag, out[i])) return 1;
+  }
+  return linear_run_impl(base, steps, n_steps, diag, out, stream);
+}
+
+int uml_linear_grad_diag(const uml_linear_step_args* a, const uml_linear_diag* diag, float* out, void* stream) {
+  UML_REQUIRE(a, "linear_grad_diag: null args");
+  if (check_linear_diag(a, diag, out)) return 1;
+  return linear_grad_diag(a, diag, out, uml::as_stream(stream));
+}
+
 int uml_linear_step(const uml_linear_step_args* a, void* stream) {
   pipe_invalidate();  // (it gathers into the first operand buffer on the main stream)
   return linear_step_impl(a, stream, StepHooks());
@@ -380,7 +429,19 @@ int uml_linear_run_reset(void) {
 
 }  // extern "C"
 
+static int linear_step_body(const uml_linear_step_args* a, void* stream, const StepHooks& hooks);
+
+// The step, then its diagnostics when asked: the bf16 path runs them inside the step (after the dW launch, before the
+// operand buffer is handed back to the gather pipeline), the exact path - and a step without rows - after its last launch.
 static int linear_step_impl(const uml_linear_step_args* a, void* stream, const StepHooks& hooks) {
+  const int rc = linear_step_body(a, stream, hooks);
+  if (rc || !hooks.diag) return rc;
+  const int64_t total = a->seg[0].n + (a->nseg > 1 ? a->seg[1].n : 0);
+  if (a->precision == 1 && total > 0) return 0;
+  return linear_grad_diag(a, hooks.diag, hooks.diag_out, uml::as_stream(stream));
+}
+
+static int linear_step_body(const uml_linear_step_args* a, void* stream, const StepHooks& hooks) {
   using namespace uml;
   const bool pregathered = hooks.pregathered;
   const cudaEvent_t operand_free = hooks.operand_free;
@@ -540,6 +601,10 @@ static int linear_step_impl(const uml_linear_step_args* a, void* stream, const S
   }
   if (rc) return rc;
   rec(a->ev[5], stream);
+  if (hooks.diag) {  // X16 and G still hold this step's operands; X16 goes back to the gather pipeline only below
+    rc = linear_grad_diag(a, hooks.diag, hooks.diag_out, as_stream(stream));
+    if (rc) return rc;
+  }
   if (operand_free) UML_CUDA(cudaEventRecord(operand_free, as_stream(stream)));  // X16 / labels32 may be overwritten
   const int64_t np = static_cast<int64_t>(a->n_classes) * a->dim;
   if (!fused) {
@@ -569,4 +634,86 @@ static int linear_step_impl(const uml_linear_step_args* a, void* stream, const S
                                nullptr, stream);
   rec(a->ev[7], stream);
   return rc;
+}
+
+// ---------------------------------------------------------------------------------------------------------------------
+// gradient diagnostics of one step (uml_linear_run_diag, uml_linear_grad_diag)
+static bool aligned16(const void* ptr) { return (reinterpret_cast<uintptr_t>(ptr) & 15) == 0; }
+
+// the image run (nullptr: none) and the text run (nullptr: none) of a step
+static void diag_runs(const uml_linear_step_args* a, const uml_linear_diag* d, const uml_segment** img, const uml_segment** txt) {
+  *img = d->has_img ? &a->seg[0] : nullptr;
+  *txt = a->nseg > (d->has_img ? 1 : 0) ? &a->seg[d->has_img ? 1 : 0] : nullptr;
+}
+
+// bf16 scratch: [slots | A partials (cap planes of C * D) | B partials (cap planes)]
+static int64_t diag_partials_offset() { return 4 * static_cast<int64_t>(uml::grad_diag_partial_slots()); }
+static int64_t diag_partial_cap(const uml_linear_step_args* a, const uml_linear_diag* d) {
+  return (d->scratch_floats - diag_partials_offset()) / (2 * static_cast<int64_t>(a->n_classes) * a->dim);
+}
+
+static int check_linear_diag(const uml_linear_step_args* a, const uml_linear_diag* d, const float* out) {
+  UML_REQUIRE(a && d && d->scratch && out, "linear_grad_diag: null diagnostics buffer");
+  UML_REQUIRE(a->nseg >= 1 && a->nseg <= UML_MAX_SEGMENTS && (d->has_img == 0 || d->has_img == 1) &&
+                  !(a->nseg == 2 && !d->has_img),
+              "linear_grad_diag: seg[0] is the image run (has_img) and a second run is the text run");
+  UML_REQUIRE(!a->dp_allreduce && !a->dW_out, "linear_grad_diag: data-parallel steps have no per-step diagnostics");
+  UML_REQUIRE(a->precision == 0 || a->precision == 1, "linear_grad_diag: precision must be 0 or 1");
+  UML_REQUIRE(a->dim > 0 && a->n_classes > 0 && a->dim % (a->precision ? 8 : 4) == 0,
+              "linear_grad_diag: dim must be a multiple of %d", a->precision ? 8 : 4);
+  const uml_segment *img, *txt;
+  diag_runs(a, d, &img, &txt);
+  UML_REQUIRE(!txt || txt->n == 0 || txt->loss_weight > 0.f,
+              "linear_grad_diag: alpha %g <= 0, the text-loss gradient cannot be recovered from G",
+              static_cast<double>(txt ? txt->loss_weight : 0.f));
+  UML_REQUIRE(!img || img->n == 0 || img->loss_weight == 1.f, "linear_grad_diag: the image run's loss weight must be 1");
+  UML_REQUIRE(a->G && aligned16(a->G) && a->ldg % (a->precision ? 64 : 4) == 0 && a->ldg >= a->n_classes,
+              "linear_grad_diag: G must be 16-byte aligned with ldg a multiple of %d", a->precision ? 64 : 4);
+  if (a->precision == 0) {
+    for (int k = 0; k < a->nseg; ++k)
+      UML_REQUIRE(a->seg[k].n == 0 || (a->seg[k].rows && aligned16(a->seg[k].rows) && a->seg[k].ld % 4 == 0),
+                  "linear_grad_diag: run %d rows must be 16-byte aligned with ld a multiple of 4", k);
+  } else {
+    UML_REQUIRE(a->X16 && aligned16(a->X16), "linear_grad_diag: X16 must be 16-byte aligned");
+  }
+  const int64_t need = a->precision == 0 ? uml_linear_diag_scratch_floats(0, 1, a->dim, a->n_classes)
+                                         : diag_partials_offset() + 2 * static_cast<int64_t>(a->n_classes) * a->dim;
+  UML_REQUIRE(aligned16(d->scratch) && d->scratch_floats >= need, "linear_grad_diag: scratch holds %lld floats, %lld needed",
+              static_cast<long long>(d->scratch_floats), static_cast<long long>(need));
+  return 0;
+}
+
+static int linear_grad_diag(const uml_linear_step_args* a, const uml_linear_diag* d, float* out, cudaStream_t st) {
+  using namespace uml;
+  const uml_segment *img, *txt;
+  diag_runs(a, d, &img, &txt);
+  const int64_t n0 = img ? img->n : 0, n1 = txt ? txt->n : 0;
+  const float alpha = txt ? txt->loss_weight : 1.f;
+  if (n0 + n1 == 0) {
+    UML_CUDA(cudaMemsetAsync(out, 0, 4 * sizeof(float), st));
+    return 0;
+  }
+  if (a->precision == 0) {
+    const float* rows[2] = {img ? static_cast<const float*>(img->rows) : nullptr, txt ? static_cast<const float*>(txt->rows) : nullptr};
+    const int64_t* idx[2] = {img ? img->idx : nullptr, txt ? txt->idx : nullptr};
+    const int64_t ld[2] = {img ? img->ld : 0, txt ? txt->ld : 0};
+    return grad_diag_f32_one(rows, idx, ld, n0, n1, a->dim, a->n_classes, static_cast<const float*>(a->G), a->ldg, alpha,
+                             d->scratch, out, st);
+  }
+  // bf16: A over rows [0, n0) of X16 and G, B over rows [n0, n0 + n1) - 16-byte aligned sub-ranges (dim % 8 == 0,
+  // ldg % 64 == 0) - each as split-K partials into scratch, then one reduction and the finish
+  const int64_t n = static_cast<int64_t>(a->n_classes) * a->dim, cap = diag_partial_cap(a, d);
+  float* pa = d->scratch + diag_partials_offset();
+  float* pb = pa + cap * n;
+  const uint16_t* G = static_cast<const uint16_t*>(a->G);
+  int32_t na = 0, nb = 0;
+  if (n0 > 0) {
+    na = static_cast<int32_t>(std::min<int64_t>(cap, std::max(1, uml_tc_dw_splits(n0, a->dim, a->n_classes))));
+    if (uml_head_bwd_dw_bf16(G, a->ldg, a->X16, n0, a->dim, a->n_classes, pa, na, st)) return 1;
+  }
+  if (n1 > 0) {
+    nb = static_cast<int32_t>(std::min<int64_t>(cap, std::max(1, uml_tc_dw_splits(n1, a->dim, a->n_classes))));
+    if (uml_head_bwd_dw_bf16(G + n0 * a->ldg, a->ldg, a->X16 + n0 * a->dim, n1, a->dim, a->n_classes, pb, nb, st)) return 1;
+  }
+  return grad_diag_partials_one(n0 > 0 ? pa : nullptr, na, pb, nb, n, n1, alpha, d->scratch, out, st);
 }

@@ -27,6 +27,7 @@
 #include <cstdlib>
 
 #include "common.cuh"
+#include "grad_diag.cuh"
 
 namespace uml {
 namespace sweep {
@@ -75,12 +76,13 @@ __device__ __forceinline__ float seg_scale(const SweepDev& p, int head, bool is_
   return p.scale_dev ? p.scale_dev[2 * head + (is_txt ? 1 : 0)] : p.scale[is_txt ? 1 : 0];
 }
 
-// bank row and bank label of logical row r (image run first, then the text run) of head `head`
+// bank row and bank label of logical row r (image run first, then the text run) of head `head`; a run without a
+// permutation is dense (the single-run diagnostics of uml_linear_grad_diag: sequential batches, adapter output Z)
 __device__ __forceinline__ int64_t bank_row(const SweepDev& p, int head, int64_t r, bool& is_txt) {
   is_txt = r >= p.n0;
   const int64_t l = is_txt ? r - p.n0 : r;
   const int64_t* pm = is_txt ? p.perm[1][head] : p.perm[0][head];
-  return pm[(is_txt ? p.pos[1] : p.pos[0]) + l];
+  return pm ? pm[(is_txt ? p.pos[1] : p.pos[0]) + l] : l;
 }
 __device__ __forceinline__ const float* row_ptr(const SweepDev& p, int head, int64_t r) {
   if (p.zrows != nullptr && r < p.n0) return p.zrows + head * p.z_stride + r * p.z_ld;
@@ -1632,6 +1634,72 @@ __global__ void __launch_bounds__(32) sweep_grad_diag_finish_kernel(const __grid
   out[4 * head + j] = static_cast<float>(s);
 }
 
+// 6b. the same four sums for a single run on the bf16 tensor-core path (uml::grad_diag_partials_one): A and B arrive as
+//     the split-K partials of two dW GEMMs ([na][n] and [nb][n], n = C * D, n % 4 == 0; na == 0: no image rows, A = 0).
+//     Grid-strided over float4 groups of elements, each element's partials summed in split order; every block writes
+//     its sums to its own slot of `part`, finished by sweep_grad_diag_finish_kernel (units = blocks): no float atomics,
+//     a fixed order for the fixed grid.                                                 grid (kDiagPartialBlocks), 256
+constexpr int kDiagPartialBlocks = 296;
+
+__global__ void __launch_bounds__(256) linear_grad_diag_partials_kernel(const float* __restrict__ pa, int na,
+                                                                        const float* __restrict__ pb, int nb, int64_t n,
+                                                                        float* __restrict__ part) {
+  __shared__ float red[8][3];
+  __shared__ int red_n[8];
+  const int64_t n4 = n / 4;
+  const float4* a4 = reinterpret_cast<const float4*>(pa);
+  const float4* b4 = reinterpret_cast<const float4*>(pb);
+  float dot = 0.f, aa = 0.f, bb = 0.f;
+  int agree = 0;
+  for (int64_t q = static_cast<int64_t>(blockIdx.x) * blockDim.x + threadIdx.x; q < n4;
+       q += static_cast<int64_t>(gridDim.x) * blockDim.x) {
+    float4 x = make_float4(0.f, 0.f, 0.f, 0.f), y = x;
+    for (int s = 0; s < na; ++s) {
+      const float4 v = a4[s * n4 + q];
+      x.x += v.x; x.y += v.y; x.z += v.z; x.w += v.w;
+    }
+    for (int s = 0; s < nb; ++s) {
+      const float4 v = b4[s * n4 + q];
+      y.x += v.x; y.y += v.y; y.z += v.z; y.w += v.w;
+    }
+    const float xs[4] = {x.x, x.y, x.z, x.w}, ys[4] = {y.x, y.y, y.z, y.w};
+#pragma unroll
+    for (int k = 0; k < 4; ++k) {
+      dot = fmaf(xs[k], ys[k], dot);
+      aa = fmaf(xs[k], xs[k], aa);
+      bb = fmaf(ys[k], ys[k], bb);
+      agree += ((xs[k] > 0.f) - (xs[k] < 0.f)) == ((ys[k] > 0.f) - (ys[k] < 0.f));  // torch.sign: 0 only equals 0
+    }
+  }
+  const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
+  dot = warp_sum(dot);
+  aa = warp_sum(aa);
+  bb = warp_sum(bb);
+  agree = warp_sum_i(agree);
+  if (lane == 0) {
+    red[warp][0] = dot;
+    red[warp][1] = aa;
+    red[warp][2] = bb;
+    red_n[warp] = agree;
+  }
+  __syncthreads();
+  if (threadIdx.x == 0) {
+    float s0 = 0.f, s1 = 0.f, s2 = 0.f;
+    int c = 0;
+    for (int w = 0; w < 8; ++w) {
+      s0 += red[w][0];
+      s1 += red[w][1];
+      s2 += red[w][2];
+      c += red_n[w];
+    }
+    float* o = part + static_cast<int64_t>(blockIdx.x) * 4;
+    o[0] = s0;
+    o[1] = s1;
+    o[2] = s2;
+    o[3] = static_cast<float>(c);  // exact: at most n / 296 elements per block, below 2^24 for any head that fits a GPU
+  }
+}
+
 // ---------------------------------------------------------------------------------------------------------------
 // 4. per-head, per-run {mean loss, hits, rows} in a fixed summation order   grid (2, K)
 // ---------------------------------------------------------------------------------------------------------------
@@ -1675,9 +1743,8 @@ int64_t uml_sweep_diag_scratch_floats(int32_t n_heads, int32_t dim, int32_t n_cl
   return static_cast<int64_t>(n_heads) * ((dim + 127) / 128) * ((n_classes + 63) / 64) * 4;
 }
 
-// Step i's gradient diagnostics (uml_sweep_run_diag): enqueued after the step's last update launch and before the next
-// step's first launch, so G and the rows (bank rows or Z) are still the step's own.
-static int launch_grad_diag(const uml::sweep::SweepDev& p, const uml_sweep_diag* dg, int K, int i, bool timed, cudaStream_t st) {
+// the tensor-core diagnostics pass and its finish over the running heads of p: out[head] for every running head
+static int launch_grad_diag_kernels(const uml::sweep::SweepDev& p, float* scratch, float* out, int K, cudaStream_t st) {
   using namespace uml;
   using namespace uml::sweep;
   static const cudaError_t attr =
@@ -1686,11 +1753,18 @@ static int launch_grad_diag(const uml::sweep::SweepDev& p, const uml_sweep_diag*
   const int per_head = ((p.dim + 127) / 128) * ((p.n_classes + 63) / 64);
   const int64_t units = static_cast<int64_t>(__builtin_popcount(p.active_mask)) * per_head;
   const unsigned g = static_cast<unsigned>(std::min<int64_t>(units, sm_count()));
+  sweep_grad_diag_tc_kernel<<<g, 256, kTcDiagSmemBytes, st>>>(p, scratch);
+  UML_CUDA(cudaGetLastError());
+  sweep_grad_diag_finish_kernel<<<K, 32, 0, st>>>(p, scratch, per_head, out);
+  UML_CUDA(cudaGetLastError());
+  return 0;
+}
+
+// Step i's gradient diagnostics (uml_sweep_run_diag): enqueued after the step's last update launch and before the next
+// step's first launch, so G and the rows (bank rows or Z) are still the step's own.
+static int launch_grad_diag(const uml::sweep::SweepDev& p, const uml_sweep_diag* dg, int K, int i, bool timed, cudaStream_t st) {
   if (timed && dg->ev[0]) UML_CUDA(cudaEventRecord(static_cast<cudaEvent_t>(dg->ev[0]), st));
-  sweep_grad_diag_tc_kernel<<<g, 256, kTcDiagSmemBytes, st>>>(p, dg->scratch);
-  UML_CUDA(cudaGetLastError());
-  sweep_grad_diag_finish_kernel<<<K, 32, 0, st>>>(p, dg->scratch, per_head, dg->out + static_cast<int64_t>(i) * K * 4);
-  UML_CUDA(cudaGetLastError());
+  if (launch_grad_diag_kernels(p, dg->scratch, dg->out + static_cast<int64_t>(i) * K * 4, K, st)) return 1;
   g_sweep_launches += 2;
   if (timed && dg->ev[1]) UML_CUDA(cudaEventRecord(static_cast<cudaEvent_t>(dg->ev[1]), st));
   return 0;
@@ -2143,3 +2217,42 @@ int uml_sweep_run_diag(const uml_sweep_args* a, const uml_sweep_adapter_args* ad
 }
 
 }  // extern "C"
+
+// Single-run diagnostics (grad_diag.cuh); the caller has checked the arguments.
+int uml::grad_diag_f32_one(const float* const rows[2], const int64_t* const idx[2], const int64_t ld[2], int64_t n0,
+                           int64_t n1, int32_t dim, int32_t n_classes, const float* G, int64_t ldg, float alpha,
+                           float* scratch, float* out, cudaStream_t st) {
+  uml::sweep::SweepDev p;
+  memset(&p, 0, sizeof(p));
+  for (int s = 0; s < 2; ++s) {
+    p.bank[s] = rows[s];
+    p.perm[s][0] = idx[s];
+    p.ld[s] = ld[s];
+  }
+  p.n0 = n0;
+  p.n1 = n1;
+  p.G = const_cast<float*>(G);  // (read only)
+  p.ldg = ldg;
+  p.dim = dim;
+  p.n_classes = n_classes;
+  p.alpha[0] = alpha;
+  p.active_mask = 1u;
+  return launch_grad_diag_kernels(p, scratch, out, 1, st);
+}
+
+int uml::grad_diag_partials_one(const float* pa, int32_t na, const float* pb, int32_t nb, int64_t n, int64_t n1, float alpha,
+                                float* slots, float* out, cudaStream_t st) {
+  using namespace uml::sweep;
+  linear_grad_diag_partials_kernel<<<kDiagPartialBlocks, 256, 0, st>>>(pa, na, pb, nb, n, slots);
+  UML_CUDA(cudaGetLastError());
+  SweepDev p;
+  memset(&p, 0, sizeof(p));
+  p.n1 = n1;
+  p.alpha[0] = alpha;
+  p.active_mask = 1u;
+  sweep_grad_diag_finish_kernel<<<1, 32, 0, st>>>(p, slots, kDiagPartialBlocks, out);
+  UML_CUDA(cudaGetLastError());
+  return 0;
+}
+
+int32_t uml::grad_diag_partial_slots() { return uml::sweep::kDiagPartialBlocks; }

@@ -64,4 +64,9 @@ _add("--sweep-batched-adapter", action="store_true", default=False,
           "'linear') also train in lock step (five launches per step of all heads) instead of one after the other")
 _add("--grad-diagnostics", action="store_true", default=False,
      help="log the reference's gradient probes (train/grad_direction_sim, img_grad_norm, txt_grad_norm, "
-          "grad_agreement_rate): every step for batched sweep groups, at evaluation cadence for single runs")
+          "grad_agreement_rate): every step for batched sweep groups, at evaluation cadence for single runs "
+          "(every step with --grad-diagnostics-every-step)")
+_add("--grad-diagnostics-every-step", action="store_true", default=False,
+     help="--grad-diagnostics, and single runs log the probes at every step as well, computed on the device from the "
+          "step's own rows at the weights before its update (exact and bf16 path, adapter heads included); data-parallel "
+          "runs, alpha <= 0 with text rows and head widths that are not multiples of 4 keep the evaluation cadence")

@@ -112,9 +112,24 @@ def ensure_dp_p2p(max_floats: int):
     _P2P_FLOATS = int(max_floats)
 
 
+def diag_blockers(model, world_size: int = 1, alpha: Optional[float] = None, has_txt: bool = True):
+    """Why a single run cannot log per-step gradient diagnostics (``StepEngine(grad_diagnostics=True)``; empty list:
+    it can).  The text-loss gradient is recovered from G, whose text rows carry alpha; the device passes read rows of
+    the head's width (bank rows, or the adapter output Z) in 16-byte units; the probes of a data-parallel step would
+    need the global gradients of both modalities."""
+    why = []
+    if int(world_size) > 1:
+        why.append("data-parallel runs have no per-step gradient diagnostics")
+    if alpha is not None and has_txt and float(alpha) <= 0:
+        why.append("gradient diagnostics need alpha > 0 when there are text rows")
+    if int(model.shared_dim) % 4:
+        why.append("gradient diagnostics need feature widths that are multiples of 4")
+    return why
+
+
 class StepEngine:
     def __init__(self, model, optimizer, device, max_img_rows: int, max_txt_rows: int, log_slots: int = 128,
-                 precision: str = "auto", dist_group=None, world_size: int = 1):
+                 precision: str = "auto", dist_group=None, world_size: int = 1, grad_diagnostics: bool = False):
         if precision not in ("auto", "fp32", "bf16"):
             raise ValueError("precision must be auto, fp32 or bf16")
         self.model, self.opt, self.device = model, optimizer, torch.device(device)
@@ -137,7 +152,18 @@ class StepEngine:
         self.ws32: Optional[ops.HeadWorkspace] = None
         self.ws16: Optional[ops.HeadWorkspace] = None
         self.log_slots = int(log_slots)
-        self.stats_log = torch.zeros((self.log_slots, 2, 4), device=self.device, dtype=torch.float32)
+        # grad_diagnostics: the reference's four gradient probes of every step (uml_linear_run_diag), stored beside the
+        # step's two uml_seg_stats records so that one copy reads both back
+        self.grad_diag = bool(grad_diagnostics)
+        if self.grad_diag:
+            why = diag_blockers(model, self.world)
+            if why:
+                raise ValueError("StepEngine: no per-step gradient diagnostics: " + "; ".join(why))
+            self._log = torch.zeros((self.log_slots, 3, 4), device=self.device, dtype=torch.float32)
+            self.stats_log, self.diag_log = self._log[:, :2], self._log[:, 2]
+            self._diag_scratch = None
+        else:
+            self._log = self.stats_log = torch.zeros((self.log_slots, 2, 4), device=self.device, dtype=torch.float32)
         self.slot_modalities = [None] * self.log_slots
         self.dW = None       # fp32 gradient buffer (data-parallel / unfused paths)
         self.Z = self.dZ = None
@@ -228,6 +254,52 @@ class StepEngine:
     def invalidate_shadow(self):
         """Call after the weights were changed outside the engine (e.g. load_state_dict)."""
         self._w16_valid = False
+
+    # ------------------------------------------------------------------------------------ per-step diagnostics
+    def _diag_struct(self, has_img: bool, bf16: bool):
+        """The uml_linear_diag struct of a step (scratch grown for the path on first use)."""
+        from .._lib import LinearDiag, load
+        need = int(load().uml_linear_diag_scratch_floats(int(bf16), self.max_rows, self.D, self.C))
+        if self._diag_scratch is None or self._diag_scratch.numel() < need:
+            self._diag_scratch = torch.empty(need, device=self.device, dtype=torch.float32)
+        d = LinearDiag()
+        d.scratch, d.scratch_floats, d.has_img = self._diag_scratch.data_ptr(), self._diag_scratch.numel(), int(has_img)
+        return d
+
+    @staticmethod
+    def _diag_launches(n_i: int, n_t: int, bf16: bool) -> int:
+        """Exact path: the diagnostics pass and its finish; bf16: a dW GEMM per modality with rows, reduction, finish."""
+        if n_i + n_t == 0:
+            return 0
+        return 2 + ((n_i > 0) + (n_t > 0) if bf16 else 0)
+
+    def _grad_diag_after(self, slot, bf16, runs):
+        """Diagnostics of the step the host just dispatched kernel by kernel, whose G and rows (X16 on the bf16 path) are
+        still in place.  ``runs``: (rows, idx, n, loss weight) of the image run (None: no image rows), then of the text
+        run; rows and idx are unused on the bf16 path."""
+        import ctypes as C
+        from .._lib import LAUNCH_COUNT, LinearStepArgs, check, load
+        a = LinearStepArgs()
+        a.dim, a.n_classes, a.precision = self.D, self.C, int(bf16)
+        k = 0
+        for r in runs:
+            if r is None:
+                continue
+            rows, idx, n, w = r
+            seg = a.seg[k]
+            seg.n, seg.loss_weight = n, w
+            if rows is not None:
+                seg.rows, seg.ld = rows.data_ptr(), rows.stride(0)
+                seg.idx = idx.data_ptr() if idx is not None else None
+            k += 1
+        a.nseg = k
+        ws = self.ws16 if bf16 else self.ws32
+        a.G, a.ldg = ws.G.data_ptr(), ws.ldg
+        a.X16 = self.X16.data_ptr() if bf16 else None
+        d = self._diag_struct(runs[0] is not None, bf16)
+        check(load().uml_linear_grad_diag(C.byref(a), C.byref(d), self.diag_log[slot].data_ptr(),
+                                          torch.cuda.current_stream().cuda_stream))
+        LAUNCH_COUNT[0] += self._diag_launches(runs[0][2] if runs[0] else 0, runs[1][2] if runs[1] else 0, bf16)
 
     # ------------------------------------------------------------------------------------ step
     def step(self, img: Optional[IndexBatch], txt: Optional[IndexBatch], alpha: float, slot: int,
@@ -348,6 +420,10 @@ class StepEngine:
         # (a step the fused exact-path kernel took is one launch instead of four)
         LAUNCH_COUNT[0] += self._kernels_per_step(k, bf16) - 3 * ((load().uml_head_step_fused_count() - f0) & 0x7fffffff)
         self._w16_valid = bf16
+        if self.grad_diag:  # G and the step's rows are still in place
+            check(load().uml_linear_grad_diag(C.byref(a), C.byref(self._diag_struct(n_i > 0, bf16)), self.diag_log[slot].data_ptr(),
+                                              torch.cuda.current_stream().cuda_stream))
+            LAUNCH_COUNT[0] += self._diag_launches(n_i, n_t, bf16)
 
     def run(self, batches, alpha, lrs, slot0):
         """Enqueue ``len(batches)`` consecutive iterations with as few host calls as possible.
@@ -381,7 +457,7 @@ class StepEngine:
             wst["step"] -= 1
             # how many following steps share this path (same modalities, same arithmetic)?
             m = j
-            steps = []
+            steps, diag_out = [], []
             ready, ready_seq, vouched = None, -1, True  # the newest 'indices uploaded' event among the chunk's batches
             while m < n_all:
                 ig, tg = batches[m]
@@ -414,6 +490,8 @@ class StepEngine:
                 slot = (slot0 + m) % self.log_slots
                 self.slot_modalities[slot] = (ig is not None and ig.n > 0, tg is not None and tg.n > 0)
                 rs.stats = self.stats_log[slot].data_ptr()
+                if self.grad_diag:
+                    diag_out.append(self.diag_log[slot].data_ptr())
                 if self.profile is not None:
                     names = ("gather_bf16", "head_fwd_ce_bf16" if bf16 else "head_fwd_ce_f32",
                              "head_bwd_dw_bf16" if bf16 else "head_bwd_dw_f32", "adamw_step_partials")
@@ -434,7 +512,13 @@ class StepEngine:
             a.idx_ready = ready.cuda_event if (vouched and ready is not None) else None
             arr = (RunStep * len(steps))(*steps)
             f0 = load().uml_head_step_fused_count()
-            check(load().uml_linear_run(C.byref(a), arr, len(steps), torch.cuda.current_stream().cuda_stream))
+            if self.grad_diag:
+                outs = (C.c_void_p * len(steps))(*diag_out)
+                check(load().uml_linear_run_diag(C.byref(a), arr, len(steps), C.byref(self._diag_struct(img_g is not None, bf16)),
+                                                 outs, torch.cuda.current_stream().cuda_stream))
+                LAUNCH_COUNT[0] += sum(self._diag_launches(int(rs.n[0]), int(rs.n[1]), bf16) for rs in steps)
+            else:
+                check(load().uml_linear_run(C.byref(a), arr, len(steps), torch.cuda.current_stream().cuda_stream))
             LAUNCH_COUNT[0] += self._kernels_per_step(k, bf16) * len(steps) - (0 if self._w16_valid or not bf16 else len(steps) - 1)
             LAUNCH_COUNT[0] -= 3 * ((load().uml_head_step_fused_count() - f0) & 0x7fffffff)
             self._w16_valid = bf16
@@ -496,6 +580,11 @@ class StepEngine:
                 ops.gemm_tn(self.dZ, rows, None, k=n_i, m=self.D, n=self.Dv, b_row_idx=idx, P=Wp.data,
                             update=self.opt.update_struct(Wp), ldc=Wp.data.stride(0))
         self._w16_valid = False
+        if self.grad_diag:  # the image side reads what the head saw: Z for an adapter head
+            ri = runs[0] if img is not None and n_i else None
+            rt = runs[-1] if txt is not None and n_t else None
+            self._grad_diag_after(slot, False, [(r.rows, r.idx, r.n, r.loss_weight) if r is not None else None
+                                                for r in (ri, rt)])
 
     def _apply_scalar(self, param, grad_view):
         if self.world > 1:
@@ -574,6 +663,8 @@ class StepEngine:
             self._timed("adamw_step_partials", ops.adamw_step_partials, W, self.partials, splits, st["m"], st["v"],
                         lr=g["lr"], step=st["step"], weight_decay=g["weight_decay"], betas=g["betas"], eps=g["eps"],
                         decoupled=(self.opt.name == "adamw"), shadow=self.W16)
+        if self.grad_diag:  # X16 and ws.G still hold the step's operands
+            self._grad_diag_after(slot, True, [(None, None, n_i, wi) if n_i else None, (None, None, n_t, wt) if n_t else None])
 
     # ------------------------------------------------------------------------------------ bf16 + adapter
     def _step_bf16_adapter(self, img, txt, n_i, n_t, wi, wt, slot):
@@ -650,6 +741,8 @@ class StepEngine:
             if side is not None:
                 torch.cuda.current_stream(dev).wait_event(self._dp_ev[1])
             self._apply_partials(Wp, self.partials_p, ps, self.Wp16, "dWp")
+        if self.grad_diag:  # X16 still holds [Z ; T] (the bf16 Z the head saw) and ws.G the step's G
+            self._grad_diag_after(slot, True, [(None, None, n_i, wi) if n_i else None, (None, None, n_t, wt) if n_t else None])
 
     def _apply_partials(self, param, partials, splits, shadow, buf_name):
         """Optimizer step of ``param`` from split-K partials (summed in the same kernel), with the
@@ -719,33 +812,36 @@ class StepEngine:
     def copy_slot_to_host(self, slot):
         """Asynchronous D2H of one step's stats record into a pinned host ring (no host sync)."""
         if self.host_log is None:
-            self.host_log = torch.zeros((self.log_slots, 2, 4), dtype=torch.float32).pin_memory()
+            self.host_log = torch.zeros(self._log.shape, dtype=torch.float32).pin_memory()
         slot %= self.log_slots
-        self.host_log[slot].copy_(self.stats_log[slot], non_blocking=True)
+        self.host_log[slot].copy_(self._log[slot], non_blocking=True)
 
     def copy_slots_to_host(self, slot0, n):
         """copy_slot_to_host for n consecutive steps with one asynchronous copy per contiguous run of ring slots."""
         if self.host_log is None:
-            self.host_log = torch.zeros((self.log_slots, 2, 4), dtype=torch.float32).pin_memory()
+            self.host_log = torch.zeros(self._log.shape, dtype=torch.float32).pin_memory()
         s = slot0 % self.log_slots
         while n > 0:
             k = min(n, self.log_slots - s)
-            self.host_log[s:s + k].copy_(self.stats_log[s:s + k], non_blocking=True)
+            self.host_log[s:s + k].copy_(self._log[s:s + k], non_blocking=True)
             n -= k
             s = 0
 
     def read_log(self, slots, from_host_ring=False):
         """Per-step stats for the given slots: one synchronising D2H of the device log, or - when every
-        step already pushed its record with ``copy_slot_to_host`` - a stream sync and a host read."""
+        step already pushed its record with ``copy_slot_to_host`` - a stream sync and a host read.  With
+        grad_diagnostics every record also carries ``"grad_diag"``: the step's four gradient-probe sums
+        (dot, |A|^2, |B|^2, sign agreements) for ``ops.grad_diag_record``."""
         from .._lib import load as _load_lib
         if self.world > 1 and _P2P_FLOATS and _load_lib().uml_dp_p2p_failed():
             raise RuntimeError("data-parallel step: a peer rank stopped answering the NVLink gradient exchange (UML_DP_TIMEOUT_S); "
                                "the affected steps applied no update - the replicas may no longer agree, restart from a checkpoint")
         if from_host_ring and self.host_log is not None:
             torch.cuda.current_stream().synchronize()
-            raw = self.host_log.clone()
+            raw_all = self.host_log.clone()
         else:
-            raw = self.stats_log.cpu()
+            raw_all = self._log.cpu()
+        raw = raw_all[:, :2]
         if self.ws16 is not None and _load_lib().uml_fwd_x_failed(self.ws16.fac.data_ptr()):
             raise RuntimeError("tensor-core step: a CTA waited a second for its peers (forward statistics exchange or the dW "
                                "kernel's split-K update); the affected step's results are undefined - restart from a checkpoint")
@@ -763,5 +859,7 @@ class StepEngine:
             if has_t:
                 n = max(1, int(ints[s, k, 3]))
                 rec["text_loss"], rec["text_acc"] = float(raw[s, k, 0]), int(ints[s, k, 2]) / n
+            if self.grad_diag:
+                rec["grad_diag"] = tuple(float(x) for x in raw_all[s, 2])
             out.append(rec)
         return out

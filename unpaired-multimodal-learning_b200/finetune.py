@@ -32,7 +32,7 @@ from .engine.optimizer.default import HYPER_DICT
 from .engine.optimizer.optim import build_optimizer
 from .engine.optimizer.scheduler import build_lr_scheduler
 from .engine.tools.utils import Tee, makedirs, set_random_seed
-from .engine.trainer import StepEngine
+from .engine.trainer import StepEngine, diag_blockers
 from .features import img_outdir, load_feature_bank, load_image_bank, load_text_bank, text_outdir
 
 EVAL_FREQ = 100  # evaluate on the val bank every 100 iterations (early stopping)
@@ -239,9 +239,20 @@ def train(model, image_loader, text_loader, val_loader, test_loader, optimizer, 
     def per_rank(loader, bs):  # a sharded (per-rank) loader's batch size already is the local one
         return bs if (loader is not None and getattr(loader, "shard_of", None)) else -(-bs // world)
 
+    # --grad-diagnostics-every-step (trace["grad_diagnostics"] == "step"): the reference's four gradient probes of every
+    # step, computed on the device from the step's own G and rows and read back with its losses
+    want_every_step = bool(getattr(args, "grad_diagnostics_every_step", False) or
+                           (trace is not None and trace.get("grad_diagnostics") == "step"))
+    every_step = want_every_step
+    if every_step:
+        why = diag_blockers(model, world, alpha, text_loader is not None)
+        if why:
+            print("=> --grad-diagnostics-every-step: " + "; ".join(why) + "; the gradient probes are logged at "
+                  "evaluation cadence instead")
+            every_step = False
     engine = StepEngine(model, optimizer, device, per_rank(image_loader, bs_i), per_rank(text_loader, bs_t),
                         log_slots=min(max(int(eval_freq), 1), int(max_iters)) + 1, precision=precision,
-                        dist_group=None, world_size=world)
+                        dist_group=None, world_size=world, grad_diagnostics=every_step)
     model._trained_bf16 = bool(engine._use_bf16(engine.max_rows))  # validate() follows the training path's precision
     if trace is not None:
         trace["engine"] = engine
@@ -259,18 +270,26 @@ def train(model, image_loader, text_loader, val_loader, test_loader, optimizer, 
             return
         recs = engine.read_log([s for s, _ in pending], from_host_ring=(stats_to_host == "step"))
         for (slot, lr), rec in zip(pending, recs):
+            sums = rec.pop("grad_diag", None)
+            diag = {}
+            if sums is not None:
+                has_i, has_t = engine.slot_modalities[slot % engine.log_slots]
+                diag = ops.grad_diag_record(*sums, engine.W.numel(), has_i and has_t)
+                if trace is not None:
+                    trace.setdefault("grad_diag", []).append((slot, diag))
             if trace is not None:
                 trace.setdefault("stats", []).append(dict(rec, lr=lr))
             if logger is not None:
                 logger.log({"train/image_loss": rec["image_loss"], "train/text_loss": rec["text_loss"],
-                            "train/image_acc": rec["img_acc"], "train/text_acc": rec["text_acc"], "train/lr": lr})
+                            "train/image_acc": rec["img_acc"], "train/text_acc": rec["text_acc"], "train/lr": lr, **diag})
         last = recs[-1]
         pending.clear()
 
     # Steps are enqueued in chunks that end at the next evaluation point, so that the host issues ONE library
     # call per chunk instead of a Python round trip per kernel; the loaders are advanced in the reference's order
     # (image batch, then text batch, per step) so the sampler stream is unchanged.
-    grad_diag = bool(getattr(args, "grad_diagnostics", False) or (trace is not None and trace.get("grad_diagnostics")))
+    grad_diag = bool(getattr(args, "grad_diagnostics", False) or (trace is not None and trace.get("grad_diagnostics")) or
+                     want_every_step) and not every_step
     if grad_diag and engine.adapter:  # StepEngine.grad_diagnostics covers the linear head only
         print("=> --grad-diagnostics: no gradient probes for a single run of a head with an image adapter (batched "
               "sweeps with --sweep-batched-adapter log them); training continues without them")
@@ -876,6 +895,8 @@ def main(args, alphas=None):
     args.use_clip = args.vision_model == "" and args.language_model == ""
     if getattr(args, "sweep_batched_adapter", False):
         args.sweep_batched = True
+    if getattr(args, "grad_diagnostics_every_step", False):  # (batched groups log the probes every step already)
+        args.grad_diagnostics = True
     encoder_name = args.clip_encoder if args.use_clip else f"{args.vision_model}-{args.language_model}"
     alpha_list = [float(a) for a in alphas] if alphas else [args.alpha]
     savepaths = [savedir(args.result_dir, args.dataset, encoder_name, args.train_shot, args.seed, args.text_type,
