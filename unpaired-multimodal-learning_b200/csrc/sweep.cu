@@ -11,15 +11,17 @@
 // own epoch permutation (device int64) at the common position `pos` - the heads share bank and batch sizes, so their
 // epochs turn over on the same steps.
 //
-// The two contractions exist in three forms:
-//   * tensor cores (default when rows are 16-byte aligned): tcgen05.mma kind::tf32 with every operand split into two tf32
-//     terms, i.e. fp32-level accuracy (section "Tensor-core forms" below); W, m, v of the update move through a TMA
-//     slot ring; softmax / CE in the logits epilogue when a head has at most eight class tiles (a cluster).  Measured on
-//     B200 with K = 30 heads of 1000 x 512: 0.134 ms per step of all heads (logits + softmax/CE 44 us, dW + update +
-//     statistics 76 = 0.76 of the HBM copy peak); with the separate softmax launch 0.139 ms (logits 36, softmax/CE 15);
-//   * FFMA with cp.async staging (UML_SWEEP_TC=0, and the dW + update of steps with more than 64 rows): 0.219 ms
-//     (logits 73, softmax/CE 15, dW + update 123 = 0.47 of the HBM peak, stats 7);
-//   * FFMA, register-staged (any alignment; UML_SWEEP_ASYNC=0): 0.268 ms.
+// The two contractions exist in three forms, chosen per call from the inputs:
+//   * tensor cores when the rows are 16-byte aligned (dim % 4 == 0, banks and G 16-byte aligned, bank_ld and ldg
+//     multiples of 4): tcgen05.mma kind::tf32 with every operand split into two tf32 terms, i.e. fp32-level accuracy
+//     (section "Tensor-core forms" below); W, m, v of the update move through a TMA slot ring.  Softmax / CE run in the
+//     logits epilogue when a head has at most eight class tiles (a cluster, <= 1024 classes), in a separate launch
+//     otherwise; the dW + update runs here for steps of at most 64 rows.  Measured on B200 with K = 30 heads of
+//     1000 x 512: 0.134 ms per step of all heads (logits + softmax/CE 44 us, dW + update + statistics 76 = 0.76 of the
+//     HBM copy peak); with the separate softmax launch 0.139 ms (logits 36, softmax/CE 15);
+//   * FFMA with cp.async staging: the same aligned rows with UML_SWEEP_TC=0, and the dW + update of steps with more
+//     than 64 rows: 0.219 ms (logits 73, softmax/CE 15, dW + update 123 = 0.47 of the HBM peak, stats 7);
+//   * FFMA, register-staged: rows that are not 16-byte aligned.  0.268 ms when aligned rows were forced onto it.
 // Per head the arithmetic of the FFMA forms is the single-head fp32 path's (simt.cu): sequential-k FFMA logits, the
 // same softmax / CE / argmax row kernel, dW summed over rows in order, torch.optim's update rules in the epilogue.  In
 // every form a head's result depends neither on its slot in the group nor on its neighbours.
@@ -978,7 +980,7 @@ __device__ __forceinline__ void tmem_ldn(uint32_t taddr, uint32_t (&v)[8]) {
                : "memory");
 }
 
-// kNT update threads per CTA plus one TMA warp and one statistics warp.  The update costs ~50 instructions per parameter (IEEE sqrt and division),
+// 512 update threads per CTA plus one TMA warp and one statistics warp.  The update costs ~50 instructions per parameter (IEEE sqrt and division),
 // so the read-back needs warps to hide its dependency chains as much as it needs bytes in flight (8 warps per SM left the
 // slots waiting for arithmetic), and nothing in it may wait for anything but its own data: an update warp waits for a
 // slot's loads, updates its share in place and arrives on the slot's `done` barrier; the TMA warp waits for that
@@ -1049,12 +1051,12 @@ __device__ __forceinline__ void g_tile_split(unsigned char* gs) {
   }
 }
 
-template <int kNT>
-__global__ void __launch_bounds__(kNT + 64, 1)
+constexpr int kTcDwThreads = 512;  // update threads per CTA; the TMA and statistics warps come on top
+
+__global__ void __launch_bounds__(kTcDwThreads + 64, 1)
     sweep_dw_update_tc_kernel(const __grid_constant__ SweepDev p, const __grid_constant__ CUtensorMap tm_w,
                               const __grid_constant__ CUtensorMap tm_m, const __grid_constant__ CUtensorMap tm_v) {
-  static_assert(kNT == 256 || kNT == 512, "8 or 4 classes of a stage per thread");
-  constexpr int BM = 128, BN = 64, kR = 64, NS = kTcDwSlots, kWarps = kNT / 32;
+  constexpr int BM = 128, BN = 64, kR = 64, NS = kTcDwSlots, kNT = kTcDwThreads, kWarps = kNT / 32;
   const int D = p.dim, C = p.n_classes;
   const int n_dt = (D + BM - 1) / BM, n_ct = (C + BN - 1) / BN, per_head = n_dt * n_ct;
   const int n_units = __popc(p.active_mask) * per_head;
@@ -1226,7 +1228,7 @@ __global__ void __launch_bounds__(kNT + 64, 1)
     sync_update_warps();
     if (t == 0) mma_unit(0);
 
-    constexpr int kCpt = 16 / (kNT / 128);  // classes of a stage per thread
+    constexpr int kCpt = 4;  // classes of a stage per thread: 16 warps, four lane quadrants x four class groups
     const int q = warp & 3, h = warp >> 2;  // TMEM lane quadrant (dims 32 q + lane), classes kCpt h + [0, kCpt) of a stage
     const uint32_t slot0 = smem_u32(slots) + static_cast<uint32_t>(((h * kCpt) * BM + q * 32 + lane) * 4);
     int gs = 0;  // stages read back so far (slot ring position)
@@ -1732,6 +1734,11 @@ __global__ void __launch_bounds__(256) sweep_stats_kernel(const __grid_constant_
 
 static long long g_sweep_launches = 0;  // kernels launched by uml_sweep_run in this process (launch accounting of the callers)
 
+// host-side view of the [K][rows][cols] W, m, v slabs for the tensor-core dW kernel's slot ring (v stays zero for SGD)
+struct SlabMaps {
+  CUtensorMap w, m, v;
+};
+
 extern "C" {
 
 int uml_sweep_launch_count(void) { return static_cast<int>(g_sweep_launches & 0x7fffffff); }
@@ -1743,13 +1750,32 @@ int64_t uml_sweep_diag_scratch_floats(int32_t n_heads, int32_t dim, int32_t n_cl
   return static_cast<int64_t>(n_heads) * ((dim + 127) / 128) * ((n_classes + 63) / 64) * 4;
 }
 
+// Dynamic shared memory of the tensor-core kernels, set by the first call in the process.
+static cudaError_t tc_smem_attributes() {
+  using namespace uml::sweep;
+  static const cudaError_t attr = [] {
+    const cudaFuncAttribute smem = cudaFuncAttributeMaxDynamicSharedMemorySize;
+    cudaError_t e = cudaFuncSetAttribute(sweep_logits_tc_kernel<false>, smem, kTcLgSmemBytes);
+    if (e == cudaSuccess) e = cudaFuncSetAttribute(sweep_logits_tc_kernel<true>, smem, kTcLgSmemBytes);
+    if (e == cudaSuccess) e = cudaFuncSetAttribute(sweep_dw_update_tc_kernel, smem, kTcDwSmemBytes);
+    if (e == cudaSuccess) e = cudaFuncSetAttribute(sweep_dz_tc_kernel, smem, kTcDzSmemBytes);
+    if (e == cudaSuccess) e = cudaFuncSetAttribute(sweep_grad_diag_tc_kernel, smem, kTcDiagSmemBytes);
+    return e;
+  }();
+  return attr;
+}
+
+// Records ev[e] on st; ev is NULL outside the timed (last) step of a call.
+static int mark(void* const* ev, int e, cudaStream_t st) {
+  if (ev && ev[e]) UML_CUDA(cudaEventRecord(static_cast<cudaEvent_t>(ev[e]), st));
+  return 0;
+}
+
 // the tensor-core diagnostics pass and its finish over the running heads of p: out[head] for every running head
 static int launch_grad_diag_kernels(const uml::sweep::SweepDev& p, float* scratch, float* out, int K, cudaStream_t st) {
   using namespace uml;
   using namespace uml::sweep;
-  static const cudaError_t attr =
-      cudaFuncSetAttribute(sweep_grad_diag_tc_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, kTcDiagSmemBytes);
-  UML_CUDA(attr);
+  UML_CUDA(tc_smem_attributes());
   const int per_head = ((p.dim + 127) / 128) * ((p.n_classes + 63) / 64);
   const int64_t units = static_cast<int64_t>(__builtin_popcount(p.active_mask)) * per_head;
   const unsigned g = static_cast<unsigned>(std::min<int64_t>(units, sm_count()));
@@ -1763,256 +1789,44 @@ static int launch_grad_diag_kernels(const uml::sweep::SweepDev& p, float* scratc
 // Step i's gradient diagnostics (uml_sweep_run_diag): enqueued after the step's last update launch and before the next
 // step's first launch, so G and the rows (bank rows or Z) are still the step's own.
 static int launch_grad_diag(const uml::sweep::SweepDev& p, const uml_sweep_diag* dg, int K, int i, bool timed, cudaStream_t st) {
-  if (timed && dg->ev[0]) UML_CUDA(cudaEventRecord(static_cast<cudaEvent_t>(dg->ev[0]), st));
+  void* const* ev = timed ? dg->ev : nullptr;
+  if (mark(ev, 0, st)) return 1;
   if (launch_grad_diag_kernels(p, dg->scratch, dg->out + static_cast<int64_t>(i) * K * 4, K, st)) return 1;
   g_sweep_launches += 2;
-  if (timed && dg->ev[1]) UML_CUDA(cudaEventRecord(static_cast<cudaEvent_t>(dg->ev[1]), st));
+  return mark(ev, 1, st);
+}
+
+// The checks uml_sweep_run and uml_sweep_adapter_run share, in this order; `who` names the entry point in the messages.
+static int check_sweep_args(const char* who, const uml_sweep_args* a, int32_t n_steps, const int64_t* rows, const float* lr) {
+  using uml::sweep::kMaxHeads;
+  UML_REQUIRE(a && rows && lr && n_steps >= 0, "%s: null argument", who);
+  UML_REQUIRE(a->n_heads >= 1 && a->n_heads <= kMaxHeads, "%s: 1..%d heads", who, kMaxHeads);
+  UML_REQUIRE(a->dim > 0 && a->n_classes > 0 && a->ldg >= a->n_classes, "%s: bad shape", who);
+  UML_REQUIRE(a->kind >= 1 && a->kind <= 3, "%s: optimizer kind must be 1 (AdamW), 2 (Adam) or 3 (SGD)", who);
+  UML_REQUIRE(a->W && a->m && (a->kind == 3 || a->v) && a->G && a->row_loss && a->row_correct && a->stats,
+              "%s: null buffer", who);
+  UML_REQUIRE(a->head_stride >= static_cast<int64_t>(a->n_classes) * a->dim, "%s: head_stride too small", who);
   return 0;
 }
 
-static int sweep_run_impl(const uml_sweep_args* a, const uml_sweep_diag* dg, int32_t n_steps, const int64_t* rows,
-                          const float* lr, void* stream) {
-  using namespace uml;
-  using namespace uml::sweep;
-  UML_REQUIRE(a && rows && lr && n_steps >= 0, "sweep_run: null argument");
-  const int K = a->n_heads;
-  UML_REQUIRE(K >= 1 && K <= kMaxHeads, "sweep_run: 1..%d heads", kMaxHeads);
-  UML_REQUIRE(a->dim > 0 && a->n_classes > 0 && a->ldg >= a->n_classes, "sweep_run: bad shape");
-  UML_REQUIRE(a->kind >= 1 && a->kind <= 3, "sweep_run: optimizer kind must be 1 (AdamW), 2 (Adam) or 3 (SGD)");
-  UML_REQUIRE(a->W && a->m && (a->kind == 3 || a->v) && a->G && a->row_loss && a->row_correct && a->stats,
-              "sweep_run: null buffer");
-  UML_REQUIRE(a->head_stride >= static_cast<int64_t>(a->n_classes) * a->dim, "sweep_run: head_stride too small");
-  if (a->dim % 4 == 0) {  // the vector epilogue's alignment contract
-    UML_REQUIRE(a->head_stride % 4 == 0 && (reinterpret_cast<uintptr_t>(a->W) & 15) == 0 &&
-                    (reinterpret_cast<uintptr_t>(a->m) & 15) == 0 && (reinterpret_cast<uintptr_t>(a->v) & 15) == 0,
-                "sweep_run: W, m, v slabs must be 16-byte aligned");
-  }
-  cudaStream_t st = as_stream(stream);
-  SweepDev p;
-  memset(&p, 0, sizeof(p));
-  uint32_t mask = 0;
-  for (int k = 0; k < K; ++k) {
-    if (!a->active[k]) continue;
-    mask |= 1u << k;
-    for (int s = 0; s < 2; ++s) p.perm[s][k] = a->perm[s][k];
-    p.alpha[k] = a->alpha[k];
-    p.wd[k] = a->weight_decay[k];
-  }
-  if (mask == 0 || n_steps == 0) return 0;
-  for (int s = 0; s < 2; ++s) {
-    p.bank[s] = a->bank[s];
-    p.labels[s] = a->labels[s];
-    p.ld[s] = a->bank_ld[s];
-    p.scale[s] = a->scale[s];
-  }
-  p.W = a->W;
-  p.m = a->m;
-  p.v = a->v;
-  p.head_stride = a->head_stride;
-  p.G = a->G;
-  p.ldg = a->ldg;
-  p.row_loss = a->row_loss;
-  p.row_correct = a->row_correct;
-  p.dim = a->dim;
-  p.n_classes = a->n_classes;
-  p.active_mask = mask;
-  p.vec_rows = a->dim % 4 == 0;  // weight rows: covered by the slab alignment check above
-  for (int s = 0; s < 2; ++s)
-    if (a->bank[s] && ((reinterpret_cast<uintptr_t>(a->bank[s]) & 15) != 0 || a->bank_ld[s] % 4 != 0)) p.vec_rows = 0;
-  // The cp.async variants of the two GEMM launches are the default when rows are 16-byte aligned (same results, 30 heads:
-  // 0.219 against 0.268 ms per step); UML_SWEEP_ASYNC=0 selects the synchronous kernels
-  static const bool want_async = [] {
-    const char* e = getenv("UML_SWEEP_ASYNC");
-    return !(e != nullptr && e[0] == '0');
-  }();
-  const bool use_async = want_async && p.vec_rows && a->ldg % 4 == 0 && (reinterpret_cast<uintptr_t>(a->G) & 15) == 0;
-  if (use_async) {
-    static const cudaError_t attr = cudaFuncSetAttribute(sweep_logits_async_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                                                         kLogitsSmemBytes);
-    UML_CUDA(attr);
-  }
-  // tensor-core forms (3xTF32, see above) whenever the async forms' alignment contract holds; UML_SWEEP_TC=0 keeps the FFMA kernels
-  static const bool want_tc = [] {
-    const char* e = getenv("UML_SWEEP_TC");
-    return !(e != nullptr && e[0] == '0');
-  }();
-  const bool use_tc = want_tc && use_async;
-  if (use_tc) {
-    static const cudaError_t attr1 = [] {
-      cudaError_t e = cudaFuncSetAttribute(sweep_logits_tc_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, kTcLgSmemBytes);
-      if (e == cudaSuccess)
-        e = cudaFuncSetAttribute(sweep_logits_tc_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, kTcLgSmemBytes);
-      return e;
-    }();
-    UML_CUDA(attr1);
-    static const cudaError_t attr2 = [] {
-      cudaError_t e = cudaFuncSetAttribute(sweep_dw_update_tc_kernel<256>, cudaFuncAttributeMaxDynamicSharedMemorySize, kTcDwSmemBytes);
-      if (e == cudaSuccess)
-        e = cudaFuncSetAttribute(sweep_dw_update_tc_kernel<512>, cudaFuncAttributeMaxDynamicSharedMemorySize, kTcDwSmemBytes);
-      return e;
-    }();
-    UML_CUDA(attr2);
-  }
-  // UML_SWEEP_TC_DW=0 keeps the FFMA dW + update launch next to the tensor-core logits; UML_SWEEP_DW_THREADS its CTA size
-  static const bool want_tc_dw = [] {
-    const char* e = getenv("UML_SWEEP_TC_DW");
-    return !(e != nullptr && e[0] == '0');
-  }();
-  static const int dw_threads = [] {
-    const char* e = getenv("UML_SWEEP_DW_THREADS");
-    return (e && atoi(e) == 256) ? 256 : 512;
-  }();
-  const bool use_tc_dw = use_tc && want_tc_dw;
-  static const bool want_fused_softmax = [] {  // UML_SWEEP_FUSED_SOFTMAX=0 keeps the separate softmax / CE launch
-    const char* e = getenv("UML_SWEEP_FUSED_SOFTMAX");
-    return !(e != nullptr && e[0] == '0');
-  }();
-  CUtensorMap tm_w, tm_m, tm_v;  // [K][C][D] views of the W, m, v slabs for the dW kernel's slot ring
-  memset(&tm_w, 0, sizeof(tm_w));
-  memset(&tm_m, 0, sizeof(tm_m));
-  memset(&tm_v, 0, sizeof(tm_v));
-  if (use_tc) {
-    const uint64_t d = static_cast<uint64_t>(a->dim), c = static_cast<uint64_t>(a->n_classes), k = static_cast<uint64_t>(K);
-    const uint64_t hs = static_cast<uint64_t>(a->head_stride) * 4;
-    if (make_tmap_3d(&tm_w, a->W, CU_TENSOR_MAP_DATA_TYPE_FLOAT32, d, c, k, d * 4, hs, 128, 16, 1)) return 1;
-    if (make_tmap_3d(&tm_m, a->m, CU_TENSOR_MAP_DATA_TYPE_FLOAT32, d, c, k, d * 4, hs, 128, 16, 1)) return 1;
-    if (a->kind != 3 && make_tmap_3d(&tm_v, a->v, CU_TENSOR_MAP_DATA_TYPE_FLOAT32, d, c, k, d * 4, hs, 128, 16, 1)) return 1;
-  }
-  p.kind = a->kind;
-  p.beta1 = a->beta1;
-  p.beta2 = a->beta2;
-  p.eps = a->eps;
-  p.momentum = a->momentum;
-  int64_t pos[2] = {a->pos[0], a->pos[1]};
-  for (int i = 0; i < n_steps; ++i) {
-    const int64_t n0 = rows[2 * i], n1 = rows[2 * i + 1], R = n0 + n1;
-    UML_REQUIRE(n0 >= 0 && n1 >= 0 && R > 0 && R <= a->max_rows, "sweep_run: step %d has %lld rows (capacity %lld)", i,
-                static_cast<long long>(R), static_cast<long long>(a->max_rows));
-    for (int s = 0; s < 2; ++s) {
-      const int64_t n = s ? n1 : n0;
-      if (n == 0) continue;
-      UML_REQUIRE(a->bank[s] && a->labels[s] && pos[s] >= 0 && pos[s] + n <= a->perm_len[s],
-                  "sweep_run: step %d runs past the end of permutation %d", i, s);
-      for (int k = 0; k < K; ++k)
-        UML_REQUIRE(!((mask >> k) & 1u) || a->perm[s][k], "sweep_run: head %d has no permutation %d", k, s);
-    }
-    p.n0 = n0;
-    p.n1 = n1;
-    p.pos[0] = pos[0];
-    p.pos[1] = pos[1];
-    p.g_stride = a->max_rows * a->ldg;
-    p.row_stride = a->max_rows;
-    p.stats = a->stats + static_cast<int64_t>(i) * K * 2;
-    const double t = static_cast<double>(a->step + i);
-    const double bc1 = 1.0 - pow(static_cast<double>(a->beta1), t);
-    const double bc2 = 1.0 - pow(static_cast<double>(a->beta2), t);
-    p.bc2_sqrt_inv = static_cast<float>(1.0 / sqrt(bc2));
-    p.first_step = (a->step + i) <= 1;
-    for (int k = 0; k < K; ++k) {
-      const float l = lr[static_cast<int64_t>(i) * K + k];
-      p.lr[k] = l;
-      p.step_size[k] = static_cast<float>(static_cast<double>(l) / bc1);
-      p.decay[k] = static_cast<float>(1.0 - static_cast<double>(l) * static_cast<double>(a->weight_decay[k]));
-    }
-    const unsigned rt = static_cast<unsigned>((R + 63) / 64), ct = static_cast<unsigned>((a->n_classes + 63) / 64);
-    const bool timed = i == n_steps - 1;
-    auto mark = [&](int e) -> int {
-      if (timed && a->ev[e]) UML_CUDA(cudaEventRecord(static_cast<cudaEvent_t>(a->ev[e]), st));
-      return 0;
-    };
-    if (mark(0)) return 1;
-    // up to eight class tiles per head: they form a cluster and finish the rows (softmax / CE) in the logits epilogue
-    const unsigned n_ctile = static_cast<unsigned>((a->n_classes + 127) / 128);
-    // (any tile count up to eight: clusters of 3, 6 and 7 are covered by tests/test_sweep_gpu.py)
-    const bool fuse_softmax = use_tc && want_fused_softmax && n_ctile <= 8;
-    if (fuse_softmax)
-      UML_CUDA(launch_kernel(sweep_logits_tc_kernel<true>, dim3(n_ctile, rt, K), dim3(256), kTcLgSmemBytes, st,
-                             static_cast<int>(n_ctile), p));
-    else if (use_tc)
-      sweep_logits_tc_kernel<false><<<dim3(n_ctile, rt, K), 256, kTcLgSmemBytes, st>>>(p);
-    else if (use_async)
-      sweep_logits_async_kernel<<<dim3(ct, rt, K), 256, kLogitsSmemBytes, st>>>(p);
-    else
-      sweep_logits_kernel<<<dim3(ct, rt, K), 256, 0, st>>>(p);
-    UML_CUDA(cudaGetLastError());
-    ++g_sweep_launches;
-    if (mark(1) || mark(2)) return 1;
-    if (!fuse_softmax) {
-      sweep_softmax_kernel<<<dim3(static_cast<unsigned>(R), K), 256, 0, st>>>(p);
-      UML_CUDA(cudaGetLastError());
-      ++g_sweep_launches;
-    }
-    if (mark(3) || mark(4)) return 1;
-    if (use_tc_dw && R <= 64) {  // (larger steps: the feature tile of the tensor-core form holds 64 rows)
-      const int64_t units = static_cast<int64_t>(__builtin_popcount(mask)) * ((a->dim + 127) / 128) * ((a->n_classes + 63) / 64);
-      const unsigned g = static_cast<unsigned>(std::min<int64_t>(units, sm_count()));
-      if (dw_threads == 256) sweep_dw_update_tc_kernel<256><<<g, 256 + 64, kTcDwSmemBytes, st>>>(p, tm_w, tm_m, tm_v);
-      else sweep_dw_update_tc_kernel<512><<<g, 512 + 64, kTcDwSmemBytes, st>>>(p, tm_w, tm_m, tm_v);
-    }
-    else if (use_async)
-      sweep_dw_update_async_kernel<<<dim3((a->dim + 63) / 64, (a->n_classes + 63) / 64, K), 256, 0, st>>>(p);
-    else
-      sweep_dw_update_kernel<<<dim3((a->dim + 63) / 64, (a->n_classes + 63) / 64, K), 256, 0, st>>>(p);
-    UML_CUDA(cudaGetLastError());
-    ++g_sweep_launches;
-    if (mark(5) || mark(6)) return 1;
-    if (!(use_tc_dw && R <= 64)) {  // (the tensor-core dW launch carries a statistics warp)
-      sweep_stats_kernel<<<dim3(2, K), 256, 0, st>>>(p);
-      UML_CUDA(cudaGetLastError());
-      ++g_sweep_launches;
-    }
-    if (mark(7)) return 1;
-    if (dg && launch_grad_diag(p, dg, K, i, timed, st)) return 1;
-    pos[0] += n0;
-    pos[1] += n1;
-  }
-  return 0;
-}
-
-int uml_sweep_run(const uml_sweep_args* a, int32_t n_steps, const int64_t* rows, const float* lr, void* stream) {
-  return sweep_run_impl(a, nullptr, n_steps, rows, lr, stream);
-}
-
-static int sweep_adapter_run_impl(const uml_sweep_args* a, const uml_sweep_adapter_args* ad, const uml_sweep_diag* dg,
-                                  int32_t n_steps, const int64_t* rows, const float* lr, void* stream) {
-  using namespace uml;
-  using namespace uml::sweep;
-  UML_REQUIRE(a && ad && rows && lr && n_steps >= 0, "sweep_adapter_run: null argument");
-  const int K = a->n_heads;
-  UML_REQUIRE(K >= 1 && K <= kMaxHeads, "sweep_adapter_run: 1..%d heads", kMaxHeads);
-  UML_REQUIRE(a->dim > 0 && a->n_classes > 0 && a->ldg >= a->n_classes, "sweep_adapter_run: bad shape");
-  UML_REQUIRE(a->kind >= 1 && a->kind <= 3, "sweep_adapter_run: optimizer kind must be 1 (AdamW), 2 (Adam) or 3 (SGD)");
-  UML_REQUIRE(a->W && a->m && (a->kind == 3 || a->v) && a->G && a->row_loss && a->row_correct && a->stats,
-              "sweep_adapter_run: null buffer");
-  UML_REQUIRE(a->head_stride >= static_cast<int64_t>(a->n_classes) * a->dim, "sweep_adapter_run: head_stride too small");
-  const bool adapter = ad->img_dim > 0, temps = ad->scale_param != nullptr;
-  // tensor-core forms only: 16-byte rows and operands, one 64-row feature tile, softmax / CE in the logits epilogue
-  UML_REQUIRE(a->dim % 4 == 0 && ad->img_dim % 4 == 0 && ad->img_dim >= 0, "sweep_adapter_run: dims must be multiples of 4");
-  UML_REQUIRE(a->n_classes <= 1024, "sweep_adapter_run: at most 1024 classes (softmax / CE in the logits epilogue)");
-  UML_REQUIRE(a->max_rows >= 1 && a->max_rows <= 64, "sweep_adapter_run: at most 64 rows per step (max_rows %lld)",
-              static_cast<long long>(a->max_rows));
+// The tensor-core forms' alignment contract: W, m, v, G and the bank rows start on 16-byte boundaries, strides are
+// multiples of 4 floats.
+static int check_tc_alignment(const char* who, const uml_sweep_args* a) {
   UML_REQUIRE(a->head_stride % 4 == 0 && aligned16(a->W) && aligned16(a->m) && aligned16(a->v) && aligned16(a->G) &&
                   a->ldg % 4 == 0,
-              "sweep_adapter_run: W, m, v, G must be 16-byte aligned with strides that are multiples of 4");
+              "%s: W, m, v, G must be 16-byte aligned with strides that are multiples of 4", who);
   for (int s = 0; s < 2; ++s)
-    UML_REQUIRE(!a->bank[s] || (aligned16(a->bank[s]) && a->bank_ld[s] % 4 == 0),
-                "sweep_adapter_run: bank %d rows must be 16-byte aligned", s);
-  if (adapter) {
-    UML_REQUIRE(ad->W && ad->m && (a->kind == 3 || ad->v) && ad->Z && ad->dZ, "sweep_adapter_run: null adapter buffer");
-    UML_REQUIRE(ad->adapter_stride >= static_cast<int64_t>(a->dim) * ad->img_dim && ad->adapter_stride % 4 == 0 &&
-                    aligned16(ad->W) && aligned16(ad->m) && aligned16(ad->v),
-                "sweep_adapter_run: adapter slabs must be 16-byte aligned, adapter_stride >= dim * img_dim, a multiple of 4");
-    UML_REQUIRE(ad->ldz >= a->dim && ad->ldz % 4 == 0 && ad->max_img_rows >= 1 && aligned16(ad->Z) && aligned16(ad->dZ),
-                "sweep_adapter_run: Z / dZ must be 16-byte aligned with ldz >= dim, a multiple of 4");
-  }
-  if (temps)
-    UML_REQUIRE(ad->scale_m && (a->kind == 3 || ad->scale_v) && ad->row_dscale,
-                "sweep_adapter_run: learnable temperatures need scale_m, scale_v and row_dscale");
-  cudaStream_t st = as_stream(stream);
-  SweepDev p;
+    UML_REQUIRE(!a->bank[s] || (aligned16(a->bank[s]) && a->bank_ld[s] % 4 == 0), "%s: bank %d rows must be 16-byte aligned",
+                who, s);
+  return 0;
+}
+
+// p for the running heads of a, all but the per-step fields (sweep_step_begin).  Returns the running heads' mask; 0 when
+// there is nothing to run (no running head or no step).
+static uint32_t sweep_dev_from_args(const uml_sweep_args* a, int32_t n_steps, uml::sweep::SweepDev& p) {
   memset(&p, 0, sizeof(p));
   uint32_t mask = 0;
-  for (int k = 0; k < K; ++k) {
+  for (int k = 0; k < a->n_heads; ++k) {
     if (!a->active[k]) continue;
     mask |= 1u << k;
     for (int s = 0; s < 2; ++s) p.perm[s][k] = a->perm[s][k];
@@ -2020,11 +1834,13 @@ static int sweep_adapter_run_impl(const uml_sweep_args* a, const uml_sweep_adapt
     p.wd[k] = a->weight_decay[k];
   }
   if (mask == 0 || n_steps == 0) return 0;
+  p.vec_rows = a->dim % 4 == 0;  // weight rows: covered by the callers' slab alignment checks
   for (int s = 0; s < 2; ++s) {
     p.bank[s] = a->bank[s];
     p.labels[s] = a->labels[s];
     p.ld[s] = a->bank_ld[s];
     p.scale[s] = a->scale[s];
+    if (a->bank[s] && (!aligned16(a->bank[s]) || a->bank_ld[s] % 4 != 0)) p.vec_rows = 0;
   }
   p.W = a->W;
   p.m = a->m;
@@ -2039,12 +1855,187 @@ static int sweep_adapter_run_impl(const uml_sweep_args* a, const uml_sweep_adapt
   p.dim = a->dim;
   p.n_classes = a->n_classes;
   p.active_mask = mask;
-  p.vec_rows = 1;
   p.kind = a->kind;
   p.beta1 = a->beta1;
   p.beta2 = a->beta2;
   p.eps = a->eps;
   p.momentum = a->momentum;
+  return mask;
+}
+
+// Step i: checks its rows against the capacity and the permutations, sets its batch, statistics slot and optimizer scalars
+// in p, and moves pos past its batch.
+static int sweep_step_begin(const char* who, const uml_sweep_args* a, int i, const int64_t* rows, const float* lr,
+                            int64_t pos[2], uml::sweep::SweepDev& p) {
+  const int K = a->n_heads;
+  const int64_t n0 = rows[2 * i], n1 = rows[2 * i + 1], R = n0 + n1;
+  UML_REQUIRE(n0 >= 0 && n1 >= 0 && R > 0 && R <= a->max_rows, "%s: step %d has %lld rows (capacity %lld)", who, i,
+              static_cast<long long>(R), static_cast<long long>(a->max_rows));
+  for (int s = 0; s < 2; ++s) {
+    const int64_t n = s ? n1 : n0;
+    if (n == 0) continue;
+    UML_REQUIRE(a->bank[s] && a->labels[s] && pos[s] >= 0 && pos[s] + n <= a->perm_len[s],
+                "%s: step %d runs past the end of permutation %d", who, i, s);
+    for (int k = 0; k < K; ++k)
+      UML_REQUIRE(!((p.active_mask >> k) & 1u) || a->perm[s][k], "%s: head %d has no permutation %d", who, k, s);
+  }
+  p.n0 = n0;
+  p.n1 = n1;
+  p.pos[0] = pos[0];
+  p.pos[1] = pos[1];
+  p.stats = a->stats + static_cast<int64_t>(i) * K * 2;
+  const double t = static_cast<double>(a->step + i);
+  const double bc1 = 1.0 - pow(static_cast<double>(a->beta1), t);
+  const double bc2 = 1.0 - pow(static_cast<double>(a->beta2), t);
+  p.bc2_sqrt_inv = static_cast<float>(1.0 / sqrt(bc2));
+  p.first_step = (a->step + i) <= 1;
+  for (int k = 0; k < K; ++k) {
+    const float l = lr[static_cast<int64_t>(i) * K + k];
+    p.lr[k] = l;
+    p.step_size[k] = static_cast<float>(static_cast<double>(l) / bc1);
+    p.decay[k] = static_cast<float>(1.0 - static_cast<double>(l) * static_cast<double>(a->weight_decay[k]));
+  }
+  pos[0] += n0;
+  pos[1] += n1;
+  return 0;
+}
+
+// [K][rows][cols] views of a (W, m, v) slab triple, heads `stride` floats apart, in boxes of 16 rows x 128 floats; no v for SGD
+static int make_slab_maps(SlabMaps& tm, float* W, float* m, float* v, int kind, int64_t cols, int64_t rows, int K,
+                          int64_t stride) {
+  using uml::make_tmap_3d;
+  const uint64_t c = static_cast<uint64_t>(cols), r = static_cast<uint64_t>(rows), k = static_cast<uint64_t>(K);
+  const uint64_t hs = static_cast<uint64_t>(stride) * 4;
+  if (make_tmap_3d(&tm.w, W, CU_TENSOR_MAP_DATA_TYPE_FLOAT32, c, r, k, c * 4, hs, 128, 16, 1)) return 1;
+  if (make_tmap_3d(&tm.m, m, CU_TENSOR_MAP_DATA_TYPE_FLOAT32, c, r, k, c * 4, hs, 128, 16, 1)) return 1;
+  if (kind != 3 && make_tmap_3d(&tm.v, v, CU_TENSOR_MAP_DATA_TYPE_FLOAT32, c, r, k, c * 4, hs, 128, 16, 1)) return 1;
+  return 0;
+}
+
+// The tensor-core dW + update over the running heads of p: persistent, at most one CTA per SM.
+static void launch_dw_update_tc(const uml::sweep::SweepDev& p, const SlabMaps& tm, cudaStream_t st) {
+  using namespace uml;
+  using namespace uml::sweep;
+  const int64_t units = static_cast<int64_t>(__builtin_popcount(p.active_mask)) * ((p.dim + 127) / 128) * ((p.n_classes + 63) / 64);
+  const unsigned g = static_cast<unsigned>(std::min<int64_t>(units, sm_count()));
+  sweep_dw_update_tc_kernel<<<g, kTcDwThreads + 64, kTcDwSmemBytes, st>>>(p, tm.w, tm.m, tm.v);
+}
+
+static int sweep_run_impl(const uml_sweep_args* a, const uml_sweep_diag* dg, int32_t n_steps, const int64_t* rows,
+                          const float* lr, void* stream) {
+  using namespace uml;
+  using namespace uml::sweep;
+  if (check_sweep_args("sweep_run", a, n_steps, rows, lr)) return 1;
+  if (a->dim % 4 == 0) {  // the vector epilogue's alignment contract
+    UML_REQUIRE(a->head_stride % 4 == 0 && aligned16(a->W) && aligned16(a->m) && aligned16(a->v),
+                "sweep_run: W, m, v slabs must be 16-byte aligned");
+  }
+  const int K = a->n_heads;
+  cudaStream_t st = as_stream(stream);
+  SweepDev p;
+  if (sweep_dev_from_args(a, n_steps, p) == 0) return 0;
+  // cp.async staging of the FFMA forms whenever rows and G are 16-byte aligned (30 heads: 0.219 against 0.268 ms per step
+  // for the register-staged kernels, which remain for unaligned rows)
+  const bool use_async = p.vec_rows && a->ldg % 4 == 0 && aligned16(a->G);
+  if (use_async) {
+    static const cudaError_t attr = cudaFuncSetAttribute(sweep_logits_async_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                                                         kLogitsSmemBytes);
+    UML_CUDA(attr);
+  }
+  // tensor-core forms (3xTF32, see above) whenever the async forms' alignment contract holds; UML_SWEEP_TC=0 keeps the FFMA kernels
+  static const bool want_tc = [] {
+    const char* e = getenv("UML_SWEEP_TC");
+    return !(e != nullptr && e[0] == '0');
+  }();
+  const bool use_tc = want_tc && use_async;
+  SlabMaps tm{};  // [K][C][D] views of the W, m, v slabs
+  if (use_tc) {
+    UML_CUDA(tc_smem_attributes());
+    if (make_slab_maps(tm, a->W, a->m, a->v, a->kind, a->dim, a->n_classes, K, a->head_stride)) return 1;
+  }
+  // up to eight class tiles per head: they form a cluster and finish the rows (softmax / CE) in the logits epilogue
+  // (any tile count up to eight: clusters of 3, 6 and 7 are covered by tests/test_sweep_gpu.py)
+  const unsigned n_ctile = static_cast<unsigned>((a->n_classes + 127) / 128);
+  const bool fuse_softmax = use_tc && n_ctile <= 8;
+  int64_t pos[2] = {a->pos[0], a->pos[1]};
+  for (int i = 0; i < n_steps; ++i) {
+    if (sweep_step_begin("sweep_run", a, i, rows, lr, pos, p)) return 1;
+    const int64_t R = p.n0 + p.n1;
+    const unsigned rt = static_cast<unsigned>((R + 63) / 64), ct = static_cast<unsigned>((a->n_classes + 63) / 64);
+    const bool timed = i == n_steps - 1;
+    void* const* ev = timed ? a->ev : nullptr;
+    if (mark(ev, 0, st)) return 1;
+    if (fuse_softmax)
+      UML_CUDA(launch_kernel(sweep_logits_tc_kernel<true>, dim3(n_ctile, rt, K), dim3(256), kTcLgSmemBytes, st,
+                             static_cast<int>(n_ctile), p));
+    else if (use_tc)
+      sweep_logits_tc_kernel<false><<<dim3(n_ctile, rt, K), 256, kTcLgSmemBytes, st>>>(p);
+    else if (use_async)
+      sweep_logits_async_kernel<<<dim3(ct, rt, K), 256, kLogitsSmemBytes, st>>>(p);
+    else
+      sweep_logits_kernel<<<dim3(ct, rt, K), 256, 0, st>>>(p);
+    UML_CUDA(cudaGetLastError());
+    ++g_sweep_launches;
+    if (mark(ev, 1, st) || mark(ev, 2, st)) return 1;
+    if (!fuse_softmax) {
+      sweep_softmax_kernel<<<dim3(static_cast<unsigned>(R), K), 256, 0, st>>>(p);
+      UML_CUDA(cudaGetLastError());
+      ++g_sweep_launches;
+    }
+    if (mark(ev, 3, st) || mark(ev, 4, st)) return 1;
+    const bool tc_dw = use_tc && R <= 64;  // (larger steps: the feature tile of the tensor-core form holds 64 rows)
+    if (tc_dw)
+      launch_dw_update_tc(p, tm, st);
+    else if (use_async)
+      sweep_dw_update_async_kernel<<<dim3((a->dim + 63) / 64, (a->n_classes + 63) / 64, K), 256, 0, st>>>(p);
+    else
+      sweep_dw_update_kernel<<<dim3((a->dim + 63) / 64, (a->n_classes + 63) / 64, K), 256, 0, st>>>(p);
+    UML_CUDA(cudaGetLastError());
+    ++g_sweep_launches;
+    if (mark(ev, 5, st) || mark(ev, 6, st)) return 1;
+    if (!tc_dw) {  // (the tensor-core dW launch carries a statistics warp)
+      sweep_stats_kernel<<<dim3(2, K), 256, 0, st>>>(p);
+      UML_CUDA(cudaGetLastError());
+      ++g_sweep_launches;
+    }
+    if (mark(ev, 7, st)) return 1;
+    if (dg && launch_grad_diag(p, dg, K, i, timed, st)) return 1;
+  }
+  return 0;
+}
+
+int uml_sweep_run(const uml_sweep_args* a, int32_t n_steps, const int64_t* rows, const float* lr, void* stream) {
+  return sweep_run_impl(a, nullptr, n_steps, rows, lr, stream);
+}
+
+static int sweep_adapter_run_impl(const uml_sweep_args* a, const uml_sweep_adapter_args* ad, const uml_sweep_diag* dg,
+                                  int32_t n_steps, const int64_t* rows, const float* lr, void* stream) {
+  using namespace uml;
+  using namespace uml::sweep;
+  UML_REQUIRE(ad, "sweep_adapter_run: null argument");
+  if (check_sweep_args("sweep_adapter_run", a, n_steps, rows, lr)) return 1;
+  const bool adapter = ad->img_dim > 0, temps = ad->scale_param != nullptr;
+  // tensor-core forms only: 16-byte rows and operands, one 64-row feature tile, softmax / CE in the logits epilogue
+  UML_REQUIRE(a->dim % 4 == 0 && ad->img_dim % 4 == 0 && ad->img_dim >= 0, "sweep_adapter_run: dims must be multiples of 4");
+  UML_REQUIRE(a->n_classes <= 1024, "sweep_adapter_run: at most 1024 classes (softmax / CE in the logits epilogue)");
+  UML_REQUIRE(a->max_rows >= 1 && a->max_rows <= 64, "sweep_adapter_run: at most 64 rows per step (max_rows %lld)",
+              static_cast<long long>(a->max_rows));
+  if (check_tc_alignment("sweep_adapter_run", a)) return 1;
+  if (adapter) {
+    UML_REQUIRE(ad->W && ad->m && (a->kind == 3 || ad->v) && ad->Z && ad->dZ, "sweep_adapter_run: null adapter buffer");
+    UML_REQUIRE(ad->adapter_stride >= static_cast<int64_t>(a->dim) * ad->img_dim && ad->adapter_stride % 4 == 0 &&
+                    aligned16(ad->W) && aligned16(ad->m) && aligned16(ad->v),
+                "sweep_adapter_run: adapter slabs must be 16-byte aligned, adapter_stride >= dim * img_dim, a multiple of 4");
+    UML_REQUIRE(ad->ldz >= a->dim && ad->ldz % 4 == 0 && ad->max_img_rows >= 1 && aligned16(ad->Z) && aligned16(ad->dZ),
+                "sweep_adapter_run: Z / dZ must be 16-byte aligned with ldz >= dim, a multiple of 4");
+  }
+  if (temps)
+    UML_REQUIRE(ad->scale_m && (a->kind == 3 || ad->scale_v) && ad->row_dscale,
+                "sweep_adapter_run: learnable temperatures need scale_m, scale_v and row_dscale");
+  const int K = a->n_heads;
+  cudaStream_t st = as_stream(stream);
+  SweepDev p;
+  if (sweep_dev_from_args(a, n_steps, p) == 0) return 0;
   if (temps) {
     p.scale_dev = ad->scale_param;
     p.scale_m = ad->scale_m;
@@ -2056,74 +2047,19 @@ static int sweep_adapter_run_impl(const uml_sweep_args* a, const uml_sweep_adapt
     p.z_ld = ad->ldz;
     p.z_stride = ad->max_img_rows * ad->ldz;
   }
-  static const cudaError_t attr = [] {
-    cudaError_t e = cudaFuncSetAttribute(sweep_logits_tc_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, kTcLgSmemBytes);
-    if (e == cudaSuccess)
-      e = cudaFuncSetAttribute(sweep_logits_tc_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, kTcLgSmemBytes);
-    if (e == cudaSuccess)
-      e = cudaFuncSetAttribute(sweep_dw_update_tc_kernel<512>, cudaFuncAttributeMaxDynamicSharedMemorySize, kTcDwSmemBytes);
-    if (e == cudaSuccess) e = cudaFuncSetAttribute(sweep_dz_tc_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, kTcDzSmemBytes);
-    return e;
-  }();
-  UML_CUDA(attr);
-  // [K][rows][dim] views of the slabs for the dW kernel's slot ring: the head (C x D) and the adapter (D x Dv)
-  CUtensorMap tm_w, tm_m, tm_v, tma_w, tma_m, tma_v;
-  memset(&tm_v, 0, sizeof(tm_v));
-  memset(&tma_w, 0, sizeof(tma_w));
-  memset(&tma_m, 0, sizeof(tma_m));
-  memset(&tma_v, 0, sizeof(tma_v));
-  {
-    const uint64_t d = static_cast<uint64_t>(a->dim), c = static_cast<uint64_t>(a->n_classes), k = static_cast<uint64_t>(K);
-    const uint64_t hs = static_cast<uint64_t>(a->head_stride) * 4;
-    if (make_tmap_3d(&tm_w, a->W, CU_TENSOR_MAP_DATA_TYPE_FLOAT32, d, c, k, d * 4, hs, 128, 16, 1)) return 1;
-    if (make_tmap_3d(&tm_m, a->m, CU_TENSOR_MAP_DATA_TYPE_FLOAT32, d, c, k, d * 4, hs, 128, 16, 1)) return 1;
-    if (a->kind != 3 && make_tmap_3d(&tm_v, a->v, CU_TENSOR_MAP_DATA_TYPE_FLOAT32, d, c, k, d * 4, hs, 128, 16, 1)) return 1;
-    if (adapter) {
-      const uint64_t dv = static_cast<uint64_t>(ad->img_dim), as = static_cast<uint64_t>(ad->adapter_stride) * 4;
-      if (make_tmap_3d(&tma_w, ad->W, CU_TENSOR_MAP_DATA_TYPE_FLOAT32, dv, d, k, dv * 4, as, 128, 16, 1)) return 1;
-      if (make_tmap_3d(&tma_m, ad->m, CU_TENSOR_MAP_DATA_TYPE_FLOAT32, dv, d, k, dv * 4, as, 128, 16, 1)) return 1;
-      if (a->kind != 3 && make_tmap_3d(&tma_v, ad->v, CU_TENSOR_MAP_DATA_TYPE_FLOAT32, dv, d, k, dv * 4, as, 128, 16, 1))
-        return 1;
-    }
-  }
-  const int n_act = __builtin_popcount(mask);
+  UML_CUDA(tc_smem_attributes());
+  // the head's [K][C][D] and the adapter's [K][D][Dv] slabs
+  SlabMaps tm{}, tma{};
+  if (make_slab_maps(tm, a->W, a->m, a->v, a->kind, a->dim, a->n_classes, K, a->head_stride)) return 1;
+  if (adapter && make_slab_maps(tma, ad->W, ad->m, ad->v, a->kind, ad->img_dim, a->dim, K, ad->adapter_stride)) return 1;
   int64_t pos[2] = {a->pos[0], a->pos[1]};
   for (int i = 0; i < n_steps; ++i) {
-    const int64_t n0 = rows[2 * i], n1 = rows[2 * i + 1], R = n0 + n1;
-    UML_REQUIRE(n0 >= 0 && n1 >= 0 && R > 0 && R <= a->max_rows, "sweep_adapter_run: step %d has %lld rows (capacity %lld)", i,
-                static_cast<long long>(R), static_cast<long long>(a->max_rows));
-    UML_REQUIRE(!adapter || n0 <= ad->max_img_rows, "sweep_adapter_run: step %d has %lld image rows (Z holds %lld)", i,
-                static_cast<long long>(n0), static_cast<long long>(ad->max_img_rows));
-    for (int s = 0; s < 2; ++s) {
-      const int64_t n = s ? n1 : n0;
-      if (n == 0) continue;
-      UML_REQUIRE(a->bank[s] && a->labels[s] && pos[s] >= 0 && pos[s] + n <= a->perm_len[s],
-                  "sweep_adapter_run: step %d runs past the end of permutation %d", i, s);
-      for (int k = 0; k < K; ++k)
-        UML_REQUIRE(!((mask >> k) & 1u) || a->perm[s][k], "sweep_adapter_run: head %d has no permutation %d", k, s);
-    }
-    p.n0 = n0;
-    p.n1 = n1;
-    p.pos[0] = pos[0];
-    p.pos[1] = pos[1];
-    p.stats = a->stats + static_cast<int64_t>(i) * K * 2;
-    const double t = static_cast<double>(a->step + i);
-    const double bc1 = 1.0 - pow(static_cast<double>(a->beta1), t);
-    const double bc2 = 1.0 - pow(static_cast<double>(a->beta2), t);
-    p.bc2_sqrt_inv = static_cast<float>(1.0 / sqrt(bc2));
-    p.first_step = (a->step + i) <= 1;
-    for (int k = 0; k < K; ++k) {
-      const float l = lr[static_cast<int64_t>(i) * K + k];
-      p.lr[k] = l;
-      p.step_size[k] = static_cast<float>(static_cast<double>(l) / bc1);
-      p.decay[k] = static_cast<float>(1.0 - static_cast<double>(l) * static_cast<double>(a->weight_decay[k]));
-    }
+    if (sweep_step_begin("sweep_adapter_run", a, i, rows, lr, pos, p)) return 1;
+    UML_REQUIRE(!adapter || p.n0 <= ad->max_img_rows, "sweep_adapter_run: step %d has %lld image rows (Z holds %lld)", i,
+                static_cast<long long>(p.n0), static_cast<long long>(ad->max_img_rows));
     const bool timed = i == n_steps - 1;
-    auto mark = [&](int e) -> int {
-      if (timed && ad->ev[e]) UML_CUDA(cudaEventRecord(static_cast<cudaEvent_t>(ad->ev[e]), st));
-      return 0;
-    };
-    const bool with_adapter = adapter && n0 > 0;
+    void* const* ev = timed ? ad->ev : nullptr;
+    const bool with_adapter = adapter && p.n0 > 0;
     // the adapter's side of the step: its rows are the image rows, its "classes" the head's input dims
     SweepDev pa = p;
     pa.zrows = nullptr;
@@ -2137,7 +2073,7 @@ static int sweep_adapter_run_impl(const uml_sweep_args* a, const uml_sweep_adapt
     pa.v = ad->v;
     pa.head_stride = ad->adapter_stride;
     pa.stats = nullptr;
-    if (mark(0)) return 1;
+    if (mark(ev, 0, st)) return 1;
     if (with_adapter) {  // Z_k = X_img Wp_k^T: the logits kernel without softmax, the adapter as its weight
       pa.G = ad->Z;
       pa.ldg = ad->ldz;
@@ -2146,41 +2082,33 @@ static int sweep_adapter_run_impl(const uml_sweep_args* a, const uml_sweep_adapt
       UML_CUDA(cudaGetLastError());
       ++g_sweep_launches;
     }
-    if (mark(1) || mark(2)) return 1;
+    if (mark(ev, 1, st) || mark(ev, 2, st)) return 1;
     const unsigned n_ctile = static_cast<unsigned>((a->n_classes + 127) / 128);
     UML_CUDA(launch_kernel(sweep_logits_tc_kernel<true>, dim3(n_ctile, 1, K), dim3(256), kTcLgSmemBytes, st,
                            static_cast<int>(n_ctile), p));
     ++g_sweep_launches;
-    if (mark(3) || mark(4)) return 1;
+    if (mark(ev, 3, st) || mark(ev, 4, st)) return 1;
     if (with_adapter) {  // dZ from the head's weights before their update
       sweep_dz_tc_kernel<<<dim3(static_cast<unsigned>((a->dim + 127) / 128), K), 256, kTcDzSmemBytes, st>>>(p, ad->dZ, ad->ldz,
                                                                                                         ad->max_img_rows * ad->ldz);
       UML_CUDA(cudaGetLastError());
       ++g_sweep_launches;
     }
-    if (mark(5) || mark(6)) return 1;
-    {
-      const int64_t units = static_cast<int64_t>(n_act) * ((a->dim + 127) / 128) * ((a->n_classes + 63) / 64);
-      const unsigned g = static_cast<unsigned>(std::min<int64_t>(units, sm_count()));
-      sweep_dw_update_tc_kernel<512><<<g, 512 + 64, kTcDwSmemBytes, st>>>(p, tm_w, tm_m, tm_v);
-      UML_CUDA(cudaGetLastError());
-      ++g_sweep_launches;
-    }
-    if (mark(7) || mark(8)) return 1;
+    if (mark(ev, 5, st) || mark(ev, 6, st)) return 1;
+    launch_dw_update_tc(p, tm, st);
+    UML_CUDA(cudaGetLastError());
+    ++g_sweep_launches;
+    if (mark(ev, 7, st) || mark(ev, 8, st)) return 1;
     if (with_adapter) {  // dWp_k = dZ_k^T X_img with the update; the statistics warp is off (pa.stats == NULL)
       pa.G = ad->dZ;
       pa.ldg = ad->ldz;
       pa.g_stride = ad->max_img_rows * ad->ldz;
-      const int64_t units = static_cast<int64_t>(n_act) * ((ad->img_dim + 127) / 128) * ((a->dim + 63) / 64);
-      const unsigned g = static_cast<unsigned>(std::min<int64_t>(units, sm_count()));
-      sweep_dw_update_tc_kernel<512><<<g, 512 + 64, kTcDwSmemBytes, st>>>(pa, tma_w, tma_m, tma_v);
+      launch_dw_update_tc(pa, tma, st);
       UML_CUDA(cudaGetLastError());
       ++g_sweep_launches;
     }
-    if (mark(9)) return 1;
+    if (mark(ev, 9, st)) return 1;
     if (dg && launch_grad_diag(p, dg, K, i, timed, st)) return 1;  // (Z is overwritten by the next step's first launch)
-    pos[0] += n0;
-    pos[1] += n1;
   }
   return 0;
 }
@@ -2198,12 +2126,7 @@ int uml_sweep_run_diag(const uml_sweep_args* a, const uml_sweep_adapter_args* ad
   UML_REQUIRE(K >= 1 && K <= kMaxHeads, "sweep_run_diag: 1..%d heads", kMaxHeads);
   UML_REQUIRE(dg->out && dg->scratch, "sweep_run_diag: null diagnostics buffer");
   UML_REQUIRE(a->dim > 0 && a->dim % 4 == 0 && a->n_classes > 0, "sweep_run_diag: dim must be a multiple of 4");
-  UML_REQUIRE(aligned16(a->W) && aligned16(a->m) && aligned16(a->v) && a->head_stride % 4 == 0 && aligned16(a->G) &&
-                  a->ldg % 4 == 0,
-              "sweep_run_diag: W, m, v, G must be 16-byte aligned with strides that are multiples of 4");
-  for (int s = 0; s < 2; ++s)
-    UML_REQUIRE(!a->bank[s] || (aligned16(a->bank[s]) && a->bank_ld[s] % 4 == 0),
-                "sweep_run_diag: bank %d rows must be 16-byte aligned", s);
+  if (check_tc_alignment("sweep_run_diag", a)) return 1;
   if (ad && ad->img_dim > 0)
     UML_REQUIRE(aligned16(ad->Z) && ad->ldz % 4 == 0, "sweep_run_diag: Z must be 16-byte aligned with ldz a multiple of 4");
   for (int k = 0; k < K; ++k)  // G's text rows carry alpha: the plain text-loss gradient is G / alpha
